@@ -27,6 +27,11 @@ separately (table_build_ms), not inside the step.
 --impl reference times the CPU oracle with every host core on the same workload: each step votes on the next few
 entries of a FIXED list of 64 evenly spread reference points (the same points on every box and at every --gpus)
 and clusters them.  The oracle is test infrastructure: it is only ever the baseline here.
+
+--dump-outputs DIR writes what the last timed step returned to its caller, the best poses and their votes of every
+model, as DIR/poses.npy (float32, K x 4 x 4) and DIR/votes.npy (float64: exact for the uint32 counts); with a model
+library, DIR/poses_model<k>.npy and DIR/votes_model<k>.npy.  The inputs are fixed files and seeded synthetic clouds,
+so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -160,8 +165,7 @@ class ClockSampler:
 
 
 def oracle_table(wl, model=None):
-    from oracle import binding as ob
-    ob.build()
+    from oracle import binding as ob  # loads the library build() made: the benchmark compiles nothing into the tree
     th = host_threads()  # the container is built sharded by key over the host cores: same buckets, seconds instead of minutes
     feats = ob.ppf_estimation(wl.model if model is None else model, n_threads=th)
     hm = ob.HashMap(wl.angle_step, wl.dist_step).set_input_feature_cloud(feats, n_threads=th)
@@ -209,6 +213,15 @@ def vote_refs(hm, wl, model, refs, threads):
     return hm.vote_refs(model, wl.scene, refs, n_threads=threads)
 
 
+def dump_outputs(out_dir, results, n_models):
+    """results: {model index: (poses, votes)} of one align.  At most 3 poses per model: a few KB for every workload."""
+    os.makedirs(out_dir, exist_ok=True)
+    for k, (poses, votes) in results.items():
+        suffix = f"_model{k}" if n_models > 1 else ""
+        np.save(os.path.join(out_dir, f"poses{suffix}.npy"), np.asarray(poses, np.float32).reshape(-1, 4, 4))
+        np.save(os.path.join(out_dir, f"votes{suffix}.npy"), np.asarray(votes, np.float64))
+
+
 def workload_config(wl, gpus):
     """`config` of the JSON line: the workload only — identical in the B200 arm and the reference arm"""
     m = wl.library()[0]
@@ -234,9 +247,10 @@ def run_reference(args, wl):
         refs = [refs_all[(k * per_step + j) % len(refs_all)] for j in range(per_step)]
         t0 = time.perf_counter()
         step_pairs = step_votes = 0
-        for m, (_, hm_k) in zip(library, tables):
+        results = {}
+        for k_m, (m, (_, hm_k)) in enumerate(zip(library, tables)):
             hyps, st = vote_refs(hm_k, wl, m, refs, threads)
-            ob.cluster(hyps, wl.pos_thr, wl.rot_thr)
+            results[k_m] = ob.cluster(hyps, wl.pos_thr, wl.rot_thr)[:2]
             step_pairs += st["pairs_in_radius"]
             step_votes += st["votes"]
         dt = time.perf_counter() - t0
@@ -263,6 +277,8 @@ def run_reference(args, wl):
         "ms_per_pose_extrapolated": 1e3 * total_s / max(1, len(used)) * wl.n_ref,
         "votes_per_sec": votes / total_s,  # the sample-independent rate (pairs differ in cost by orders of magnitude)
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, results, len(library))
     print(json.dumps(line), flush=True)
 
 
@@ -333,9 +349,9 @@ def run_b200(args, wl):
         group.connect([np.frombuffer(h, np.uint8) for h in handles])
 
     def align(ds, collect=None):
-        """vote (this rank's shard) -> exchange -> cluster, once per model of this rank; returns the last (poses, votes)."""
-        res = (np.zeros((0, 4, 4), np.float32), np.zeros(0, np.uint32))
-        for dm, table in zip(dms, tables):
+        """vote (this rank's shard) -> exchange -> cluster, once per model of this rank; returns {model: (poses, votes)}."""
+        results = {}
+        for k_m, dm, table in zip(my_models, dms, tables):
             if p2p:
                 group.vote(dm, table, ds, wl.ref_rate)
             else:
@@ -346,15 +362,15 @@ def run_b200(args, wl):
                     collect[k] = collect.get(k, 0) + v
                 collect["vote_ms"] = collect.get("vote_ms", 0.0) + ctx.timings()["vote_ms"]
             if p2p:
-                res = group.cluster(dm, table, ds, wl.ref_rate, wl.pos_thr, wl.rot_thr)
+                results[k_m] = group.cluster(dm, table, ds, wl.ref_rate, wl.pos_thr, wl.rot_thr)
             elif world > 1 and (not lib_mode or lib_sharded):
                 with torch.cuda.stream(stream):
                     ordered = sharding.all_gather_hypotheses(local_buf, n_ref, world, dist)
-                res = ctx.cluster(None, wl.pos_thr, wl.rot_thr, device_ptr=ordered.data_ptr(), n=n_ref)
+                results[k_m] = ctx.cluster(None, wl.pos_thr, wl.rot_thr, device_ptr=ordered.data_ptr(), n=n_ref)
                 del ordered
             else:
-                res = ctx.cluster(None, wl.pos_thr, wl.rot_thr, device_ptr=local_buf.data_ptr(), n=n_ref)
-        return res
+                results[k_m] = ctx.cluster(None, wl.pos_thr, wl.rot_thr, device_ptr=local_buf.data_ptr(), n=n_ref)
+        return results
 
     def barrier():
         if world > 1:
@@ -370,14 +386,14 @@ def run_b200(args, wl):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             l0 = ctx.launch_count
             e0.record(stream)
-            poses, votes = align(make_scene())
+            results = align(make_scene())
             e1.record(stream)
             e1.synchronize()
             total += e0.elapsed_time(e1)
             launches += ctx.launch_count - l0
             if not lib_mode:
                 vote_ms.append(ctx.timings()["vote_ms"])
-        return total, vote_ms, launches, poses, votes
+        return total, vote_ms, launches, results
 
     # ---- resident-input measurement ---------------------------------------------------------------
     sampler = ClockSampler(local)
@@ -391,16 +407,20 @@ def run_b200(args, wl):
         stats.setdefault(k, 0)
     barrier()
     sampler.samples.clear()
-    total_ms, vote_ms, launches, poses, votes = timed_steps(lambda: ds_resident, args.steps)
+    total_ms, vote_ms, launches, results = timed_steps(lambda: ds_resident, args.steps)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    poses, votes = results[my_models[-1]]
+    # model-parallel ranks each hold their own models' results; otherwise every rank holds the same ones
+    if args.dump_outputs and (rank == 0 or (lib_mode and not lib_sharded)):
+        dump_outputs(args.dump_outputs, results, len(library))
 
     # ---- end to end through the host-buffer API: H2D scene every step, poses read back -------------
     def upload():
         return ctx.upload_cloud((scene_pinned.data_ptr(), n_s), stride=6, normal_offset=3)
     timed_steps(upload, min(args.warmup, 3))
     barrier()
-    e2e_total_ms, _, _, _, _ = timed_steps(upload, args.steps)
+    e2e_total_ms, _, _, _ = timed_steps(upload, args.steps)
     barrier()
 
     # whole-job numbers: max over ranks of the time, sum over ranks of the work
@@ -517,7 +537,11 @@ def main():
                          "reference points of each align shared by all GPUs")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="several GPUs: records written into every peer's buffer by the vote epilogue (default) or NCCL all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the poses and votes the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     from yolo_ppf_pose_estimation_b200 import workloads
     wl = workloads.load(args.workload)

@@ -1039,3 +1039,19 @@ def test_cpp_pcl_shim_end_to_end(tmp_path, ctx, bottle, scene_crop, dev_bottle, 
                         env=dict(os.environ, B200PPF_DEVICES="0,0"))
     assert r2.returncode == 0, r2.stdout + r2.stderr
     assert r2.stdout.strip().splitlines()[:9] == lines[:9]
+
+
+def test_bench_dump_outputs_are_the_align_result(tmp_path, ctx, dev_bottle, dev_crop, table_fused):
+    """bench.py --dump-outputs on c1 (the 1 cm bottle against the crop, every 5th scene point a reference): the poses and
+    votes of its last timed step are those b200ppf_register returns on the same clouds, and those its JSON line reports."""
+    import json
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c1", "--steps", "2", "--warmup", "3",
+                        "--no-cpu", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600,
+                       env=dict(os.environ, BENCH_CLOCKS="0"))
+    assert r.returncode == 0, r.stderr
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2
+    _, poses, votes = ctx.register(dev_bottle, table_fused, dev_crop, ref_rate=5)
+    dumped_poses, dumped_votes = np.load(tmp_path / "poses.npy"), np.load(tmp_path / "votes.npy")
+    assert len(votes) > 0 and np.array_equal(dumped_poses, poses) and np.array_equal(dumped_votes, votes.astype(np.float64))
+    assert line["result"]["votes"] == [int(v) for v in dumped_votes]

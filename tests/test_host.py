@@ -321,14 +321,31 @@ def test_header_is_plain_c(tmp_path):
     assert r.returncode == 0, r.stderr
 
 
-def test_bench_reference_arm_prints_the_contract_line():
+def test_bench_reference_arm_prints_the_contract_line(tmp_path, oracle):
+    """The reference arm prints the JSON line, and --dump-outputs writes the clustering of its last step: the oracle's
+    on that step's reference points."""
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "c1",
-                        "--steps", "1", "--warmup", "0", "--cpu-sample", "8"], capture_output=True, text=True, timeout=600)
+                        "--steps", "1", "--warmup", "0", "--cpu-sample", "8", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "pairs/s" and line["higher_is_better"] is True
     assert line["value"] > 0 and line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and "workload" in line["config"]
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    from yolo_ppf_pose_estimation_b200 import workloads
+    wl = workloads.load("c1")
+    refs = bench.sample_list(wl)[:8]  # the one step's reference points, in the order it votes on them
+    assert sorted(refs) == line["sample_refs"]
+    hm = oracle.HashMap(wl.angle_step, wl.dist_step).set_input_feature_cloud(oracle.ppf_estimation(wl.model))
+    hyps, _ = hm.vote_refs(wl.model, wl.scene, refs, n_threads=oracle.host_threads())
+    poses, votes, _, _ = oracle.cluster(hyps, wl.pos_thr, wl.rot_thr)
+    dumped_poses, dumped_votes = np.load(tmp_path / "poses.npy"), np.load(tmp_path / "votes.npy")
+    assert dumped_poses.dtype == np.float32 and dumped_votes.dtype == np.float64 and len(votes) > 0
+    assert np.array_equal(dumped_poses, poses) and np.array_equal(dumped_votes, votes)
 
 
 def test_bench_arms_print_the_same_config_and_a_fixed_cpu_sample():
