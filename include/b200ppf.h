@@ -399,8 +399,9 @@ int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf
  * What this is NOT: the reference's Matching_S2B feeds the edge cloud to its detector's match_S2B; the PCL
  * matching here votes on the object cloud only, so the edges are extracted only when edges_out asks for them.
  * The pose is PPFRegistration::align's (PCL arithmetic), not cv::ppf_match_3d::PPF3DDetector's — that engine is
- * the b200cv_* interface.  PCL's clusterPoses returns at most three poses, so at most three are refined
- * (icp_poses > 3 is clamped); sor_stddev_mul has no default in the reference (argv[5]): 1.0 is this library's. */
+ * the b200cv_* interface, and b200cv_match_object below runs this same chain with it, edges included.  PCL's
+ * clusterPoses returns at most three poses, so at most three are refined (icp_poses > 3 is clamped); sor_stddev_mul
+ * has no default in the reference (argv[5]): 1.0 is this library's. */
 typedef struct b200ppf_object_params {
     float leaf;             /* Subsampling leaf size (CLI argument 4 of the reference) */
     int sor_mean_k;         /* 50 */
@@ -472,6 +473,12 @@ int b200cv_detector_match(b200cv_detector *d, const float *scene, size_t n, size
 int b200cv_detector_match_s2b(b200cv_detector *d, const float *scene, size_t n, size_t stride_floats, const float *edge,
                               size_t n_edge, size_t edge_stride_floats, double relative_scene_sample_step,
                               double relative_scene_distance, b200cv_pose *results, size_t cap, size_t *n_results);
+/* match / match_S2B on device clouds of the detector's context (b200ppf_cloud: the normals, not the curvature, are read):
+ * edge == NULL -> match, else match_S2B.  The same results, bit for bit, as the host calls on the clouds'
+ * b200ppf_cloud_download rows; the last-match queries below report this call. */
+int b200cv_detector_match_cloud(b200cv_detector *d, const b200ppf_cloud *scene, const b200ppf_cloud *edge,
+                                double relative_scene_sample_step, double relative_scene_distance, b200cv_pose *results,
+                                size_t cap, size_t *n_results);
 /* parity hooks: one bucket of the table (ppfInd = i * n_sampled + j, ascending), the whole table, the per-reference poses
  * of the last match before clustering, the accumulator (n_sampled * num_angles words) of one reference point */
 int b200cv_detector_bucket(b200cv_detector *d, size_t bucket, uint32_t *ppf_ind, size_t cap, size_t *n_found);
@@ -481,6 +488,36 @@ int b200cv_detector_debug_accumulator(b200cv_detector *d, const float *scene, si
                                       const float *edge, size_t n_edge, size_t edge_stride_floats,
                                       double relative_scene_sample_step, double relative_scene_distance, size_t reference,
                                       uint32_t *acc);
+
+/* ---- one YOLO box with the engine the reference calls ----------------------------------------------------------------
+ * src/YOLO_cropping_ppf_test.cpp:91-122 per detected object, as one call on device handles: the pre-processing of
+ * b200ppf_match_object (SceneCropping -> Subsampling -> OutlierProcessing -> NormalEstimation -> EdgeExtraction ->
+ * PointCloudXYZNormalToMat, the same stages and results) -> Matching_S2B (include/CloudProcessing.h:481-495:
+ * match_S2B(object, edges, results, 0.05, 0.05); use_edges = 0 runs Matching, :428-442, whose step is 1/14) -> ICP of
+ * the first icp_poses pose clusters against model (the reference's models[id]: the full model, not the detector's
+ * sampled one; :508-530) -> resultsSub[0].  d is trained (b200cv_detector_train); scene and model are clouds of d's
+ * context.  Nothing is copied to the host between the stages.  result: pose / residual / votes of resultsSub[0], the
+ * number of pose clusters (n_poses), the stage sizes and device times; match_ms covers scene sampling, voting and
+ * clustering.  object_out / edges_out (optional) receive the object cloud and its edges (edges when use_edges, or when
+ * edges_out asks and edge_curvature > 0); free them with b200ppf_cloud_free.  Errors: an untrained detector, an empty
+ * crop or edge cloud and a match without a pose cluster are B200PPF_ERR_STATE (the reference exits there, :502-507);
+ * clouds of another context, and use_edges with edge_curvature <= 0, are B200PPF_ERR_INVALID. */
+typedef struct b200cv_object_params {
+    float leaf;                         /* Subsampling leaf size (CLI argument 4 of the reference) */
+    int sor_mean_k;                     /* 50 */
+    double sor_stddev_mul;              /* CLI argument 5; 1.0 here */
+    int normal_k;                       /* 30 */
+    float edge_curvature;               /* 0.03 */
+    int use_edges;                      /* 1: Matching_S2B (default, what main() calls), 0: Matching */
+    double relative_scene_sample_step;  /* 0.05 (:481); Matching uses 1/14 (:428) */
+    double relative_scene_distance;     /* 0.05 */
+    int icp_poses;                      /* 5 (:508), clamped to the clusters returned; 0 = no ICP */
+    b200ppf_icp_params icp;             /* (100, 0.005, 2.5, 8) */
+} b200cv_object_params;
+void b200cv_object_params_default(b200cv_object_params *params);
+int b200cv_match_object(b200cv_detector *d, const b200ppf_cloud *scene, const float corners12[12], const b200ppf_cloud *model,
+                        const b200cv_object_params *params, b200ppf_object_result *result, b200ppf_cloud **object_out,
+                        b200ppf_cloud **edges_out);
 
 #ifdef __cplusplus
 }

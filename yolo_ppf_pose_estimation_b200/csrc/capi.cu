@@ -1039,6 +1039,51 @@ int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf
     return B200PPF_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+struct OwnedCloud {  // intermediate clouds live until the call returns
+    b200ppf_cloud *c = nullptr;
+    ~OwnedCloud() { if (c) b200ppf_cloud_free(c); }
+    b200ppf_cloud *release() { b200ppf_cloud *r = c; c = nullptr; return r; }
+};
+
+// the pre-processing both per-object calls share: SceneCropping -> Subsampling -> OutlierProcessing -> NormalEstimation ->
+// EdgeExtraction (with_edges) -> PointCloudXYZNormalToMat, stage sizes and times into res
+int match_object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const float *corners12, float leaf, int sor_mean_k,
+                      double sor_stddev_mul, int normal_k, float edge_curvature, bool with_edges, b200ppf_object_result *res,
+                      OwnedCloud *object, OwnedCloud *edges) {
+    OwnedCloud cropped, sampled;
+    int rc = b200ppf_crop_pyramid(ctx, scene, corners12, &cropped.c, nullptr);
+    if (rc) return rc;
+    res->crop_ms = ctx->timings.prep_ms;
+    res->n_cropped = (uint32_t)cropped.c->n;
+    if (cropped.c->n == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match object: no scene point inside the box's frustum");
+    const float leaf3[3] = {leaf, leaf, leaf};
+    if ((rc = b200ppf_voxel_grid(ctx, cropped.c, leaf3, &sampled.c))) return rc;
+    res->voxel_ms = ctx->timings.prep_ms;
+    res->n_sampled = (uint32_t)sampled.c->n;
+    if ((rc = b200ppf_statistical_outlier_removal(ctx, sampled.c, sor_mean_k, sor_stddev_mul, &object->c, nullptr, nullptr, nullptr)))
+        return rc;
+    res->outlier_ms = ctx->timings.prep_ms;
+    res->n_filtered = (uint32_t)object->c->n;
+    if ((rc = b200ppf_normal_estimation(ctx, object->c, normal_k, nullptr, B200PPF_COVARIANCE_SHIFTED))) return rc;
+    res->normals_ms = ctx->timings.prep_ms;
+    if (with_edges) {
+        if ((rc = b200ppf_curvature_edges(ctx, object->c, edge_curvature, &edges->c))) return rc;
+        res->edges_ms = ctx->timings.prep_ms;
+        res->n_edges = (uint32_t)edges->c->n;
+    }
+    if ((rc = b200ppf_normalize_normals(ctx, object->c))) return rc;
+    if (edges->c && (rc = b200ppf_normalize_normals(ctx, edges->c))) return rc;
+    return B200PPF_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 void b200ppf_object_params_default(b200ppf_object_params *p) {
     if (!p) return;
     p->leaf = 0.01f;
@@ -1065,33 +1110,11 @@ int b200ppf_match_object(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const flo
     if (params) p = *params;
     memset(res, 0, sizeof(*res));
     const auto t0 = std::chrono::steady_clock::now();
-    struct Owned {  // intermediate clouds live until the call returns
-        b200ppf_cloud *c = nullptr;
-        ~Owned() { if (c) b200ppf_cloud_free(c); }
-        b200ppf_cloud *release() { b200ppf_cloud *r = c; c = nullptr; return r; }
-    } cropped, sampled, object, edges;
-    int rc = b200ppf_crop_pyramid(ctx, scene, corners12, &cropped.c, nullptr);
+    OwnedCloud object, edges;
+    // the edge cloud does not enter the PCL matching: extracted on request only
+    int rc = match_object_prep(ctx, scene, corners12, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k, p.edge_curvature,
+                               p.edge_curvature > 0.0f && edges_out, res, &object, &edges);
     if (rc) return rc;
-    res->crop_ms = ctx->timings.prep_ms;
-    res->n_cropped = (uint32_t)cropped.c->n;
-    if (cropped.c->n == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match object: no scene point inside the box's frustum");
-    const float leaf3[3] = {p.leaf, p.leaf, p.leaf};
-    if ((rc = b200ppf_voxel_grid(ctx, cropped.c, leaf3, &sampled.c))) return rc;
-    res->voxel_ms = ctx->timings.prep_ms;
-    res->n_sampled = (uint32_t)sampled.c->n;
-    if ((rc = b200ppf_statistical_outlier_removal(ctx, sampled.c, p.sor_mean_k, p.sor_stddev_mul, &object.c, nullptr, nullptr, nullptr)))
-        return rc;
-    res->outlier_ms = ctx->timings.prep_ms;
-    res->n_filtered = (uint32_t)object.c->n;
-    if ((rc = b200ppf_normal_estimation(ctx, object.c, p.normal_k, nullptr, B200PPF_COVARIANCE_SHIFTED))) return rc;
-    res->normals_ms = ctx->timings.prep_ms;
-    if (p.edge_curvature > 0.0f && edges_out) {  // the edge cloud does not enter the PCL matching: extracted on request only
-        if ((rc = b200ppf_curvature_edges(ctx, object.c, p.edge_curvature, &edges.c))) return rc;
-        res->edges_ms = ctx->timings.prep_ms;
-        res->n_edges = (uint32_t)edges.c->n;
-    }
-    if ((rc = b200ppf_normalize_normals(ctx, object.c))) return rc;
-    if (edges.c && (rc = b200ppf_normalize_normals(ctx, edges.c))) return rc;
     float final16[16], poses16[3 * 16];
     uint32_t votes[3] = {0, 0, 0};
     size_t n_poses = 0;
@@ -1112,6 +1135,81 @@ int b200ppf_match_object(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const flo
     memcpy(res->pose, refined, 16 * sizeof(double));  // resultsSub[0]
     res->residual = residuals[0];
     res->votes = votes[0];
+    res->total_wall_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (object_out) *object_out = object.release();
+    if (edges_out) *edges_out = edges.release();
+    return B200PPF_OK;
+}
+
+void b200cv_object_params_default(b200cv_object_params *p) {
+    if (!p) return;
+    p->leaf = 0.01f;
+    p->sor_mean_k = 50;                   // OutlierProcessing(50, thresh), src/YOLO_cropping_ppf_test.cpp:98
+    p->sor_stddev_mul = 1.0;
+    p->normal_k = 30;                     // NormalEstimation(30), :101
+    p->edge_curvature = 0.03f;            // EdgeExtraction(0.03), :103
+    p->use_edges = 1;                     // Matching_S2B, :120
+    p->relative_scene_sample_step = 0.05;  // match_S2B(object, edges, results, 0.05, 0.05), include/CloudProcessing.h:481-495
+    p->relative_scene_distance = 0.05;
+    p->icp_poses = 5;                     // N = 5, include/CloudProcessing.h:508
+    p->icp = b200ppf_icp_params{100, 0.005f, 2.5f, 8};
+}
+
+int b200cv_match_object(b200cv_detector *d, const b200ppf_cloud *scene, const float *corners12, const b200ppf_cloud *model,
+                        const b200cv_object_params *params, b200ppf_object_result *res, b200ppf_cloud **object_out,
+                        b200ppf_cloud **edges_out) {
+    if (object_out) *object_out = nullptr;
+    if (edges_out) *edges_out = nullptr;
+    if (!d) return fail_msg(nullptr, B200PPF_ERR_INVALID, "cv match object: null detector");
+    b200ppf_ctx *ctx = cv_detector_context(d);
+    if (!scene || !corners12 || !model || !res) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match object: null argument");
+    if (!cv_detector_trained(d)) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match object: the detector is not trained");
+    if (scene->ctx != ctx || model->ctx != ctx)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match object: the clouds belong to another context than the detector");
+    b200cv_object_params p;
+    b200cv_object_params_default(&p);
+    if (params) p = *params;
+    if (p.use_edges && !(p.edge_curvature > 0.0f))
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match object: Matching_S2B needs the edge cloud, edge_curvature must be positive");
+    DeviceGuard guard(ctx->device);
+    memset(res, 0, sizeof(*res));
+    const auto t0 = std::chrono::steady_clock::now();
+    OwnedCloud object, edges;
+    int rc = match_object_prep(ctx, scene, corners12, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k, p.edge_curvature,
+                               p.use_edges || (p.edge_curvature > 0.0f && edges_out), res, &object, &edges);
+    if (rc) return rc;
+    if (p.use_edges && edges.c->n == 0)
+        return fail_msg(ctx, B200PPF_ERR_STATE, "cv match object: the object has no edge point for Matching_S2B to pair with");
+    const size_t cap = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
+    std::vector<b200cv_pose> poses(cap);
+    size_t n_clusters = 0;
+    cudaEvent_t ev[2] = {nullptr, nullptr};  // the context's events are taken by the stages inside the match
+    PPF_CUDA(ctx, cudaEventCreate(&ev[0]));
+    if (cudaEventCreate(&ev[1]) != cudaSuccess) {
+        cudaEventDestroy(ev[0]);
+        return fail_msg(ctx, B200PPF_ERR_CUDA, "cv match object: cudaEventCreate failed");
+    }
+    cudaEventRecord(ev[0], ctx->stream);
+    rc = b200cv_detector_match_cloud(d, object.c, p.use_edges ? edges.c : nullptr, p.relative_scene_sample_step,
+                                     p.relative_scene_distance, poses.data(), cap, &n_clusters);
+    cudaEventRecord(ev[1], ctx->stream);
+    if (rc == B200PPF_OK && cudaEventSynchronize(ev[1]) == cudaSuccess) cudaEventElapsedTime(&res->match_ms, ev[0], ev[1]);
+    cudaEventDestroy(ev[0]);
+    cudaEventDestroy(ev[1]);
+    if (rc) return rc;
+    res->n_poses = (uint32_t)n_clusters;
+    if (n_clusters == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match object: the matching returned no pose");  // reference: exit(0), :502-507
+    const size_t n_icp = std::min<size_t>(n_clusters, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
+    const size_t n_keep = std::max<size_t>(n_icp, 1);
+    std::vector<double> refined(16 * n_keep), residuals(n_keep, 0.0);
+    for (size_t k = 0; k < n_keep; ++k) memcpy(refined.data() + 16 * k, poses[k].pose, 16 * sizeof(double));
+    if (n_icp) {
+        if ((rc = b200ppf_icp_refine(ctx, model, object.c, &p.icp, refined.data(), n_icp, residuals.data(), nullptr))) return rc;
+        res->icp_ms = ctx->timings.icp_ms;
+    }
+    memcpy(res->pose, refined.data(), 16 * sizeof(double));  // resultsSub[0]
+    res->residual = residuals[0];
+    res->votes = poses[0].num_votes;
     res->total_wall_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (object_out) *object_out = object.release();
     if (edges_out) *edges_out = edges.release();

@@ -158,11 +158,40 @@ struct SampleRange {
     int ns;
 };
 
-__global__ void cv_cell_index_kernel(const float *__restrict__ pc, uint32_t n, uint32_t stride, SampleRange r,
-                                     uint32_t *__restrict__ cell) {
+// where samplePCByQuantization reads its points from: the same kernels serve both, so a device cloud and its downloaded
+// rows go through identical arithmetic
+struct RowPoints {  // host input uploaded as is: rows of `stride` floats [x y z nx ny nz ...]
+    const float *pc;
+    uint32_t stride;
+    __device__ __forceinline__ void xyz(uint32_t i, float p[3]) const {
+        const float *r = pc + (size_t)i * stride;
+        p[0] = r[0], p[1] = r[1], p[2] = r[2];
+    }
+    __device__ __forceinline__ void row(uint32_t i, float p[6]) const {
+        const float *r = pc + (size_t)i * stride;
+#pragma unroll
+        for (int k = 0; k < 6; ++k) p[k] = r[k];
+    }
+};
+struct CloudPoints {  // b200ppf_cloud: x y z in pos, the normal in nrm.xyz; nrm.w holds the curvature and is never read
+    const float4 *pos, *nrm;
+    __device__ __forceinline__ void xyz(uint32_t i, float p[3]) const {
+        const float4 v = pos[i];
+        p[0] = v.x, p[1] = v.y, p[2] = v.z;
+    }
+    __device__ __forceinline__ void row(uint32_t i, float p[6]) const {
+        xyz(i, p);
+        const float4 q = nrm[i];
+        p[3] = q.x, p[4] = q.y, p[5] = q.z;
+    }
+};
+
+template <class Points>
+__global__ void cv_cell_index_kernel(const Points pts, uint32_t n, SampleRange r, uint32_t *__restrict__ cell) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const float *p = pc + (size_t)i * stride;
+    float p[3];
+    pts.xyz(i, p);
     // (int)((float)numSamplesDim * (x - xrange[0]) / xr), index = xc * ns * ns + yc * ns + zc — upstream's stride, under which a
     // coordinate on the upper bound (cell ns) lands in a neighbouring cell's list
     const int xc = (int)((float)r.ns * (p[0] - r.lo[0]) / r.ext[0]);
@@ -177,15 +206,16 @@ __global__ void cv_cell_heads_kernel(const uint32_t *__restrict__ sorted_cell, u
 }
 
 // one thread per occupied cell: the cell's points averaged in input order, in double
-__global__ void cv_cell_average_kernel(const float *__restrict__ pc, uint32_t stride, const uint32_t *__restrict__ order,
-                                       const uint32_t *__restrict__ head, const uint32_t *__restrict__ rank, uint32_t n,
-                                       float *__restrict__ out6) {
+template <class Points>
+__global__ void cv_cell_average_kernel(const Points pts, const uint32_t *__restrict__ order, const uint32_t *__restrict__ head,
+                                       const uint32_t *__restrict__ rank, uint32_t n, float *__restrict__ out6) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n || !head[i]) return;
     double a[6] = {0, 0, 0, 0, 0, 0};
     uint32_t q = i, cnt = 0;
     do {
-        const float *p = pc + (size_t)order[q] * stride;
+        float p[6];
+        pts.row(order[q], p);
 #pragma unroll
         for (int k = 0; k < 6; ++k) a[k] += (double)p[k];
         ++cnt;
@@ -423,9 +453,10 @@ void bbox6(const float *pc, size_t n, size_t stride, float r[6]) {
         }
 }
 
-// samplePCByQuantization of a host cloud -> device rows of 6 floats (caller frees with cudaFree) and their count
-int cv_sample(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, const float range[6], float sample_step, float **d_out,
-              size_t *n_out) {
+// samplePCByQuantization over the box `range` -> device rows of 6 floats (caller frees with cudaFree) and their count
+template <class Points>
+int cv_sample_points(b200ppf_ctx *ctx, const Points &pts, size_t n, const float range[6], float sample_step, float **d_out,
+                     size_t *n_out) {
     *d_out = nullptr;
     *n_out = 0;
     if (n == 0) return B200PPF_OK;
@@ -440,18 +471,15 @@ int cv_sample(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, cons
             return fail_msg(ctx, B200PPF_ERR_INVALID, "cv sample: the cloud's bounding box is flat or not finite (upstream divides by its extent)");
     }
     const uint32_t nn = (uint32_t)n;
-    StreamBuf<float> d_pc(ctx);
     StreamBuf<uint32_t> cell0(ctx), cell1(ctx), ord0(ctx), ord1(ctx), head(ctx), rank(ctx);
-    PPF_CUDA(ctx, d_pc.alloc(n * stride));
     PPF_CUDA(ctx, cell0.alloc(n));
     PPF_CUDA(ctx, cell1.alloc(n));
     PPF_CUDA(ctx, ord0.alloc(n));
     PPF_CUDA(ctx, ord1.alloc(n));
     PPF_CUDA(ctx, head.alloc(n));
     PPF_CUDA(ctx, rank.alloc(n));
-    PPF_CUDA(ctx, cudaMemcpyAsync(d_pc, host, n * stride * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     const unsigned g = (nn + 255) / 256;
-    PPF_LAUNCH(ctx, cv_cell_index_kernel, g, 256, 0, d_pc.p, nn, (uint32_t)stride, r, cell0.p);
+    PPF_LAUNCH(ctx, cv_cell_index_kernel<Points>, g, 256, 0, pts, nn, r, cell0.p);
     int bits = 1;
     const uint64_t max_cell = (uint64_t)(r.ns + 1) * (r.ns + 1) * (r.ns + 1);
     while ((1ull << bits) < max_cell && bits < 32) ++bits;
@@ -465,7 +493,7 @@ int cv_sample(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, cons
     if (rc) return rc;
     float *out = nullptr;
     PPF_CUDA(ctx, cudaMalloc(&out, std::max<size_t>(1, cells) * 6 * sizeof(float)));
-    cv_cell_average_kernel<<<g, 256, 0, ctx->stream>>>(d_pc.p, (uint32_t)stride, os, head.p, rank.p, nn, out);
+    cv_cell_average_kernel<Points><<<g, 256, 0, ctx->stream>>>(pts, os, head.p, rank.p, nn, out);
     ctx->launches++;
     if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
         cudaFree(out);
@@ -474,6 +502,26 @@ int cv_sample(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, cons
     *d_out = out;
     *n_out = cells;
     return B200PPF_OK;
+}
+
+// samplePCByQuantization of a host cloud: its rows uploaded as they are
+int cv_sample(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, const float range[6], float sample_step, float **d_out,
+              size_t *n_out) {
+    *d_out = nullptr;
+    *n_out = 0;
+    if (n == 0) return B200PPF_OK;
+    StreamBuf<float> d_pc(ctx);
+    PPF_CUDA(ctx, d_pc.alloc(n * stride));
+    PPF_CUDA(ctx, cudaMemcpyAsync(d_pc, host, n * stride * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    return cv_sample_points(ctx, RowPoints{d_pc.p, (uint32_t)stride}, n, range, sample_step, d_out, n_out);
+}
+
+// samplePCByQuantization of a device cloud over its own bounding box: bbox_min / bbox_max are the exact, order-free
+// min / max of pos that every producer of a cloud sets (the host upload, cloud_bbox_from_device after the device
+// stages), so the result equals that of the cloud's downloaded rows bit for bit
+int cv_sample_cloud(b200ppf_ctx *ctx, const b200ppf_cloud *c, float sample_step, float **d_out, size_t *n_out) {
+    const float range[6] = {c->bbox_min[0], c->bbox_max[0], c->bbox_min[1], c->bbox_max[1], c->bbox_min[2], c->bbox_max[2]};
+    return cv_sample_points(ctx, CloudPoints{c->pos, c->nrm}, c->n, range, sample_step, d_out, n_out);
 }
 
 void cv_free_match(b200cv_detector *d) {
@@ -729,6 +777,9 @@ int cv_cluster(b200cv_detector *d, const b200cv_pose *d_poses, uint32_t refs, b2
 
 }  // namespace
 
+b200ppf_ctx *cv_detector_context(const b200cv_detector *d) { return d->ctx; }
+bool cv_detector_trained(const b200cv_detector *d) { return d->d_offsets != nullptr; }
+
 }  // namespace b200ppf
 
 using namespace b200ppf;
@@ -882,23 +933,56 @@ int b200cv_detector_table_export(b200cv_detector *d, uint32_t *offsets, uint32_t
     return B200PPF_OK;
 }
 
-static int cv_match_impl(b200cv_detector *d, const float *scene, size_t n, size_t stride, const float *edge, size_t n_edge,
-                         size_t edge_stride, double relative_scene_sample_step, double relative_scene_distance,
-                         b200cv_pose *results, size_t cap, size_t *n_results, uint32_t *acc_dump, size_t dump_ref) {
-    if (!d || !scene || !n_results || (cap && !results)) return fail_msg(d ? d->ctx : nullptr, B200PPF_ERR_INVALID, "cv match: null argument");
+// the checks every match makes; *step = the reference stride of relativeSceneSampleStep
+static int cv_match_begin(b200cv_detector *d, b200cv_pose *results, size_t cap, size_t *n_results, double relative_scene_sample_step,
+                          double relative_scene_distance, int *step) {
+    if (!d || !n_results || (cap && !results)) return fail_msg(d ? d->ctx : nullptr, B200PPF_ERR_INVALID, "cv match: null argument");
     *n_results = 0;
     b200ppf_ctx *ctx = d->ctx;
     if (!d->d_offsets) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match: the detector is not trained");
-    if (stride < 6 || (edge && edge_stride < 6) || n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: clouds are N x 6 [x y z nx ny nz]");
     if (!(relative_scene_sample_step > 0) || !(relative_scene_distance > 0))
         return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: the scene steps must be positive");
+    *step = (int)(1.0 / relative_scene_sample_step);
+    if (*step < 1) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: relativeSceneSampleStep must not exceed 1");
+    return B200PPF_OK;
+}
+
+// everything after sampling, whichever input the sampled clouds came from: the last-match state (sampled scene on the
+// host, per-reference poses), voting, clustering
+static int cv_match_sampled(b200cv_detector *d, int step, b200cv_pose *results, size_t cap, size_t *n_results, uint32_t *acc_dump,
+                            size_t dump_ref) {
+    b200ppf_ctx *ctx = d->ctx;
+    d->h_scene.resize(d->n_scene * 6);
+    PPF_CUDA(ctx, cudaMemcpyAsync(d->h_scene.data(), d->d_scene, d->n_scene * 6 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    const size_t refs = (d->n_scene + step - 1) / step;
+    d->raw.clear();
+    if (refs == 0) return B200PPF_OK;
+    b200cv_pose *d_poses = nullptr;
+    int rc = cv_vote(d, (uint32_t)step, (uint32_t)refs, acc_dump, (uint32_t)dump_ref, &d_poses);
+    if (rc) return rc;
+    size_t ncl = 0;
+    rc = cv_cluster(d, d_poses, (uint32_t)refs, results, cap, &ncl);
+    cudaFreeAsync(d_poses, ctx->stream);
+    if (rc) return rc;
+    *n_results = ncl;
+    return B200PPF_OK;
+}
+
+static int cv_match_impl(b200cv_detector *d, const float *scene, size_t n, size_t stride, const float *edge, size_t n_edge,
+                         size_t edge_stride, double relative_scene_sample_step, double relative_scene_distance,
+                         b200cv_pose *results, size_t cap, size_t *n_results, uint32_t *acc_dump, size_t dump_ref) {
+    if (!scene) return fail_msg(d ? d->ctx : nullptr, B200PPF_ERR_INVALID, "cv match: null argument");
+    int step = 0;
+    int rc = cv_match_begin(d, results, cap, n_results, relative_scene_sample_step, relative_scene_distance, &step);
+    if (rc) return rc;
+    b200ppf_ctx *ctx = d->ctx;
+    if (stride < 6 || (edge && edge_stride < 6) || n == 0)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: clouds are N x 6 [x y z nx ny nz]");
     DevGuard guard(ctx->device);
     cv_free_match(d);
-    const int step = (int)(1.0 / relative_scene_sample_step);
-    if (step < 1) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: relativeSceneSampleStep must not exceed 1");
     float r[6];
     bbox6(scene, n, stride, r);
-    int rc = cv_sample(ctx, scene, n, stride, r, (float)relative_scene_distance, &d->d_scene, &d->n_scene);
+    rc = cv_sample(ctx, scene, n, stride, r, (float)relative_scene_distance, &d->d_scene, &d->n_scene);
     if (rc) return rc;
     d->second_is_scene = edge == nullptr;
     if (edge) {
@@ -910,20 +994,34 @@ static int cv_match_impl(b200cv_detector *d, const float *scene, size_t n, size_
         d->d_second = d->d_scene;
         d->n_second = d->n_scene;
     }
-    d->h_scene.resize(d->n_scene * 6);
-    PPF_CUDA(ctx, cudaMemcpyAsync(d->h_scene.data(), d->d_scene, d->n_scene * 6 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    const size_t refs = (d->n_scene + step - 1) / step;
-    d->raw.clear();
-    if (refs == 0) return B200PPF_OK;
-    b200cv_pose *d_poses = nullptr;
-    rc = cv_vote(d, (uint32_t)step, (uint32_t)refs, acc_dump, (uint32_t)dump_ref, &d_poses);
+    return cv_match_sampled(d, step, results, cap, n_results, acc_dump, dump_ref);
+}
+
+int b200cv_detector_match_cloud(b200cv_detector *d, const b200ppf_cloud *scene, const b200ppf_cloud *edge,
+                                double relative_scene_sample_step, double relative_scene_distance, b200cv_pose *results, size_t cap,
+                                size_t *n_results) {
+    int step = 0;
+    int rc = cv_match_begin(d, results, cap, n_results, relative_scene_sample_step, relative_scene_distance, &step);
     if (rc) return rc;
-    size_t ncl = 0;
-    rc = cv_cluster(d, d_poses, (uint32_t)refs, results, cap, &ncl);
-    cudaFreeAsync(d_poses, ctx->stream);
+    b200ppf_ctx *ctx = d->ctx;
+    if (!scene) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match cloud: null scene");
+    if (scene->ctx != ctx || (edge && edge->ctx != ctx))
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match cloud: the clouds belong to another context than the detector");
+    if (scene->n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match cloud: empty scene cloud");
+    if (edge && edge->n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match_S2B: empty edge cloud");
+    DevGuard guard(ctx->device);
+    cv_free_match(d);
+    rc = cv_sample_cloud(ctx, scene, (float)relative_scene_distance, &d->d_scene, &d->n_scene);
     if (rc) return rc;
-    *n_results = ncl;
-    return B200PPF_OK;
+    d->second_is_scene = edge == nullptr;
+    if (edge) {
+        rc = cv_sample_cloud(ctx, edge, (float)relative_scene_distance, &d->d_second, &d->n_second);
+        if (rc) return rc;
+    } else {
+        d->d_second = d->d_scene;
+        d->n_second = d->n_scene;
+    }
+    return cv_match_sampled(d, step, results, cap, n_results, nullptr, 0);
 }
 
 int b200cv_detector_match(b200cv_detector *d, const float *scene, size_t n, size_t stride, double relative_scene_sample_step,

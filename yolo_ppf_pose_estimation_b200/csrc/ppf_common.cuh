@@ -58,7 +58,7 @@ struct b200ppf_cloud {
     size_t n = 0;
     float4 *pos = nullptr;  // x y z 1
     float4 *nrm = nullptr;  // nx ny nz 0
-    float bbox_min[3] = {0, 0, 0}, bbox_max[3] = {0, 0, 0};
+    float bbox_min[3] = {0, 0, 0}, bbox_max[3] = {0, 0, 0};  // exact min / max of pos: every producer of a cloud sets them
 };
 
 struct b200ppf_features {
@@ -178,6 +178,10 @@ int k5_transform(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, const float *pose
 int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cloud *scene, int max_iterations,
                   float tolerance, float rejection_scale, int num_levels, double *poses16_host, size_t n_poses,
                   double *residuals_host, uint64_t *iterations_host);
+
+// the context of an OpenCV-engine detector and whether it holds a trained model (k7_cvppf.cu)
+b200ppf_ctx *cv_detector_context(const b200cv_detector *d);
+bool cv_detector_trained(const b200cv_detector *d);
 
 // exclusive scan of 0/1 flags on the context stream (prep.cu): rank[k] = set flags before k; total on the host
 int flag_scan_u32(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, uint32_t *total_host);
