@@ -23,6 +23,11 @@
 //             The scene phase's own cell compares phases per entry; tables whose 2*pi/step is not an
 //             integer bin every entry in fixed point with guard bands, the literal double-precision
 //             form inside the bands.
+//   D  fold   tables of 2 M+ entries, flushes of FOLD_MIN_PAIRS+ candidates: a pair on the constant-shift path keeps
+//             only its own cell in phase C and leaves a code (key, q, cell) in the drained candidate queue.  The codes
+//             are sorted; for every (bucket, shift s) they touch, a warp reads off per cell how many pairs vote on it
+//             with that shift (prefix / suffix counts of the cells at q = s and q = s - 1) and walks the cell once,
+//             adding count x pairs.  Sums of integers in any order: the accumulators are those of one walk per pair.
 // The accumulator slice is bin-major (word = bin * pitch + row, pitch a multiple of 32): the bank of a vote
 // is (row mod 32) whatever the scene pair, and the table build orders every phase cell so that 32
 // consecutive entries hit 32 different banks.
@@ -63,6 +68,12 @@ constexpr int CAND_CAP = B200PPF_CAND_CAP;  // in-radius candidates buffered bet
 #endif
 constexpr int VOTE_UNROLL = B200PPF_VOTE_UNROLL;
 static_assert(CAND_CAP >= 2 * VOTE_THREADS_LARGE, "flush threshold must leave one sweep iteration of room");
+#ifndef B200PPF_FOLD_MIN_PAIRS
+#define B200PPF_FOLD_MIN_PAIRS 1024
+#endif
+constexpr uint32_t FOLD_MIN_PAIRS = B200PPF_FOLD_MIN_PAIRS;  // flushes with fewer candidates keep one walk per pair
+constexpr size_t FOLD_MIN_ENTRIES = 1u << 21;  // tables below this walk short buckets: folding does not repay its sort
+static_assert((CAND_CAP & (CAND_CAP - 1)) == 0, "the fold codes of a flush are sorted in place (bitonic)");
 
 // One in-radius scene pair with a non-empty bucket.  Phase-sorted tables: the bucket's merged words are
 // [off, off + len); those below k_below lie under the scene pair's phase (shift constant c_below), those from
@@ -85,6 +96,8 @@ struct __align__(16) WorkItem {
 constexpr size_t queue_bytes(int threads) { return CAND_CAP * sizeof(uint32_t) + (size_t)threads * sizeof(WorkItem); }
 constexpr size_t SMALL_SHAPE_SMEM_MAX = 111 * 1024;  // two such CTAs (+ static + system reserve) share one SM
 constexpr size_t STATIC_RESERVE = 2048;  // static shared + the 1 KB the system reserves per CTA
+// the folded groups of a flush (at most two per fold code) live where the consumed work items were
+static_assert(2 * CAND_CAP * sizeof(uint32_t) <= VOTE_THREADS_SMALL * sizeof(WorkItem), "fold groups must fit the item queue");
 
 struct VoteArgs {
     const float4 *pos, *nrm;    // scene, original order (reference points are addressed by index)
@@ -122,6 +135,7 @@ struct VoteArgs {
     uint32_t signal_slot, signal_value;
     uint32_t *done_counter;
     int no_sub_phase;  // debug (B200PPF_NO_SUB_PHASE): compare every own-cell entry in full
+    uint32_t fold_qbits;  // bits of q in a fold code (key, q, cell); 0: every pair walks its own bucket
 };
 
 __device__ __forceinline__ unsigned long long shfl_xor_u64(unsigned long long v, int o) {
@@ -160,6 +174,10 @@ __device__ __forceinline__ void red_shared_inc_if_lt(uint32_t addr, uint32_t k, 
                  : "memory");
 }
 
+// count of a merged word times the scene pairs that cast it: one pair's item (the constant 1) or a folded group
+__device__ __forceinline__ uint32_t times(uint32_t cnt, std::integral_constant<uint32_t, 1>) { return cnt; }
+__device__ __forceinline__ uint32_t times(uint32_t cnt, uint32_t pairs) { return cnt * pairs; }
+
 // One vote of the per-entry path of tables without phase cells (alpha mode A), in fixed point (ppf_math.cuh,
 // alpha_bin_fixed):  X = A_m - C_s  (wraps like the angle),  hi = mulhi(X, T_fix) = bin.position,
 // (bin, frac) = hi * 2^(32-s).  The increment is unconditional — a select is cheaper than a divergent branch —
@@ -191,12 +209,13 @@ __device__ __forceinline__ void vote_exact(const BinParams &bp, uint32_t acc_add
 }
 
 // one (reference point, accumulator slice) task; ref_i = reference slot of this launch
-template <int MODE, bool SEAM, bool BULK, int THREADS>
+// FOLD: the table folds (phase D); the other tables run a kernel without it
+template <int MODE, bool SEAM, bool BULK, int THREADS, bool FOLD>
 __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_i, const uint32_t slice,
                                           uint32_t *next_task) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ Frame s_sg;
-    __shared__ uint32_t s_ncand, s_nitems, s_next, s_scratch;
+    __shared__ uint32_t s_ncand, s_nitems, s_next, s_scratch, s_nfold, s_ngroups;
     __shared__ uint32_t s_cls[8];  // work items per length class of the current round
     __shared__ uint32_t s_run_start[9], s_run_end[9];
     __shared__ unsigned long long s_best[(THREADS / 32)];
@@ -229,6 +248,8 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
         s_ncand = 0;
         s_nitems = 0;
         s_next = 0;
+        s_nfold = 0;
+        s_ngroups = 0;
     }
     if (tid < 4) s_stat[tid] = 0;
     if (tid >= 64 && tid < 72) s_cls[tid - 64] = 0;
@@ -257,9 +278,50 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
     const uint32_t fmask = (1u << a.bp.fix_shift) - 1u;
     uint32_t st_examined = 0, st_in_radius = 0, st_nonempty = 0, st_votes = 0, st_skipped = 0;
 
-    // phases B + C over the buffered candidates
+    // shift range [kb, ke) of merged words mp[]: add count * mult at umin(hot word - c, hot word - c + one turn).  The
+    // arrays carry ENTRY_PAD readable words past the end, so the partial batch loads unclamped.  mult is the constant 1
+    // for one scene pair's item, the number of folded pairs for a folded group (D).
+    auto shift_range = [&](const uint32_t *mp, uint32_t kb, uint32_t ke, uint32_t c0v, auto mult) {
+        const uint32_t c1v = c0v - wrap_bytes;
+        uint32_t k0 = kb + lane;
+        auto vote = [&](uint32_t w) {
+            const uint32_t off = w & 0xFFFFFFu;
+            red_shared_add(acc_addr + min(off - c0v, off - c1v), times(w >> 24, mult));
+        };
+        // long ranges: 8 x 32 words in flight per lane (the gathers are latency-bound)
+        for (; k0 - lane + 64 * VOTE_UNROLL <= ke; k0 += 64 * VOTE_UNROLL) {  // warp-uniform: a double batch
+            uint32_t hw[2 * VOTE_UNROLL];
+#pragma unroll
+            for (int u = 0; u < 2 * VOTE_UNROLL; ++u) hw[u] = __ldg(mp + k0 + u * 32);
+#pragma unroll
+            for (int u = 0; u < 2 * VOTE_UNROLL; ++u) vote(hw[u]);
+        }
+        if (k0 - lane + 32 * VOTE_UNROLL <= ke) {  // warp-uniform: one more full batch
+            uint32_t hw[VOTE_UNROLL];
+#pragma unroll
+            for (int u = 0; u < VOTE_UNROLL; ++u) hw[u] = __ldg(mp + k0 + u * 32);
+#pragma unroll
+            for (int u = 0; u < VOTE_UNROLL; ++u) vote(hw[u]);
+            k0 += 32 * VOTE_UNROLL;
+        }
+        if (k0 - lane < ke) {  // warp-uniform: a partial batch remains; votes are predicated
+            uint32_t hw[VOTE_UNROLL];
+#pragma unroll
+            for (int u = 0; u < VOTE_UNROLL; ++u) hw[u] = __ldg(mp + k0 + u * 32);
+#pragma unroll
+            for (int u = 0; u < VOTE_UNROLL; ++u) {
+                const uint32_t off = hw[u] & 0xFFFFFFu;
+                red_shared_add_if_lt(acc_addr + min(off - c0v, off - c1v), times(hw[u] >> 24, mult), k0 + u * 32, ke);
+            }
+        }
+    };
+
+    // phases B + C (+ D) over the buffered candidates
     auto flush = [&]() {
         const uint32_t ncand = s_ncand;
+        // Fold the constant-shift walks of this flush's pairs (D below): on tables of FOLD_MIN_ENTRIES+ entries, when the
+        // flush holds enough pairs to share buckets.  Light reference points keep one walk per pair.
+        const bool fold = FOLD && BULK && ncand >= FOLD_MIN_PAIRS;
         for (uint32_t c0 = 0; c0 < ncand; c0 += THREADS) {
             // ---- B: pair features -> work items -------------------------------------------------
             const uint32_t c = c0 + tid;
@@ -267,6 +329,8 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
             // phase's cell [ma, mb) into below / above, and the cell's own unmerged entries are [oa, ob)
             uint32_t o0 = 0, oa = 0, ob = 0, oF = 0, q = 0, c_s = 0, phi = 0, sub_range = 0;
             uint32_t m0 = 0, ma = 0, mb = 0, mF = 0;
+            uint32_t code = 0;  // folding pair: (key, q, cell)
+            bool folds = false;
             float alpha_s = 0.0f;
             if (tid < THREADS && c < ncand) {
                 const uint32_t s = cand[c];
@@ -304,6 +368,11 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                                     mb = __ldg(mo + cell + 1);
                                     oa = __ldg(so + cell);
                                     ob = __ldg(so + cell + 1);
+                                    if (fold) {  // the shift ranges go to a folded group; the item keeps the own cell
+                                        folds = true;
+                                        code = (((key << a.fold_qbits) | q) << lf) | cell;
+                                        m0 = ma = mb = mF = 0;
+                                    }
                                 }
                             }
                         }
@@ -325,6 +394,15 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 }
             }
             __syncthreads();
+            if (fold) {  // every candidate of the round has been read: the fold codes take the front of the queue
+                const uint32_t fm = __ballot_sync(0xFFFFFFFFu, folds);
+                if (fm) {
+                    uint32_t b = 0;
+                    if (lane == (uint32_t)(__ffs(fm) - 1)) b = atomicAdd(&s_nfold, __popc(fm));
+                    b = __shfl_sync(0xFFFFFFFFu, b, __ffs(fm) - 1);
+                    if (folds) cand[b + __popc(fm & ((1u << lane) - 1u))] = code;
+                }
+            }
             if (push) {
                 uint32_t slot = rank;
 #pragma unroll
@@ -361,45 +439,10 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 const WorkItem wi = items[w];
                 const uint32_t len = wi.len;
                 const uint32_t *mp = a.merged_w + wi.off;
-                // shift range [kb, ke) of merged words: count votes at umin(hot word - c, hot word - c + one turn).  The
-                // arrays carry ENTRY_PAD readable words past the end, so the partial batch loads unclamped.
-                auto shift_range = [&](uint32_t kb, uint32_t ke, uint32_t c0v) {
-                    const uint32_t c1v = c0v - wrap_bytes;
-                    uint32_t k0 = kb + lane;
-                    auto vote = [&](uint32_t w) {
-                        const uint32_t off = w & 0xFFFFFFu;
-                        red_shared_add(acc_addr + min(off - c0v, off - c1v), w >> 24);
-                    };
-                    // long ranges: 8 x 32 words in flight per lane (the gathers are latency-bound)
-                    for (; k0 - lane + 64 * VOTE_UNROLL <= ke; k0 += 64 * VOTE_UNROLL) {  // warp-uniform: a double batch
-                        uint32_t hw[2 * VOTE_UNROLL];
-#pragma unroll
-                        for (int u = 0; u < 2 * VOTE_UNROLL; ++u) hw[u] = __ldg(mp + k0 + u * 32);
-#pragma unroll
-                        for (int u = 0; u < 2 * VOTE_UNROLL; ++u) vote(hw[u]);
-                    }
-                    if (k0 - lane + 32 * VOTE_UNROLL <= ke) {  // warp-uniform: one more full batch
-                        uint32_t hw[VOTE_UNROLL];
-#pragma unroll
-                        for (int u = 0; u < VOTE_UNROLL; ++u) hw[u] = __ldg(mp + k0 + u * 32);
-#pragma unroll
-                        for (int u = 0; u < VOTE_UNROLL; ++u) vote(hw[u]);
-                        k0 += 32 * VOTE_UNROLL;
-                    }
-                    if (k0 - lane < ke) {  // warp-uniform: a partial batch remains; votes are predicated
-                        uint32_t hw[VOTE_UNROLL];
-#pragma unroll
-                        for (int u = 0; u < VOTE_UNROLL; ++u) hw[u] = __ldg(mp + k0 + u * 32);
-#pragma unroll
-                        for (int u = 0; u < VOTE_UNROLL; ++u) {
-                            const uint32_t off = hw[u] & 0xFFFFFFu;
-                            red_shared_add_if_lt(acc_addr + min(off - c0v, off - c1v), hw[u] >> 24, k0 + u * 32, ke);
-                        }
-                    }
-                };
                 if (BULK) {
-                    if (wi.k_below) shift_range(0u, wi.k_below, wi.c_below);
-                    if (wi.k_above < len) shift_range(wi.k_above, len, wi.c_below - unit);
+                    const std::integral_constant<uint32_t, 1> one;
+                    if (wi.k_below) shift_range(mp, 0u, wi.k_below, wi.c_below, one);
+                    if (wi.k_above < len) shift_range(mp, wi.k_above, len, wi.c_below - unit, one);
                 }
                 if (wi.e_len) {
                     // per-entry range [0, e_end) of the unmerged entry arrays
@@ -530,6 +573,93 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
             if (tid >= 64 && tid < 72) s_cls[tid - 64] = 0;
             __syncthreads();
         }
+        const uint32_t n = fold ? s_nfold : 0u;
+        if (n) {
+            // ---- D: folded shift ranges ------------------------------------------------------------
+            // A folding pair (q, c) votes on cell k of its bucket with shift q + 1 below c and q above it, so the pairs
+            // of one bucket that vote on cell k with shift s number
+            //     m_s(k) = #{q = s, c < k} + #{q = s - 1 (mod N_T), c > k},
+            // and one walk of the cell adding count * m_s(k) casts all their votes.  The codes (key, q, c) are sorted
+            // (bitonic, in place), so both terms are differences of lower bounds.
+            const uint32_t qb = a.fold_qbits, qmask = (1u << qb) - 1u, ncell = 1u << lf;
+            uint32_t np = 32;
+            while (np < n) np <<= 1;
+            for (uint32_t i = n + tid; i < np; i += THREADS) cand[i] = 0xFFFFFFFFu;  // codes have at most 31 bits
+            __syncthreads();
+            for (uint32_t k = 2; k <= np; k <<= 1)
+                for (uint32_t j = k >> 1; j > 0; j >>= 1) {
+                    for (uint32_t i = tid; i < np / 2; i += THREADS) {
+                        const uint32_t lo = ((i & ~(j - 1u)) << 1) | (i & (j - 1u)), hi = lo + j;
+                        const uint32_t x = cand[lo], y = cand[hi];
+                        if ((x > y) == ((lo & k) == 0)) {
+                            cand[lo] = y;
+                            cand[hi] = x;
+                        }
+                    }
+                    __syncthreads();
+                }
+            auto first_at_least = [&](uint32_t x) {
+                uint32_t lo = 0, len = n;
+                while (len) {
+                    const uint32_t half = len >> 1;
+                    if (cand[lo + half] < x) {
+                        lo += half + 1;
+                        len -= half + 1;
+                    } else {
+                        len = half;
+                    }
+                }
+                return lo;
+            };
+            // one group (key, s) per s that some run (key, q) touches: s = q, and s = q + 1 when no run (key, q + 1) exists
+            uint32_t *groups = reinterpret_cast<uint32_t *>(items);  // the round's items are consumed
+            for (uint32_t i = tid; i < n; i += THREADS) {
+                const uint32_t run = cand[i] >> lf;
+                if (i == 0 || (cand[i - 1] >> lf) != run) {
+                    const uint32_t q = run & qmask;
+                    const uint32_t next = ((run - q) | (q + 1u == a.bp.n_turn ? 0u : q + 1u)) << lf;
+                    const uint32_t p = first_at_least(next);
+                    const bool alone = p == n || (cand[p] >> lf) != (next >> lf);
+                    const uint32_t slot = atomicAdd(&s_ngroups, alone ? 2u : 1u);
+                    groups[slot] = run << lf;
+                    if (alone) groups[slot + 1] = next;
+                }
+            }
+            __syncthreads();
+            const uint32_t ngroups = s_ngroups;
+            for (;;) {
+                uint32_t w = 0;
+                if (lane == 0) w = atomicAdd(&s_next, 1u);
+                w = __shfl_sync(0xFFFFFFFFu, w, 0);
+                if (w >= ngroups) break;
+                const uint32_t g = groups[w], run = g >> lf, s = run & qmask;
+                const uint32_t gp = ((run - s) | (s == 0 ? a.bp.n_turn - 1u : s - 1u)) << lf;
+                // lane k < 16: first code >= (key, s, k); lane 16 + k: first code >= (key, s - 1, k + 1)
+                const uint32_t kk = lane & 15u;
+                const uint32_t pos = first_at_least(lane < 16 ? g + kk : gp + kk + 1u);
+                const uint32_t m = (pos - __shfl_sync(0xFFFFFFFFu, pos, 0)) +
+                                   (__shfl_sync(0xFFFFFFFFu, pos, 15 + ncell) - __shfl_sync(0xFFFFFFFFu, pos, 16 + kk));
+                // lane k <= ncell: start of cell k of the bucket in the merged words
+                const uint32_t mo = __ldg(slice_moffsets + ((size_t)(run >> qb) << lf) + min(lane, ncell));
+                const uint32_t m_prev = __shfl_up_sync(0xFFFFFFFFu, m, 1), m_next = __shfl_down_sync(0xFFFFFFFFu, m, 1);
+                // consecutive cells with the same multiplier are one range
+                const bool live = lane < ncell && m != 0;
+                uint32_t starts = __ballot_sync(0xFFFFFFFFu, live && (lane == 0 || m_prev != m));
+                const uint32_t ends = __ballot_sync(0xFFFFFFFFu, live && (lane + 1 == ncell || m_next != m));
+                while (starts) {
+                    const uint32_t b = __ffs(starts) - 1, e = __ffs(ends & (0xFFFFFFFFu << b)) - 1;
+                    shift_range(a.merged_w, __shfl_sync(0xFFFFFFFFu, mo, b), __shfl_sync(0xFFFFFFFFu, mo, e + 1), unit * s,
+                                __shfl_sync(0xFFFFFFFFu, m, b));
+                    starts &= starts - 1;
+                }
+            }
+            __syncthreads();
+            if (tid == 0) {
+                s_next = 0;
+                s_nfold = 0;
+                s_ngroups = 0;
+            }
+        }
         if (tid == 0) s_ncand = 0;
         __syncthreads();
     };
@@ -658,7 +788,7 @@ __global__ void ref_cost_kernel(const float4 *__restrict__ pos, const uint32_t *
     inv_cost[r] = n_s - n;  // ascending sort = heaviest first; equal costs keep reference order (stable sort)
 }
 
-template <int MODE, bool SEAM, bool BULK, int THREADS>
+template <int MODE, bool SEAM, bool BULK, int THREADS, bool FOLD>
 __global__ void __launch_bounds__(THREADS, THREADS == 1024 ? 1 : B200PPF_VOTE_MINBLOCKS)
 ppf_vote_kernel(const VoteArgs a) {
     // Either one CTA per (reference point, slice) — the grid is (positions, slices) — or persistent CTAs on a queue
@@ -673,7 +803,7 @@ ppf_vote_kernel(const VoteArgs a) {
         const uint32_t task = s_task;
         if (task >= total) break;
         const uint32_t pos = task % a.ref_count;
-        vote_task<MODE, SEAM, BULK, THREADS>(a, a.ref_order ? a.ref_order[pos] : pos, task / a.ref_count,
+        vote_task<MODE, SEAM, BULK, THREADS, FOLD>(a, a.ref_order ? a.ref_order[pos] : pos, task / a.ref_count,
                                              persistent ? &s_task : nullptr);
         if (!persistent) break;
     }
@@ -860,6 +990,13 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
     a.signal_slot = a.signal_value = 0;
     a.done_counter = nullptr;
     a.no_sub_phase = getenv("B200PPF_NO_SUB_PHASE") ? 1 : 0;
+    // folded shift ranges: phase-sorted tables of FOLD_MIN_ENTRIES+ entries whose fold codes (key, q, cell) fit 31 bits
+    a.fold_qbits = 0;
+    if (a.bp.bulk && a.bp.mode == ALPHA_MODE_A && t->info.n_entries >= FOLD_MIN_ENTRIES) {
+        auto bits = [](uint32_t x) { uint32_t b = 0; while (b < 32 && (x >> b) != 0) ++b; return b; };
+        const uint32_t qbits = bits(a.bp.n_turn - 1u);
+        if (bits(a.kp.key_space - 1u) + qbits + a.bp.cells_log2 <= 31) a.fold_qbits = qbits;
+    }
     for (int g = 0; g < MAX_PEERS; ++g) {
         a.peer_peaks[g] = nullptr;
         a.peer_flags[g] = nullptr;
@@ -899,22 +1036,23 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
         if (rc) return rc;
         a.ref_order = in_alt ? order_alt.p : order.p;
     }
-#define LAUNCH_VOTE_T(M, S, B, T)                                                                                  \
+#define LAUNCH_VOTE_T(M, S, B, T, F)                                                                                  \
     do {                                                                                                            \
-        PPF_CUDA(ctx, cudaFuncSetAttribute(ppf_vote_kernel<M, S, B, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+        PPF_CUDA(ctx, cudaFuncSetAttribute(ppf_vote_kernel<M, S, B, T, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                            (int)smem));                                                             \
-        PPF_LAUNCH(ctx, (ppf_vote_kernel<M, S, B, T>), grid_dim, T, smem, a);                                       \
+        PPF_LAUNCH(ctx, (ppf_vote_kernel<M, S, B, T, F>), grid_dim, T, smem, a);                                       \
     } while (0)
-#define LAUNCH_VOTE(M, S, B)                                                            \
+#define LAUNCH_VOTE(M, S, B, F)                                                          \
     do {                                                                                 \
-        if (threads == VOTE_THREADS_SMALL) LAUNCH_VOTE_T(M, S, B, VOTE_THREADS_SMALL);  \
-        else LAUNCH_VOTE_T(M, S, B, VOTE_THREADS_LARGE);                                \
+        if (threads == VOTE_THREADS_SMALL) LAUNCH_VOTE_T(M, S, B, VOTE_THREADS_SMALL, F);  \
+        else LAUNCH_VOTE_T(M, S, B, VOTE_THREADS_LARGE, F);                            \
     } while (0)
     const int threads = vote_threads(t);
-    if (ctx->alpha_mode == ALPHA_MODE_B) LAUNCH_VOTE(ALPHA_MODE_B, false, false);
-    else if (a.bp.bulk) LAUNCH_VOTE(ALPHA_MODE_A, false, true);  // an integer T has no separate seam band
-    else if (a.bp.seam_guard) LAUNCH_VOTE(ALPHA_MODE_A, true, false);
-    else LAUNCH_VOTE(ALPHA_MODE_A, false, false);
+    if (ctx->alpha_mode == ALPHA_MODE_B) LAUNCH_VOTE(ALPHA_MODE_B, false, false, false);
+    else if (a.bp.bulk && a.fold_qbits) LAUNCH_VOTE(ALPHA_MODE_A, false, true, true);
+    else if (a.bp.bulk) LAUNCH_VOTE(ALPHA_MODE_A, false, true, false);  // an integer T has no separate seam band
+    else if (a.bp.seam_guard) LAUNCH_VOTE(ALPHA_MODE_A, true, false, false);
+    else LAUNCH_VOTE(ALPHA_MODE_A, false, false, false);
 #undef LAUNCH_VOTE_T
 #undef LAUNCH_VOTE
     cudaEventRecord(ctx->ev_vote[2], ctx->stream);
