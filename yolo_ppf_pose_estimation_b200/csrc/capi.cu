@@ -24,17 +24,36 @@ int fail_msg(b200ppf_ctx *ctx, int code, const char *msg) {
     return code;
 }
 
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) {
-        cudaGetDevice(&prev);
-        if (prev != dev) cudaSetDevice(dev);
-        else prev = -1;
-    }
-    ~DeviceGuard() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
+int cloud_alloc(b200ppf_ctx *ctx, size_t n, CloudPtr *out) {
+    CloudPtr c(new (std::nothrow) b200ppf_cloud());
+    if (!c) return fail_msg(ctx, B200PPF_ERR_NOMEM, "cloud: out of host memory");
+    c->ctx = ctx;
+    c->n = n;
+    PPF_CUDA(ctx, cudaMallocAsync(&c->pos, std::max<size_t>(1, 2 * n) * sizeof(float4), ctx->stream));
+    c->nrm = c->pos + n;
+    *out = std::move(c);
+    return B200PPF_OK;
+}
+
+std::array<TableArray, 8> table_arrays(b200ppf_table *t) {
+    const uint64_t total_keys = (uint64_t)t->info.key_space * t->info.n_slices;
+    const bool cells = t->bp.cells_log2 != 0, merged = cells && t->info.n_entries != 0;
+    const size_t n_sub = cells ? (size_t)(total_keys << t->bp.cells_log2) + 1 : 0, ne = t->info.n_entries;
+    return {{{&t->offsets, (size_t)total_keys + 1, 0, true},
+             {&t->sub_offsets, n_sub, 0, cells},
+             {&t->entry_w, ne, ENTRY_PAD, true},
+             {&t->entry_am, ne, ENTRY_PAD, true},
+             {reinterpret_cast<uint32_t **>(&t->entry_alpha), ne, 0, true},
+             {&t->entry_idx, ne, 0, true},
+             {&t->merged_w, merged ? t->n_merged : 0, ENTRY_PAD, merged},
+             {&t->msub_offsets, merged ? n_sub : 0, 0, merged}}};
+}
+
+cudaError_t table_array_alloc(cudaStream_t stream, const TableArray &a) {
+    cudaError_t e = cudaMallocAsync(a.slot, std::max<size_t>(1, a.words + a.pad) * sizeof(uint32_t), stream);
+    if (e == cudaSuccess && a.pad) e = cudaMemsetAsync(*a.slot + a.words, 0, a.pad * sizeof(uint32_t), stream);
+    return e;
+}
 
 }  // namespace b200ppf
 
@@ -170,18 +189,8 @@ int b200ppf_cloud_upload(b200ppf_ctx *ctx, const float *host, size_t n, size_t s
     if (stride < 6 || noff < 3 || noff + 3 > stride)
         return fail_msg(ctx, B200PPF_ERR_INVALID, "cloud upload: stride/normal offset do not describe [x y z .. nx ny nz]");
     // AoS -> float4 SoA staging in the context's grow-only pinned buffer, dropping non-finite points
-    const size_t need = std::max<size_t>(1, 2 * n) * sizeof(float4);
-    if (ctx->stage_bytes < need) {
-        if (ctx->stage) cudaFreeHost(ctx->stage);
-        ctx->stage = nullptr;
-        ctx->stage_bytes = 0;
-        PPF_CUDA(ctx, cudaMallocHost(&ctx->stage, need));
-        ctx->stage_bytes = need;
-    }
-    float4 *stage = static_cast<float4 *>(ctx->stage);
-    b200ppf_cloud *c = new (std::nothrow) b200ppf_cloud();
-    if (!c) return fail_msg(ctx, B200PPF_ERR_NOMEM, "cloud upload: out of host memory");
-    c->ctx = ctx;
+    PPF_CUDA(ctx, grow_buffer(&ctx->stage, &ctx->stage_cap, std::max<size_t>(1, 2 * n), /*pinned=*/true));
+    float4 *stage = ctx->stage;
     size_t m = 0;
     float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
     float4 *sp = stage, *sn = stage + n;
@@ -200,25 +209,20 @@ int b200ppf_cloud_upload(b200ppf_ctx *ctx, const float *host, size_t n, size_t s
         }
         ++m;
     }
-    c->n = m;
+    CloudPtr c;
+    int rc = cloud_alloc(ctx, m, &c);
+    if (rc) return rc;
     for (int k = 0; k < 3; ++k) {
         c->bbox_min[k] = m ? lo[k] : 0.0f;
         c->bbox_max[k] = m ? hi[k] : 0.0f;
     }
-    // one stream-ordered allocation holds both arrays (pos | nrm)
-    cudaError_t e = cudaMallocAsync(&c->pos, std::max<size_t>(1, 2 * m) * sizeof(float4), ctx->stream);
-    if (e == cudaSuccess) c->nrm = c->pos + m;
     cudaEventRecord(ctx->ev[0], ctx->stream);
-    if (e == cudaSuccess && m) e = cudaMemcpyAsync(c->pos, sp, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess && m) e = cudaMemcpyAsync(c->nrm, sn, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream);
+    if (m) PPF_CUDA(ctx, cudaMemcpyAsync(c->pos, sp, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
+    if (m) PPF_CUDA(ctx, cudaMemcpyAsync(c->nrm, sn, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
     cudaEventRecord(ctx->ev[1], ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);  // the staging buffer is reused by the next upload
-    if (e != cudaSuccess) {
-        b200ppf_cloud_free(c);
-        return fail_msg(ctx, e == cudaErrorMemoryAllocation ? B200PPF_ERR_NOMEM : B200PPF_ERR_CUDA, cudaGetErrorString(e));
-    }
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the staging buffer is reused by the next upload
     cudaEventElapsedTime(&ctx->timings.upload_ms, ctx->ev[0], ctx->ev[1]);
-    *out = c;
+    *out = c.release();
     return B200PPF_OK;
 }
 
@@ -541,33 +545,28 @@ int b200ppf_table_save(b200ppf_ctx *ctx, const b200ppf_table *t, const char *pat
     h.info = t->info;
     h.kp = t->kp;
     h.bp = t->bp;
-    const uint64_t total_keys = (uint64_t)t->info.key_space * t->info.n_slices;
-    h.n_offsets = total_keys + 1;
-    h.n_sub_offsets = t->sub_offsets ? (total_keys << t->bp.cells_log2) + 1 : 0;
+    const std::array<TableArray, 8> arrs = table_arrays(const_cast<b200ppf_table *>(t));  // read only
+    h.n_offsets = arrs[0].words;
+    h.n_sub_offsets = arrs[1].words;
     h.n_entries = t->info.n_entries;
-    h.n_merged = t->merged_w ? t->n_merged : 0;
-    constexpr int NA = 8;
-    const uint32_t *arrays[NA] = {t->offsets, t->sub_offsets, t->entry_w, t->entry_am,
-                                  reinterpret_cast<const uint32_t *>(t->entry_alpha), t->entry_idx, t->merged_w, t->msub_offsets};
-    const uint64_t lengths[NA] = {h.n_offsets, h.n_sub_offsets, h.n_entries, h.n_entries, h.n_entries, h.n_entries, h.n_merged,
-                                  t->msub_offsets ? h.n_sub_offsets : 0};
-    std::vector<std::vector<uint32_t>> host(NA);
-    for (int a = 0; a < NA; ++a) {
-        host[a].resize(lengths[a]);
-        if (lengths[a])
-            PPF_CUDA(ctx, cudaMemcpyAsync(host[a].data(), arrays[a], lengths[a] * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+    h.n_merged = arrs[6].words;
+    std::vector<std::vector<uint32_t>> host(arrs.size());
+    for (size_t a = 0; a < arrs.size(); ++a) {
+        host[a].resize(arrs[a].words);
+        if (arrs[a].words)
+            PPF_CUDA(ctx, cudaMemcpyAsync(host[a].data(), *arrs[a].slot, arrs[a].words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                                           ctx->stream));
     }
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     // the parameter block (info, kp, bp: everything behind the checksum field) and then the six arrays
     uint64_t sum = mix_bytes(0x42323030u, reinterpret_cast<const char *>(&h) + offsetof(TableFileHeader, info),
                              sizeof(h) - offsetof(TableFileHeader, info));
-    for (int a = 0; a < NA; ++a) sum = mix_bytes(sum, host[a].data(), host[a].size() * sizeof(uint32_t));
+    for (const std::vector<uint32_t> &a : host) sum = mix_bytes(sum, a.data(), a.size() * sizeof(uint32_t));
     h.checksum = sum;
     FileCloser fc{fopen(path, "wb")};
     if (!fc.f) return fail_msg(ctx, B200PPF_ERR_IO, "table save: cannot open the file for writing");
     bool ok = fwrite(&h, sizeof(h), 1, fc.f) == 1;
-    for (int a = 0; a < NA && ok; ++a)
+    for (size_t a = 0; a < host.size() && ok; ++a)
         if (!host[a].empty()) ok = fwrite(host[a].data(), sizeof(uint32_t), host[a].size(), fc.f) == host[a].size();
     ok = ok && fflush(fc.f) == 0;
     if (!ok) return fail_msg(ctx, B200PPF_ERR_IO, "table save: short write");
@@ -597,19 +596,27 @@ int b200ppf_table_load(b200ppf_ctx *ctx, const char *path, b200ppf_table **out) 
                       h.info.n_alpha >= 1 && h.bp.n_alpha == h.info.n_alpha &&
                       h.kp.slice_rows == h.info.slice_rows && h.kp.n_slices == h.info.n_slices;
     if (!sane) return fail_msg(ctx, B200PPF_ERR_IO, "table load: inconsistent header");
-    constexpr int NA = 8;
     const bool has_merged = h.bp.cells_log2 != 0 && h.n_entries != 0;
     if (h.n_merged > h.n_entries || (has_merged ? h.n_merged == 0 : h.n_merged != 0) || h.info.n_merged != h.n_merged)
         return fail_msg(ctx, B200PPF_ERR_IO, "table load: inconsistent header");
-    const uint64_t lengths[NA] = {h.n_offsets, h.n_sub_offsets, h.n_entries, h.n_entries, h.n_entries, h.n_entries, h.n_merged,
-                                  has_merged ? h.n_sub_offsets : 0};
-    std::vector<std::vector<uint32_t>> host(NA);
+    TablePtr t(new (std::nothrow) b200ppf_table());
+    if (!t) return fail_msg(ctx, B200PPF_ERR_NOMEM, "table load: out of host memory");
+    t->ctx = ctx;
+    t->info = h.info;
+    t->kp = h.kp;
+    t->bp = h.bp;
+    t->feature_mode = (int)h.feature_mode;
+    t->n_merged = h.n_merged;
+    // the header is consistent: these are the lengths it states
+    const std::array<TableArray, 8> arrs = table_arrays(t.get());
+    std::vector<std::vector<uint32_t>> host(arrs.size());
     // the parameter block (info, kp, bp: everything behind the checksum field) and then the six arrays
     uint64_t sum = mix_bytes(0x42323030u, reinterpret_cast<const char *>(&h) + offsetof(TableFileHeader, info),
                              sizeof(h) - offsetof(TableFileHeader, info));
-    for (int a = 0; a < NA; ++a) {
-        host[a].resize(lengths[a]);
-        if (lengths[a] && fread(host[a].data(), sizeof(uint32_t), lengths[a], fc.f) != lengths[a])
+    for (size_t a = 0; a < arrs.size(); ++a) {
+        const size_t words = arrs[a].words;
+        host[a].resize(words);
+        if (words && fread(host[a].data(), sizeof(uint32_t), words, fc.f) != words)
             return fail_msg(ctx, B200PPF_ERR_IO, "table load: truncated file");
         sum = mix_bytes(sum, host[a].data(), host[a].size() * sizeof(uint32_t));
     }
@@ -621,35 +628,15 @@ int b200ppf_table_load(b200ppf_ctx *ctx, const char *path, b200ppf_table **out) 
         return fail_msg(ctx, B200PPF_ERR_IO, msg);
     }
 
-    b200ppf_table *t = new (std::nothrow) b200ppf_table();
-    if (!t) return fail_msg(ctx, B200PPF_ERR_NOMEM, "table load: out of host memory");
-    t->ctx = ctx;
-    t->info = h.info;
-    t->kp = h.kp;
-    t->bp = h.bp;
-    t->feature_mode = (int)h.feature_mode;
-    t->n_merged = h.n_merged;
-    uint32_t **dev[NA] = {&t->offsets, &t->sub_offsets, &t->entry_w, &t->entry_am,
-                          reinterpret_cast<uint32_t **>(&t->entry_alpha), &t->entry_idx, &t->merged_w, &t->msub_offsets};
-    for (int a = 0; a < NA; ++a) {
-        if (a == 1 && !h.n_sub_offsets) continue;
-        if (a >= 6 && !has_merged) continue;
-        const size_t pad = (a == 2 || a == 3 || a == 6) ? b200ppf::ENTRY_PAD : 0;
-        const size_t words = std::max<size_t>(1, lengths[a] + pad);
-        cudaError_t e = cudaMallocAsync(dev[a], words * sizeof(uint32_t), ctx->stream);
-        if (e == cudaSuccess && pad) e = cudaMemsetAsync(*dev[a] + lengths[a], 0, pad * sizeof(uint32_t), ctx->stream);
-        if (e == cudaSuccess && lengths[a])
-            e = cudaMemcpyAsync(*dev[a], host[a].data(), lengths[a] * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-        if (e != cudaSuccess) {
-            b200ppf_table_free(t);
-            return fail_msg(ctx, e == cudaErrorMemoryAllocation ? B200PPF_ERR_NOMEM : B200PPF_ERR_CUDA, cudaGetErrorString(e));
-        }
+    for (size_t a = 0; a < arrs.size(); ++a) {
+        if (!arrs[a].used) continue;
+        PPF_CUDA(ctx, table_array_alloc(ctx->stream, arrs[a]));
+        if (arrs[a].words)
+            PPF_CUDA(ctx, cudaMemcpyAsync(*arrs[a].slot, host[a].data(), arrs[a].words * sizeof(uint32_t), cudaMemcpyHostToDevice,
+                                          ctx->stream));
     }
-    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
-        b200ppf_table_free(t);
-        return fail_msg(ctx, B200PPF_ERR_CUDA, "table load: upload failed");
-    }
-    *out = t;
+    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) return fail_msg(ctx, B200PPF_ERR_CUDA, "table load: upload failed");
+    *out = t.release();
     return B200PPF_OK;
 }
 
@@ -658,7 +645,7 @@ int b200ppf_table_clone(b200ppf_ctx *dst, const b200ppf_table *src, b200ppf_tabl
     if (!src || !out) return fail_msg(dst, B200PPF_ERR_INVALID, "table clone: null argument");
     *out = nullptr;
     if (src->ctx) cudaStreamSynchronize(src->ctx->stream);  // the source table's build has finished (device guard is dst's)
-    b200ppf_table *t = new (std::nothrow) b200ppf_table();
+    TablePtr t(new (std::nothrow) b200ppf_table());
     if (!t) return fail_msg(dst, B200PPF_ERR_NOMEM, "table clone: out of host memory");
     t->ctx = dst;
     t->info = src->info;
@@ -666,37 +653,17 @@ int b200ppf_table_clone(b200ppf_ctx *dst, const b200ppf_table *src, b200ppf_tabl
     t->bp = src->bp;
     t->feature_mode = src->feature_mode;
     t->n_merged = src->n_merged;
-    const uint64_t total_keys = (uint64_t)src->info.key_space * src->info.n_slices;
-    const size_t n_sub = src->sub_offsets ? (size_t)(total_keys << src->bp.cells_log2) + 1 : 0, ne = src->info.n_entries;
     const int src_dev = src->ctx ? src->ctx->device : dst->device;
-    struct Arr {
-        uint32_t *const *from;
-        uint32_t **to;
-        size_t words, pad;
-    } arrs[8] = {{&src->offsets, &t->offsets, (size_t)total_keys + 1, 0},
-                 {&src->sub_offsets, &t->sub_offsets, n_sub, 0},
-                 {&src->entry_w, &t->entry_w, ne, b200ppf::ENTRY_PAD},
-                 {&src->entry_am, &t->entry_am, ne, b200ppf::ENTRY_PAD},
-                 {reinterpret_cast<uint32_t *const *>(&src->entry_alpha), reinterpret_cast<uint32_t **>(&t->entry_alpha), std::max<size_t>(1, ne), 0},
-                 {&src->entry_idx, &t->entry_idx, std::max<size_t>(1, ne), 0},
-                 {&src->merged_w, &t->merged_w, src->merged_w ? src->n_merged : 0, b200ppf::ENTRY_PAD},
-                 {&src->msub_offsets, &t->msub_offsets, src->msub_offsets ? n_sub : 0, 0}};
-    for (const Arr &a : arrs) {
-        if (!*a.from) continue;
-        cudaError_t e = cudaMallocAsync(a.to, (a.words + a.pad) * sizeof(uint32_t), dst->stream);
-        if (e == cudaSuccess && a.pad) e = cudaMemsetAsync(*a.to + a.words, 0, a.pad * sizeof(uint32_t), dst->stream);
-        if (e == cudaSuccess && a.words)
-            e = cudaMemcpyPeerAsync(*a.to, dst->device, *a.from, src_dev, a.words * sizeof(uint32_t), dst->stream);
-        if (e != cudaSuccess) {
-            b200ppf_table_free(t);
-            return fail_msg(dst, e == cudaErrorMemoryAllocation ? B200PPF_ERR_NOMEM : B200PPF_ERR_CUDA, cudaGetErrorString(e));
-        }
+    const std::array<TableArray, 8> from = table_arrays(const_cast<b200ppf_table *>(src)), to = table_arrays(t.get());  // src: read only
+    for (size_t a = 0; a < to.size(); ++a) {
+        if (!to[a].used) continue;
+        PPF_CUDA(dst, table_array_alloc(dst->stream, to[a]));
+        if (to[a].words)
+            PPF_CUDA(dst, cudaMemcpyPeerAsync(*to[a].slot, dst->device, *from[a].slot, src_dev, to[a].words * sizeof(uint32_t),
+                                              dst->stream));
     }
-    if (cudaStreamSynchronize(dst->stream) != cudaSuccess) {
-        b200ppf_table_free(t);
-        return fail_msg(dst, B200PPF_ERR_CUDA, "table clone: copy failed");
-    }
-    *out = t;
+    if (cudaStreamSynchronize(dst->stream) != cudaSuccess) return fail_msg(dst, B200PPF_ERR_CUDA, "table clone: copy failed");
+    *out = t.release();
     return B200PPF_OK;
 }
 
@@ -705,11 +672,10 @@ void b200ppf_table_free(b200ppf_table *t) {
     DeviceGuard guard(t->ctx ? t->ctx->device : 0);
     // the arrays come from the device's stream-ordered pool (k2_build, load, clone): they go back to it, so that the
     // next build re-uses the memory instead of asking the driver for gigabytes again
-    void *arrays[8] = {t->offsets, t->sub_offsets, t->entry_w, t->entry_am, t->entry_idx, t->entry_alpha, t->merged_w, t->msub_offsets};
-    for (void *p : arrays) {
-        if (!p) continue;
-        if (t->ctx) cudaFreeAsync(p, t->ctx->stream);
-        else cudaFree(p);
+    for (const TableArray &a : table_arrays(t)) {
+        if (!*a.slot) continue;
+        if (t->ctx) cudaFreeAsync(*a.slot, t->ctx->stream);
+        else cudaFree(*a.slot);
     }
     delete t;
 }
@@ -746,17 +712,15 @@ int b200ppf_hyp_buffer_create(b200ppf_ctx *ctx, size_t n_records, b200ppf_hypoth
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle travels as 64 bytes");
     b200ppf_hypothesis *p = nullptr;
     PPF_CUDA(ctx, cudaMalloc(&p, std::max<size_t>(1, n_records) * sizeof(b200ppf_hypothesis)));  // cudaMalloc: IPC-exportable
+    std::unique_ptr<b200ppf_hypothesis, cudaError_t (*)(void *)> owner(p, cudaFree);
     PPF_CUDA(ctx, cudaMemset(p, 0, std::max<size_t>(1, n_records) * sizeof(b200ppf_hypothesis)));
     if (ipc_handle) {
         cudaIpcMemHandle_t h;
         cudaError_t e = cudaIpcGetMemHandle(&h, p);
-        if (e != cudaSuccess) {
-            cudaFree(p);
-            return fail_msg(ctx, B200PPF_ERR_CUDA, cudaGetErrorString(e));
-        }
+        if (e != cudaSuccess) return fail_msg(ctx, B200PPF_ERR_CUDA, cudaGetErrorString(e));
         memcpy(ipc_handle, &h, 64);
     }
-    *buffer = p;
+    *buffer = owner.release();
     return B200PPF_OK;
 }
 
@@ -799,13 +763,7 @@ int b200ppf_vote(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_tab
                  size_t ref_first, size_t ref_step, size_t ref_count, b200ppf_hypothesis *hyps_host) {
     CHECK_CTX(ctx);
     if (ref_count && !hyps_host) return fail_msg(ctx, B200PPF_ERR_INVALID, "vote: null output pointer");
-    if (ctx->hyps_cap < ref_count) {
-        if (ctx->d_hyps) cudaFree(ctx->d_hyps);
-        ctx->d_hyps = nullptr;
-        ctx->hyps_cap = 0;
-        PPF_CUDA(ctx, cudaMalloc(&ctx->d_hyps, ref_count * sizeof(b200ppf_hypothesis)));
-        ctx->hyps_cap = ref_count;
-    }
+    PPF_CUDA(ctx, grow_buffer(&ctx->d_hyps, &ctx->hyps_cap, ref_count));
     b200ppf_hypothesis *const target = ctx->d_hyps;
     int rc = k3_vote(ctx, model, t, scene, ref_first, ref_step, ref_count, &target, 1, 0, 1);
     if (rc) return rc;
@@ -1023,13 +981,7 @@ int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf
     if (ref_rate == 0) ref_rate = 1;
     const size_t ref_count = (scene->n + ref_rate - 1) / ref_rate;
     if (ref_count == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "register: empty scene");
-    if (ctx->hyps_cap < ref_count) {
-        if (ctx->d_hyps) cudaFree(ctx->d_hyps);
-        ctx->d_hyps = nullptr;
-        ctx->hyps_cap = 0;
-        PPF_CUDA(ctx, cudaMalloc(&ctx->d_hyps, ref_count * sizeof(b200ppf_hypothesis)));
-        ctx->hyps_cap = ref_count;
-    }
+    PPF_CUDA(ctx, grow_buffer(&ctx->d_hyps, &ctx->hyps_cap, ref_count));
     b200ppf_hypothesis *const reg_target = ctx->d_hyps;
     int rc = k3_vote(ctx, model, t, scene, 0, ref_rate, ref_count, &reg_target, 1, 0, 1);
     if (rc) return rc;

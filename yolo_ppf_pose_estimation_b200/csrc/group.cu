@@ -53,18 +53,6 @@ using namespace b200ppf;
 
 namespace {
 
-struct DevGuard {
-    int prev = -1;
-    explicit DevGuard(int dev) {
-        cudaGetDevice(&prev);
-        if (prev != dev) cudaSetDevice(dev);
-        else prev = -1;
-    }
-    ~DevGuard() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 constexpr size_t FLAG_WORDS = 2 * MAX_PEERS + 16;  // two flag sets, the done counter, two queue counters
 constexpr size_t DONE_WORD = 2 * MAX_PEERS, QUEUE_WORD = 2 * MAX_PEERS + 8;
 
@@ -78,7 +66,7 @@ int group_alloc(b200ppf_ctx *ctx, int rank, int world, size_t n_records, b200ppf
     g->rank = rank;
     g->world = world;
     g->n_records = std::max<size_t>(1, n_records);
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     cudaError_t e = cudaSuccess;
     for (int s = 0; s < 2 && e == cudaSuccess; ++s) {  // cudaMalloc: exportable through CUDA IPC
         e = cudaMalloc(&g->own[s], g->n_records * sizeof(unsigned long long));
@@ -108,7 +96,7 @@ int b200ppf_group_create(b200ppf_ctx *ctx, int rank, int world, size_t n_records
     if (rc) return rc;
     if (handles) {
         static_assert(B200PPF_GROUP_HANDLE_BYTES == 3 * sizeof(cudaIpcMemHandle_t), "three IPC handles travel as one blob");
-        DevGuard guard(ctx->device);
+        DeviceGuard guard(ctx->device);
         b200ppf_group *g = *out;
         void *bufs[3] = {g->own[0], g->own[1], g->own_flags};
         for (int k = 0; k < 3; ++k) {
@@ -127,7 +115,7 @@ int b200ppf_group_create(b200ppf_ctx *ctx, int rank, int world, size_t n_records
 
 int b200ppf_group_connect(b200ppf_group *g, const unsigned char *all_handles) {
     if (!g || !all_handles) return fail_msg(g ? g->ctx : nullptr, B200PPF_ERR_INVALID, "group connect: null argument");
-    DevGuard guard(g->ctx->device);
+    DeviceGuard guard(g->ctx->device);
     for (int r = 0; r < g->world; ++r) {
         if (r == g->rank) continue;
         void *p[3] = {nullptr, nullptr, nullptr};
@@ -150,7 +138,7 @@ int b200ppf_group_connect(b200ppf_group *g, const unsigned char *all_handles) {
 
 void b200ppf_group_destroy(b200ppf_group *g) {
     if (!g) return;
-    DevGuard guard(g->ctx->device);
+    DeviceGuard guard(g->ctx->device);
     cudaStreamSynchronize(g->ctx->stream);
     for (int r = 0; r < g->world; ++r)
         if (g->opened[r]) {
@@ -176,7 +164,7 @@ int b200ppf_group_vote(b200ppf_group *g, const b200ppf_cloud *model, const b200p
     const size_t n_ref = (scene->n + ref_rate - 1) / ref_rate;
     if (n_ref == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "group vote: empty scene");
     if (n_ref > g->n_records) return fail_msg(ctx, B200PPF_ERR_INVALID, "group vote: more reference points than the group's buffers hold");
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     const int set = (int)(g->step & 1u);
     g->step += 1;
     // Clear the OTHER set for the next step now: its last users finished before they raised the flags this rank waited for
@@ -208,7 +196,7 @@ int b200ppf_group_cluster(b200ppf_group *g, const b200ppf_cloud *model, const b2
     if (g->step == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "group cluster: no vote has been issued");
     if (ref_rate == 0) ref_rate = 1;
     const size_t n_ref = (scene->n + ref_rate - 1) / ref_rate;
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     const int set = (int)((g->step - 1) & 1u);
     int rc = k3_group_wait(ctx, g->own_flags + set * MAX_PEERS, g->world, g->step);
     if (rc) return rc;
@@ -249,7 +237,7 @@ int b200ppf_multi_create(const int *devices, int n_devices, b200ppf_multi **out)
     }
     // every device may store into every other device's buffers
     for (int a = 0; a < n_devices; ++a) {
-        DevGuard guard(devices[a]);
+        DeviceGuard guard(devices[a]);
         for (int b = 0; b < n_devices; ++b) {
             if (a == b || devices[a] == devices[b]) continue;
             int can = 0;
@@ -401,7 +389,7 @@ int b200ppf_multi_register(b200ppf_multi *m, size_t ref_rate, float pos_thr, flo
     if (rc) return multi_fail(m, 0, rc);
     // the other devices only have to drain before their buffers are reused two steps from now; keep the steps aligned
     for (int g = 1; g < G; ++g) {
-        DevGuard guard(m->ctx[g]->device);
+        DeviceGuard guard(m->ctx[g]->device);
         const int set = (int)((m->group[g]->step - 1) & 1u);
         rc = k3_group_wait(m->ctx[g], m->group[g]->own_flags + set * MAX_PEERS, G, m->group[g]->step);
         if (rc) return multi_fail(m, g, rc);

@@ -386,7 +386,7 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
     if (n > 65535) return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "table build: more than 65535 model points (pair index is 32-bit)");
     const size_t count = n * n;
 
-    b200ppf_table *t = new b200ppf_table();
+    TablePtr t(new b200ppf_table());
     t->ctx = ctx;
     t->feature_mode = ctx->feature_mode;
     b200ppf_table_info &info = t->info;
@@ -395,20 +395,15 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
     info.dist_step = dist_step;
     info.n_alpha = num_alpha_bins(angle_step, ctx->nalpha_rule);
     info.nalpha_rule = (uint32_t)ctx->nalpha_rule;
-    if (info.n_alpha == 0) {
-        delete t;
-        return fail_msg(ctx, B200PPF_ERR_INVALID, "table build: angle step larger than 2*pi");
-    }
+    if (info.n_alpha == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "table build: angle step larger than 2*pi");
     // accumulator slices: rows per slice bounded by the shared-memory budget of the voting kernel.  The slice is held
     // bin-major with a pitch of 32-row multiples (k3_vote.cu), acc_cols columns (the FLOOR rules carry a spare one).
     t->bp = make_bin_params(angle_step, ctx->alpha_mode, ctx->nalpha_rule);
     {
         size_t budget = k3_accumulator_budget(ctx);
         size_t rows_max = budget / ((size_t)t->bp.acc_cols * sizeof(uint32_t)) / 32 * 32;
-        if (rows_max == 0) {
-            delete t;
+        if (rows_max == 0)
             return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "table build: angle step too fine for 32 accumulator rows in shared memory");
-        }
         if (const char *e = getenv("B200PPF_SLICE_ROWS")) {
             size_t v = (size_t)atoll(e);
             if (v > 0 && v < rows_max) rows_max = v;
@@ -425,8 +420,8 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
     kp.n_slices = info.n_slices;
     kp.row_pitch = (info.slice_rows + 31u) / 32u * 32u;
 
-    int *d_range = nullptr;  // lo[4], hi[4], max_f4_bits, out_of_range, bad_alpha, pad
-    PPF_CUDA(ctx, cudaMallocAsync(&d_range, 12 * sizeof(int), ctx->stream));
+    StreamBuf<int> d_range(ctx);  // lo[4], hi[4], max_f4_bits, out_of_range, bad_alpha, pad
+    PPF_CUDA(ctx, d_range.alloc(12));
     int h_range[12] = {INT_MAX, INT_MAX, INT_MAX, INT_MAX, INT_MIN, INT_MIN, INT_MIN, INT_MIN, -1, 0, 0, 0};
     PPF_CUDA(ctx, cudaMemcpyAsync(d_range, h_range, sizeof(h_range), cudaMemcpyHostToDevice, ctx->stream));
 
@@ -478,11 +473,8 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
         unsigned __int128 ks = 1;
         for (int k = 0; k < 4; ++k) ks *= (unsigned __int128)(uint32_t)kp.size[k];
         unsigned __int128 total = ks * info.n_slices + 1;
-        if (total >= ((unsigned __int128)1 << 31)) {
-            cudaFreeAsync(d_range, ctx->stream);
-            delete t;
+        if (total >= ((unsigned __int128)1 << 31))
             return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "table build: discretisation too fine (packed key space exceeds 2^31)");
-        }
         kp.key_space = (uint32_t)ks;
         // phase cells multiply the sort-key space: halve them until it fits 31 bits and 1 Gi offsets
         if (const char *e = getenv("B200PPF_PHASE_CELLS_LOG2")) {
@@ -511,92 +503,53 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
     info.phase_cells = 1u << cells_log2;
 
     // ---- keys ---------------------------------------------------------------------------------
-    uint32_t *keys[2] = {nullptr, nullptr}, *idx[2] = {nullptr, nullptr}, *alp[2] = {nullptr, nullptr};
-    unsigned long long *d_cnt = nullptr;
-    auto cleanup = [&]() {
-        if (d_cnt) cudaFreeAsync(d_cnt, ctx->stream);
-        d_cnt = nullptr;
-        for (int b = 0; b < 2; ++b) {
-            if (keys[b]) cudaFreeAsync(keys[b], ctx->stream);
-            if (idx[b]) cudaFreeAsync(idx[b], ctx->stream);
-            if (alp[b]) cudaFreeAsync(alp[b], ctx->stream);
-        }
-        if (d_range) cudaFreeAsync(d_range, ctx->stream);
-    };
-#define K2_TRY(expr)                       \
-    do {                                   \
-        int _rc = (expr);                  \
-        if (_rc != B200PPF_OK) {           \
-            cleanup();                     \
-            b200ppf_table_free(t);         \
-            return _rc;                    \
-        }                                  \
-    } while (0)
-#define K2_CUDA(expr)                                                               \
-    do {                                                                            \
-        cudaError_t _e = (expr);                                                    \
-        if (_e != cudaSuccess) {                                                    \
-            cleanup();                                                              \
-            b200ppf_table_free(t);                                                  \
-            char _b[256];                                                           \
-            snprintf(_b, sizeof(_b), "%s failed: %s", #expr, cudaGetErrorString(_e)); \
-            return fail_msg(ctx, _e == cudaErrorMemoryAllocation ? B200PPF_ERR_NOMEM : B200PPF_ERR_CUDA, _b); \
-        }                                                                           \
-    } while (0)
-    for (int b = 0; b < 2; ++b) {
-        K2_CUDA(cudaMallocAsync(&keys[b], count * sizeof(uint32_t), ctx->stream));
-        K2_CUDA(cudaMallocAsync(&idx[b], count * sizeof(uint32_t), ctx->stream));
-        K2_CUDA(cudaMallocAsync(&alp[b], count * sizeof(uint32_t), ctx->stream));
-    }
+    StreamBuf<uint32_t> keys0(ctx), keys1(ctx), idx0(ctx), idx1(ctx), alp0(ctx), alp1(ctx);
+    PPF_CUDA(ctx, keys0.alloc(count));
+    PPF_CUDA(ctx, idx0.alloc(count));
+    PPF_CUDA(ctx, alp0.alloc(count));
+    PPF_CUDA(ctx, keys1.alloc(count));
+    PPF_CUDA(ctx, idx1.alloc(count));
+    PPF_CUDA(ctx, alp1.alloc(count));
+    uint32_t *keys[2] = {keys0, keys1}, *idx[2] = {idx0, idx1}, *alp[2] = {alp0, alp1};
     if (feat) {
         int blocks = (int)std::min<size_t>((count + 255) / 256, (size_t)ctx->sm_count * 32);
-        auto launch = [&]() -> int {
-            PPF_LAUNCH(ctx, keys_from_features_kernel, blocks, 256, 0, reinterpret_cast<const float *>(feat->d),
-                       (uint32_t)n, kp, t->bp, keys[0], alp[0]);
-            return B200PPF_OK;
-        };
-        K2_TRY(launch());
+        PPF_LAUNCH(ctx, keys_from_features_kernel, blocks, 256, 0, reinterpret_cast<const float *>(feat->d), (uint32_t)n, kp,
+                   t->bp, keys[0], alp[0]);
     } else {
         dim3 grid((unsigned)((n + FTJ - 1) / FTJ), (unsigned)((n + FTI - 1) / FTI));
-        auto launch = [&]() -> int {
-            PPF_LAUNCH(ctx, keys_from_cloud_kernel, grid, FTJ, 0, model->pos, model->nrm, (uint32_t)n,
-                       ctx->feature_mode, kp, t->bp, keys[0], alp[0], d_range + 8, d_range + 9);
-            return B200PPF_OK;
-        };
-        K2_TRY(launch());
+        PPF_LAUNCH(ctx, keys_from_cloud_kernel, grid, FTJ, 0, model->pos, model->nrm, (uint32_t)n, ctx->feature_mode, kp, t->bp,
+                   keys[0], alp[0], d_range + 8, d_range + 9);
     }
     cudaEventRecord(ctx->ev[1], ctx->stream);
 
     // ---- sort -----------------------------------------------------------------------------------
     bool in_alt = false;
-    K2_TRY(radix_sort_u32(ctx, keys[0], keys[1], idx[0], idx[1], alp[0], alp[1], count, (int)info.key_bits,
-                          /*v0_iota=*/true, &in_alt));
+    int rc = radix_sort_u32(ctx, keys[0], keys[1], idx[0], idx[1], alp[0], alp[1], count, (int)info.key_bits,
+                            /*v0_iota=*/true, &in_alt);
+    if (rc) return rc;
     const int s = in_alt ? 1 : 0;
     cudaEventRecord(ctx->ev[2], ctx->stream);
 
     // ---- CSR ------------------------------------------------------------------------------------
-    K2_CUDA(cudaMallocAsync(&t->offsets, ((size_t)total_keys + 1) * sizeof(uint32_t), ctx->stream));
-    if (cells_log2) K2_CUDA(cudaMallocAsync(&t->sub_offsets, ((size_t)total_sub + 1) * sizeof(uint32_t), ctx->stream));
-    {
-        auto launch = [&]() -> int {
-            PPF_LAUNCH(ctx, csr_offsets_kernel, (total_keys + 1 + 255) / 256, 256, 0, keys[s], (uint32_t)count,
-                       total_keys, cells_log2 + merge_bits, t->offsets);
-            if (cells_log2)
-                PPF_LAUNCH(ctx, csr_sub_offsets_kernel, (total_sub + 1 + 255) / 256, 256, 0, keys[s], t->offsets, total_sub,
-                           cells_log2, merge_bits, t->sub_offsets);
-            return B200PPF_OK;
-        };
-        K2_TRY(launch());
-    }
+    // each array is allocated once what sizes it is known, with the length and pad table_arrays gives it
+    auto alloc_arrays = [&](int first, int last) -> int {
+        const std::array<TableArray, 8> arrs = table_arrays(t.get());
+        for (int a = first; a <= last; ++a)
+            if (arrs[a].used) PPF_CUDA(ctx, table_array_alloc(ctx->stream, arrs[a]));
+        return B200PPF_OK;
+    };
+    if ((rc = alloc_arrays(0, 1))) return rc;  // offsets, sub_offsets
+    PPF_LAUNCH(ctx, csr_offsets_kernel, (total_keys + 1 + 255) / 256, 256, 0, keys[s], (uint32_t)count, total_keys,
+               cells_log2 + merge_bits, t->offsets);
+    if (cells_log2)
+        PPF_LAUNCH(ctx, csr_sub_offsets_kernel, (total_sub + 1 + 255) / 256, 256, 0, keys[s], t->offsets, total_sub, cells_log2,
+                   merge_bits, t->sub_offsets);
     uint32_t n_entries = 0;
-    K2_CUDA(cudaMemcpyAsync(&n_entries, t->offsets + total_keys, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    K2_CUDA(cudaMemcpyAsync(h_range, d_range, sizeof(h_range), cudaMemcpyDeviceToHost, ctx->stream));
-    K2_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (!feat && h_range[9] != 0) {
-        cleanup();
-        b200ppf_table_free(t);
+    PPF_CUDA(ctx, cudaMemcpyAsync(&n_entries, t->offsets + total_keys, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(h_range, d_range, sizeof(h_range), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (!feat && h_range[9] != 0)
         return fail_msg(ctx, B200PPF_ERR_STATE, "table build: a model pair feature left the analytic key range (non-unit normals?)");
-    }
     info.n_entries = n_entries;
     {
         int bits = h_range[8];
@@ -605,94 +558,60 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
         info.max_dist = bits < 0 ? -1.0f : mx;  // PCL: max_dist_ starts at -1
     }
     // the voting kernel reads whole batches: ENTRY_PAD readable (zero) words follow the last entry
-    K2_CUDA(cudaMallocAsync(&t->entry_w, ((size_t)n_entries + ENTRY_PAD) * sizeof(uint32_t), ctx->stream));
-    K2_CUDA(cudaMallocAsync(&t->entry_am, ((size_t)n_entries + ENTRY_PAD) * sizeof(uint32_t), ctx->stream));
-    K2_CUDA(cudaMemsetAsync(t->entry_w + n_entries, 0, ENTRY_PAD * sizeof(uint32_t), ctx->stream));
-    K2_CUDA(cudaMemsetAsync(t->entry_am + n_entries, 0, ENTRY_PAD * sizeof(uint32_t), ctx->stream));
-    K2_CUDA(cudaMallocAsync(&t->entry_idx, std::max<size_t>(1, n_entries) * sizeof(uint32_t), ctx->stream));
-    K2_CUDA(cudaMallocAsync(&t->entry_alpha, std::max<size_t>(1, n_entries) * sizeof(float), ctx->stream));
-    K2_CUDA(cudaMallocAsync(&d_cnt, sizeof(unsigned long long), ctx->stream));
-    K2_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), ctx->stream));
-    {
-        auto launch = [&]() -> int {
-            if (n_entries) {
-                // per-entry arrays in sorted order: (key, cell, [bin of alpha_m,] i, j)
-                PPF_LAUNCH(ctx, entries_kernel, (n_entries + 255) / 256, 256, 0, idx[s], alp[s], n_entries, (uint32_t)n,
-                           info.slice_rows, kp.row_pitch, t->bp, t->entry_w, t->entry_am, t->entry_alpha, d_range + 10);
-                PPF_CUDA(ctx, cudaMemcpyAsync(t->entry_idx, idx[s], (size_t)n_entries * sizeof(uint32_t),
-                                              cudaMemcpyDeviceToDevice, ctx->stream));
-            }
-            PPF_LAUNCH(ctx, count_nonempty_kernel, (kp.key_space + 255) / 256, 256, 0, t->offsets, kp.key_space, info.n_slices, d_cnt);
-            return B200PPF_OK;
-        };
-        K2_TRY(launch());
+    if ((rc = alloc_arrays(2, 5))) return rc;  // entry_w, entry_am, entry_alpha, entry_idx
+    StreamBuf<unsigned long long> d_cnt(ctx);
+    PPF_CUDA(ctx, d_cnt.alloc(1));
+    PPF_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), ctx->stream));
+    if (n_entries) {
+        // per-entry arrays in sorted order: (key, cell, [bin of alpha_m,] i, j)
+        PPF_LAUNCH(ctx, entries_kernel, (n_entries + 255) / 256, 256, 0, idx[s], alp[s], n_entries, (uint32_t)n, info.slice_rows,
+                   kp.row_pitch, t->bp, t->entry_w, t->entry_am, t->entry_alpha, d_range + 10);
+        PPF_CUDA(ctx, cudaMemcpyAsync(t->entry_idx, idx[s], (size_t)n_entries * sizeof(uint32_t), cudaMemcpyDeviceToDevice,
+                                      ctx->stream));
     }
+    PPF_LAUNCH(ctx, count_nonempty_kernel, (kp.key_space + 255) / 256, 256, 0, t->offsets, kp.key_space, info.n_slices, d_cnt);
     // ---- merged votes + bank order (phase-sorted tables) ---------------------------------------------
-    t->n_merged = 0;
     if (cells_log2 && n_entries) {
         // the free halves of the sort buffers hold the run heads, their ranks and the unordered merged words
         uint32_t *head = keys[1 - s], *rank = idx[1 - s], *mw_tmp = alp[1 - s];
         uint32_t n_merged = n_entries;
-        {
-            auto launch = [&]() -> int {
-                if (merge_bits)
-                    PPF_LAUNCH(ctx, merge_heads_kernel, (n_entries + 255) / 256, 256, 0, keys[s], idx[s], n_entries, (uint32_t)n, head);
-                return B200PPF_OK;
-            };
-            K2_TRY(launch());
-        }
         if (merge_bits) {
-            K2_TRY(flag_scan_u32(ctx, head, n_entries, rank, &n_merged));
-        }
-        K2_CUDA(cudaMallocAsync(&t->merged_w, ((size_t)n_merged + ENTRY_PAD) * sizeof(uint32_t), ctx->stream));
-        K2_CUDA(cudaMemsetAsync(t->merged_w + n_merged, 0, ENTRY_PAD * sizeof(uint32_t), ctx->stream));
-        K2_CUDA(cudaMallocAsync(&t->msub_offsets, ((size_t)total_sub + 1) * sizeof(uint32_t), ctx->stream));
-        {
-            auto launch = [&]() -> int {
-                if (merge_bits) {
-                    PPF_LAUNCH(ctx, merge_words_kernel, (n_entries + 255) / 256, 256, 0, head, rank, t->entry_w, n_entries, mw_tmp);
-                    PPF_LAUNCH(ctx, merge_offsets_kernel, (total_sub + 1 + 255) / 256, 256, 0, t->sub_offsets, total_sub, rank,
-                               n_entries, n_merged, t->msub_offsets);
-                } else {  // no room for the bin in the sort key: one word per entry, count 1
-                    PPF_LAUNCH(ctx, merge_identity_kernel, (n_entries + 255) / 256, 256, 0, t->entry_w, n_entries, mw_tmp);
-                    PPF_CUDA(ctx, cudaMemcpyAsync(t->msub_offsets, t->sub_offsets, ((size_t)total_sub + 1) * sizeof(uint32_t),
-                                                  cudaMemcpyDeviceToDevice, ctx->stream));
-                }
-                if (!getenv("B200PPF_NO_BANK_SPREAD")) {
-                    const unsigned blocks = (unsigned)std::min<size_t>(((size_t)total_sub + 32 * SPREAD_WARPS - 1) /
-                                                                           (32 * SPREAD_WARPS),
-                                                                       (size_t)ctx->sm_count * 16);
-                    PPF_LAUNCH(ctx, bank_order_kernel, blocks, SPREAD_WARPS * 32, 0, t->msub_offsets, total_sub, mw_tmp, t->merged_w);
-                } else {
-                    PPF_CUDA(ctx, cudaMemcpyAsync(t->merged_w, mw_tmp, (size_t)n_merged * sizeof(uint32_t), cudaMemcpyDeviceToDevice,
-                                                  ctx->stream));
-                }
-                return B200PPF_OK;
-            };
-            K2_TRY(launch());
+            PPF_LAUNCH(ctx, merge_heads_kernel, (n_entries + 255) / 256, 256, 0, keys[s], idx[s], n_entries, (uint32_t)n, head);
+            if ((rc = flag_scan_u32(ctx, head, n_entries, rank, &n_merged))) return rc;
         }
         t->n_merged = n_merged;
+        if ((rc = alloc_arrays(6, 7))) return rc;  // merged_w, msub_offsets
+        if (merge_bits) {
+            PPF_LAUNCH(ctx, merge_words_kernel, (n_entries + 255) / 256, 256, 0, head, rank, t->entry_w, n_entries, mw_tmp);
+            PPF_LAUNCH(ctx, merge_offsets_kernel, (total_sub + 1 + 255) / 256, 256, 0, t->sub_offsets, total_sub, rank, n_entries,
+                       n_merged, t->msub_offsets);
+        } else {  // no room for the bin in the sort key: one word per entry, count 1
+            PPF_LAUNCH(ctx, merge_identity_kernel, (n_entries + 255) / 256, 256, 0, t->entry_w, n_entries, mw_tmp);
+            PPF_CUDA(ctx, cudaMemcpyAsync(t->msub_offsets, t->sub_offsets, ((size_t)total_sub + 1) * sizeof(uint32_t),
+                                          cudaMemcpyDeviceToDevice, ctx->stream));
+        }
+        if (!getenv("B200PPF_NO_BANK_SPREAD")) {
+            const unsigned blocks = (unsigned)std::min<size_t>(((size_t)total_sub + 32 * SPREAD_WARPS - 1) / (32 * SPREAD_WARPS),
+                                                               (size_t)ctx->sm_count * 16);
+            PPF_LAUNCH(ctx, bank_order_kernel, blocks, SPREAD_WARPS * 32, 0, t->msub_offsets, total_sub, mw_tmp, t->merged_w);
+        } else {
+            PPF_CUDA(ctx, cudaMemcpyAsync(t->merged_w, mw_tmp, (size_t)n_merged * sizeof(uint32_t), cudaMemcpyDeviceToDevice,
+                                          ctx->stream));
+        }
     }
     info.n_merged = t->n_merged;
     unsigned long long h_cnt = 0;
-    K2_CUDA(cudaMemcpyAsync(&h_cnt, d_cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, ctx->stream));
-    K2_CUDA(cudaMemcpyAsync(h_range, d_range, sizeof(h_range), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(&h_cnt, d_cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(h_range, d_range, sizeof(h_range), cudaMemcpyDeviceToHost, ctx->stream));
     cudaEventRecord(ctx->ev[3], ctx->stream);
-    K2_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (h_range[10] != 0) {
-        cleanup();
-        b200ppf_table_free(t);
-        return fail_msg(ctx, B200PPF_ERR_INVALID,
-                        "table build: an alpha_m lies outside [-pi, pi] (not produced by PPFEstimation::compute)");
-    }
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (h_range[10] != 0)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "table build: an alpha_m lies outside [-pi, pi] (not produced by PPFEstimation::compute)");
     info.n_keys = h_cnt;
-    cleanup();
     cudaEventElapsedTime(&ctx->timings.keys_ms, ctx->ev[0], ctx->ev[1]);
     cudaEventElapsedTime(&ctx->timings.sort_ms, ctx->ev[1], ctx->ev[2]);
     cudaEventElapsedTime(&ctx->timings.csr_ms, ctx->ev[2], ctx->ev[3]);
-#undef K2_TRY
-#undef K2_CUDA
-    *out = t;
+    *out = t.release();
     return B200PPF_OK;
 }
 
@@ -732,8 +651,8 @@ int k2_query_key(b200ppf_ctx *ctx, const b200ppf_table *t, const int32_t *d4, ui
 
 int k2_alpha_m(b200ppf_ctx *ctx, const b200ppf_table *t, float *host) {
     const size_t n = t->info.n_model, count = n * n;
-    float *d = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&d, count * sizeof(float), ctx->stream));
+    StreamBuf<float> d(ctx);
+    PPF_CUDA(ctx, d.alloc(count));
     int blocks = (int)std::min<size_t>((count + 255) / 256, (size_t)ctx->sm_count * 16);
     PPF_LAUNCH(ctx, fill_nan_kernel, blocks, 256, 0, d, count);
     if (t->info.n_entries)
@@ -741,7 +660,6 @@ int k2_alpha_m(b200ppf_ctx *ctx, const b200ppf_table *t, float *host) {
                    t->entry_alpha, (uint32_t)t->info.n_entries, d);
     PPF_CUDA(ctx, cudaMemcpyAsync(host, d, count * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    PPF_CUDA(ctx, cudaFreeAsync(d, ctx->stream));
     return B200PPF_OK;
 }
 

@@ -949,12 +949,8 @@ float radius_sq_bound(float r) {
 int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *scene, size_t ref_first,
                 size_t ref_step, size_t ref_count, uint32_t *acc_dump, const VoteQueue *queue = nullptr) {
     const float radius = t->info.max_dist * 0.5f;
-    struct GridOwner {  // the grid goes back to the pool on every return path, the launch macros' error returns included
-        b200ppf_ctx *ctx;
-        SceneGrid g;
-        ~GridOwner() { scene_grid_free(ctx, &g); }
-    } owner{ctx, SceneGrid()};
-    SceneGrid &grid = owner.g;
+    SceneGrid grid;
+    std::unique_ptr<SceneGrid, SceneGridFree> grid_owner(&grid, SceneGridFree{ctx});
     int rc = scene_grid_build(ctx, scene, radius, &grid);
     if (rc) return rc;
     VoteArgs a;
@@ -1061,13 +1057,7 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
 
 int ensure_vote_scratch(b200ppf_ctx *ctx, size_t ref_count) {
     if (!ctx->d_stats) PPF_CUDA(ctx, cudaMalloc(&ctx->d_stats, 4 * sizeof(unsigned long long)));
-    if (ctx->peaks_cap < ref_count) {
-        if (ctx->d_peaks) cudaFree(ctx->d_peaks);
-        ctx->d_peaks = nullptr;
-        ctx->peaks_cap = 0;
-        PPF_CUDA(ctx, cudaMalloc(&ctx->d_peaks, ref_count * sizeof(unsigned long long)));
-        ctx->peaks_cap = ref_count;
-    }
+    PPF_CUDA(ctx, grow_buffer(&ctx->d_peaks, &ctx->peaks_cap, ref_count));
     PPF_CUDA(ctx, cudaMemsetAsync(ctx->d_stats, 0, 4 * sizeof(unsigned long long), ctx->stream));
     PPF_CUDA(ctx, cudaMemsetAsync(ctx->d_peaks, 0, ref_count * sizeof(unsigned long long), ctx->stream));
     return B200PPF_OK;
@@ -1150,22 +1140,18 @@ int k3_debug_alpha_bins(b200ppf_ctx *ctx, float angle_step, int alpha_mode, int 
         }
         return B200PPF_OK;
     }
-    float *d_am = nullptr, *d_as = nullptr;
-    uint32_t *d_f = nullptr, *d_e = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&d_am, n * sizeof(float), ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&d_as, n * sizeof(float), ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&d_f, n * sizeof(uint32_t), ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&d_e, n * sizeof(uint32_t), ctx->stream));
+    StreamBuf<float> d_am(ctx), d_as(ctx);
+    StreamBuf<uint32_t> d_f(ctx), d_e(ctx);
+    PPF_CUDA(ctx, d_am.alloc(n));
+    PPF_CUDA(ctx, d_as.alloc(n));
+    PPF_CUDA(ctx, d_f.alloc(n));
+    PPF_CUDA(ctx, d_e.alloc(n));
     PPF_CUDA(ctx, cudaMemcpyAsync(d_am, alpha_m, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     PPF_CUDA(ctx, cudaMemcpyAsync(d_as, alpha_s, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     PPF_LAUNCH(ctx, debug_alpha_bins_kernel, (unsigned)((n + 255) / 256), 256, 0, bp, d_am, d_as, (uint32_t)n, d_f, d_e);
     PPF_CUDA(ctx, cudaMemcpyAsync(fast, d_f, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaMemcpyAsync(exact, d_e, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFreeAsync(d_am, ctx->stream);
-    cudaFreeAsync(d_as, ctx->stream);
-    cudaFreeAsync(d_f, ctx->stream);
-    cudaFreeAsync(d_e, ctx->stream);
     return B200PPF_OK;
 }
 
@@ -1259,21 +1245,18 @@ int k3_debug_pairs(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud
                    uint8_t *in_radius, int32_t *d4, float *alpha_s) {
     if (!t || !scene || s_r >= scene->n) return fail_msg(ctx, B200PPF_ERR_INVALID, "debug pairs: bad arguments");
     const size_t n = scene->n;
-    uint8_t *d_in = nullptr;
-    int *d_d = nullptr;
-    float *d_a = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&d_in, n, ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&d_d, n * 4 * sizeof(int), ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&d_a, n * sizeof(float), ctx->stream));
+    StreamBuf<uint8_t> d_in(ctx);
+    StreamBuf<int> d_d(ctx);
+    StreamBuf<float> d_a(ctx);
+    PPF_CUDA(ctx, d_in.alloc(n));
+    PPF_CUDA(ctx, d_d.alloc(n * 4));
+    PPF_CUDA(ctx, d_a.alloc(n));
     PPF_LAUNCH(ctx, ppf_debug_pairs_kernel, (unsigned)((n + 255) / 256), 256, 0, scene->pos, scene->nrm, (uint32_t)n,
                (uint32_t)s_r, t->kp, t->feature_mode, t->info.max_dist * 0.5f, d_in, d_d, d_a);
     PPF_CUDA(ctx, cudaMemcpyAsync(in_radius, d_in, n, cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaMemcpyAsync(d4, d_d, n * 4 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaMemcpyAsync(alpha_s, d_a, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFreeAsync(d_in, ctx->stream);
-    cudaFreeAsync(d_d, ctx->stream);
-    cudaFreeAsync(d_a, ctx->stream);
     return B200PPF_OK;
 }
 

@@ -502,13 +502,8 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
     // state .. cl_size are contiguous: one memset clears state (UNDECIDED), leader ids, assignments, cluster sums
     PPF_CUDA(ctx, cudaMemsetAsync(state, 0, (o_cell - o_state) * sizeof(uint32_t), st));
     PPF_CUDA(ctx, cudaMemsetAsync(small, 0, (16 + 48) * sizeof(uint32_t), st));
-    if (ctx->assign_cap < n) {
-        if (ctx->d_assign) cudaFree(ctx->d_assign);
-        ctx->d_assign = nullptr;
-        ctx->assign_cap = ctx->assign_n = 0;
-        PPF_CUDA(ctx, cudaMalloc(&ctx->d_assign, n * sizeof(uint32_t)));
-        ctx->assign_cap = n;
-    }
+    ctx->assign_n = 0;
+    PPF_CUDA(ctx, grow_buffer(&ctx->d_assign, &ctx->assign_cap, n));
     ctx->assign_n = n;
 
     // small[0] = max votes, small[1] = undecided counter, small[2] = n_clusters, small[3..5] = top, small[6..8] = votes

@@ -32,8 +32,8 @@ int k5_transform(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, const float *pose
     if (out_stride_floats < 3) return fail_msg(ctx, B200PPF_ERR_INVALID, "transform: output stride must be >= 3 floats");
     Pose16 P;
     memcpy(P.m, pose16, sizeof(P.m));
-    float *d = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&d, n * 3 * sizeof(float), ctx->stream));
+    StreamBuf<float> d(ctx);
+    PPF_CUDA(ctx, d.alloc(n * 3));
     cudaEventRecord(ctx->ev[0], ctx->stream);
     PPF_LAUNCH(ctx, transform_cloud_kernel, (unsigned)((n + 255) / 256), 256, 0, cloud->pos, (uint32_t)n, P, d, 3u);
     cudaEventRecord(ctx->ev[1], ctx->stream);
@@ -42,7 +42,6 @@ int k5_transform(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, const float *pose
                                     n, cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->timings.transform_ms, ctx->ev[0], ctx->ev[1]);
-    PPF_CUDA(ctx, cudaFreeAsync(d, ctx->stream));
     return B200PPF_OK;
 }
 

@@ -805,8 +805,8 @@ int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cl
     const size_t o_win = take(P * nd * sizeof(unsigned long long));
     const size_t o_cs = take(P * (ICP_CELLS_MAX + 1) * sizeof(uint32_t)), o_cf = take(P * ICP_CELLS_MAX * sizeof(uint32_t));
     const size_t o_items = take(P * nd * sizeof(float4));
-    unsigned char *slab = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&slab, off, ctx->stream));
+    StreamBuf<unsigned char> slab(ctx);
+    PPF_CUDA(ctx, slab.alloc(off));
     IcpArgs a;
     a.mpos = model->pos;
     a.mnrm = model->nrm;
@@ -867,7 +867,6 @@ int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cl
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->timings.icp_ms, ctx->ev[0], ctx->ev[1]);
     if (iterations_host) *iterations_host = it;
-    PPF_CUDA(ctx, cudaFreeAsync(slab, ctx->stream));
     return B200PPF_OK;
 }
 

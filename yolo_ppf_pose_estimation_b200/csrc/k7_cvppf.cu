@@ -453,7 +453,7 @@ void bbox6(const float *pc, size_t n, size_t stride, float r[6]) {
         }
 }
 
-// samplePCByQuantization over the box `range` -> device rows of 6 floats (caller frees with cudaFree) and their count
+// samplePCByQuantization over the box `range` -> device rows of 6 floats (cudaMalloc: the caller frees them) and their count
 template <class Points>
 int cv_sample_points(b200ppf_ctx *ctx, const Points &pts, size_t n, const float range[6], float sample_step, float **d_out,
                      size_t *n_out) {
@@ -493,13 +493,12 @@ int cv_sample_points(b200ppf_ctx *ctx, const Points &pts, size_t n, const float 
     if (rc) return rc;
     float *out = nullptr;
     PPF_CUDA(ctx, cudaMalloc(&out, std::max<size_t>(1, cells) * 6 * sizeof(float)));
+    std::unique_ptr<float, cudaError_t (*)(void *)> owner(out, cudaFree);
     cv_cell_average_kernel<Points><<<g, 256, 0, ctx->stream>>>(pts, os, head.p, rank.p, nn, out);
     ctx->launches++;
-    if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
-        cudaFree(out);
+    if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess)
         return fail_msg(ctx, B200PPF_ERR_CUDA, "cv sample: kernel failed");
-    }
-    *d_out = out;
+    *d_out = owner.release();
     *n_out = cells;
     return B200PPF_OK;
 }
@@ -542,26 +541,13 @@ void cv_free_model(b200cv_detector *d) {
     d->m = d->table_size = d->n_nodes = 0;
 }
 
-struct DevGuard {
-    int prev = -1;
-    explicit DevGuard(int dev) {
-        cudaGetDevice(&prev);
-        if (prev != dev) cudaSetDevice(dev);
-        else prev = -1;
-    }
-    ~DevGuard() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 // the voting launch of match / match_S2B over the detector's sampled clouds
-int cv_vote(b200cv_detector *d, uint32_t step, uint32_t refs, uint32_t *acc_dump_host, uint32_t dump_ref, b200cv_pose **d_poses_out) {
+int cv_vote(b200cv_detector *d, uint32_t step, uint32_t refs, uint32_t *acc_dump_host, uint32_t dump_ref, StreamBuf<b200cv_pose> &poses) {
     b200ppf_ctx *ctx = d->ctx;
     const int num_angles = (int)std::floor(2 * PI_D / d->angle_step);
     const size_t acc_len = d->m * (size_t)num_angles;
     const unsigned grid = (unsigned)std::min<size_t>(refs, (size_t)ctx->sm_count * 2);
     StreamBuf<uint32_t> acc(ctx), dump(ctx);
-    StreamBuf<b200cv_pose> poses(ctx);
     PPF_CUDA(ctx, acc.alloc(acc_len * grid));
     PPF_CUDA(ctx, cudaMemsetAsync(acc, 0, acc_len * grid * sizeof(uint32_t), ctx->stream));
     PPF_CUDA(ctx, poses.alloc(refs));
@@ -599,7 +585,6 @@ int cv_vote(b200cv_detector *d, uint32_t step, uint32_t refs, uint32_t *acc_dump
         PPF_CUDA(ctx, cudaMemcpyAsync(acc_dump_host, dump, acc_len * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->timings.vote_ms, ctx->ev[0], ctx->ev[1]);
-    if (d_poses_out) *d_poses_out = poses.release();  // the caller clusters them on the device and frees them
     return B200PPF_OK;
 }
 
@@ -807,7 +792,7 @@ int b200cv_detector_create(b200ppf_ctx *ctx, double relative_sampling_step, doub
 
 void b200cv_detector_free(b200cv_detector *d) {
     if (!d) return;
-    DevGuard guard(d->ctx->device);
+    DeviceGuard guard(d->ctx->device);
     cudaStreamSynchronize(d->ctx->stream);
     cv_free_match(d);
     cv_free_model(d);
@@ -825,7 +810,7 @@ int b200cv_detector_train(b200cv_detector *d, const float *model, size_t n, size
     if (!d || !model) return fail_msg(d ? d->ctx : nullptr, B200PPF_ERR_INVALID, "cv train: null argument");
     b200ppf_ctx *ctx = d->ctx;
     if (stride < 6 || n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv train: the model is N x 6 [x y z nx ny nz], N >= 1");
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     cv_free_model(d);
     float r[6];
     bbox6(model, n, stride, r);
@@ -909,7 +894,7 @@ int b200cv_detector_bucket(b200cv_detector *d, size_t bucket, uint32_t *ppf_ind,
     *n_found = 0;
     if (!d->d_offsets || bucket >= d->table_size) return B200PPF_OK;
     b200ppf_ctx *ctx = d->ctx;
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     uint32_t off[2];
     PPF_CUDA(ctx, cudaMemcpyAsync(off, d->d_offsets + bucket, sizeof(off), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -925,7 +910,7 @@ int b200cv_detector_bucket(b200cv_detector *d, size_t bucket, uint32_t *ppf_ind,
 int b200cv_detector_table_export(b200cv_detector *d, uint32_t *offsets, uint32_t *nodes, float *alpha_m) {
     if (!d || !d->d_offsets) return fail_msg(d ? d->ctx : nullptr, B200PPF_ERR_STATE, "cv export: the detector is not trained");
     b200ppf_ctx *ctx = d->ctx;
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     if (offsets) PPF_CUDA(ctx, cudaMemcpyAsync(offsets, d->d_offsets, (d->table_size + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     if (nodes) PPF_CUDA(ctx, cudaMemcpyAsync(nodes, d->d_nodes, d->n_nodes * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     if (alpha_m) PPF_CUDA(ctx, cudaMemcpyAsync(alpha_m, d->d_alpha, d->m * d->m * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
@@ -957,12 +942,11 @@ static int cv_match_sampled(b200cv_detector *d, int step, b200cv_pose *results, 
     const size_t refs = (d->n_scene + step - 1) / step;
     d->raw.clear();
     if (refs == 0) return B200PPF_OK;
-    b200cv_pose *d_poses = nullptr;
-    int rc = cv_vote(d, (uint32_t)step, (uint32_t)refs, acc_dump, (uint32_t)dump_ref, &d_poses);
+    StreamBuf<b200cv_pose> d_poses(ctx);  // per reference point, clustered on the device
+    int rc = cv_vote(d, (uint32_t)step, (uint32_t)refs, acc_dump, (uint32_t)dump_ref, d_poses);
     if (rc) return rc;
     size_t ncl = 0;
     rc = cv_cluster(d, d_poses, (uint32_t)refs, results, cap, &ncl);
-    cudaFreeAsync(d_poses, ctx->stream);
     if (rc) return rc;
     *n_results = ncl;
     return B200PPF_OK;
@@ -978,7 +962,7 @@ static int cv_match_impl(b200cv_detector *d, const float *scene, size_t n, size_
     b200ppf_ctx *ctx = d->ctx;
     if (stride < 6 || (edge && edge_stride < 6) || n == 0)
         return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: clouds are N x 6 [x y z nx ny nz]");
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     cv_free_match(d);
     float r[6];
     bbox6(scene, n, stride, r);
@@ -1009,7 +993,7 @@ int b200cv_detector_match_cloud(b200cv_detector *d, const b200ppf_cloud *scene, 
         return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match cloud: the clouds belong to another context than the detector");
     if (scene->n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match cloud: empty scene cloud");
     if (edge && edge->n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match_S2B: empty edge cloud");
-    DevGuard guard(ctx->device);
+    DeviceGuard guard(ctx->device);
     cv_free_match(d);
     rc = cv_sample_cloud(ctx, scene, (float)relative_scene_distance, &d->d_scene, &d->n_scene);
     if (rc) return rc;

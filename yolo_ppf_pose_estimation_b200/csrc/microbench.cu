@@ -115,22 +115,15 @@ int microbench_atoms(b200ppf_ctx *ctx, int pattern, double *atoms_per_sec) {
     *atoms_per_sec = 0.0;
     const bool large = pattern >= 8;
     const int p = pattern & 7;
-    unsigned long long *sink = nullptr;
-    uint32_t *table = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&sink, sizeof(unsigned long long), ctx->stream));
+    StreamBuf<unsigned long long> sink(ctx);
+    StreamBuf<uint32_t> table(ctx);
+    PPF_CUDA(ctx, sink.alloc(1));
     if (p >= 5) {
-        cudaError_t e = cudaMallocAsync(&table, (size_t)MB_TABLE_WORDS * sizeof(uint32_t), ctx->stream);
-        if (e != cudaSuccess) {
-            cudaFreeAsync(sink, ctx->stream);
-            return fail_msg(ctx, B200PPF_ERR_NOMEM, "microbench: table allocation failed");
-        }
+        if (table.alloc(MB_TABLE_WORDS) != cudaSuccess) return fail_msg(ctx, B200PPF_ERR_NOMEM, "microbench: table allocation failed");
         mb_fill_table_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table, p == 5 ? 0 : (p == 6 ? 1 : 3));
         ctx->launches++;
     }
-    const int rc = large ? run_rate<1024>(ctx, p, table, sink, atoms_per_sec) : run_rate<512>(ctx, p, table, sink, atoms_per_sec);
-    if (table) cudaFreeAsync(table, ctx->stream);
-    cudaFreeAsync(sink, ctx->stream);
-    return rc;
+    return large ? run_rate<1024>(ctx, p, table, sink, atoms_per_sec) : run_rate<512>(ctx, p, table, sink, atoms_per_sec);
 }
 
 }  // namespace b200ppf

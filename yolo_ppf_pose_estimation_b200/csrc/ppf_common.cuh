@@ -6,6 +6,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <array>
+#include <memory>
 #include <string>
 
 #include "../../include/b200ppf.h"
@@ -49,8 +51,8 @@ struct b200ppf_ctx {
     size_t assign_cap = 0;  // capacity of d_assign
     uint32_t n_clusters = 0;
     // grow-only pinned staging buffer of cloud uploads
-    void *stage = nullptr;
-    size_t stage_bytes = 0;
+    float4 *stage = nullptr;
+    size_t stage_cap = 0;
 };
 
 struct b200ppf_cloud {
@@ -130,6 +132,55 @@ struct StreamBuf {
     }
     operator T *() const { return p; }
 };
+
+// a context buffer kept across calls and grown on demand (cudaMalloc, or pinned host memory): its contents are not
+// kept, and after a failed allocation the pointer is null and the capacity 0
+template <typename T>
+cudaError_t grow_buffer(T **p, size_t *cap, size_t count, bool pinned = false) {
+    if (*cap >= count) return cudaSuccess;
+    if (*p) pinned ? cudaFreeHost(*p) : cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    const cudaError_t e = pinned ? cudaMallocHost(reinterpret_cast<void **>(p), count * sizeof(T)) : cudaMalloc(p, count * sizeof(T));
+    if (e == cudaSuccess) *cap = count;
+    return e;
+}
+
+// makes `dev` the current device for the scope
+struct DeviceGuard {
+    int prev = -1;
+    explicit DeviceGuard(int dev) {
+        cudaGetDevice(&prev);
+        if (prev != dev) cudaSetDevice(dev);
+        else prev = -1;
+    }
+    ~DeviceGuard() {
+        if (prev >= 0) cudaSetDevice(prev);
+    }
+};
+
+// a handle owned through its C ABI free function, e.g. a cloud under construction until it is released to the caller
+template <auto Free>
+struct FreeWith {
+    template <typename T>
+    void operator()(T *p) const { Free(p); }
+};
+using CloudPtr = std::unique_ptr<b200ppf_cloud, FreeWith<b200ppf_cloud_free>>;
+using TablePtr = std::unique_ptr<b200ppf_table, FreeWith<b200ppf_table_free>>;
+
+// a cloud of n points whose arrays are allocated (pos | nrm in one stream-ordered allocation) but not filled
+int cloud_alloc(b200ppf_ctx *ctx, size_t n, CloudPtr *out);
+
+// one device array of a table: where its pointer lives, its length in 32-bit words and the readable zero words behind it
+struct TableArray {
+    uint32_t **slot;
+    size_t words, pad;
+    bool used;  // whether the table has this array at all
+};
+// the eight arrays of a table in file order, as its info, kp, bp and n_merged size them
+std::array<TableArray, 8> table_arrays(b200ppf_table *t);
+// allocates one array from the stream-ordered pool (at least one word) and zeroes its pad
+cudaError_t table_array_alloc(cudaStream_t stream, const TableArray &a);
 
 // ---- stage entry points implemented in the k*.cu files (host functions) ----------------------
 int k1_features_compute(b200ppf_ctx *ctx, const b200ppf_cloud *model, b200ppf_signature *out);
@@ -230,6 +281,10 @@ struct SceneGrid {
 uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp);
 int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius, SceneGrid *out);
 void scene_grid_free(b200ppf_ctx *ctx, SceneGrid *g);
+struct SceneGridFree {
+    b200ppf_ctx *ctx;
+    void operator()(SceneGrid *g) const { scene_grid_free(ctx, g); }
+};
 
 // hand-written LSD radix sort (radix_sort.cu): keys ascending, stable, two 32-bit payload streams.
 // All buffers are device pointers of n elements; *_alt are the ping-pong partners.  On return

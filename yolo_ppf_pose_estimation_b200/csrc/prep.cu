@@ -36,22 +36,6 @@ namespace {
 
 constexpr int SCAN_BLOCK = 1024;
 
-// an output cloud under construction: freed unless released to the caller
-struct CloudOwner {
-    b200ppf_cloud *c = nullptr;
-    CloudOwner() = default;
-    CloudOwner(const CloudOwner &) = delete;
-    CloudOwner &operator=(const CloudOwner &) = delete;
-    ~CloudOwner() {
-        if (c) b200ppf_cloud_free(c);
-    }
-    b200ppf_cloud *release() {
-        b200ppf_cloud *r = c;
-        c = nullptr;
-        return r;
-    }
-};
-
 // ---- exclusive scan of 0/1 flags (three launches; same shape as K4's leader index) ----------------------------
 __global__ void __launch_bounds__(SCAN_BLOCK)
 flag_count_kernel(const uint32_t *__restrict__ flags, uint32_t n, uint32_t *__restrict__ block_sums) {
@@ -191,22 +175,6 @@ int cloud_bbox_from_device(b200ppf_ctx *ctx, b200ppf_cloud *c) {
         c->bbox_min[k] = float_unorder(h[k]);
         c->bbox_max[k] = float_unorder(h[3 + k]);
     }
-    return B200PPF_OK;
-}
-
-// a cloud of n points whose arrays are allocated (pos | nrm in one allocation) but not filled
-int cloud_alloc(b200ppf_ctx *ctx, size_t n, b200ppf_cloud **out) {
-    b200ppf_cloud *c = new (std::nothrow) b200ppf_cloud();
-    if (!c) return fail_msg(ctx, B200PPF_ERR_NOMEM, "pre-processing: out of host memory");
-    c->ctx = ctx;
-    c->n = n;
-    cudaError_t e = cudaMallocAsync(&c->pos, std::max<size_t>(1, 2 * n) * sizeof(float4), ctx->stream);
-    if (e != cudaSuccess) {
-        delete c;
-        return fail_msg(ctx, B200PPF_ERR_NOMEM, "pre-processing: device allocation of the output cloud failed");
-    }
-    c->nrm = c->pos + n;
-    *out = c;
     return B200PPF_OK;
 }
 
@@ -609,19 +577,17 @@ float knn_cell_edge(const b200ppf_cloud *c, int k) {
 template <int MODE>
 int knn_run(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, KnnArgs a) {
     SceneGrid grid;
+    std::unique_ptr<SceneGrid, SceneGridFree> grid_owner(&grid, SceneGridFree{ctx});
     int rc = scene_grid_build(ctx, cloud, knn_cell_edge(cloud, a.k), &grid);
-    if (rc == B200PPF_OK) {
-        a.pos = cloud->pos;
-        a.gpos = grid.pos;
-        a.cell_start = grid.cell_start;
-        a.orig = grid.orig;
-        a.gp = grid.gp;
-        a.cell = 1.0f / grid.gp.inv_cell;
-        a.n = (uint32_t)cloud->n;
-        rc = knn_launch<MODE>(ctx, a);
-    }
-    scene_grid_free(ctx, &grid);
-    return rc;
+    if (rc != B200PPF_OK) return rc;
+    a.pos = cloud->pos;
+    a.gpos = grid.pos;
+    a.cell_start = grid.cell_start;
+    a.orig = grid.orig;
+    a.gp = grid.gp;
+    a.cell = 1.0f / grid.gp.inv_cell;
+    a.n = (uint32_t)cloud->n;
+    return knn_launch<MODE>(ctx, a);
 }
 
 // ---- P3: statistical outlier removal --------------------------------------------------------------------------
@@ -684,12 +650,12 @@ int compact_cloud(b200ppf_ctx *ctx, const b200ppf_cloud *in, const uint32_t *fla
     uint32_t m = 0;
     int rc = flag_scan(ctx, flags, n, rank, &m);
     if (rc != B200PPF_OK) return rc;
-    CloudOwner c;
-    if ((rc = cloud_alloc(ctx, m, &c.c)) != B200PPF_OK) return rc;
+    CloudPtr c;
+    if ((rc = cloud_alloc(ctx, m, &c)) != B200PPF_OK) return rc;
     if (kept_host && m) PPF_CUDA(ctx, index.alloc(m));
-    if (n) PPF_LAUNCH(ctx, compact_kernel, (n + 255) / 256, 256, 0, in->pos, in->nrm, flags, rank, n, c.c->pos, c.c->nrm, index);
+    if (n) PPF_LAUNCH(ctx, compact_kernel, (n + 255) / 256, 256, 0, in->pos, in->nrm, flags, rank, n, c->pos, c->nrm, index);
     if (index) PPF_CUDA(ctx, cudaMemcpyAsync(kept_host, index, (size_t)m * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if ((rc = cloud_bbox_from_device(ctx, c.c)) != B200PPF_OK) return rc;  // synchronises the stream
+    if ((rc = cloud_bbox_from_device(ctx, c.get())) != B200PPF_OK) return rc;  // synchronises the stream
     *out = c.release();
     return B200PPF_OK;
 }
@@ -763,15 +729,8 @@ int flag_scan_u32(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t 
 // host entry points (called from capi.cu)
 
 int prep_upload_xyz(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, b200ppf_cloud **out) {
-    const size_t need = std::max<size_t>(1, n) * sizeof(float4);
-    if (ctx->stage_bytes < need) {
-        if (ctx->stage) cudaFreeHost(ctx->stage);
-        ctx->stage = nullptr;
-        ctx->stage_bytes = 0;
-        PPF_CUDA(ctx, cudaMallocHost(&ctx->stage, need));
-        ctx->stage_bytes = need;
-    }
-    float4 *sp = static_cast<float4 *>(ctx->stage);
+    PPF_CUDA(ctx, grow_buffer(&ctx->stage, &ctx->stage_cap, std::max<size_t>(1, n), /*pinned=*/true));
+    float4 *sp = ctx->stage;
     size_t m = 0;
     float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
     for (size_t i = 0; i < n; ++i) {
@@ -783,15 +742,15 @@ int prep_upload_xyz(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride
             hi[k] = std::max(hi[k], p[k]);
         }
     }
-    CloudOwner c;
-    int rc = cloud_alloc(ctx, m, &c.c);
+    CloudPtr c;
+    int rc = cloud_alloc(ctx, m, &c);
     if (rc != B200PPF_OK) return rc;
     for (int k = 0; k < 3; ++k) {
-        c.c->bbox_min[k] = m ? lo[k] : 0.0f;
-        c.c->bbox_max[k] = m ? hi[k] : 0.0f;
+        c->bbox_min[k] = m ? lo[k] : 0.0f;
+        c->bbox_max[k] = m ? hi[k] : 0.0f;
     }
-    if (m) PPF_CUDA(ctx, cudaMemcpyAsync(c.c->pos, sp, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
-    if (m) PPF_CUDA(ctx, cudaMemsetAsync(c.c->nrm, 0, m * sizeof(float4), ctx->stream));
+    if (m) PPF_CUDA(ctx, cudaMemcpyAsync(c->pos, sp, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
+    if (m) PPF_CUDA(ctx, cudaMemsetAsync(c->nrm, 0, m * sizeof(float4), ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the staging buffer is reused by the next upload
     *out = c.release();
     return B200PPF_OK;
@@ -813,8 +772,10 @@ int prep_voxel_grid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *leaf
     const uint32_t n = (uint32_t)in->n;
     EventTimer timer(ctx);
     if (n == 0) {
-        int rc = cloud_alloc(ctx, 0, out);
+        CloudPtr c;
+        int rc = cloud_alloc(ctx, 0, &c);
         timer.stop();
+        *out = c.release();
         return rc;
     }
     VoxelParams vp;
@@ -824,11 +785,11 @@ int prep_voxel_grid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *leaf
     for (int k = 0; k < 3; ++k) d[k] = (int64_t)((in->bbox_max[k] - in->bbox_min[k]) * vp.inv[k]) + 1;
     const bool overflow = d[0] * d[1] * d[2] > (int64_t)INT32_MAX;
     if (overflow) {
-        CloudOwner c;
-        int rc = cloud_alloc(ctx, n, &c.c);
+        CloudPtr c;
+        int rc = cloud_alloc(ctx, n, &c);
         if (rc != B200PPF_OK) return rc;
-        PPF_LAUNCH(ctx, copy_cloud_kernel, (n + 255) / 256, 256, 0, in->pos, in->nrm, n, c.c->pos, c.c->nrm);
-        for (int k = 0; k < 3; ++k) c.c->bbox_min[k] = in->bbox_min[k], c.c->bbox_max[k] = in->bbox_max[k];
+        PPF_LAUNCH(ctx, copy_cloud_kernel, (n + 255) / 256, 256, 0, in->pos, in->nrm, n, c->pos, c->nrm);
+        for (int k = 0; k < 3; ++k) c->bbox_min[k] = in->bbox_min[k], c->bbox_max[k] = in->bbox_max[k];
         timer.stop();
         ctx->error = "voxel grid: leaf size is too small for the input dataset, integer indices would overflow; input returned unchanged";
         *out = c.release();
@@ -862,11 +823,11 @@ int prep_voxel_grid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *leaf
     uint32_t m = 0;
     if ((rc = flag_scan(ctx, head, n, rank, &m)) != B200PPF_OK) return rc;
     PPF_CUDA(ctx, starts.alloc((size_t)m + 1));
-    CloudOwner c;
-    if ((rc = cloud_alloc(ctx, m, &c.c)) != B200PPF_OK) return rc;
+    CloudPtr c;
+    if ((rc = cloud_alloc(ctx, m, &c)) != B200PPF_OK) return rc;
     PPF_LAUNCH(ctx, voxel_starts_kernel, gb, 256, 0, head, rank, n, m, starts);
-    PPF_LAUNCH(ctx, voxel_centroid_kernel, (m + 127) / 128, 128, 0, in->pos, order, starts, m, c.c->pos, c.c->nrm);
-    if ((rc = cloud_bbox_from_device(ctx, c.c)) != B200PPF_OK) return rc;
+    PPF_LAUNCH(ctx, voxel_centroid_kernel, (m + 127) / 128, 128, 0, in->pos, order, starts, m, c->pos, c->nrm);
+    if ((rc = cloud_bbox_from_device(ctx, c.get())) != B200PPF_OK) return rc;
     timer.stop();
     *out = c.release();
     return B200PPF_OK;

@@ -220,10 +220,10 @@ int radix_sort_impl(b200ppf_ctx *ctx, uint32_t *keys, uint32_t *keys_alt, uint32
     constexpr uint32_t TILE = WARPS * ROUNDS * 32;
     const uint32_t ntiles = (uint32_t)((n + TILE - 1) / TILE);
     const uint32_t nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK;
-    uint32_t *hist = nullptr, *chunk_tot = nullptr, *digit_base = nullptr;
-    PPF_CUDA(ctx, cudaMallocAsync(&hist, (size_t)ntiles * RADIX * sizeof(uint32_t), ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&chunk_tot, (size_t)nchunks * RADIX * sizeof(uint32_t), ctx->stream));
-    PPF_CUDA(ctx, cudaMallocAsync(&digit_base, RADIX * sizeof(uint32_t), ctx->stream));
+    StreamBuf<uint32_t> hist(ctx), chunk_tot(ctx), digit_base(ctx);
+    PPF_CUDA(ctx, hist.alloc((size_t)ntiles * RADIX));
+    PPF_CUDA(ctx, chunk_tot.alloc((size_t)nchunks * RADIX));
+    PPF_CUDA(ctx, digit_base.alloc(RADIX));
 
     const bool has_v0 = v0 != nullptr && v0_alt != nullptr, has_v1 = v1 != nullptr && v1_alt != nullptr;
     bool iota = has_v0 && v0_iota;
@@ -259,9 +259,6 @@ int radix_sort_impl(b200ppf_ctx *ctx, uint32_t *keys, uint32_t *keys_alt, uint32
         t = v1i; v1i = v1o; v1o = t;
         in_alt = !in_alt;
     }
-    PPF_CUDA(ctx, cudaFreeAsync(hist, ctx->stream));
-    PPF_CUDA(ctx, cudaFreeAsync(chunk_tot, ctx->stream));
-    PPF_CUDA(ctx, cudaFreeAsync(digit_base, ctx->stream));
     *result_in_alt = in_alt;
     return B200PPF_OK;
 }
