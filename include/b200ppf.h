@@ -462,6 +462,9 @@ int b200cv_detector_create(b200ppf_ctx *ctx, double relative_sampling_step, doub
 void b200cv_detector_free(b200cv_detector *d);
 /* setSearchParams(positionThreshold, rotationThreshold): a negative value keeps the default */
 int b200cv_detector_set_search_params(b200cv_detector *d, double position_threshold, double rotation_threshold);
+/* trainModel.  The model must sample to 2 .. 46340 points: the table's m^2 pair slots and its power-of-two bucket count
+ * are 32-bit, so m^2 <= 2^31.  A larger sampled model is refused with B200PPF_ERR_UNSUPPORTED right after sampling,
+ * before any table memory is allocated, and leaves the detector untrained (it can be trained again). */
 int b200cv_detector_train(b200cv_detector *d, const float *model, size_t n, size_t stride_floats);
 int b200cv_detector_get_info(const b200cv_detector *d, b200cv_info *info);
 int b200cv_detector_model_points(const b200cv_detector *d, float *out6);  /* n_sampled x 6 */

@@ -137,6 +137,9 @@ def _declare(L):
     L.oracle_cv_match_s2b.restype = sz
     L.oracle_cv_table_size.argtypes = [vp]
     L.oracle_cv_table_size.restype = sz
+    L.oracle_cv_table_export.argtypes = [vp, vp, vp]
+    L.oracle_cv_num_angles.argtypes = [vp]
+    L.oracle_cv_num_angles.restype = C.c_int
     L.oracle_cv_bucket.argtypes = [vp, sz, vp, sz]
     L.oracle_cv_bucket.restype = sz
     L.oracle_cv_accumulator.argtypes = [vp, vp, sz, vp, sz, C.c_double, sz, vp]
@@ -559,10 +562,23 @@ class CvDetector:
             lib().oracle_cv_bucket(self._h, int(b), _p(out), n)
         return out
 
-    def accumulator(self, scene, sampled_index, relative_scene_distance, num_angles=30, edge=None):
+    @property
+    def num_angles(self):
+        """accumulator columns of the trained detector: floor(2 pi / angle_step)"""
+        return int(lib().oracle_cv_num_angles(self._h))
+
+    def table_export(self):
+        """(offsets (table_size + 1,), nodes (M * (M - 1),)): the buckets as a CSR, nodes ascending inside a bucket"""
+        off = np.zeros(self.table_size + 1, np.uint32)
+        nodes = np.zeros(max(1, self.n_model * (self.n_model - 1)), np.uint32)
+        lib().oracle_cv_table_export(self._h, _p(off), _p(nodes))
+        return off, nodes[:self.n_model * (self.n_model - 1)]
+
+    def accumulator(self, scene, sampled_index, relative_scene_distance, edge=None):
+        """accumulator (M, num_angles) of the sampled scene point sampled_index"""
         scene = _f32(scene)
         edge = None if edge is None else _f32(edge)
-        acc = np.zeros((self.n_model, num_angles), np.uint32)
+        acc = np.zeros((self.n_model, self.num_angles), np.uint32)
         lib().oracle_cv_accumulator(self._h, _p(scene), scene.shape[0], _p(edge) if edge is not None else None,
                                     0 if edge is None else edge.shape[0], float(relative_scene_distance), int(sampled_index), _p(acc))
         return acc

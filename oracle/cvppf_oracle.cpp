@@ -503,6 +503,21 @@ size_t oracle_cv_match_s2b(const oracle_cv_detector *d, const float *scene, size
 
 size_t oracle_cv_table_size(const oracle_cv_detector *d) { return d->table_size; }
 
+/* the whole table as a CSR over the buckets: offsets (table_size + 1), nodes (ppfInd, ascending inside a bucket) */
+void oracle_cv_table_export(const oracle_cv_detector *d, uint32_t *offsets, uint32_t *nodes) {
+    size_t at = 0;
+    for (size_t b = 0; b < d->buckets.size(); ++b) {
+        offsets[b] = (uint32_t)at;
+        const size_t first = at;
+        for (const auto &node : d->buckets[b]) nodes[at++] = node.second;
+        std::sort(nodes + first, nodes + at);
+    }
+    offsets[d->buckets.size()] = (uint32_t)at;
+}
+
+/* columns of an accumulator: numAngles = floor(2 pi / angle_step), as match() sizes it (one fewer than asked for 13, 25, ...) */
+int oracle_cv_num_angles(const oracle_cv_detector *d) { return (int)std::floor(2 * PI / d->angle_step); }
+
 size_t oracle_cv_bucket(const oracle_cv_detector *d, size_t bucket, uint32_t *ppf_ind, size_t cap) {
     if (bucket >= d->buckets.size()) return 0;
     std::vector<uint32_t> v;

@@ -2,11 +2,13 @@
 actually calls (include/CloudProcessing.h:205-236, :442).  It is the checker of a row that is not built on the device
 yet (SURVEY.md §8f rank 4); these tests pin what can be pinned offline: the hash against published MurmurHash3 vectors,
 the sampling and the pair feature against numpy restatements, and the whole train / match / cluster chain against a
-known rigid motion."""
+known rigid motion.  The rest of the chain is compared with tests/cvppf_reference.py in test_cvppf_reference_host.py."""
 import struct
 
 import numpy as np
 import pytest
+
+import cvppf_reference as cr
 
 
 def test_murmur3_x86_32_known_answers(oracle):
@@ -43,22 +45,16 @@ def test_pair_feature_and_hash(oracle, bottle_5mm):
 
 
 def test_sample_by_quantization(oracle, bottle_5mm):
-    step = 0.05
-    out = oracle.cv_sample(bottle_5mm, step)
-    pc = bottle_5mm
-    ns = int(1.0 / float(np.float32(step)))  # (int)(1.0 / sampleStep) with a float step: 19, not 20, for 0.05f
-    assert ns == 19
-    lo, hi = pc[:, :3].min(0), pc[:, :3].max(0)
-    cells = (np.float32(ns) * (pc[:, :3] - lo) / (hi - lo)).astype(np.int32)  # float32 arithmetic, truncation
-    index = cells[:, 0] * ns * ns + cells[:, 1] * ns + cells[:, 2]            # upstream's stride (ns, not ns + 1)
-    order = np.argsort(index, kind="stable")
-    starts = np.flatnonzero(np.r_[True, index[order][1:] != index[order][:-1]])
-    counts = np.diff(np.r_[starts, index.size])
-    mean = np.add.reduceat(pc[order].astype(np.float64), starts, axis=0) / counts[:, None]
-    mean[:, 3:] /= np.linalg.norm(mean[:, 3:], axis=1, keepdims=True)
-    assert out.shape == mean.shape and 100 < out.shape[0] < pc.shape[0]
-    assert np.abs(out - mean).max() < 1e-6
-    assert np.abs(np.linalg.norm(out[:, 3:], axis=1) - 1).max() < 1e-6
+    """float32 cell arithmetic, upstream's stride ns (a coordinate on the upper bound shares a neighbour's list), averages
+    in double in input order: the restatement in tests/cvppf_reference.py and the oracle agree bit for bit"""
+    assert int(1.0 / float(np.float32(0.05))) == 19  # (int)(1.0 / sampleStep) with a float step: 19 cells, not 20
+    for step in (0.05, 0.04, 0.1, 1.0 / 8.5):
+        out = cr.sample(bottle_5mm, np.float32(step))
+        assert np.array_equal(out.view(np.uint32), oracle.cv_sample(bottle_5mm, step).view(np.uint32)), step
+        assert 100 < out.shape[0] < bottle_5mm.shape[0]
+        assert np.abs(np.linalg.norm(out[:, 3:], axis=1) - 1).max() < 1e-6
+        index, ns = cr.sample_cells(bottle_5mm, np.float32(step))
+        assert index.max() >= ns * ns * ns  # the points on the upper bound of x exist and land past the last full cell
 
 
 def _rigid(axis, angle, t):

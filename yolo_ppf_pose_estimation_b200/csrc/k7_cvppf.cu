@@ -820,9 +820,11 @@ int b200cv_detector_train(b200cv_detector *d, const float *model, size_t n, size
     int rc = cv_sample(ctx, model, n, stride, r, (float)d->sampling_step_relative, &d->d_model, &d->m);
     if (rc) return rc;
     const size_t m = d->m;
-    if (m < 2 || m > 65535) {
+    // the table addresses its m^2 pair slots and its power-of-two bucket count with 32-bit words: m^2 <= 2^31 keeps both in
+    // range (46341^2 > 2^31 would round the bucket count up to 2^32); refused before any of the O(m^2) buffers is allocated
+    if (m < 2 || m > 46340) {
         cv_free_model(d);
-        return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "cv train: 2 .. 65535 sampled model points");
+        return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "cv train: 2 .. 46340 sampled model points (m^2 pair slots in 32-bit offsets)");
     }
     d->h_model.resize(m * 6);
     PPF_CUDA(ctx, cudaMemcpyAsync(d->h_model.data(), d->d_model, m * 6 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
