@@ -45,6 +45,11 @@ class IcpParams(C.Structure):
                 ("num_levels", C.c_int)]
 
 
+class IcpJob(C.Structure):
+    _fields_ = [("model", C.c_void_p), ("scene", C.c_void_p), ("poses16", C.c_void_p), ("n_poses", C.c_size_t),
+                ("residuals", C.c_void_p)]
+
+
 class ObjectParams(C.Structure):
     _fields_ = [("leaf", C.c_float), ("sor_mean_k", C.c_int), ("sor_stddev_mul", C.c_double), ("normal_k", C.c_int),
                 ("edge_curvature", C.c_float), ("ref_rate", C.c_uint32), ("pos_thr", C.c_float), ("rot_thr", C.c_float),
@@ -145,6 +150,7 @@ SYMBOLS = {
     "b200ppf_cluster_device": (_i, [_vp, _vp, _sz, _f, _f, _vp, _vp, C.POINTER(_sz)]),
     "b200ppf_cluster_assignment": (_i, [_vp, _vp, _sz, C.POINTER(_sz)]),
     "b200ppf_icp_refine": (_i, [_vp, _vp, _vp, C.POINTER(IcpParams), _vp, _sz, _vp, C.POINTER(C.c_uint64)]),
+    "b200ppf_icp_refine_batch": (_i, [_vp, C.POINTER(IcpJob), _sz, C.POINTER(IcpParams), C.POINTER(C.c_uint64)]),
     "b200ppf_transform": (_i, [_vp, _vp, _vp, _vp, _sz]),
     "b200ppf_cloud_upload_xyz": (_i, [_vp, _vp, _sz, _sz, C.POINTER(_vp)]),
     "b200ppf_cloud_download": (_i, [_vp, _vp, _vp, _sz, _sz, _sz]),
@@ -157,10 +163,12 @@ SYMBOLS = {
     "b200ppf_normalize_normals": (_i, [_vp, _vp]),
     "b200ppf_frustum_corners": (_i, [_vp, _i, _i, _i, _i, _i, _i, C.c_double, C.c_double, C.c_double, C.c_double, _vp]),
     "b200ppf_crop_pyramid": (_i, [_vp, _vp, _vp, C.POINTER(_vp), _vp]),
+    "b200ppf_crop_pyramids": (_i, [_vp, _vp, _vp, _sz, _vp]),
     "b200ppf_debug_knn_host": (_i, [_vp, _sz, _sz, _i, _i, _f, _vp, _i, _vp, _vp, _vp, _vp]),
     "b200ppf_object_params_default": (None, [C.POINTER(ObjectParams)]),
     "b200ppf_match_object": (_i, [_vp, _vp, _vp, _vp, _vp, C.POINTER(ObjectParams), C.POINTER(ObjectResult), C.POINTER(_vp),
                                   C.POINTER(_vp)]),
+    "b200ppf_match_frame": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(ObjectParams), C.POINTER(ObjectResult), _vp]),
     "b200ppf_register": (_i, [_vp, _vp, _vp, _vp, _sz, _f, _f, _vp, _vp, _vp, C.POINTER(_sz)]),
     "b200cv_detector_create": (_i, [_vp, C.c_double, C.c_double, C.c_double, C.POINTER(_vp)]),
     "b200cv_detector_free": (None, [_vp]),
@@ -175,6 +183,7 @@ SYMBOLS = {
     "b200cv_object_params_default": (None, [C.POINTER(CvObjectParams)]),
     "b200cv_match_object": (_i, [_vp, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(ObjectResult), C.POINTER(_vp),
                                  C.POINTER(_vp)]),
+    "b200cv_match_frame": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(ObjectResult), _vp]),
     "b200cv_detector_bucket": (_i, [_vp, _sz, _vp, _sz, C.POINTER(_sz)]),
     "b200cv_detector_table_export": (_i, [_vp, _vp, _vp, _vp]),
     "b200cv_detector_raw_poses": (_i, [_vp, _vp, _sz, C.POINTER(_sz)]),
@@ -322,6 +331,14 @@ class Context:
         out = Cloud(self, h)
         return out, kept[:out.size].copy()
 
+    def crop_pyramids(self, cloud: "Cloud", corners):
+        """SceneCropping for K boxes in one pass over the frame: corners (K, 4, 3) or (K, 12) -> K Clouds, cloud k as
+        crop_pyramid(cloud, corners[k]) makes it"""
+        c12 = np.ascontiguousarray(corners, np.float32).reshape(-1, 12)
+        out = (C.c_void_p * max(1, c12.shape[0]))()
+        self.check(lib().b200ppf_crop_pyramids(self._h, cloud._h, _p(c12), c12.shape[0], out))
+        return [Cloud(self, C.c_void_p(out[k])) for k in range(c12.shape[0])]
+
     def voxel_grid(self, cloud: "Cloud", leaf) -> "Cloud":
         """pcl::VoxelGrid<PointXYZ>::filter (Subsampling)"""
         leaf3 = np.ascontiguousarray(np.broadcast_to(np.asarray(leaf, np.float32), (3,)))
@@ -364,9 +381,9 @@ class Context:
         """CloudProcessor::PointCloudXYZNormalToMat's re-normalisation, in place"""
         self.check(lib().b200ppf_normalize_normals(self._h, cloud._h))
 
-    def _object_call(self, params_cls, default_fn, call, overrides):
-        """the per-object calls: defaults, then overrides (fields of params_cls; icp_* for the ICP) ->
-        (result dict, object Cloud, edges Cloud or None)"""
+    @staticmethod
+    def _params(params_cls, default_fn, overrides):
+        """defaults, then overrides (fields of params_cls; icp_* for the ICP)"""
         prm = params_cls()
         default_fn(C.byref(prm))
         for k, v in overrides.items():
@@ -374,12 +391,34 @@ class Context:
                 setattr(prm.icp, k[4:], v)
             else:
                 setattr(prm, k, v)
+        return prm
+
+    @staticmethod
+    def _result(res):
+        out = {n: getattr(res, n) for n, _ in ObjectResult._fields_ if n != "pose"}
+        out["pose"] = np.array(res.pose, np.float64).reshape(4, 4)
+        return out
+
+    def _object_call(self, params_cls, default_fn, call, overrides):
+        """the per-object calls: -> (result dict, object Cloud, edges Cloud or None)"""
+        prm = self._params(params_cls, default_fn, overrides)
         res = ObjectResult()
         obj, edg = C.c_void_p(), C.c_void_p()
         self.check(call(C.byref(prm), C.byref(res), C.byref(obj), C.byref(edg)))
-        out = {n: getattr(res, n) for n, _ in ObjectResult._fields_ if n != "pose"}
-        out["pose"] = np.array(res.pose, np.float64).reshape(4, 4)
-        return out, Cloud(self, obj), (Cloud(self, edg) if edg.value else None)
+        return self._result(res), Cloud(self, obj), (Cloud(self, edg) if edg.value else None)
+
+    def _frame_call(self, params_cls, default_fn, call, corners, overrides):
+        """the frame calls: -> (result dicts, one per box, int32 status per box)"""
+        c12 = np.ascontiguousarray(corners, np.float32).reshape(-1, 12)
+        prm = self._params(params_cls, default_fn, overrides)
+        res = (ObjectResult * max(1, c12.shape[0]))()
+        status = np.zeros(max(1, c12.shape[0]), np.int32)
+        self.check(call(c12.shape[0], _p(c12), C.byref(prm), res, _p(status)))
+        return [self._result(res[k]) for k in range(c12.shape[0])], status[:c12.shape[0]]
+
+    @staticmethod
+    def _handles(objs, n):
+        return (C.c_void_p * max(1, n))(*[None if o is None else o._h for o in objs])
 
     def match_object(self, scene: "Cloud", corners, model: "Cloud", table: "Table", **overrides):
         """One YOLO box start to finish (src/YOLO_cropping_ppf_test.cpp:91-122) on device handles:
@@ -395,6 +434,22 @@ class Context:
         c12 = np.ascontiguousarray(corners, np.float32).reshape(12)
         return self._object_call(CvObjectParams, lib().b200cv_object_params_default,
                                  lambda *a: lib().b200cv_match_object(detector._h, scene._h, _p(c12), model._h, *a), overrides)
+
+    def cv_match_frame(self, scene: "Cloud", corners, detectors, models, **overrides):
+        """every box of a frame in one call (b200cv_match_frame): corners (K, 4, 3), detectors / models one per box ->
+        (K result dicts as cv_match_object gives them, status per box: 0 or the per-object call's error code).
+        crop_ms, icp_ms and total_wall_ms are the frame's, repeated in every result."""
+        n = len(detectors)
+        dets, mods = self._handles(detectors, n), self._handles(models, n)
+        return self._frame_call(CvObjectParams, lib().b200cv_object_params_default,
+                                lambda k, c, *a: lib().b200cv_match_frame(self._h, scene._h, k, c, dets, mods, *a), corners, overrides)
+
+    def match_frame(self, scene: "Cloud", corners, models, tables, **overrides):
+        """match_object for every box of a frame in one call (b200ppf_match_frame), as cv_match_frame"""
+        n = len(models)
+        mods, tabs = self._handles(models, n), self._handles(tables, n)
+        return self._frame_call(ObjectParams, lib().b200ppf_object_params_default,
+                                lambda k, c, *a: lib().b200ppf_match_frame(self._h, scene._h, k, c, mods, tabs, *a), corners, overrides)
 
     # ---- K1 / K2 -------------------------------------------------------------------------------
     def features_compute(self, model: "Cloud") -> "Features":
@@ -430,6 +485,21 @@ class Context:
         self.check(lib().b200ppf_icp_refine(self._h, model._h, scene._h, C.byref(prm), _p(P), P.shape[0], _p(res),
                                             C.byref(it)))
         return P, res, int(it.value)
+
+    def icp_refine_batch(self, jobs, max_iterations=100, tolerance=0.005, rejection_scale=2.5, num_levels=8):
+        """several registerModelToScene problems in one call: jobs = [(model, scene, poses), ...] ->
+        ([(refined (P,4,4), residuals) per job], total iterations)"""
+        arrays = []
+        for _, _, p in jobs:
+            P = np.ascontiguousarray(np.asarray(p, np.float64).reshape(-1, 4, 4)).copy()
+            arrays.append((P, np.zeros(P.shape[0], np.float64)))
+        js = (IcpJob * max(1, len(jobs)))()
+        for k, ((m, s, _), (P, r)) in enumerate(zip(jobs, arrays)):
+            js[k] = IcpJob(m._h, s._h, P.ctypes.data, P.shape[0], r.ctypes.data)
+        it = C.c_uint64(0)
+        prm = IcpParams(max_iterations, tolerance, rejection_scale, num_levels)
+        self.check(lib().b200ppf_icp_refine_batch(self._h, js, len(jobs), C.byref(prm), C.byref(it)))
+        return arrays, int(it.value)
 
     def table_load(self, path) -> "Table":
         """LoadTrainedDetector: rebuild a saved table on this context's device (no K1/K2)."""

@@ -950,6 +950,22 @@ int b200ppf_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float 
     return prep_crop_pyramid(ctx, in, corners12, out, kept_host);
 }
 
+int b200ppf_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, size_t n_boxes,
+                          b200ppf_cloud **out) {
+    CHECK_CTX(ctx);
+    if (!in || !corners12 || !out) return fail_msg(ctx, B200PPF_ERR_INVALID, "crop: null argument");
+    if (n_boxes < 1 || n_boxes > 64) return fail_msg(ctx, B200PPF_ERR_INVALID, "crop: n_boxes must be in 1 .. 64");
+    for (size_t b = 0; b < n_boxes; ++b) out[b] = nullptr;
+    if (in->ctx != ctx) return fail_msg(ctx, B200PPF_ERR_INVALID, "crop: the cloud belongs to another context");
+    for (size_t k = 0; k < 12 * n_boxes; ++k)
+        if (!std::isfinite(corners12[k])) {
+            char msg[96];
+            snprintf(msg, sizeof(msg), "crop: box %zu: non-finite corner", k / 12);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+    return prep_crop_pyramids(ctx, in, corners12, n_boxes, out);
+}
+
 int b200ppf_debug_knn_host(const float *xyz, size_t n, size_t stride, int k, int mode, float cell_edge, const float *viewpoint3,
                            int cov_mode, uint32_t *idx, float *d2, float *mean_dist, float *normals4) {
     if ((n && !xyz) || stride < 3 || k < 1 || k > 128 || (size_t)k > std::max<size_t>(1, n) || mode < 0 || mode > 2 ||
@@ -970,6 +986,26 @@ int b200ppf_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200p
     if (params) p = *params;
     return k6_icp_refine(ctx, model, scene, p.max_iterations, p.tolerance, p.rejection_scale, p.num_levels, poses16,
                          n_poses, residuals, iterations);
+}
+
+int b200ppf_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_icp_params *params,
+                             uint64_t *iterations) {
+    CHECK_CTX(ctx);
+    if (n_jobs && !jobs) return fail_msg(ctx, B200PPF_ERR_INVALID, "icp batch: null jobs");
+    for (size_t j = 0; j < n_jobs; ++j) {
+        char msg[128];
+        const b200ppf_icp_job &jb = jobs[j];
+        const char *why = !jb.model || !jb.scene || (jb.n_poses && !jb.poses16) ? "null argument"
+                          : jb.model->ctx != ctx || jb.scene->ctx != ctx       ? "a cloud belongs to another context"
+                                                                                : nullptr;
+        if (why) {
+            snprintf(msg, sizeof(msg), "icp batch: job %zu: %s", j, why);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+    }
+    b200ppf_icp_params p = {100, 0.005f, 2.5f, 8};  // the reference's ICP(100, 0.005f, 2.5f, 8)
+    if (params) p = *params;
+    return k6_icp_refine_batch(ctx, jobs, n_jobs, p.max_iterations, p.tolerance, p.rejection_scale, p.num_levels, iterations);
 }
 
 int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_table *t,
@@ -1001,19 +1037,14 @@ struct OwnedCloud {  // intermediate clouds live until the call returns
     b200ppf_cloud *release() { b200ppf_cloud *r = c; c = nullptr; return r; }
 };
 
-// the pre-processing both per-object calls share: SceneCropping -> Subsampling -> OutlierProcessing -> NormalEstimation ->
-// EdgeExtraction (with_edges) -> PointCloudXYZNormalToMat, stage sizes and times into res
-int match_object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const float *corners12, float leaf, int sor_mean_k,
-                      double sor_stddev_mul, int normal_k, float edge_curvature, bool with_edges, b200ppf_object_result *res,
-                      OwnedCloud *object, OwnedCloud *edges) {
-    OwnedCloud cropped, sampled;
-    int rc = b200ppf_crop_pyramid(ctx, scene, corners12, &cropped.c, nullptr);
-    if (rc) return rc;
-    res->crop_ms = ctx->timings.prep_ms;
-    res->n_cropped = (uint32_t)cropped.c->n;
-    if (cropped.c->n == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match object: no scene point inside the box's frustum");
+// the pre-processing after the crop, shared by the per-object and the frame calls: Subsampling -> OutlierProcessing ->
+// NormalEstimation -> EdgeExtraction (with_edges) -> PointCloudXYZNormalToMat, stage sizes and times into res
+int object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *cropped, float leaf, int sor_mean_k, double sor_stddev_mul, int normal_k,
+                float edge_curvature, bool with_edges, b200ppf_object_result *res, OwnedCloud *object, OwnedCloud *edges) {
+    OwnedCloud sampled;
     const float leaf3[3] = {leaf, leaf, leaf};
-    if ((rc = b200ppf_voxel_grid(ctx, cropped.c, leaf3, &sampled.c))) return rc;
+    int rc;
+    if ((rc = b200ppf_voxel_grid(ctx, cropped, leaf3, &sampled.c))) return rc;
     res->voxel_ms = ctx->timings.prep_ms;
     res->n_sampled = (uint32_t)sampled.c->n;
     if ((rc = b200ppf_statistical_outlier_removal(ctx, sampled.c, sor_mean_k, sor_stddev_mul, &object->c, nullptr, nullptr, nullptr)))
@@ -1029,6 +1060,95 @@ int match_object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const float 
     }
     if ((rc = b200ppf_normalize_normals(ctx, object->c))) return rc;
     if (edges->c && (rc = b200ppf_normalize_normals(ctx, edges->c))) return rc;
+    return B200PPF_OK;
+}
+
+// SceneCropping, then the above: what both per-object calls run before matching
+int match_object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const float *corners12, float leaf, int sor_mean_k,
+                      double sor_stddev_mul, int normal_k, float edge_curvature, bool with_edges, b200ppf_object_result *res,
+                      OwnedCloud *object, OwnedCloud *edges) {
+    OwnedCloud cropped;
+    int rc = b200ppf_crop_pyramid(ctx, scene, corners12, &cropped.c, nullptr);
+    if (rc) return rc;
+    res->crop_ms = ctx->timings.prep_ms;
+    res->n_cropped = (uint32_t)cropped.c->n;
+    if (cropped.c->n == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match object: no scene point inside the box's frustum");
+    return object_prep(ctx, cropped.c, leaf, sor_mean_k, sor_stddev_mul, normal_k, edge_curvature, with_edges, res, object, edges);
+}
+
+// a CUDA or memory failure ends a frame call; any other failure of a box's chain is that box's status
+bool fatal(int rc) { return rc == B200PPF_ERR_CUDA || rc == B200PPF_ERR_NOMEM; }
+
+// One frame call: crop all boxes in one pass, run `match(b, object, edges, refined, residuals, &n_icp)` per box after its
+// pre-processing (it fills the box's result and returns its top poses), then one batched ICP over every box that reached
+// it.  models[b] is what box b's poses are refined against.
+template <class Match>
+int match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                const b200ppf_cloud *const *models, float leaf, int sor_mean_k, double sor_stddev_mul, int normal_k,
+                float edge_curvature, const b200ppf_icp_params &icp, b200ppf_object_result *results, int *status, Match match) {
+    const auto t0 = std::chrono::steady_clock::now();
+    for (size_t b = 0; b < n_boxes; ++b) {
+        memset(&results[b], 0, sizeof(results[b]));
+        status[b] = B200PPF_OK;
+    }
+    std::vector<OwnedCloud> crops(n_boxes), objects(n_boxes), edges(n_boxes);
+    {
+        std::vector<b200ppf_cloud *> out(n_boxes, nullptr);
+        const int rc = b200ppf_crop_pyramids(ctx, scene, corners12, n_boxes, out.data());
+        for (size_t b = 0; b < n_boxes; ++b) crops[b].c = out[b];
+        if (rc) return rc;
+    }
+    const float crop_ms = ctx->timings.prep_ms;
+    std::vector<std::vector<double>> refined(n_boxes), residuals(n_boxes);
+    std::vector<b200ppf_icp_job> jobs;
+    for (size_t b = 0; b < n_boxes; ++b) {
+        b200ppf_object_result *res = &results[b];
+        res->n_cropped = (uint32_t)crops[b].c->n;
+        int rc = B200PPF_OK;
+        size_t n_icp = 0;
+        if (crops[b].c->n == 0)
+            rc = fail_msg(ctx, B200PPF_ERR_STATE, "match frame: no scene point inside the box's frustum");
+        if (!rc)
+            rc = object_prep(ctx, crops[b].c, leaf, sor_mean_k, sor_stddev_mul, normal_k, edge_curvature, edge_curvature > 0.0f, res,
+                             &objects[b], &edges[b]);
+        b200ppf_cloud_free(crops[b].release());  // the frame's crops go back to the pool as soon as their box is through
+        if (!rc) rc = match(b, objects[b].c, edges[b].c, &refined[b], &residuals[b], &n_icp);
+        if (fatal(rc)) return rc;
+        status[b] = rc;
+        if (!rc && n_icp) jobs.push_back(b200ppf_icp_job{models[b], objects[b].c, refined[b].data(), n_icp, residuals[b].data()});
+    }
+    float icp_ms = 0.0f;
+    if (!jobs.empty()) {
+        if (int rc = b200ppf_icp_refine_batch(ctx, jobs.data(), jobs.size(), &icp, nullptr)) return rc;
+        icp_ms = ctx->timings.icp_ms;
+    }
+    const float wall = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    for (size_t b = 0; b < n_boxes; ++b) {
+        b200ppf_object_result *res = &results[b];
+        if (!status[b]) {
+            memcpy(res->pose, refined[b].data(), 16 * sizeof(double));  // resultsSub[0]
+            res->residual = residuals[b][0];
+        }
+        res->crop_ms = crop_ms;
+        res->icp_ms = jobs.empty() ? 0.0f : icp_ms;
+        res->total_wall_ms = wall;
+    }
+    return B200PPF_OK;
+}
+
+// the frame calls' argument checks shared by both engines
+int frame_args(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, const void *per_box,
+               const b200ppf_cloud *const *models, const b200ppf_object_result *results, const int *status) {
+    if (!scene || !corners12 || !per_box || !models || !results || !status)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "match frame: null argument");
+    if (n_boxes < 1 || n_boxes > 64) return fail_msg(ctx, B200PPF_ERR_INVALID, "match frame: n_boxes must be in 1 .. 64");
+    if (scene->ctx != ctx) return fail_msg(ctx, B200PPF_ERR_INVALID, "match frame: the scene belongs to another context");
+    for (size_t b = 0; b < n_boxes; ++b)
+        if (!models[b] || models[b]->ctx != ctx) {
+            char msg[128];
+            snprintf(msg, sizeof(msg), "match frame: box %zu: the model is NULL or belongs to another context", b);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
     return B200PPF_OK;
 }
 
@@ -1166,6 +1286,103 @@ int b200cv_match_object(b200cv_detector *d, const b200ppf_cloud *scene, const fl
     if (object_out) *object_out = object.release();
     if (edges_out) *edges_out = edges.release();
     return B200PPF_OK;
+}
+
+int b200cv_match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                       b200cv_detector *const *detectors, const b200ppf_cloud *const *models, const b200cv_object_params *params,
+                       b200ppf_object_result *results, int *status) {
+    CHECK_CTX(ctx);
+    if (int rc = frame_args(ctx, scene, n_boxes, corners12, detectors, models, results, status)) return rc;
+    for (size_t b = 0; b < n_boxes; ++b) {
+        char msg[128];
+        if (!detectors[b] || cv_detector_context(detectors[b]) != ctx) {
+            snprintf(msg, sizeof(msg), "cv match frame: box %zu: the detector is NULL or belongs to another context", b);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+        if (!cv_detector_trained(detectors[b])) {
+            snprintf(msg, sizeof(msg), "cv match frame: box %zu: the detector is not trained", b);
+            return fail_msg(ctx, B200PPF_ERR_STATE, msg);
+        }
+    }
+    b200cv_object_params p;
+    b200cv_object_params_default(&p);
+    if (params) p = *params;
+    if (p.use_edges && !(p.edge_curvature > 0.0f))
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match frame: Matching_S2B needs the edge cloud, edge_curvature must be positive");
+    const size_t cap = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
+    std::vector<b200cv_pose> poses(cap);
+    cudaEvent_t ev[2] = {nullptr, nullptr};  // the context's events are taken by the stages inside the match
+    PPF_CUDA(ctx, cudaEventCreate(&ev[0]));
+    if (cudaEventCreate(&ev[1]) != cudaSuccess) {
+        cudaEventDestroy(ev[0]);
+        return fail_msg(ctx, B200PPF_ERR_CUDA, "cv match frame: cudaEventCreate failed");
+    }
+    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *edges, std::vector<double> *refined,
+                     std::vector<double> *residuals, size_t *n_icp) {
+        b200ppf_object_result *res = &results[b];
+        if (p.use_edges && edges->n == 0)
+            return fail_msg(ctx, B200PPF_ERR_STATE, "cv match frame: the object has no edge point for Matching_S2B to pair with");
+        size_t n_clusters = 0;
+        cudaEventRecord(ev[0], ctx->stream);
+        int rc = b200cv_detector_match_cloud(detectors[b], object, p.use_edges ? edges : nullptr, p.relative_scene_sample_step,
+                                             p.relative_scene_distance, poses.data(), cap, &n_clusters);
+        cudaEventRecord(ev[1], ctx->stream);
+        if (rc == B200PPF_OK && cudaEventSynchronize(ev[1]) == cudaSuccess) cudaEventElapsedTime(&res->match_ms, ev[0], ev[1]);
+        if (rc) return rc;
+        res->n_poses = (uint32_t)n_clusters;
+        if (n_clusters == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match frame: the matching returned no pose");
+        *n_icp = std::min<size_t>(n_clusters, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
+        const size_t n_keep = std::max<size_t>(*n_icp, 1);
+        refined->resize(16 * n_keep);
+        residuals->assign(n_keep, 0.0);
+        for (size_t k = 0; k < n_keep; ++k) memcpy(refined->data() + 16 * k, poses[k].pose, 16 * sizeof(double));
+        res->votes = poses[0].num_votes;
+        return B200PPF_OK;
+    };
+    const int rc = match_frame(ctx, scene, n_boxes, corners12, models, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k,
+                               p.edge_curvature, p.icp, results, status, match);
+    cudaEventDestroy(ev[0]);
+    cudaEventDestroy(ev[1]);
+    return rc;
+}
+
+int b200ppf_match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                        const b200ppf_cloud *const *models, const b200ppf_table *const *tables, const b200ppf_object_params *params,
+                        b200ppf_object_result *results, int *status) {
+    CHECK_CTX(ctx);
+    if (int rc = frame_args(ctx, scene, n_boxes, corners12, tables, models, results, status)) return rc;
+    for (size_t b = 0; b < n_boxes; ++b)
+        if (!tables[b] || tables[b]->ctx != ctx) {
+            char msg[128];
+            snprintf(msg, sizeof(msg), "match frame: box %zu: the table is NULL or belongs to another context", b);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+    b200ppf_object_params p;
+    b200ppf_object_params_default(&p);
+    if (params) p = *params;
+    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *, std::vector<double> *refined,
+                     std::vector<double> *residuals, size_t *n_icp) {
+        b200ppf_object_result *res = &results[b];
+        float final16[16], poses16[3 * 16];
+        uint32_t votes[3] = {0, 0, 0};
+        size_t n_poses = 0;
+        if (int rc = b200ppf_register(ctx, models[b], tables[b], object, p.ref_rate, p.pos_thr, p.rot_thr, final16, poses16, votes,
+                                      &n_poses))
+            return rc;
+        b200ppf_timings tm;
+        b200ppf_get_timings(ctx, &tm);
+        res->match_ms = tm.grid_ms + tm.vote_ms + tm.pose_ms + tm.cluster_ms;
+        res->n_poses = (uint32_t)n_poses;
+        if (n_poses == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match frame: the matching returned no pose");
+        refined->resize(3 * 16);
+        residuals->assign(3, 0.0);
+        for (size_t k = 0; k < n_poses * 16; ++k) (*refined)[k] = (double)poses16[k];
+        *n_icp = std::min<size_t>(n_poses, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
+        res->votes = votes[0];
+        return B200PPF_OK;
+    };
+    return match_frame(ctx, scene, n_boxes, corners12, models, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k, p.edge_curvature,
+                       p.icp, results, status, match);
 }
 
 }  // extern "C"

@@ -12,6 +12,8 @@
 // One persistent thread-block CLUSTER (8 CTAs x 1024 threads, one SM each) per pose hypothesis runs the whole
 // refinement — every pyramid level and every iteration — in ONE launch: the reference refines its five best
 // poses, and an iteration is far too small (<= 20 k points) to be worth a kernel launch, let alone several.
+// Several jobs (models and scenes) share launches: every pose reads its clouds and scratch slices from a descriptor, and
+// the poses whose models want the same cluster size run in one launch (b200ppf_icp_refine_batch).
 // The samples are strided over the cluster; sums and histograms are combined through distributed shared
 // memory (every CTA adds the eight partials in rank order, so all of them hold bit-identical state and take
 // the same branches); cluster.sync() is the only inter-SM synchronisation.  FP64 is scarce on this part
@@ -28,6 +30,11 @@
 // -fmad=false), so the only differences are libm's double sin/cos and the order of the reductions.
 #include <cooperative_groups.h>
 
+#include <algorithm>
+#include <cstdlib>
+#include <utility>
+#include <vector>
+
 #include "ppf_common.cuh"
 
 namespace b200ppf {
@@ -43,16 +50,12 @@ constexpr int ICP_WARPS = ICP_THREADS / 32;
 constexpr uint32_t ICP_CELLS_MAX = 1u << 16;  // grid cells per level (scanned by the CTA)
 constexpr int NEQ = 29;                       // 21 (upper A) + 6 (b) + 1 (squared error) + 1 (matches)
 
-struct IcpArgs {
+// one pose of a launch: its clouds, and its slices of the call's scratch slab (sized by its own clouds)
+struct IcpPose {
     const float4 *mpos, *mnrm;
     const float4 *spos, *snrm;
     uint32_t n_model, n_scene;
-    int max_iterations, num_levels;
-    float tolerance, rejection_scale;
-    double *poses;       // [n_poses][16] in: start, out: refined
-    double *residuals;   // [n_poses]
-    unsigned long long *iterations;
-    // per-pose scratch (pose p uses slice p)
+    uint32_t slot;               // index of the pose in the call's poses / residuals
     float *src_norm, *dst_norm;  // [n_model][6], [n_scene][6]  normalised clouds
     float *src_t;                // [n_model][6]  level samples under the level's start pose
     float *moved;                // [n_model][3]
@@ -63,6 +66,15 @@ struct IcpArgs {
     uint32_t *cell_start;        // [ICP_CELLS_MAX + 1]
     uint32_t *cell_fill;         // [ICP_CELLS_MAX]
     float4 *items;               // [n_scene]  cell-sorted level scene samples {x, y, z, sample index}
+};
+
+struct IcpArgs {
+    const IcpPose *pose;  // [gridDim.y]: the cluster of blockIdx.y refines pose[blockIdx.y]
+    int max_iterations, num_levels;
+    float tolerance, rejection_scale;
+    double *poses;       // [n_poses][16] in: start, out: refined
+    double *residuals;   // [n_poses]
+    unsigned long long *iterations;
 };
 
 struct GridDev {  // any exact nearest-neighbour structure gives the same matches: the grid itself is fp32
@@ -341,21 +353,26 @@ __global__ void __launch_bounds__(ICP_THREADS, 1) icp_refine_kernel(const IcpArg
     __shared__ int s_flag, s_iter;
     __shared__ float s_bb[ICP_WARPS][6];
 
+    __shared__ IcpPose s_job;
+
     cg::cluster_group cluster = cg::this_cluster();
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t rank = cluster.block_rank(), csize = cluster.num_blocks();
     const uint32_t first = rank * ICP_THREADS + tid, stride = csize * ICP_THREADS;  // this thread's samples
-    const uint32_t p = blockIdx.y;
-    const uint32_t n = a.n_model, nd = a.n_scene;
-    float *src = a.src_norm + (size_t)p * n * 6, *dst = a.dst_norm + (size_t)p * nd * 6;
-    float *src_t = a.src_t + (size_t)p * n * 6, *moved = a.moved + (size_t)p * n * 3;
-    int *nn = a.nn + (size_t)p * n;
-    int *nn_prev = a.nn_prev + (size_t)p * n;
-    float *d2 = a.d2 + (size_t)p * n;
-    unsigned long long *winner = a.winner + (size_t)p * nd;
-    uint32_t *cell_start = a.cell_start + (size_t)p * (ICP_CELLS_MAX + 1);
-    uint32_t *cell_fill = a.cell_fill + (size_t)p * ICP_CELLS_MAX;
-    float4 *items = a.items + (size_t)p * nd;
+    if (tid == 0) s_job = a.pose[blockIdx.y];
+    __syncthreads();
+    const uint32_t p = s_job.slot;
+    const uint32_t n = s_job.n_model, nd = s_job.n_scene;
+    const float4 *const mpos = s_job.mpos, *const mnrm = s_job.mnrm, *const spos = s_job.spos, *const snrm = s_job.snrm;
+    float *src = s_job.src_norm, *dst = s_job.dst_norm;
+    float *src_t = s_job.src_t, *moved = s_job.moved;
+    int *nn = s_job.nn;
+    int *nn_prev = s_job.nn_prev;
+    float *d2 = s_job.d2;
+    unsigned long long *winner = s_job.winner;
+    uint32_t *cell_start = s_job.cell_start;
+    uint32_t *cell_fill = s_job.cell_fill;
+    float4 *items = s_job.items;
     double start_pose[16];
     for (int k = 0; k < 16; ++k) start_pose[k] = a.poses[(size_t)p * 16 + k];
 
@@ -363,7 +380,7 @@ __global__ void __launch_bounds__(ICP_THREADS, 1) icp_refine_kernel(const IcpArg
     double acc[NEQ];
     for (int k = 0; k < NEQ; ++k) acc[k] = 0.0;
     for (uint32_t i = first; i < n; i += stride) {
-        const float4 q = a.mpos[i], r = a.mnrm[i];
+        const float4 q = mpos[i], r = mnrm[i];
         const float in[6] = {q.x, q.y, q.z, r.x, r.y, r.z};
         float out[6];
         transform_point(start_pose, in, out, true);
@@ -373,7 +390,7 @@ __global__ void __launch_bounds__(ICP_THREADS, 1) icp_refine_kernel(const IcpArg
         acc[2] += out[2];
     }
     for (uint32_t i = first; i < nd; i += stride) {
-        const float4 q = a.spos[i], r = a.snrm[i];
+        const float4 q = spos[i], r = snrm[i];
         dst[6 * (size_t)i] = q.x;
         dst[6 * (size_t)i + 1] = q.y;
         dst[6 * (size_t)i + 2] = q.z;
@@ -780,18 +797,48 @@ __global__ void __launch_bounds__(ICP_THREADS, 1) icp_refine_kernel(const IcpArg
     }
 }
 
+// CTAs per pose cluster for a model of n points.  An iteration is a chain of ~20 cluster-wide synchronisations around little
+// arithmetic, so the cluster is only as large as the model needs: one CTA per 1 024 model points, at most ICP_CLUSTER (the
+// reference's 543-point bottle runs in a single CTA, whose cluster barrier is a block barrier).  The cluster size fixes the
+// order of the reductions, so a pose gives the same bits whatever else shares its launch.
+int icp_cluster_size(size_t n_model) {
+    int csize = 1;
+    while (csize < ICP_CLUSTER && (size_t)csize * ICP_THREADS < n_model) csize *= 2;
+    if (const char *e = getenv("B200PPF_ICP_CLUSTER")) csize = std::max(1, std::min(ICP_CLUSTER, atoi(e)));
+    return csize;
+}
+
 }  // namespace
 
-int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cloud *scene, int max_iterations,
-                  float tolerance, float rejection_scale, int num_levels, double *poses16_host, size_t n_poses,
-                  double *residuals_host, uint64_t *iterations_host) {
-    if (n_poses == 0) return B200PPF_OK;
-    if (n_poses > 65535) return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "icp: more than 65535 poses per call");
-    if (model->n == 0 || scene->n == 0) return fail_msg(ctx, B200PPF_ERR_INVALID, "icp: empty cloud");
+int k6_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, int max_iterations, float tolerance,
+                        float rejection_scale, int num_levels, uint64_t *iterations_host) {
+    char msg[160];
+    auto bad = [&](int code, size_t j, const char *what) {  // the single call's messages name no job
+        if (n_jobs == 1) snprintf(msg, sizeof(msg), "icp: %s", what);
+        else snprintf(msg, sizeof(msg), "icp: job %zu: %s", j, what);
+        return fail_msg(ctx, code, msg);
+    };
+    size_t P = 0;
+    for (size_t j = 0; j < n_jobs; ++j) {
+        if (jobs[j].n_poses == 0) continue;
+        if (jobs[j].n_poses > 65535) return bad(B200PPF_ERR_UNSUPPORTED, j, "more than 65535 poses per call");
+        if (jobs[j].model->n == 0 || jobs[j].scene->n == 0) return bad(B200PPF_ERR_INVALID, j, "empty cloud");
+        P += jobs[j].n_poses;
+    }
+    if (P == 0) return B200PPF_OK;
     if (max_iterations < 1 || num_levels < 1 || num_levels > 30 || !(tolerance >= 0.0f))
         return fail_msg(ctx, B200PPF_ERR_INVALID, "icp: bad parameters");
-    const size_t n = model->n, nd = scene->n, P = n_poses;
-    // one slab for all scratch
+    // one launch per cluster size, sizes ascending; within a launch the poses keep job order
+    std::vector<std::pair<int, size_t>> order;  // (cluster size, job)
+    for (size_t j = 0; j < n_jobs; ++j)
+        if (jobs[j].n_poses) order.push_back({icp_cluster_size(jobs[j].model->n), j});
+    std::stable_sort(order.begin(), order.end(), [](const auto &x, const auto &y) { return x.first < y.first; });
+    for (size_t g = 0, e = 0; g < order.size(); g = e) {
+        size_t poses = 0;
+        for (e = g; e < order.size() && order[e].first == order[g].first; ++e) poses += jobs[order[e].second].n_poses;
+        if (poses > 65535) return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "icp: more than 65535 poses of one cluster size per call");
+    }
+    // one slab for all scratch: the call's poses, residuals, iteration counter and descriptors, then each pose's slices
     size_t off = 0;
     auto take = [&](size_t bytes) {
         const size_t o = off;
@@ -799,21 +846,54 @@ int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cl
         return o;
     };
     const size_t o_poses = take(P * 16 * sizeof(double)), o_res = take(P * sizeof(double)), o_it = take(sizeof(unsigned long long));
-    const size_t o_src = take(P * n * 6 * sizeof(float)), o_dst = take(P * nd * 6 * sizeof(float));
-    const size_t o_srct = take(P * n * 6 * sizeof(float)), o_moved = take(P * n * 3 * sizeof(float));
-    const size_t o_nn = take(P * n * sizeof(int)), o_nnp = take(P * n * sizeof(int)), o_d2 = take(P * n * sizeof(float));
-    const size_t o_win = take(P * nd * sizeof(unsigned long long));
-    const size_t o_cs = take(P * (ICP_CELLS_MAX + 1) * sizeof(uint32_t)), o_cf = take(P * ICP_CELLS_MAX * sizeof(uint32_t));
-    const size_t o_items = take(P * nd * sizeof(float4));
+    const size_t o_desc = take(P * sizeof(IcpPose));
+    std::vector<size_t> job_first(n_jobs, 0), pose_off(P);  // first slot of each job; scratch offset of each slot
+    struct Slices {
+        size_t src, dst, srct, moved, nn, nnp, d2, win, cs, cf, items;
+    };
+    auto slices = [&](size_t n, size_t nd) {
+        Slices s;
+        s.src = take(n * 6 * sizeof(float)), s.dst = take(nd * 6 * sizeof(float));
+        s.srct = take(n * 6 * sizeof(float)), s.moved = take(n * 3 * sizeof(float));
+        s.nn = take(n * sizeof(int)), s.nnp = take(n * sizeof(int)), s.d2 = take(n * sizeof(float));
+        s.win = take(nd * sizeof(unsigned long long));
+        s.cs = take((ICP_CELLS_MAX + 1) * sizeof(uint32_t)), s.cf = take(ICP_CELLS_MAX * sizeof(uint32_t));
+        s.items = take(nd * sizeof(float4));
+        return s;
+    };
+    std::vector<Slices> sl(P);
+    for (size_t j = 0, slot = 0; j < n_jobs; ++j) {
+        job_first[j] = slot;
+        for (size_t k = 0; k < jobs[j].n_poses; ++k, ++slot) sl[slot] = slices(jobs[j].model->n, jobs[j].scene->n);
+    }
     StreamBuf<unsigned char> slab(ctx);
     PPF_CUDA(ctx, slab.alloc(off));
+    std::vector<IcpPose> desc;  // launch order
+    std::vector<double> poses(P * 16), residuals(P);
+    desc.reserve(P);
+    for (const auto &o : order) {
+        const b200ppf_icp_job &jb = jobs[o.second];
+        for (size_t k = 0; k < jb.n_poses; ++k) {
+            const size_t slot = job_first[o.second] + k;
+            const Slices &s = sl[slot];
+            IcpPose d;
+            d.mpos = jb.model->pos, d.mnrm = jb.model->nrm;
+            d.spos = jb.scene->pos, d.snrm = jb.scene->nrm;
+            d.n_model = (uint32_t)jb.model->n, d.n_scene = (uint32_t)jb.scene->n;
+            d.slot = (uint32_t)slot;
+            d.src_norm = reinterpret_cast<float *>(slab + s.src), d.dst_norm = reinterpret_cast<float *>(slab + s.dst);
+            d.src_t = reinterpret_cast<float *>(slab + s.srct), d.moved = reinterpret_cast<float *>(slab + s.moved);
+            d.nn = reinterpret_cast<int *>(slab + s.nn), d.nn_prev = reinterpret_cast<int *>(slab + s.nnp);
+            d.d2 = reinterpret_cast<float *>(slab + s.d2);
+            d.winner = reinterpret_cast<unsigned long long *>(slab + s.win);
+            d.cell_start = reinterpret_cast<uint32_t *>(slab + s.cs), d.cell_fill = reinterpret_cast<uint32_t *>(slab + s.cf);
+            d.items = reinterpret_cast<float4 *>(slab + s.items);
+            desc.push_back(d);
+        }
+    }
+    for (size_t j = 0; j < n_jobs; ++j)
+        if (jobs[j].n_poses) memcpy(poses.data() + 16 * job_first[j], jobs[j].poses16, jobs[j].n_poses * 16 * sizeof(double));
     IcpArgs a;
-    a.mpos = model->pos;
-    a.mnrm = model->nrm;
-    a.spos = scene->pos;
-    a.snrm = scene->nrm;
-    a.n_model = (uint32_t)n;
-    a.n_scene = (uint32_t)nd;
     a.max_iterations = max_iterations;
     a.num_levels = num_levels;
     a.tolerance = tolerance;
@@ -821,30 +901,20 @@ int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cl
     a.poses = reinterpret_cast<double *>(slab + o_poses);
     a.residuals = reinterpret_cast<double *>(slab + o_res);
     a.iterations = reinterpret_cast<unsigned long long *>(slab + o_it);
-    a.src_norm = reinterpret_cast<float *>(slab + o_src);
-    a.dst_norm = reinterpret_cast<float *>(slab + o_dst);
-    a.src_t = reinterpret_cast<float *>(slab + o_srct);
-    a.moved = reinterpret_cast<float *>(slab + o_moved);
-    a.nn = reinterpret_cast<int *>(slab + o_nn);
-    a.nn_prev = reinterpret_cast<int *>(slab + o_nnp);
-    a.d2 = reinterpret_cast<float *>(slab + o_d2);
-    a.winner = reinterpret_cast<unsigned long long *>(slab + o_win);
-    a.cell_start = reinterpret_cast<uint32_t *>(slab + o_cs);
-    a.cell_fill = reinterpret_cast<uint32_t *>(slab + o_cf);
-    a.items = reinterpret_cast<float4 *>(slab + o_items);
-    PPF_CUDA(ctx, cudaMemcpyAsync(a.poses, poses16_host, P * 16 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    IcpPose *d_desc = reinterpret_cast<IcpPose *>(slab + o_desc);
+    PPF_CUDA(ctx, cudaMemcpyAsync(a.poses, poses.data(), P * 16 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(d_desc, desc.data(), P * sizeof(IcpPose), cudaMemcpyHostToDevice, ctx->stream));
     PPF_CUDA(ctx, cudaMemsetAsync(a.iterations, 0, sizeof(unsigned long long), ctx->stream));
     cudaEventRecord(ctx->ev[0], ctx->stream);
-    {
-        // One cluster per pose: grid (csize, n_poses), cluster dimension (csize, 1, 1).  An iteration is a chain of ~20
-        // cluster-wide synchronisations around little arithmetic, so the cluster is only as large as the model needs:
-        // one CTA per 1 024 model points, at most ICP_CLUSTER (the reference's 543-point bottle runs in a single CTA,
-        // whose cluster barrier is a block barrier).
-        int csize = 1;
-        while (csize < ICP_CLUSTER && (size_t)csize * ICP_THREADS < model->n) csize *= 2;
-        if (const char *e = getenv("B200PPF_ICP_CLUSTER")) csize = std::max(1, std::min(ICP_CLUSTER, atoi(e)));
+    for (size_t g = 0, e = 0, first = 0; g < order.size(); g = e) {
+        // one cluster per pose: grid (csize, poses of this size), cluster dimension (csize, 1, 1)
+        const int csize = order[g].first;
+        size_t count = 0;
+        for (e = g; e < order.size() && order[e].first == csize; ++e) count += jobs[order[e].second].n_poses;
+        a.pose = d_desc + first;
+        first += count;
         cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)csize, (unsigned)P, 1);
+        cfg.gridDim = dim3((unsigned)csize, (unsigned)count, 1);
         cfg.blockDim = dim3(ICP_THREADS, 1, 1);
         cfg.dynamicSmemBytes = 0;
         cfg.stream = ctx->stream;
@@ -859,15 +929,26 @@ int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cl
         ctx->launches++;
     }
     cudaEventRecord(ctx->ev[1], ctx->stream);
-    PPF_CUDA(ctx, cudaMemcpyAsync(poses16_host, a.poses, P * 16 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    if (residuals_host)
-        PPF_CUDA(ctx, cudaMemcpyAsync(residuals_host, a.residuals, P * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(poses.data(), a.poses, P * 16 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(residuals.data(), a.residuals, P * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     unsigned long long it = 0;
     PPF_CUDA(ctx, cudaMemcpyAsync(&it, a.iterations, sizeof(it), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->timings.icp_ms, ctx->ev[0], ctx->ev[1]);
+    for (size_t j = 0; j < n_jobs; ++j) {
+        if (!jobs[j].n_poses) continue;
+        memcpy(jobs[j].poses16, poses.data() + 16 * job_first[j], jobs[j].n_poses * 16 * sizeof(double));
+        if (jobs[j].residuals) memcpy(jobs[j].residuals, residuals.data() + job_first[j], jobs[j].n_poses * sizeof(double));
+    }
     if (iterations_host) *iterations_host = it;
     return B200PPF_OK;
+}
+
+int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cloud *scene, int max_iterations,
+                  float tolerance, float rejection_scale, int num_levels, double *poses16_host, size_t n_poses,
+                  double *residuals_host, uint64_t *iterations_host) {
+    const b200ppf_icp_job job = {model, scene, poses16_host, n_poses, residuals_host};
+    return k6_icp_refine_batch(ctx, &job, 1, max_iterations, tolerance, rejection_scale, num_levels, iterations_host);
 }
 
 }  // namespace b200ppf

@@ -229,6 +229,9 @@ int k5_transform(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, const float *pose
 int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cloud *scene, int max_iterations,
                   float tolerance, float rejection_scale, int num_levels, double *poses16_host, size_t n_poses,
                   double *residuals_host, uint64_t *iterations_host);
+// the same for several (model, scene, poses) jobs: one launch per distinct cluster size, every pose as the single call
+int k6_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, int max_iterations, float tolerance,
+                        float rejection_scale, int num_levels, uint64_t *iterations_host);
 
 // the context of an OpenCV-engine detector and whether it holds a trained model (k7_cvppf.cu)
 b200ppf_ctx *cv_detector_context(const b200cv_detector *d);
@@ -250,6 +253,8 @@ int prep_renormalize(b200ppf_ctx *ctx, b200ppf_cloud *cloud);
 void prep_frustum_corners(const float *depth, int rows, int cols, int bx, int by, int bw, int bh, double fx, double fy,
                           double ppx, double ppy, float *corners12);
 int prep_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, b200ppf_cloud **out, uint32_t *kept_host);
+// the crop for n_boxes pyramids in one pass over the frame; out[b] as prep_crop_pyramid(corners12 + 12 * b) makes it
+int prep_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, size_t n_boxes, b200ppf_cloud **out);
 int prep_debug_knn_host(const float *xyz, size_t n, size_t stride, int k, int mode, float cell_edge, const float *viewpoint3,
                         int cov_mode, uint32_t *idx, float *d2, float *mean_dist, float *normals4);
 

@@ -26,6 +26,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <new>
+#include <string>
 #include <vector>
 
 #include "ppf_common.cuh"
@@ -44,10 +45,13 @@ flag_count_kernel(const uint32_t *__restrict__ flags, uint32_t n, uint32_t *__re
     if (threadIdx.x == 0) block_sums[blockIdx.x] = (uint32_t)c;
 }
 
+// block b of the grid scans row b: block_sums[b * n_blocks ...], total[b]
 __global__ void __launch_bounds__(SCAN_BLOCK)
 flag_scan_blocks_kernel(uint32_t *__restrict__ block_sums, uint32_t n_blocks, uint32_t *__restrict__ total) {
     __shared__ uint32_t warp_tot[32];
     __shared__ uint32_t carry;
+    block_sums += (size_t)blockIdx.x * n_blocks;
+    total += blockIdx.x;
     if (threadIdx.x == 0) carry = 0;
     __syncthreads();
     for (uint32_t base = 0; base < n_blocks; base += SCAN_BLOCK) {
@@ -667,16 +671,100 @@ struct PyramidPlanes {
     double d[5];
 };
 
-__global__ void __launch_bounds__(256)
-pyramid_flag_kernel(const float4 *__restrict__ pos, uint32_t n, PyramidPlanes pl, uint32_t *__restrict__ flags) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float4 p = pos[i];
+// the one inside test of both crops, so that a point falls the same way for a box alone and in a frame of boxes
+__device__ __forceinline__ bool pyramid_contains(const PyramidPlanes &pl, const float4 p) {
     const double x = p.x, y = p.y, z = p.z;
     bool in = true;
 #pragma unroll
     for (int f = 0; f < 5; ++f) in = in && (pl.n[f][0] * x + pl.n[f][1] * y + pl.n[f][2] * z <= pl.d[f]);
-    flags[i] = in ? 1u : 0u;
+    return in;
+}
+
+__global__ void __launch_bounds__(256)
+pyramid_flag_kernel(const float4 *__restrict__ pos, uint32_t n, PyramidPlanes pl, uint32_t *__restrict__ flags) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    flags[i] = pyramid_contains(pl, pos[i]) ? 1u : 0u;
+}
+
+// ---- P0 for up to 64 boxes: one tile of SCAN_BLOCK points per block ------------------------------------------
+constexpr int MAX_BOXES = 64;
+
+// membership mask of every point, the tile's count per box (counts[b * n_tiles + tile]) and each box's bounding box
+// (lo[3 * b ..], hi[3 * b ..] as order-preserving words): the bounds of a box's points are those of its cloud
+__global__ void __launch_bounds__(SCAN_BLOCK)
+pyramids_mask_kernel(const float4 *__restrict__ pos, uint32_t n, const PyramidPlanes *__restrict__ planes, int n_boxes,
+                     unsigned long long *__restrict__ mask, uint32_t *__restrict__ counts, uint32_t *__restrict__ lo,
+                     uint32_t *__restrict__ hi) {
+    __shared__ PyramidPlanes s_pl[MAX_BOXES];
+    __shared__ uint32_t s_cnt[MAX_BOXES], s_lo[MAX_BOXES][3], s_hi[MAX_BOXES][3];
+    for (int t = threadIdx.x; t < n_boxes * (int)(sizeof(PyramidPlanes) / sizeof(double)); t += SCAN_BLOCK)
+        reinterpret_cast<double *>(s_pl)[t] = reinterpret_cast<const double *>(planes)[t];
+    for (int b = threadIdx.x; b < n_boxes; b += SCAN_BLOCK) {
+        s_cnt[b] = 0;
+        for (int k = 0; k < 3; ++k) s_lo[b][k] = 0xFFFFFFFFu, s_hi[b][k] = 0u;
+    }
+    __syncthreads();
+    const uint32_t i = blockIdx.x * SCAN_BLOCK + threadIdx.x, lane = threadIdx.x & 31;
+    const float4 p = i < n ? pos[i] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    unsigned long long m = 0;
+    if (i < n)
+        for (int b = 0; b < n_boxes; ++b)
+            if (pyramid_contains(s_pl[b], p)) m |= 1ull << b;
+    if (i < n) mask[i] = m;
+    const uint32_t c[3] = {float_order(p.x), float_order(p.y), float_order(p.z)};
+    for (int b = 0; b < n_boxes; ++b) {
+        const bool in = (m >> b) & 1ull;
+        const uint32_t bal = __ballot_sync(0xFFFFFFFFu, in);
+        if (!bal) continue;  // warp-uniform
+        for (int k = 0; k < 3; ++k) {
+            const uint32_t l = __reduce_min_sync(0xFFFFFFFFu, in ? c[k] : 0xFFFFFFFFu);
+            const uint32_t h = __reduce_max_sync(0xFFFFFFFFu, in ? c[k] : 0u);
+            if (lane == 0) atomicMin(&s_lo[b][k], l), atomicMax(&s_hi[b][k], h);
+        }
+        if (lane == 0) atomicAdd(&s_cnt[b], (uint32_t)__popc(bal));
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b < n_boxes; b += SCAN_BLOCK) {
+        counts[(size_t)b * gridDim.x + blockIdx.x] = s_cnt[b];
+        if (s_cnt[b])
+            for (int k = 0; k < 3; ++k) atomicMin(lo + 3 * b + k, s_lo[b][k]), atomicMax(hi + 3 * b + k, s_hi[b][k]);
+    }
+}
+
+// every point into each of its boxes' clouds at (scanned tile offset + rank in the tile): input order, as compaction
+// keeps it.  out[b] / out[n_boxes + b] are cloud b's pos / nrm arrays.
+__global__ void __launch_bounds__(SCAN_BLOCK)
+pyramids_scatter_kernel(const float4 *__restrict__ pos, const float4 *__restrict__ nrm, uint32_t n,
+                        const unsigned long long *__restrict__ mask, int n_boxes, const uint32_t *__restrict__ tile_off,
+                        float4 *const *__restrict__ out) {
+    __shared__ uint32_t s_warp[MAX_BOXES][32];  // box b: points of warps before w in this tile
+    const uint32_t i = blockIdx.x * SCAN_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned long long m = i < n ? mask[i] : 0ull;
+    for (int b = 0; b < n_boxes; ++b) {
+        const uint32_t bal = __ballot_sync(0xFFFFFFFFu, (m >> b) & 1ull);
+        if (lane == 0) s_warp[b][warp] = (uint32_t)__popc(bal);
+    }
+    __syncthreads();
+    for (uint32_t t = threadIdx.x; t < (uint32_t)n_boxes * 32; t += SCAN_BLOCK) {  // one warp per box row: exclusive scan
+        const uint32_t v = s_warp[t >> 5][lane];
+        uint32_t incl = v;
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+            if (lane >= (uint32_t)o) incl += u;
+        }
+        s_warp[t >> 5][lane] = incl - v;
+    }
+    __syncthreads();
+    const float4 p = m ? pos[i] : make_float4(0.0f, 0.0f, 0.0f, 0.0f), q = m ? nrm[i] : p;
+    for (int b = 0; b < n_boxes; ++b) {
+        const bool in = (m >> b) & 1ull;
+        const uint32_t bal = __ballot_sync(0xFFFFFFFFu, in);
+        if (!in) continue;
+        const uint32_t r = tile_off[(size_t)b * gridDim.x + blockIdx.x] + s_warp[b][warp] + __popc(bal & ((1u << lane) - 1u));
+        out[b][r] = p;
+        out[n_boxes + b][r] = q;
+    }
 }
 
 // ---- P6 ---------------------------------------------------------------------------------------------------------
@@ -940,7 +1028,10 @@ void prep_frustum_corners(const float *depth, int rows, int cols, int bx, int by
     }
 }
 
-int prep_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, b200ppf_cloud **out, uint32_t *kept_host) {
+namespace {
+
+// the five half-spaces of the pyramid {origin, four corners}; 0, or B200PPF_ERR_* with the reason in *why
+int pyramid_planes(const float *corners12, PyramidPlanes *pl, const char **why) {
     double c[4][3], m[3] = {0, 0, 0};
     for (int i = 0; i < 4; ++i)
         for (int k = 0; k < 3; ++k) c[i][k] = corners12[3 * i + k], m[k] += 0.25 * corners12[3 * i + k];
@@ -950,27 +1041,40 @@ int prep_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *co
         o[2] = a[0] * b[1] - a[1] * b[0];
     };
     auto dot = [](const double *a, const double *b) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; };
-    PyramidPlanes pl;
     const int cyc[4] = {0, 1, 3, 2};  // left_top -> left_bot -> right_bot -> right_top
     for (int s = 0; s < 4; ++s) {  // side faces contain the apex (the origin): d = 0; the corners' centroid is inside
-        cross(c[cyc[s]], c[cyc[(s + 1) & 3]], pl.n[s]);
-        if (dot(pl.n[s], m) > 0)
-            for (int k = 0; k < 3; ++k) pl.n[s][k] = -pl.n[s][k];
-        pl.d[s] = 0.0;
+        cross(c[cyc[s]], c[cyc[(s + 1) & 3]], pl->n[s]);
+        if (dot(pl->n[s], m) > 0)
+            for (int k = 0; k < 3; ++k) pl->n[s][k] = -pl->n[s][k];
+        pl->d[s] = 0.0;
     }
     double e1[3], e2[3];
     for (int k = 0; k < 3; ++k) e1[k] = c[1][k] - c[0][k], e2[k] = c[2][k] - c[0][k];
-    cross(e1, e2, pl.n[4]);
-    pl.d[4] = dot(pl.n[4], c[0]);
-    if (pl.d[4] < 0) {  // the apex is inside
-        for (int k = 0; k < 3; ++k) pl.n[4][k] = -pl.n[4][k];
-        pl.d[4] = -pl.d[4];
+    cross(e1, e2, pl->n[4]);
+    pl->d[4] = dot(pl->n[4], c[0]);
+    if (pl->d[4] < 0) {  // the apex is inside
+        for (int k = 0; k < 3; ++k) pl->n[4][k] = -pl->n[4][k];
+        pl->d[4] = -pl->d[4];
     }
-    const double nn = std::sqrt(dot(pl.n[4], pl.n[4]));
-    if (!(nn > 0.0) || !(pl.d[4] > 0.0)) return fail_msg(ctx, B200PPF_ERR_INVALID, "crop: the four corners do not span a base in front of the camera");
+    const double nn = std::sqrt(dot(pl->n[4], pl->n[4]));
+    if (!(nn > 0.0) || !(pl->d[4] > 0.0)) {
+        *why = "the four corners do not span a base in front of the camera";
+        return B200PPF_ERR_INVALID;
+    }
     // the reference's corners share one z; a base that is not planar would make the hull a different solid
-    if (std::fabs(dot(pl.n[4], c[3]) - pl.d[4]) > 1e-6 * nn * (std::fabs(c[3][0]) + std::fabs(c[3][1]) + std::fabs(c[3][2]) + 1.0))
-        return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "crop: the four corners are not coplanar");
+    if (std::fabs(dot(pl->n[4], c[3]) - pl->d[4]) > 1e-6 * nn * (std::fabs(c[3][0]) + std::fabs(c[3][1]) + std::fabs(c[3][2]) + 1.0)) {
+        *why = "the four corners are not coplanar";
+        return B200PPF_ERR_UNSUPPORTED;
+    }
+    return B200PPF_OK;
+}
+
+}  // namespace
+
+int prep_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, b200ppf_cloud **out, uint32_t *kept_host) {
+    PyramidPlanes pl;
+    const char *why = nullptr;
+    if (int rc = pyramid_planes(corners12, &pl, &why)) return fail_msg(ctx, rc, (std::string("crop: ") + why).c_str());
     const uint32_t n = (uint32_t)in->n;
     StreamBuf<uint32_t> flags(ctx);
     PPF_CUDA(ctx, flags.alloc(n));
@@ -979,6 +1083,60 @@ int prep_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *co
     int rc = compact_cloud(ctx, in, flags, out, kept_host);
     timer.stop();
     return rc;
+}
+
+int prep_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, size_t n_boxes, b200ppf_cloud **out) {
+    std::vector<PyramidPlanes> pl(n_boxes);
+    for (size_t b = 0; b < n_boxes; ++b) {
+        const char *why = nullptr;
+        if (int rc = pyramid_planes(corners12 + 12 * b, &pl[b], &why)) {
+            char msg[160];
+            snprintf(msg, sizeof(msg), "crop: box %zu: %s", b, why);
+            return fail_msg(ctx, rc, msg);
+        }
+    }
+    const uint32_t n = (uint32_t)in->n, K = (uint32_t)n_boxes, T = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    // scratch: planes, masks, tile counts (box-major, scanned in place), and the words read back: K totals, 6K bounds
+    StreamBuf<PyramidPlanes> d_pl(ctx);
+    StreamBuf<unsigned long long> mask(ctx);
+    StreamBuf<uint32_t> counts(ctx), back(ctx);
+    StreamBuf<float4 *> d_out(ctx);
+    PPF_CUDA(ctx, d_pl.alloc(K));
+    PPF_CUDA(ctx, mask.alloc(n));
+    PPF_CUDA(ctx, counts.alloc((size_t)K * T));
+    PPF_CUDA(ctx, back.alloc(7 * (size_t)K));
+    PPF_CUDA(ctx, d_out.alloc(2 * (size_t)K));
+    uint32_t *d_tot = back, *d_lo = back + K, *d_hi = back + 4 * K;
+    EventTimer timer(ctx);
+    PPF_CUDA(ctx, cudaMemcpyAsync(d_pl, pl.data(), K * sizeof(PyramidPlanes), cudaMemcpyHostToDevice, ctx->stream));
+    PPF_CUDA(ctx, cudaMemsetAsync(d_tot, 0, K * sizeof(uint32_t), ctx->stream));
+    PPF_CUDA(ctx, cudaMemsetAsync(d_lo, 0xFF, 3 * K * sizeof(uint32_t), ctx->stream));
+    PPF_CUDA(ctx, cudaMemsetAsync(d_hi, 0x00, 3 * K * sizeof(uint32_t), ctx->stream));
+    if (n) {
+        PPF_LAUNCH(ctx, pyramids_mask_kernel, T, SCAN_BLOCK, 0, in->pos, n, d_pl, (int)K, mask, counts, d_lo, d_hi);
+        PPF_LAUNCH(ctx, flag_scan_blocks_kernel, K, SCAN_BLOCK, 0, counts, T, d_tot);
+    }
+    std::vector<uint32_t> h(7 * (size_t)K);
+    PPF_CUDA(ctx, cudaMemcpyAsync(h.data(), back, h.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the one wait: the clouds are sized by the counts
+    std::vector<CloudPtr> c(K);
+    std::vector<float4 *> ptrs(2 * (size_t)K);
+    for (uint32_t b = 0; b < K; ++b) {
+        if (int rc = cloud_alloc(ctx, h[b], &c[b])) return rc;
+        for (int k = 0; k < 3; ++k) {  // cloud_bbox_from_device's values: exact bounds, zeros for an empty cloud
+            c[b]->bbox_min[k] = h[b] ? float_unorder(h[K + 3 * b + k]) : 0.0f;
+            c[b]->bbox_max[k] = h[b] ? float_unorder(h[4 * K + 3 * b + k]) : 0.0f;
+        }
+        ptrs[b] = c[b]->pos;
+        ptrs[K + b] = c[b]->nrm;
+    }
+    if (n) {
+        PPF_CUDA(ctx, cudaMemcpyAsync(d_out, ptrs.data(), ptrs.size() * sizeof(float4 *), cudaMemcpyHostToDevice, ctx->stream));
+        PPF_LAUNCH(ctx, pyramids_scatter_kernel, T, SCAN_BLOCK, 0, in->pos, in->nrm, n, mask, (int)K, counts, d_out);
+    }
+    timer.stop();
+    for (uint32_t b = 0; b < K; ++b) out[b] = c[b].release();
+    return B200PPF_OK;
 }
 
 int prep_renormalize(b200ppf_ctx *ctx, b200ppf_cloud *cloud) {
