@@ -1,10 +1,11 @@
 """GPU tests of the frame calls: every box of a frame in one call (b200ppf_crop_pyramids, b200ppf_icp_refine_batch,
-b200cv_match_frame, b200ppf_match_frame).
+b200cv_match_frame, b200ppf_match_frame), and of the per-object calls as frames of one box.
 
 Bars: the multi-box crop equals one crop per box bit for bit (rows, order, bounding box); the batched ICP equals one
 icp_refine per job bit for bit (poses, residuals, summed iterations) with one launch per distinct cluster size; a frame call
 equals the per-object calls box by box in every result field but the times; a failed box leaves the others as they would
-be alone; errors of the call itself leave the default pool's used-memory counter where it was.
+be alone; errors of the call itself leave the default pool's used-memory counter where it was; a per-object call keeps its
+own edge rule (edges for edges_out, or for Matching_S2B) and rejects handles of another context.
 """
 import ctypes
 import gc
@@ -389,3 +390,60 @@ def test_c_abi_multi_box_example(tmp_path, ctx, scene_full, bottle, reference):
         assert v[:3] == ["box", str(i), "0"] and status[i] == 0
         assert int(v[3]) == res[i]["votes"] and int(v[4]) == res[i]["n_poses"] and float(v[5]) == res[i]["residual"]
         assert np.array_equal(np.array([float(x) for x in v[6:]]), res[i]["pose"].reshape(16))
+
+
+# ---- 9. the per-object calls: a frame of one box, plus its clouds ------------------------------------------------------
+def _object_call(ctx, call, params_cls, default_fn, edges_out, **over):
+    """a per-object call through ctypes with edges_out passed or NULL (Context's wrappers always pass both)
+    -> (result dict, whether an edge cloud was handed out)"""
+    from yolo_ppf_pose_estimation_b200 import capi
+    prm = ctx._params(params_cls, default_fn, over)
+    res = capi.ObjectResult()
+    obj, edg = ctypes.c_void_p(), ctypes.c_void_p()
+    ctx.check(call(ctypes.byref(prm), ctypes.byref(res), ctypes.byref(obj), ctypes.byref(edg) if edges_out else None))
+    got_edges = bool(edg.value)
+    _free([capi.Cloud(ctx, h) for h in (obj, edg) if h.value])
+    return ctx._result(res), got_edges
+
+
+def _edges_only_when_asked(ctx, call, params_cls, default_fn, **over):
+    """edge_curvature > 0 and no engine need for the edges: they are extracted for edges_out only, and the rest of the
+    result does not depend on them"""
+    asked, got = _object_call(ctx, call, params_cls, default_fn, True, **over)
+    plain, none = _object_call(ctx, call, params_cls, default_fn, False, **over)
+    assert got and asked["n_edges"] > 0
+    assert not none and plain["n_edges"] == 0 and plain["edges_ms"] == 0.0
+    assert plain["pose"].tobytes() == asked["pose"].tobytes()
+    for f in ("residual", "votes", "n_poses", "n_cropped", "n_sampled", "n_filtered"):
+        assert plain[f] == asked[f], f
+
+
+def test_match_object_extracts_edges_for_edges_out_only(ctx, reference):
+    from yolo_ppf_pose_estimation_b200 import capi
+    r, lib = reference, capi.lib()
+    table = ctx.table_build_from_cloud(r["model"], ANGLE_STEP, DIST_STEP)
+    c12 = np.ascontiguousarray(r["cor"], np.float32).reshape(12)
+    _edges_only_when_asked(ctx, lambda *a: lib.b200ppf_match_object(ctx._h, r["scene"]._h, c12.ctypes.data, r["model"]._h, table._h, *a),
+                           capi.ObjectParams, lib.b200ppf_object_params_default, leaf=0.01, ref_rate=5)
+
+
+def test_cv_match_object_without_s2b_extracts_edges_for_edges_out_only(ctx, reference):
+    from yolo_ppf_pose_estimation_b200 import capi
+    r, lib = reference, capi.lib()
+    c12 = np.ascontiguousarray(r["cor"], np.float32).reshape(12)
+    _edges_only_when_asked(ctx, lambda *a: lib.b200cv_match_object(r["det"]._h, r["scene"]._h, c12.ctypes.data, r["model"]._h, *a),
+                           capi.CvObjectParams, lib.b200cv_object_params_default, leaf=0.01, use_edges=0,
+                           relative_scene_sample_step=1.0 / 14.0)
+
+
+def test_match_object_rejects_handles_of_another_context(ctx, reference, scene_full, bottle):
+    from yolo_ppf_pose_estimation_b200 import capi
+    r = reference
+    table = ctx.table_build_from_cloud(r["model"], ANGLE_STEP, DIST_STEP)
+    other = capi.Context(0)
+    f_scene, f_model = other.upload_xyz(scene_full[:, :3]), other.upload_cloud(bottle)
+    f_table = other.table_build_from_cloud(f_model, ANGLE_STEP, DIST_STEP)
+    assert _code(lambda: ctx.match_object(f_scene, r["cor"], r["model"], table, leaf=0.01)) == INVALID
+    assert _code(lambda: ctx.match_object(r["scene"], r["cor"], f_model, table, leaf=0.01)) == INVALID
+    assert _code(lambda: ctx.match_object(r["scene"], r["cor"], r["model"], f_table, leaf=0.01)) == INVALID
+    other.close()

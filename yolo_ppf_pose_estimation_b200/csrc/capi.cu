@@ -63,6 +63,9 @@ using namespace b200ppf;
     if (!(ctx)) return fail_msg(nullptr, B200PPF_ERR_INVALID, "null context"); \
     DeviceGuard _guard((ctx)->device)
 
+// the reference's ICP(100, 0.005f, 2.5f, 8): the default of both ICP calls and of both per-object parameter blocks
+constexpr b200ppf_icp_params ICP_DEFAULT = {100, 0.005f, 2.5f, 8};
+
 extern "C" {
 
 int b200ppf_version(void) { return B200PPF_VERSION; }
@@ -982,8 +985,7 @@ int b200ppf_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200p
     CHECK_CTX(ctx);
     if (!model || !scene || (n_poses && !poses16)) return fail_msg(ctx, B200PPF_ERR_INVALID, "icp: null argument");
     DeviceGuard guard(ctx->device);
-    b200ppf_icp_params p = {100, 0.005f, 2.5f, 8};  // the reference's ICP(100, 0.005f, 2.5f, 8)
-    if (params) p = *params;
+    const b200ppf_icp_params p = params ? *params : ICP_DEFAULT;
     return k6_icp_refine(ctx, model, scene, p.max_iterations, p.tolerance, p.rejection_scale, p.num_levels, poses16,
                          n_poses, residuals, iterations);
 }
@@ -1003,8 +1005,7 @@ int b200ppf_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size
             return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
         }
     }
-    b200ppf_icp_params p = {100, 0.005f, 2.5f, 8};  // the reference's ICP(100, 0.005f, 2.5f, 8)
-    if (params) p = *params;
+    const b200ppf_icp_params p = params ? *params : ICP_DEFAULT;
     return k6_icp_refine_batch(ctx, jobs, n_jobs, p.max_iterations, p.tolerance, p.rejection_scale, p.num_levels, iterations);
 }
 
@@ -1031,71 +1032,58 @@ int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf
 
 namespace {
 
-struct OwnedCloud {  // intermediate clouds live until the call returns
-    b200ppf_cloud *c = nullptr;
-    ~OwnedCloud() { if (c) b200ppf_cloud_free(c); }
-    b200ppf_cloud *release() { b200ppf_cloud *r = c; c = nullptr; return r; }
-};
-
-// the pre-processing after the crop, shared by the per-object and the frame calls: Subsampling -> OutlierProcessing ->
-// NormalEstimation -> EdgeExtraction (with_edges) -> PointCloudXYZNormalToMat, stage sizes and times into res
-int object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *cropped, float leaf, int sor_mean_k, double sor_stddev_mul, int normal_k,
-                float edge_curvature, bool with_edges, b200ppf_object_result *res, OwnedCloud *object, OwnedCloud *edges) {
-    OwnedCloud sampled;
-    const float leaf3[3] = {leaf, leaf, leaf};
-    int rc;
-    if ((rc = b200ppf_voxel_grid(ctx, cropped, leaf3, &sampled.c))) return rc;
+// the pre-processing after the crop: Subsampling -> OutlierProcessing -> NormalEstimation -> EdgeExtraction (with_edges) ->
+// PointCloudXYZNormalToMat, stage sizes and times into res
+template <class Params>
+int object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *cropped, const Params &p, bool with_edges, b200ppf_object_result *res,
+                CloudPtr *object, CloudPtr *edges) {
+    const float leaf3[3] = {p.leaf, p.leaf, p.leaf};
+    b200ppf_cloud *sampled_c = nullptr, *object_c = nullptr, *edges_c = nullptr;  // each owned once its call returns
+    int rc = b200ppf_voxel_grid(ctx, cropped, leaf3, &sampled_c);
+    const CloudPtr sampled(sampled_c);
+    if (rc) return rc;
     res->voxel_ms = ctx->timings.prep_ms;
-    res->n_sampled = (uint32_t)sampled.c->n;
-    if ((rc = b200ppf_statistical_outlier_removal(ctx, sampled.c, sor_mean_k, sor_stddev_mul, &object->c, nullptr, nullptr, nullptr)))
-        return rc;
+    res->n_sampled = (uint32_t)sampled->n;
+    rc = b200ppf_statistical_outlier_removal(ctx, sampled.get(), p.sor_mean_k, p.sor_stddev_mul, &object_c, nullptr, nullptr, nullptr);
+    object->reset(object_c);
+    if (rc) return rc;
     res->outlier_ms = ctx->timings.prep_ms;
-    res->n_filtered = (uint32_t)object->c->n;
-    if ((rc = b200ppf_normal_estimation(ctx, object->c, normal_k, nullptr, B200PPF_COVARIANCE_SHIFTED))) return rc;
+    res->n_filtered = (uint32_t)object_c->n;
+    if ((rc = b200ppf_normal_estimation(ctx, object_c, p.normal_k, nullptr, B200PPF_COVARIANCE_SHIFTED))) return rc;
     res->normals_ms = ctx->timings.prep_ms;
     if (with_edges) {
-        if ((rc = b200ppf_curvature_edges(ctx, object->c, edge_curvature, &edges->c))) return rc;
+        rc = b200ppf_curvature_edges(ctx, object_c, p.edge_curvature, &edges_c);
+        edges->reset(edges_c);
+        if (rc) return rc;
         res->edges_ms = ctx->timings.prep_ms;
-        res->n_edges = (uint32_t)edges->c->n;
+        res->n_edges = (uint32_t)edges_c->n;
     }
-    if ((rc = b200ppf_normalize_normals(ctx, object->c))) return rc;
-    if (edges->c && (rc = b200ppf_normalize_normals(ctx, edges->c))) return rc;
+    if ((rc = b200ppf_normalize_normals(ctx, object_c))) return rc;
+    if (edges_c && (rc = b200ppf_normalize_normals(ctx, edges_c))) return rc;
     return B200PPF_OK;
 }
 
-// SceneCropping, then the above: what both per-object calls run before matching
-int match_object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const float *corners12, float leaf, int sor_mean_k,
-                      double sor_stddev_mul, int normal_k, float edge_curvature, bool with_edges, b200ppf_object_result *res,
-                      OwnedCloud *object, OwnedCloud *edges) {
-    OwnedCloud cropped;
-    int rc = b200ppf_crop_pyramid(ctx, scene, corners12, &cropped.c, nullptr);
-    if (rc) return rc;
-    res->crop_ms = ctx->timings.prep_ms;
-    res->n_cropped = (uint32_t)cropped.c->n;
-    if (cropped.c->n == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match object: no scene point inside the box's frustum");
-    return object_prep(ctx, cropped.c, leaf, sor_mean_k, sor_stddev_mul, normal_k, edge_curvature, with_edges, res, object, edges);
-}
-
-// a CUDA or memory failure ends a frame call; any other failure of a box's chain is that box's status
+// a CUDA or memory failure ends a call; any other failure of a box's chain is that box's status
 bool fatal(int rc) { return rc == B200PPF_ERR_CUDA || rc == B200PPF_ERR_NOMEM; }
 
-// One frame call: crop all boxes in one pass, run `match(b, object, edges, refined, residuals, &n_icp)` per box after its
-// pre-processing (it fills the box's result and returns its top poses), then one batched ICP over every box that reached
-// it.  models[b] is what box b's poses are refined against.
-template <class Match>
-int match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
-                const b200ppf_cloud *const *models, float leaf, int sor_mean_k, double sor_stddev_mul, int normal_k,
-                float edge_curvature, const b200ppf_icp_params &icp, b200ppf_object_result *results, int *status, Match match) {
+// The chain of every match call, frame or per-object: crop all boxes in one pass, then per box the pre-processing and
+// `match(b, object, edges, &poses)`, the engine's matching step (it fills the box's match_ms, n_poses and votes and returns
+// its best poses, 16 doubles each, most-voted first), then one batched ICP of the top icp_poses poses of every box that
+// reached it against models[b].  When box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
+template <class Params, class Match>
+int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                const b200ppf_cloud *const *models, const Params &p, bool with_edges, b200ppf_object_result *results, int *status,
+                b200ppf_cloud **object_out, b200ppf_cloud **edges_out, Match match) {
     const auto t0 = std::chrono::steady_clock::now();
     for (size_t b = 0; b < n_boxes; ++b) {
         memset(&results[b], 0, sizeof(results[b]));
         status[b] = B200PPF_OK;
     }
-    std::vector<OwnedCloud> crops(n_boxes), objects(n_boxes), edges(n_boxes);
+    std::vector<CloudPtr> crops(n_boxes), objects(n_boxes), edges(n_boxes);
     {
         std::vector<b200ppf_cloud *> out(n_boxes, nullptr);
         const int rc = b200ppf_crop_pyramids(ctx, scene, corners12, n_boxes, out.data());
-        for (size_t b = 0; b < n_boxes; ++b) crops[b].c = out[b];
+        for (size_t b = 0; b < n_boxes; ++b) crops[b].reset(out[b]);
         if (rc) return rc;
     }
     const float crop_ms = ctx->timings.prep_ms;
@@ -1103,23 +1091,24 @@ int match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
     std::vector<b200ppf_icp_job> jobs;
     for (size_t b = 0; b < n_boxes; ++b) {
         b200ppf_object_result *res = &results[b];
-        res->n_cropped = (uint32_t)crops[b].c->n;
+        res->n_cropped = (uint32_t)crops[b]->n;
         int rc = B200PPF_OK;
-        size_t n_icp = 0;
-        if (crops[b].c->n == 0)
-            rc = fail_msg(ctx, B200PPF_ERR_STATE, "match frame: no scene point inside the box's frustum");
-        if (!rc)
-            rc = object_prep(ctx, crops[b].c, leaf, sor_mean_k, sor_stddev_mul, normal_k, edge_curvature, edge_curvature > 0.0f, res,
-                             &objects[b], &edges[b]);
-        b200ppf_cloud_free(crops[b].release());  // the frame's crops go back to the pool as soon as their box is through
-        if (!rc) rc = match(b, objects[b].c, edges[b].c, &refined[b], &residuals[b], &n_icp);
+        if (crops[b]->n == 0) rc = fail_msg(ctx, B200PPF_ERR_STATE, "match: no scene point inside the box's frustum");
+        if (!rc) rc = object_prep(ctx, crops[b].get(), p, with_edges, res, &objects[b], &edges[b]);
+        crops[b].reset();  // the frame's crops go back to the pool as soon as their box is through
+        if (!rc) rc = match(b, objects[b].get(), edges[b].get(), &refined[b]);
+        if (!rc && res->n_poses == 0)  // the reference exits there, :502-507
+            rc = fail_msg(ctx, B200PPF_ERR_STATE, "match: the matching returned no pose");
         if (fatal(rc)) return rc;
         status[b] = rc;
-        if (!rc && n_icp) jobs.push_back(b200ppf_icp_job{models[b], objects[b].c, refined[b].data(), n_icp, residuals[b].data()});
+        if (rc) continue;
+        const size_t n_icp = std::min<size_t>(res->n_poses, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
+        residuals[b].assign(std::max<size_t>(n_icp, 1), 0.0);
+        if (n_icp) jobs.push_back(b200ppf_icp_job{models[b], objects[b].get(), refined[b].data(), n_icp, residuals[b].data()});
     }
     float icp_ms = 0.0f;
     if (!jobs.empty()) {
-        if (int rc = b200ppf_icp_refine_batch(ctx, jobs.data(), jobs.size(), &icp, nullptr)) return rc;
+        if (int rc = b200ppf_icp_refine_batch(ctx, jobs.data(), jobs.size(), &p.icp, nullptr)) return rc;
         icp_ms = ctx->timings.icp_ms;
     }
     const float wall = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1130,26 +1119,122 @@ int match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
             res->residual = residuals[b][0];
         }
         res->crop_ms = crop_ms;
-        res->icp_ms = jobs.empty() ? 0.0f : icp_ms;
+        res->icp_ms = icp_ms;
         res->total_wall_ms = wall;
+    }
+    if (!status[0]) {
+        if (object_out) *object_out = objects[0].release();
+        if (edges_out) *edges_out = edges[0].release();
     }
     return B200PPF_OK;
 }
 
-// the frame calls' argument checks shared by both engines
+// the argument checks both engines share
 int frame_args(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, const void *per_box,
                const b200ppf_cloud *const *models, const b200ppf_object_result *results, const int *status) {
     if (!scene || !corners12 || !per_box || !models || !results || !status)
-        return fail_msg(ctx, B200PPF_ERR_INVALID, "match frame: null argument");
-    if (n_boxes < 1 || n_boxes > 64) return fail_msg(ctx, B200PPF_ERR_INVALID, "match frame: n_boxes must be in 1 .. 64");
-    if (scene->ctx != ctx) return fail_msg(ctx, B200PPF_ERR_INVALID, "match frame: the scene belongs to another context");
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "match: null argument");
+    if (n_boxes < 1 || n_boxes > 64) return fail_msg(ctx, B200PPF_ERR_INVALID, "match: n_boxes must be in 1 .. 64");
+    if (scene->ctx != ctx) return fail_msg(ctx, B200PPF_ERR_INVALID, "match: the scene belongs to another context");
     for (size_t b = 0; b < n_boxes; ++b)
         if (!models[b] || models[b]->ctx != ctx) {
             char msg[128];
-            snprintf(msg, sizeof(msg), "match frame: box %zu: the model is NULL or belongs to another context", b);
+            snprintf(msg, sizeof(msg), "match: box %zu: the model is NULL or belongs to another context", b);
             return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
         }
     return B200PPF_OK;
+}
+
+// b200ppf_match_frame; b200ppf_match_object is this on one box.  The PCL matching does not read the edge cloud: it is
+// extracted when the caller wants it (want_edges) and edge_curvature > 0.
+int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, const b200ppf_cloud *const *models,
+              const b200ppf_table *const *tables, const b200ppf_object_params *params, b200ppf_object_result *results, int *status,
+              bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out) {
+    CHECK_CTX(ctx);
+    if (int rc = frame_args(ctx, scene, n_boxes, corners12, tables, models, results, status)) return rc;
+    for (size_t b = 0; b < n_boxes; ++b)
+        if (!tables[b] || tables[b]->ctx != ctx) {
+            char msg[128];
+            snprintf(msg, sizeof(msg), "match: box %zu: the table is NULL or belongs to another context", b);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+    b200ppf_object_params p;
+    b200ppf_object_params_default(&p);
+    if (params) p = *params;
+    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *, std::vector<double> *poses) {
+        b200ppf_object_result *res = &results[b];
+        float poses16[3 * 16];
+        uint32_t votes[3] = {0, 0, 0};
+        size_t n_poses = 0;
+        if (int rc = b200ppf_register(ctx, models[b], tables[b], object, p.ref_rate, p.pos_thr, p.rot_thr, nullptr, poses16, votes,
+                                      &n_poses))
+            return rc;
+        b200ppf_timings tm;
+        b200ppf_get_timings(ctx, &tm);
+        res->match_ms = tm.grid_ms + tm.vote_ms + tm.pose_ms + tm.cluster_ms;
+        res->n_poses = (uint32_t)n_poses;
+        res->votes = votes[0];
+        poses->assign(poses16, poses16 + 16 * n_poses);
+        return B200PPF_OK;
+    };
+    return match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && want_edges, results, status, object_out,
+                       edges_out, match);
+}
+
+// b200cv_match_frame; b200cv_match_object is this on one box.  The edge cloud is extracted when edge_curvature > 0 and
+// Matching_S2B needs it (use_edges) or the caller wants it (want_edges).
+int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, b200cv_detector *const *detectors,
+             const b200ppf_cloud *const *models, const b200cv_object_params *params, b200ppf_object_result *results, int *status,
+             bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out) {
+    CHECK_CTX(ctx);
+    if (int rc = frame_args(ctx, scene, n_boxes, corners12, detectors, models, results, status)) return rc;
+    for (size_t b = 0; b < n_boxes; ++b) {
+        char msg[128];
+        if (!detectors[b] || cv_detector_context(detectors[b]) != ctx) {
+            snprintf(msg, sizeof(msg), "cv match: box %zu: the detector is NULL or belongs to another context", b);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+        if (!cv_detector_trained(detectors[b])) {
+            snprintf(msg, sizeof(msg), "cv match: box %zu: the detector is not trained", b);
+            return fail_msg(ctx, B200PPF_ERR_STATE, msg);
+        }
+    }
+    b200cv_object_params p;
+    b200cv_object_params_default(&p);
+    if (params) p = *params;
+    if (p.use_edges && !(p.edge_curvature > 0.0f))
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match: Matching_S2B needs the edge cloud, edge_curvature must be positive");
+    const size_t cap = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
+    std::vector<b200cv_pose> poses(cap);
+    cudaEvent_t ev[2] = {nullptr, nullptr};  // the context's events are taken by the stages inside the match
+    PPF_CUDA(ctx, cudaEventCreate(&ev[0]));
+    if (cudaEventCreate(&ev[1]) != cudaSuccess) {
+        cudaEventDestroy(ev[0]);
+        return fail_msg(ctx, B200PPF_ERR_CUDA, "cv match: cudaEventCreate failed");
+    }
+    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *edges, std::vector<double> *refined) {
+        b200ppf_object_result *res = &results[b];
+        if (p.use_edges && edges->n == 0)
+            return fail_msg(ctx, B200PPF_ERR_STATE, "cv match: the object has no edge point for Matching_S2B to pair with");
+        size_t n_clusters = 0;
+        cudaEventRecord(ev[0], ctx->stream);
+        int rc = b200cv_detector_match_cloud(detectors[b], object, p.use_edges ? edges : nullptr, p.relative_scene_sample_step,
+                                             p.relative_scene_distance, poses.data(), cap, &n_clusters);
+        cudaEventRecord(ev[1], ctx->stream);
+        if (rc == B200PPF_OK && cudaEventSynchronize(ev[1]) == cudaSuccess) cudaEventElapsedTime(&res->match_ms, ev[0], ev[1]);
+        if (rc) return rc;
+        const size_t n_kept = std::min(n_clusters, cap);
+        refined->resize(16 * n_kept);
+        for (size_t k = 0; k < n_kept; ++k) memcpy(refined->data() + 16 * k, poses[k].pose, 16 * sizeof(double));
+        res->n_poses = (uint32_t)n_clusters;
+        res->votes = n_kept ? poses[0].num_votes : 0;
+        return B200PPF_OK;
+    };
+    const int rc = match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && (p.use_edges || want_edges),
+                               results, status, object_out, edges_out, match);
+    cudaEventDestroy(ev[0]);
+    cudaEventDestroy(ev[1]);
+    return rc;
 }
 
 }  // namespace
@@ -1167,50 +1252,17 @@ void b200ppf_object_params_default(b200ppf_object_params *p) {
     p->pos_thr = 0.01f;       // PCL defaults of PPFRegistration
     p->rot_thr = 20.0f / 180.0f * 3.14159265358979f;
     p->icp_poses = 5;         // N = 5, include/CloudProcessing.h:508
-    p->icp = b200ppf_icp_params{100, 0.005f, 2.5f, 8};
+    p->icp = ICP_DEFAULT;
 }
 
 int b200ppf_match_object(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const float *corners12, const b200ppf_cloud *model,
                          const b200ppf_table *table, const b200ppf_object_params *params, b200ppf_object_result *res,
                          b200ppf_cloud **object_out, b200ppf_cloud **edges_out) {
-    if (!ctx) return fail_msg(nullptr, B200PPF_ERR_INVALID, "null context");
     if (object_out) *object_out = nullptr;
     if (edges_out) *edges_out = nullptr;
-    if (!scene || !corners12 || !model || !table || !res) return fail_msg(ctx, B200PPF_ERR_INVALID, "match object: null argument");
-    b200ppf_object_params p;
-    b200ppf_object_params_default(&p);
-    if (params) p = *params;
-    memset(res, 0, sizeof(*res));
-    const auto t0 = std::chrono::steady_clock::now();
-    OwnedCloud object, edges;
-    // the edge cloud does not enter the PCL matching: extracted on request only
-    int rc = match_object_prep(ctx, scene, corners12, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k, p.edge_curvature,
-                               p.edge_curvature > 0.0f && edges_out, res, &object, &edges);
-    if (rc) return rc;
-    float final16[16], poses16[3 * 16];
-    uint32_t votes[3] = {0, 0, 0};
-    size_t n_poses = 0;
-    if ((rc = b200ppf_register(ctx, model, table, object.c, p.ref_rate, p.pos_thr, p.rot_thr, final16, poses16, votes, &n_poses)))
-        return rc;
-    b200ppf_timings tm;
-    b200ppf_get_timings(ctx, &tm);
-    res->match_ms = tm.grid_ms + tm.vote_ms + tm.pose_ms + tm.cluster_ms;
-    res->n_poses = (uint32_t)n_poses;
-    if (n_poses == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match object: the matching returned no pose");  // reference: exit(0), :502-507
-    double refined[3 * 16], residuals[3] = {0, 0, 0};
-    for (size_t k = 0; k < n_poses * 16; ++k) refined[k] = (double)poses16[k];
-    const size_t n_icp = std::min<size_t>(n_poses, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
-    if (n_icp) {
-        if ((rc = b200ppf_icp_refine(ctx, model, object.c, &p.icp, refined, n_icp, residuals, nullptr))) return rc;
-        res->icp_ms = ctx->timings.icp_ms;
-    }
-    memcpy(res->pose, refined, 16 * sizeof(double));  // resultsSub[0]
-    res->residual = residuals[0];
-    res->votes = votes[0];
-    res->total_wall_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (object_out) *object_out = object.release();
-    if (edges_out) *edges_out = edges.release();
-    return B200PPF_OK;
+    int status = B200PPF_OK;
+    const int rc = ppf_match(ctx, scene, 1, corners12, &model, &table, params, res, &status, edges_out != nullptr, object_out, edges_out);
+    return rc ? rc : status;
 }
 
 void b200cv_object_params_default(b200cv_object_params *p) {
@@ -1224,7 +1276,7 @@ void b200cv_object_params_default(b200cv_object_params *p) {
     p->relative_scene_sample_step = 0.05;  // match_S2B(object, edges, results, 0.05, 0.05), include/CloudProcessing.h:481-495
     p->relative_scene_distance = 0.05;
     p->icp_poses = 5;                     // N = 5, include/CloudProcessing.h:508
-    p->icp = b200ppf_icp_params{100, 0.005f, 2.5f, 8};
+    p->icp = ICP_DEFAULT;
 }
 
 int b200cv_match_object(b200cv_detector *d, const b200ppf_cloud *scene, const float *corners12, const b200ppf_cloud *model,
@@ -1233,156 +1285,22 @@ int b200cv_match_object(b200cv_detector *d, const b200ppf_cloud *scene, const fl
     if (object_out) *object_out = nullptr;
     if (edges_out) *edges_out = nullptr;
     if (!d) return fail_msg(nullptr, B200PPF_ERR_INVALID, "cv match object: null detector");
-    b200ppf_ctx *ctx = cv_detector_context(d);
-    if (!scene || !corners12 || !model || !res) return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match object: null argument");
-    if (!cv_detector_trained(d)) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match object: the detector is not trained");
-    if (scene->ctx != ctx || model->ctx != ctx)
-        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match object: the clouds belong to another context than the detector");
-    b200cv_object_params p;
-    b200cv_object_params_default(&p);
-    if (params) p = *params;
-    if (p.use_edges && !(p.edge_curvature > 0.0f))
-        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match object: Matching_S2B needs the edge cloud, edge_curvature must be positive");
-    DeviceGuard guard(ctx->device);
-    memset(res, 0, sizeof(*res));
-    const auto t0 = std::chrono::steady_clock::now();
-    OwnedCloud object, edges;
-    int rc = match_object_prep(ctx, scene, corners12, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k, p.edge_curvature,
-                               p.use_edges || (p.edge_curvature > 0.0f && edges_out), res, &object, &edges);
-    if (rc) return rc;
-    if (p.use_edges && edges.c->n == 0)
-        return fail_msg(ctx, B200PPF_ERR_STATE, "cv match object: the object has no edge point for Matching_S2B to pair with");
-    const size_t cap = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
-    std::vector<b200cv_pose> poses(cap);
-    size_t n_clusters = 0;
-    cudaEvent_t ev[2] = {nullptr, nullptr};  // the context's events are taken by the stages inside the match
-    PPF_CUDA(ctx, cudaEventCreate(&ev[0]));
-    if (cudaEventCreate(&ev[1]) != cudaSuccess) {
-        cudaEventDestroy(ev[0]);
-        return fail_msg(ctx, B200PPF_ERR_CUDA, "cv match object: cudaEventCreate failed");
-    }
-    cudaEventRecord(ev[0], ctx->stream);
-    rc = b200cv_detector_match_cloud(d, object.c, p.use_edges ? edges.c : nullptr, p.relative_scene_sample_step,
-                                     p.relative_scene_distance, poses.data(), cap, &n_clusters);
-    cudaEventRecord(ev[1], ctx->stream);
-    if (rc == B200PPF_OK && cudaEventSynchronize(ev[1]) == cudaSuccess) cudaEventElapsedTime(&res->match_ms, ev[0], ev[1]);
-    cudaEventDestroy(ev[0]);
-    cudaEventDestroy(ev[1]);
-    if (rc) return rc;
-    res->n_poses = (uint32_t)n_clusters;
-    if (n_clusters == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match object: the matching returned no pose");  // reference: exit(0), :502-507
-    const size_t n_icp = std::min<size_t>(n_clusters, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
-    const size_t n_keep = std::max<size_t>(n_icp, 1);
-    std::vector<double> refined(16 * n_keep), residuals(n_keep, 0.0);
-    for (size_t k = 0; k < n_keep; ++k) memcpy(refined.data() + 16 * k, poses[k].pose, 16 * sizeof(double));
-    if (n_icp) {
-        if ((rc = b200ppf_icp_refine(ctx, model, object.c, &p.icp, refined.data(), n_icp, residuals.data(), nullptr))) return rc;
-        res->icp_ms = ctx->timings.icp_ms;
-    }
-    memcpy(res->pose, refined.data(), 16 * sizeof(double));  // resultsSub[0]
-    res->residual = residuals[0];
-    res->votes = poses[0].num_votes;
-    res->total_wall_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (object_out) *object_out = object.release();
-    if (edges_out) *edges_out = edges.release();
-    return B200PPF_OK;
+    int status = B200PPF_OK;
+    const int rc = cv_match(cv_detector_context(d), scene, 1, corners12, &d, &model, params, res, &status, edges_out != nullptr,
+                            object_out, edges_out);
+    return rc ? rc : status;
 }
 
 int b200cv_match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
                        b200cv_detector *const *detectors, const b200ppf_cloud *const *models, const b200cv_object_params *params,
                        b200ppf_object_result *results, int *status) {
-    CHECK_CTX(ctx);
-    if (int rc = frame_args(ctx, scene, n_boxes, corners12, detectors, models, results, status)) return rc;
-    for (size_t b = 0; b < n_boxes; ++b) {
-        char msg[128];
-        if (!detectors[b] || cv_detector_context(detectors[b]) != ctx) {
-            snprintf(msg, sizeof(msg), "cv match frame: box %zu: the detector is NULL or belongs to another context", b);
-            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
-        }
-        if (!cv_detector_trained(detectors[b])) {
-            snprintf(msg, sizeof(msg), "cv match frame: box %zu: the detector is not trained", b);
-            return fail_msg(ctx, B200PPF_ERR_STATE, msg);
-        }
-    }
-    b200cv_object_params p;
-    b200cv_object_params_default(&p);
-    if (params) p = *params;
-    if (p.use_edges && !(p.edge_curvature > 0.0f))
-        return fail_msg(ctx, B200PPF_ERR_INVALID, "cv match frame: Matching_S2B needs the edge cloud, edge_curvature must be positive");
-    const size_t cap = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
-    std::vector<b200cv_pose> poses(cap);
-    cudaEvent_t ev[2] = {nullptr, nullptr};  // the context's events are taken by the stages inside the match
-    PPF_CUDA(ctx, cudaEventCreate(&ev[0]));
-    if (cudaEventCreate(&ev[1]) != cudaSuccess) {
-        cudaEventDestroy(ev[0]);
-        return fail_msg(ctx, B200PPF_ERR_CUDA, "cv match frame: cudaEventCreate failed");
-    }
-    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *edges, std::vector<double> *refined,
-                     std::vector<double> *residuals, size_t *n_icp) {
-        b200ppf_object_result *res = &results[b];
-        if (p.use_edges && edges->n == 0)
-            return fail_msg(ctx, B200PPF_ERR_STATE, "cv match frame: the object has no edge point for Matching_S2B to pair with");
-        size_t n_clusters = 0;
-        cudaEventRecord(ev[0], ctx->stream);
-        int rc = b200cv_detector_match_cloud(detectors[b], object, p.use_edges ? edges : nullptr, p.relative_scene_sample_step,
-                                             p.relative_scene_distance, poses.data(), cap, &n_clusters);
-        cudaEventRecord(ev[1], ctx->stream);
-        if (rc == B200PPF_OK && cudaEventSynchronize(ev[1]) == cudaSuccess) cudaEventElapsedTime(&res->match_ms, ev[0], ev[1]);
-        if (rc) return rc;
-        res->n_poses = (uint32_t)n_clusters;
-        if (n_clusters == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "cv match frame: the matching returned no pose");
-        *n_icp = std::min<size_t>(n_clusters, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
-        const size_t n_keep = std::max<size_t>(*n_icp, 1);
-        refined->resize(16 * n_keep);
-        residuals->assign(n_keep, 0.0);
-        for (size_t k = 0; k < n_keep; ++k) memcpy(refined->data() + 16 * k, poses[k].pose, 16 * sizeof(double));
-        res->votes = poses[0].num_votes;
-        return B200PPF_OK;
-    };
-    const int rc = match_frame(ctx, scene, n_boxes, corners12, models, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k,
-                               p.edge_curvature, p.icp, results, status, match);
-    cudaEventDestroy(ev[0]);
-    cudaEventDestroy(ev[1]);
-    return rc;
+    return cv_match(ctx, scene, n_boxes, corners12, detectors, models, params, results, status, true, nullptr, nullptr);
 }
 
 int b200ppf_match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
                         const b200ppf_cloud *const *models, const b200ppf_table *const *tables, const b200ppf_object_params *params,
                         b200ppf_object_result *results, int *status) {
-    CHECK_CTX(ctx);
-    if (int rc = frame_args(ctx, scene, n_boxes, corners12, tables, models, results, status)) return rc;
-    for (size_t b = 0; b < n_boxes; ++b)
-        if (!tables[b] || tables[b]->ctx != ctx) {
-            char msg[128];
-            snprintf(msg, sizeof(msg), "match frame: box %zu: the table is NULL or belongs to another context", b);
-            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
-        }
-    b200ppf_object_params p;
-    b200ppf_object_params_default(&p);
-    if (params) p = *params;
-    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *, std::vector<double> *refined,
-                     std::vector<double> *residuals, size_t *n_icp) {
-        b200ppf_object_result *res = &results[b];
-        float final16[16], poses16[3 * 16];
-        uint32_t votes[3] = {0, 0, 0};
-        size_t n_poses = 0;
-        if (int rc = b200ppf_register(ctx, models[b], tables[b], object, p.ref_rate, p.pos_thr, p.rot_thr, final16, poses16, votes,
-                                      &n_poses))
-            return rc;
-        b200ppf_timings tm;
-        b200ppf_get_timings(ctx, &tm);
-        res->match_ms = tm.grid_ms + tm.vote_ms + tm.pose_ms + tm.cluster_ms;
-        res->n_poses = (uint32_t)n_poses;
-        if (n_poses == 0) return fail_msg(ctx, B200PPF_ERR_STATE, "match frame: the matching returned no pose");
-        refined->resize(3 * 16);
-        residuals->assign(3, 0.0);
-        for (size_t k = 0; k < n_poses * 16; ++k) (*refined)[k] = (double)poses16[k];
-        *n_icp = std::min<size_t>(n_poses, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
-        res->votes = votes[0];
-        return B200PPF_OK;
-    };
-    return match_frame(ctx, scene, n_boxes, corners12, models, p.leaf, p.sor_mean_k, p.sor_stddev_mul, p.normal_k, p.edge_curvature,
-                       p.icp, results, status, match);
+    return ppf_match(ctx, scene, n_boxes, corners12, models, tables, params, results, status, true, nullptr, nullptr);
 }
 
 }  // extern "C"
