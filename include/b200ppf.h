@@ -568,6 +568,63 @@ int b200ppf_match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_b
                         const b200ppf_cloud *const *models, const b200ppf_table *const *tables,
                         const b200ppf_object_params *params, b200ppf_object_result *results, int *status);
 
+/* ---- pose verification: how much of a pose's visible model surface the scene supports ---------------------------------
+ * The last stage of a PPF pipeline (Drost et al. 2010; Vidal et al. 2018): every candidate pose is scored against the
+ * points it should explain.  For a model cloud, a scene cloud and a pose T = [R t] (model -> scene), model point p with
+ * normal n moves to p' = R p + t, n' = R n.  It is VISIBLE when n'.(-p') > 0 (the camera sits at the origin; a zero normal
+ * counts as visible), and a visible point is an INLIER when its nearest scene point q (exact; the lowest index among
+ * equally near points) lies within inlier_dist and q's normal has n_q.n' >= cos(normal_angle).  Per pose:
+ *   inliers, visible   exact counts
+ *   fit                inliers / visible (float), 0 when nothing is visible
+ *   rms                root mean square distance of the inliers to their nearest scene points, 0 without inliers
+ * A pose's record has the same bits alone or in any batch, and on every run. */
+typedef struct b200ppf_verify_params {
+    float inlier_dist;  /* metres, > 0; default 0.01 (the reference's leaf) */
+    float normal_angle; /* radians, >= 0; default 30 degrees; >= pi: the distance alone decides */
+} b200ppf_verify_params;
+void b200ppf_verify_params_default(b200ppf_verify_params *params);
+typedef struct b200ppf_pose_fit {
+    uint32_t inliers, visible;
+    float fit; /* inliers / visible; 0 when visible == 0 */
+    float rms; /* root mean square of the inliers' distances; 0 without inliers */
+} b200ppf_pose_fit;
+/* Scores the poses of ICP jobs (the b200ppf_icp_refine_batch block: poses16 are read only, residuals are ignored) against
+ * their scenes: fits receives the sum of the jobs' n_poses records, job-major.  params NULL = the defaults.  One grid per
+ * distinct scene of the call, all built in one pass, and a launch count that does not grow with the jobs or the poses.
+ * An empty scene gives 0 inliers.  B200PPF_ERR_INVALID, before anything is allocated: NULL arrays, a cloud of another
+ * context, a non-finite pose, inlier_dist not finite and positive, normal_angle negative or NaN. */
+int b200ppf_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_verify_params *params,
+                        b200ppf_pose_fit *fits);
+
+/* The frame calls above, with every candidate pose of every box scored against the box's object cloud and the best one
+ * returned.  The same chain runs (the crop, the per-box pre-processing and matching, the one batched ICP), then ONE
+ * b200ppf_score_poses over the candidates of every box that reached the matching, each against models[b] and the box's
+ * pre-processed object cloud (what the ICP registered to).  A box's candidates are the poses the call refines: its top
+ * icp_poses clusters (clamped as for the unverified call), or with icp_poses = 0 its top cluster alone, unrefined.
+ *   results[b]   pose, residual and votes are those of the candidate with the highest fit (ties: the lower rank); every
+ *                other field is the unverified call's, bit for bit, but the frame-wide crop_ms, icp_ms and total_wall_ms
+ *                (which now includes the scoring).
+ *   candidates   NULL, or n_boxes x max(icp_poses, 1) records: box b's from b * max(icp_poses, 1), sorted by fit
+ *                descending, ties by rank ascending.  Unused slots and the slots of a failed box are zero with
+ *                rank = UINT32_MAX.  An application rejects a box's pose whose fit is too low (INTEGRATION.md §3c).
+ *   status, return codes   as the unverified call's, and B200PPF_ERR_INVALID for bad verify values (NULL = the
+ *                defaults), checked before the crop runs. */
+typedef struct b200ppf_candidate {
+    double pose[16];  /* row-major 4x4, model -> scene, after ICP when icp_poses > 0 */
+    double residual;  /* its ICP residual (0 without ICP) */
+    uint32_t votes;   /* votes of its pose cluster */
+    uint32_t rank;    /* its position among the clusters, 0 = most voted; UINT32_MAX = unused slot */
+    b200ppf_pose_fit fit;
+} b200ppf_candidate;
+int b200cv_match_frame_verified(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                                b200cv_detector *const *detectors, const b200ppf_cloud *const *models,
+                                const b200cv_object_params *params, const b200ppf_verify_params *verify,
+                                b200ppf_object_result *results, int *status, b200ppf_candidate *candidates);
+int b200ppf_match_frame_verified(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                                 const b200ppf_cloud *const *models, const b200ppf_table *const *tables,
+                                 const b200ppf_object_params *params, const b200ppf_verify_params *verify,
+                                 b200ppf_object_result *results, int *status, b200ppf_candidate *candidates);
+
 #ifdef __cplusplus
 }
 #endif

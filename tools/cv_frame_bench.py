@@ -15,7 +15,13 @@ crop and ICP are one each).  Kernel launches per call and the ICP launches among
 launches with icp_poses = 0) are counted with b200ppf_launch_count.  Every frame result must equal its serial call's bits.
 The card's name, power limit and maximum SM clock (nvidia-smi, read-only) go into every line.
 
-usage: python tools/cv_frame_bench.py [--repeat 20] [--out profiles/r4_cv_frame.jsonl]"""
+--verify: what pose verification adds.  For K = 1 and 8 boxes on both frames, --repeat b200cv_match_frame and
+b200cv_match_frame_verified calls (default parameters: 1 cm, 30 degrees), alternated after one warm-up of each, medians of
+the wall time; and b200ppf_score_poses alone on the verified call's candidates of the same boxes (each box's object cloud
+from b200cv_match_object), --repeat calls timed with CUDA events on the context's stream.  The verified results must hold
+the plain call's fields and the fits of score_poses.
+
+usage: python tools/cv_frame_bench.py [--repeat 20] [--verify] [--out profiles/r4_cv_frame.jsonl | profiles/r5_verify.jsonl]"""
 import argparse
 import json
 import os
@@ -117,11 +123,61 @@ def bench(c, name, scene, boxes, leaf, K, repeat, gpu):
             "speedup_wall": s_wall / f_wall, "frame_wall_ms_per_object": f_wall / K, "identical_to_serial": identical, "gpu": gpu}
 
 
+def bench_verify(c, name, scene, boxes, leaf, K, repeat, gpu):
+    import torch
+    cors = np.stack([b[0] for b in boxes[:K]])
+    dets, mods = [b[1] for b in boxes[:K]], [b[2] for b in boxes[:K]]
+
+    def timed(fn):
+        t0 = time.perf_counter()
+        out = fn(scene, cors, dets, mods, leaf=leaf)
+        return out, 1e3 * (time.perf_counter() - t0)
+
+    timed(c.cv_match_frame), timed(c.cv_match_frame_verified)  # warm-up
+    plain, verified = [], []
+    for _ in range(repeat):
+        plain.append(timed(c.cv_match_frame))
+        verified.append(timed(c.cv_match_frame_verified))
+    (res, status), _ = plain[-1]
+    (vres, vstatus, cands), _ = verified[-1]
+    assert status.tolist() == vstatus.tolist() == [0] * K, (status, vstatus)
+    same = all(a[f] == b[f] for a, b in zip(res, vres) for f in ("n_poses", "n_cropped", "n_sampled", "n_filtered", "n_edges"))
+    # score_poses alone on the same candidates, against the same object clouds
+    objects = [c.cv_match_object(dets[k], scene, cors[k], mods[k], leaf=leaf)[1] for k in range(K)]
+    jobs = [(mods[k], objects[k], np.stack([x["pose"] for x in cands[k]])) for k in range(K)]
+    fits = c.score_poses(jobs)
+    fits_match = all(f["fit"] == x["fit"]["fit"] and f["inliers"] == x["fit"]["inliers"] for k in range(K)
+                     for f, x in zip(fits[k], cands[k]))
+    stream = torch.cuda.ExternalStream(c.stream)
+    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(repeat)]
+    n0 = c.launch_count
+    c.score_poses(jobs)
+    launches = c.launch_count - n0
+    for e0, e1 in ev:
+        e0.record(stream)
+        c.score_poses(jobs)
+        e1.record(stream)
+    torch.cuda.synchronize()
+    score_ms = [e0.elapsed_time(e1) for e0, e1 in ev]
+    med = lambda v: float(np.median(v))  # noqa: E731
+    p_wall, v_wall = med([w for _, w in plain]), med([w for _, w in verified])
+    return {"frame": name, "boxes": K, "calls": repeat, "leaf": leaf, "verify": {"inlier_dist": 0.01, "normal_angle_deg": 30.0},
+            "candidates": int(sum(len(x) for x in cands)), "model_points": [int(m.size) for m in mods],
+            "object_points": [int(o.size) for o in objects],
+            "plain_wall_ms_median": p_wall, "verified_wall_ms_median": v_wall, "added_wall_ms": v_wall - p_wall,
+            "score_poses_device_ms_median": med(score_ms), "score_poses_launches": launches,
+            "best_rank": [int(x[0]["rank"]) for x in cands], "best_fit": [float(x[0]["fit"]["fit"]) for x in cands],
+            "fields_equal_plain": same, "fits_equal_score_poses": fits_match, "gpu": gpu}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--repeat", type=int, default=20, help="timed frame calls and serial rounds per K (after one warm-up each)")
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r4_cv_frame.jsonl"))
+    ap.add_argument("--verify", action="store_true", help="time the verified frame call and b200ppf_score_poses instead")
+    ap.add_argument("--out", default=None)
     args = ap.parse_args()
+    if args.out is None:
+        args.out = os.path.join(ROOT, "profiles", "r5_verify.jsonl" if args.verify else "r4_cv_frame.jsonl")
     if args.repeat < 1:
         ap.error("--repeat must be at least 1")
     from yolo_ppf_pose_estimation_b200 import capi
@@ -130,8 +186,8 @@ def main():
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
         for name, scene, boxes, leaf in frames(c):
-            for K in (1, 2, 4, 8):
-                line = json.dumps(bench(c, name, scene, boxes, leaf, K, args.repeat, gpu))
+            for K in ((1, 8) if args.verify else (1, 2, 4, 8)):
+                line = json.dumps((bench_verify if args.verify else bench)(c, name, scene, boxes, leaf, K, args.repeat, gpu))
                 print(line, flush=True)
                 f.write(line + "\n")
 

@@ -69,6 +69,20 @@ class CvObjectParams(C.Structure):
                 ("relative_scene_distance", C.c_double), ("icp_poses", C.c_int), ("icp", IcpParams)]
 
 
+class VerifyParams(C.Structure):
+    _fields_ = [("inlier_dist", C.c_float), ("normal_angle", C.c_float)]
+
+
+class PoseFit(C.Structure):
+    _fields_ = [("inliers", C.c_uint32), ("visible", C.c_uint32), ("fit", C.c_float), ("rms", C.c_float)]
+
+
+class Candidate(C.Structure):
+    _fields_ = [("pose", C.c_double * 16), ("residual", C.c_double), ("votes", C.c_uint32), ("rank", C.c_uint32), ("fit", PoseFit)]
+
+
+CANDIDATE_UNUSED = 0xFFFFFFFF  # rank of an unused candidate slot
+
 CV_POSE_DTYPE = np.dtype([("pose", np.float64, (16,)), ("alpha", np.float64), ("residual", np.float64), ("angle", np.float64),
                           ("t", np.float64, (3,)), ("q", np.float64, (4,)), ("model_index", np.uint32), ("num_votes", np.uint32),
                           ("alpha_index", np.uint32), ("reference_index", np.uint32)])
@@ -169,6 +183,12 @@ SYMBOLS = {
     "b200ppf_match_object": (_i, [_vp, _vp, _vp, _vp, _vp, C.POINTER(ObjectParams), C.POINTER(ObjectResult), C.POINTER(_vp),
                                   C.POINTER(_vp)]),
     "b200ppf_match_frame": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(ObjectParams), C.POINTER(ObjectResult), _vp]),
+    "b200ppf_verify_params_default": (None, [C.POINTER(VerifyParams)]),
+    "b200ppf_score_poses": (_i, [_vp, C.POINTER(IcpJob), _sz, C.POINTER(VerifyParams), C.POINTER(PoseFit)]),
+    "b200ppf_match_frame_verified": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(ObjectParams), C.POINTER(VerifyParams),
+                                          C.POINTER(ObjectResult), _vp, C.POINTER(Candidate)]),
+    "b200cv_match_frame_verified": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(VerifyParams),
+                                         C.POINTER(ObjectResult), _vp, C.POINTER(Candidate)]),
     "b200ppf_register": (_i, [_vp, _vp, _vp, _vp, _sz, _f, _f, _vp, _vp, _vp, C.POINTER(_sz)]),
     "b200cv_detector_create": (_i, [_vp, C.c_double, C.c_double, C.c_double, C.POINTER(_vp)]),
     "b200cv_detector_free": (None, [_vp]),
@@ -415,6 +435,75 @@ class Context:
         status = np.zeros(max(1, c12.shape[0]), np.int32)
         self.check(call(c12.shape[0], _p(c12), C.byref(prm), res, _p(status)))
         return [self._result(res[k]) for k in range(c12.shape[0])], status[:c12.shape[0]]
+
+    @staticmethod
+    def verify_params(**overrides):
+        """VerifyParams: the defaults (inlier_dist 0.01 m, normal_angle 30 degrees), then overrides"""
+        prm = VerifyParams()
+        lib().b200ppf_verify_params_default(C.byref(prm))
+        for k, v in overrides.items():
+            setattr(prm, k, v)
+        return prm
+
+    @staticmethod
+    def _fit(f):
+        return {"inliers": f.inliers, "visible": f.visible, "fit": f.fit, "rms": f.rms}
+
+    def _verified_frame_call(self, params_cls, default_fn, call, corners, overrides):
+        """the verified frame calls: -> (result dicts, int32 status per box, candidate dicts per box (used slots only,
+        best first))"""
+        c12 = np.ascontiguousarray(corners, np.float32).reshape(-1, 12)
+        K = c12.shape[0]
+        vover = {k: overrides.pop(k) for k in ("inlier_dist", "normal_angle") if k in overrides}
+        prm = self._params(params_cls, default_fn, overrides)
+        vp = self.verify_params(**vover)
+        slots = max(prm.icp_poses, 1)
+        res = (ObjectResult * max(1, K))()
+        status = np.zeros(max(1, K), np.int32)
+        cand = (Candidate * max(1, K * slots))()
+        self.check(call(K, _p(c12), C.byref(prm), C.byref(vp), res, _p(status), cand))
+        per_box = []
+        for b in range(K):
+            cs = [cand[b * slots + i] for i in range(slots)]
+            per_box.append([{"pose": np.array(c.pose, np.float64).reshape(4, 4), "residual": c.residual, "votes": c.votes,
+                             "rank": c.rank, "fit": self._fit(c.fit)} for c in cs if c.rank != CANDIDATE_UNUSED])
+        return [self._result(res[k]) for k in range(K)], status[:K], per_box
+
+    def score_poses(self, jobs, inlier_dist=None, normal_angle=None):
+        """b200ppf_score_poses: jobs = [(model, scene, poses (P,4,4)), ...] -> [list of P fit dicts per job]
+        (inliers, visible, fit, rms); None keeps a default (0.01 m, 30 degrees)"""
+        over = {k: v for k, v in (("inlier_dist", inlier_dist), ("normal_angle", normal_angle)) if v is not None}
+        vp = self.verify_params(**over)
+        arrays = [np.ascontiguousarray(np.asarray(p, np.float64).reshape(-1, 4, 4)) for _, _, p in jobs]
+        js = (IcpJob * max(1, len(jobs)))()
+        for k, ((m, s, _), P) in enumerate(zip(jobs, arrays)):
+            js[k] = IcpJob(m._h, s._h, P.ctypes.data, P.shape[0], None)
+        total = sum(P.shape[0] for P in arrays)
+        fits = (PoseFit * max(1, total))()
+        self.check(lib().b200ppf_score_poses(self._h, js, len(jobs), C.byref(vp), fits))
+        out, at = [], 0
+        for P in arrays:
+            out.append([self._fit(fits[at + i]) for i in range(P.shape[0])])
+            at += P.shape[0]
+        return out
+
+    def cv_match_frame_verified(self, scene: "Cloud", corners, detectors, models, **overrides):
+        """cv_match_frame with every candidate pose scored (b200cv_match_frame_verified) and the best one returned ->
+        (result dicts, status per box, candidates per box sorted by fit).  overrides: fields of CvObjectParams (icp_* for
+        the ICP), inlier_dist and normal_angle for the scoring."""
+        n = len(detectors)
+        dets, mods = self._handles(detectors, n), self._handles(models, n)
+        return self._verified_frame_call(
+            CvObjectParams, lib().b200cv_object_params_default,
+            lambda k, c, *a: lib().b200cv_match_frame_verified(self._h, scene._h, k, c, dets, mods, *a), corners, dict(overrides))
+
+    def match_frame_verified(self, scene: "Cloud", corners, models, tables, **overrides):
+        """match_frame with every candidate pose scored (b200ppf_match_frame_verified), as cv_match_frame_verified"""
+        n = len(models)
+        mods, tabs = self._handles(models, n), self._handles(tables, n)
+        return self._verified_frame_call(
+            ObjectParams, lib().b200ppf_object_params_default,
+            lambda k, c, *a: lib().b200ppf_match_frame_verified(self._h, scene._h, k, c, mods, tabs, *a), corners, dict(overrides))
 
     @staticmethod
     def _handles(objs, n):

@@ -66,6 +66,20 @@ using namespace b200ppf;
 // the reference's ICP(100, 0.005f, 2.5f, 8): the default of both ICP calls and of both per-object parameter blocks
 constexpr b200ppf_icp_params ICP_DEFAULT = {100, 0.005f, 2.5f, 8};
 
+namespace {
+
+// params (NULL = the defaults) -> *out, or B200PPF_ERR_INVALID
+int verify_params(b200ppf_ctx *ctx, const b200ppf_verify_params *params, b200ppf_verify_params *out) {
+    b200ppf_verify_params_default(out);
+    if (params) *out = *params;
+    if (!(std::isfinite(out->inlier_dist) && out->inlier_dist > 0.0f))
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "verify: inlier_dist must be finite and positive");
+    if (!(out->normal_angle >= 0.0f)) return fail_msg(ctx, B200PPF_ERR_INVALID, "verify: normal_angle must be >= 0");
+    return B200PPF_OK;
+}
+
+}  // namespace
+
 extern "C" {
 
 int b200ppf_version(void) { return B200PPF_VERSION; }
@@ -1009,6 +1023,37 @@ int b200ppf_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size
     return k6_icp_refine_batch(ctx, jobs, n_jobs, p.max_iterations, p.tolerance, p.rejection_scale, p.num_levels, iterations);
 }
 
+void b200ppf_verify_params_default(b200ppf_verify_params *p) {
+    if (!p) return;
+    p->inlier_dist = 0.01f;                              // the reference's leaf
+    p->normal_angle = 30.0f / 180.0f * 3.14159265358979f;
+}
+
+int b200ppf_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_verify_params *params,
+                        b200ppf_pose_fit *fits) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params p;
+    if (int rc = verify_params(ctx, params, &p)) return rc;
+    if (n_jobs && !jobs) return fail_msg(ctx, B200PPF_ERR_INVALID, "score poses: null jobs");
+    size_t n_poses = 0;
+    for (size_t j = 0; j < n_jobs; ++j) {
+        char msg[128];
+        const b200ppf_icp_job &jb = jobs[j];
+        const char *why = !jb.model || !jb.scene || (jb.n_poses && !jb.poses16) ? "null argument"
+                          : jb.model->ctx != ctx || jb.scene->ctx != ctx       ? "a cloud belongs to another context"
+                                                                                : nullptr;
+        for (size_t k = 0; !why && k < 16 * jb.n_poses; ++k)
+            if (!std::isfinite(jb.poses16[k])) why = "a pose is not finite";
+        if (why) {
+            snprintf(msg, sizeof(msg), "score poses: job %zu: %s", j, why);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+        n_poses += jb.n_poses;
+    }
+    if (n_poses && !fits) return fail_msg(ctx, B200PPF_ERR_INVALID, "score poses: null fits");
+    return verify_score_poses(ctx, jobs, n_jobs, p, fits);
+}
+
 int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_table *t,
                      const b200ppf_cloud *scene, size_t ref_rate, float pos_thr, float rot_thr, float *final16,
                      float *poses16, uint32_t *votes, size_t *n_out) {
@@ -1067,13 +1112,17 @@ int object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *cropped, const Params &p,
 bool fatal(int rc) { return rc == B200PPF_ERR_CUDA || rc == B200PPF_ERR_NOMEM; }
 
 // The chain of every match call, frame or per-object: crop all boxes in one pass, then per box the pre-processing and
-// `match(b, object, edges, &poses)`, the engine's matching step (it fills the box's match_ms, n_poses and votes and returns
-// its best poses, 16 doubles each, most-voted first), then one batched ICP of the top icp_poses poses of every box that
-// reached it against models[b].  When box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
+// `match(b, object, edges, &poses, &votes)`, the engine's matching step (it fills the box's match_ms and n_poses and returns
+// its best poses, 16 doubles each, most-voted first, and their clusters' votes), then one batched ICP of the top icp_poses
+// poses of every box that reached it against models[b].  With verify (checked), the candidates of every such box (the
+// refined poses, or the top pose alone without ICP) are then scored in one b200ppf_score_poses against models[b] and the
+// box's object cloud, the best one becomes the box's result, and candidates (may be NULL) receives them all, max(icp_poses,
+// 1) slots per box.  When box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
 template <class Params, class Match>
 int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
                 const b200ppf_cloud *const *models, const Params &p, bool with_edges, b200ppf_object_result *results, int *status,
-                b200ppf_cloud **object_out, b200ppf_cloud **edges_out, Match match) {
+                b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify,
+                b200ppf_candidate *candidates, Match match) {
     const auto t0 = std::chrono::steady_clock::now();
     for (size_t b = 0; b < n_boxes; ++b) {
         memset(&results[b], 0, sizeof(results[b]));
@@ -1088,6 +1137,8 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
     }
     const float crop_ms = ctx->timings.prep_ms;
     std::vector<std::vector<double>> refined(n_boxes), residuals(n_boxes);
+    std::vector<std::vector<uint32_t>> votes(n_boxes);
+    std::vector<size_t> n_cand(n_boxes, 0);
     std::vector<b200ppf_icp_job> jobs;
     for (size_t b = 0; b < n_boxes; ++b) {
         b200ppf_object_result *res = &results[b];
@@ -1096,14 +1147,16 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
         if (crops[b]->n == 0) rc = fail_msg(ctx, B200PPF_ERR_STATE, "match: no scene point inside the box's frustum");
         if (!rc) rc = object_prep(ctx, crops[b].get(), p, with_edges, res, &objects[b], &edges[b]);
         crops[b].reset();  // the frame's crops go back to the pool as soon as their box is through
-        if (!rc) rc = match(b, objects[b].get(), edges[b].get(), &refined[b]);
+        if (!rc) rc = match(b, objects[b].get(), edges[b].get(), &refined[b], &votes[b]);
+        if (!rc) res->votes = votes[b].empty() ? 0 : votes[b][0];
         if (!rc && res->n_poses == 0)  // the reference exits there, :502-507
             rc = fail_msg(ctx, B200PPF_ERR_STATE, "match: the matching returned no pose");
         if (fatal(rc)) return rc;
         status[b] = rc;
         if (rc) continue;
         const size_t n_icp = std::min<size_t>(res->n_poses, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
-        residuals[b].assign(std::max<size_t>(n_icp, 1), 0.0);
+        n_cand[b] = std::max<size_t>(n_icp, 1);
+        residuals[b].assign(n_cand[b], 0.0);
         if (n_icp) jobs.push_back(b200ppf_icp_job{models[b], objects[b].get(), refined[b].data(), n_icp, residuals[b].data()});
     }
     float icp_ms = 0.0f;
@@ -1111,16 +1164,58 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
         if (int rc = b200ppf_icp_refine_batch(ctx, jobs.data(), jobs.size(), &p.icp, nullptr)) return rc;
         icp_ms = ctx->timings.icp_ms;
     }
+    std::vector<std::vector<b200ppf_pose_fit>> fits(n_boxes);
+    std::vector<size_t> best(n_boxes, 0);  // resultsSub[0] unless verified
+    if (verify) {
+        std::vector<b200ppf_icp_job> score_jobs;
+        size_t n_scored = 0;
+        for (size_t b = 0; b < n_boxes; ++b)
+            if (!status[b]) {
+                score_jobs.push_back(b200ppf_icp_job{models[b], objects[b].get(), refined[b].data(), n_cand[b], nullptr});
+                n_scored += n_cand[b];
+            }
+        std::vector<b200ppf_pose_fit> all(n_scored);
+        if (int rc = verify_score_poses(ctx, score_jobs.data(), score_jobs.size(), *verify, all.data())) return rc;
+        size_t at = 0;
+        for (size_t b = 0; b < n_boxes; ++b) {
+            if (status[b]) continue;
+            fits[b].assign(all.begin() + at, all.begin() + at + n_cand[b]);
+            at += n_cand[b];
+            for (size_t k = 1; k < n_cand[b]; ++k)
+                if (fits[b][k].fit > fits[b][best[b]].fit) best[b] = k;
+        }
+    }
     const float wall = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     for (size_t b = 0; b < n_boxes; ++b) {
         b200ppf_object_result *res = &results[b];
         if (!status[b]) {
-            memcpy(res->pose, refined[b].data(), 16 * sizeof(double));  // resultsSub[0]
-            res->residual = residuals[b][0];
+            memcpy(res->pose, refined[b].data() + 16 * best[b], 16 * sizeof(double));
+            res->residual = residuals[b][best[b]];
+            res->votes = votes[b][best[b]];
         }
         res->crop_ms = crop_ms;
         res->icp_ms = icp_ms;
         res->total_wall_ms = wall;
+    }
+    if (verify && candidates) {
+        const size_t slots = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
+        for (size_t b = 0; b < n_boxes; ++b) {
+            b200ppf_candidate *c = candidates + b * slots;
+            memset(c, 0, slots * sizeof(*c));
+            for (size_t k = 0; k < slots; ++k) c[k].rank = UINT32_MAX;
+            if (status[b]) continue;
+            std::vector<size_t> order(n_cand[b]);
+            for (size_t k = 0; k < order.size(); ++k) order[k] = k;
+            std::stable_sort(order.begin(), order.end(), [&](size_t x, size_t y) { return fits[b][x].fit > fits[b][y].fit; });
+            for (size_t i = 0; i < order.size(); ++i) {
+                const size_t k = order[i];
+                memcpy(c[i].pose, refined[b].data() + 16 * k, 16 * sizeof(double));
+                c[i].residual = residuals[b][k];
+                c[i].votes = votes[b][k];
+                c[i].rank = (uint32_t)k;
+                c[i].fit = fits[b][k];
+            }
+        }
     }
     if (!status[0]) {
         if (object_out) *object_out = objects[0].release();
@@ -1149,7 +1244,8 @@ int frame_args(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, con
 // extracted when the caller wants it (want_edges) and edge_curvature > 0.
 int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, const b200ppf_cloud *const *models,
               const b200ppf_table *const *tables, const b200ppf_object_params *params, b200ppf_object_result *results, int *status,
-              bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out) {
+              bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify = nullptr,
+              b200ppf_candidate *candidates = nullptr) {
     CHECK_CTX(ctx);
     if (int rc = frame_args(ctx, scene, n_boxes, corners12, tables, models, results, status)) return rc;
     for (size_t b = 0; b < n_boxes; ++b)
@@ -1161,7 +1257,8 @@ int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, cons
     b200ppf_object_params p;
     b200ppf_object_params_default(&p);
     if (params) p = *params;
-    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *, std::vector<double> *poses) {
+    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *, std::vector<double> *poses,
+                     std::vector<uint32_t> *cluster_votes) {
         b200ppf_object_result *res = &results[b];
         float poses16[3 * 16];
         uint32_t votes[3] = {0, 0, 0};
@@ -1173,19 +1270,20 @@ int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, cons
         b200ppf_get_timings(ctx, &tm);
         res->match_ms = tm.grid_ms + tm.vote_ms + tm.pose_ms + tm.cluster_ms;
         res->n_poses = (uint32_t)n_poses;
-        res->votes = votes[0];
         poses->assign(poses16, poses16 + 16 * n_poses);
+        cluster_votes->assign(votes, votes + n_poses);
         return B200PPF_OK;
     };
     return match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && want_edges, results, status, object_out,
-                       edges_out, match);
+                       edges_out, verify, candidates, match);
 }
 
 // b200cv_match_frame; b200cv_match_object is this on one box.  The edge cloud is extracted when edge_curvature > 0 and
 // Matching_S2B needs it (use_edges) or the caller wants it (want_edges).
 int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, b200cv_detector *const *detectors,
              const b200ppf_cloud *const *models, const b200cv_object_params *params, b200ppf_object_result *results, int *status,
-             bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out) {
+             bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify = nullptr,
+             b200ppf_candidate *candidates = nullptr) {
     CHECK_CTX(ctx);
     if (int rc = frame_args(ctx, scene, n_boxes, corners12, detectors, models, results, status)) return rc;
     for (size_t b = 0; b < n_boxes; ++b) {
@@ -1212,7 +1310,8 @@ int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const
         cudaEventDestroy(ev[0]);
         return fail_msg(ctx, B200PPF_ERR_CUDA, "cv match: cudaEventCreate failed");
     }
-    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *edges, std::vector<double> *refined) {
+    auto match = [&](size_t b, const b200ppf_cloud *object, const b200ppf_cloud *edges, std::vector<double> *refined,
+                     std::vector<uint32_t> *cluster_votes) {
         b200ppf_object_result *res = &results[b];
         if (p.use_edges && edges->n == 0)
             return fail_msg(ctx, B200PPF_ERR_STATE, "cv match: the object has no edge point for Matching_S2B to pair with");
@@ -1225,13 +1324,16 @@ int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const
         if (rc) return rc;
         const size_t n_kept = std::min(n_clusters, cap);
         refined->resize(16 * n_kept);
-        for (size_t k = 0; k < n_kept; ++k) memcpy(refined->data() + 16 * k, poses[k].pose, 16 * sizeof(double));
+        cluster_votes->resize(n_kept);
+        for (size_t k = 0; k < n_kept; ++k) {
+            memcpy(refined->data() + 16 * k, poses[k].pose, 16 * sizeof(double));
+            (*cluster_votes)[k] = poses[k].num_votes;
+        }
         res->n_poses = (uint32_t)n_clusters;
-        res->votes = n_kept ? poses[0].num_votes : 0;
         return B200PPF_OK;
     };
     const int rc = match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && (p.use_edges || want_edges),
-                               results, status, object_out, edges_out, match);
+                               results, status, object_out, edges_out, verify, candidates, match);
     cudaEventDestroy(ev[0]);
     cudaEventDestroy(ev[1]);
     return rc;
@@ -1301,6 +1403,26 @@ int b200ppf_match_frame(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_b
                         const b200ppf_cloud *const *models, const b200ppf_table *const *tables, const b200ppf_object_params *params,
                         b200ppf_object_result *results, int *status) {
     return ppf_match(ctx, scene, n_boxes, corners12, models, tables, params, results, status, true, nullptr, nullptr);
+}
+
+int b200cv_match_frame_verified(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                                b200cv_detector *const *detectors, const b200ppf_cloud *const *models,
+                                const b200cv_object_params *params, const b200ppf_verify_params *verify,
+                                b200ppf_object_result *results, int *status, b200ppf_candidate *candidates) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params v;
+    if (int rc = verify_params(ctx, verify, &v)) return rc;
+    return cv_match(ctx, scene, n_boxes, corners12, detectors, models, params, results, status, true, nullptr, nullptr, &v, candidates);
+}
+
+int b200ppf_match_frame_verified(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                                 const b200ppf_cloud *const *models, const b200ppf_table *const *tables,
+                                 const b200ppf_object_params *params, const b200ppf_verify_params *verify,
+                                 b200ppf_object_result *results, int *status, b200ppf_candidate *candidates) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params v;
+    if (int rc = verify_params(ctx, verify, &v)) return rc;
+    return ppf_match(ctx, scene, n_boxes, corners12, models, tables, params, results, status, true, nullptr, nullptr, &v, candidates);
 }
 
 }  // extern "C"

@@ -232,6 +232,9 @@ int k6_icp_refine(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_cl
 // the same for several (model, scene, poses) jobs: one launch per distinct cluster size, every pose as the single call
 int k6_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, int max_iterations, float tolerance,
                         float rejection_scale, int num_levels, uint64_t *iterations_host);
+// the pose scores of b200ppf_score_poses (verify.cu) for checked arguments: fits of the jobs' poses, job-major
+int verify_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_verify_params &params,
+                       b200ppf_pose_fit *fits);
 
 // the context of an OpenCV-engine detector and whether it holds a trained model (k7_cvppf.cu)
 b200ppf_ctx *cv_detector_context(const b200cv_detector *d);
@@ -282,8 +285,11 @@ struct SceneGrid {
     uint32_t *orig = nullptr;        // cell-sorted position -> original scene index
 };
 
-// grid geometry for a bounding box and a search radius (host); returns the number of cells
-uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp);
+// grid geometry for a bounding box and a search radius (host), coarsened until it has at most max_cells cells; returns the
+// number of cells (0 for a non-finite box or radius)
+uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp, uint32_t max_cells = 1u << 22);
+// cell_start[c] (c = 0 .. n_cells) = the first of the n ascending sorted_ids that is >= c
+int grid_cell_starts(b200ppf_ctx *ctx, const uint32_t *sorted_ids, uint32_t n, uint32_t n_cells, uint32_t *cell_start);
 int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius, SceneGrid *out);
 void scene_grid_free(b200ppf_ctx *ctx, SceneGrid *g);
 struct SceneGridFree {

@@ -19,8 +19,6 @@ namespace b200ppf {
 
 namespace {
 
-constexpr uint32_t MAX_CELLS = 1u << 22;
-
 __global__ void grid_cell_ids_kernel(const float4 *__restrict__ pos, uint32_t n, GridParams g,
                                      uint32_t *__restrict__ cell_ids) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -63,7 +61,7 @@ void scene_grid_free(b200ppf_ctx *ctx, SceneGrid *g) {
     g->orig = nullptr;
 }
 
-uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp) {
+uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp, uint32_t max_cells) {
     GridParams &g = *gp;
     // cell edge: the search radius plus a margin that absorbs the rounding of the cell coordinate
     double cell = (radius > 0.0f ? (double)radius : 1e-3) * 1.001;
@@ -76,7 +74,7 @@ uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float r
     for (int guard = 0;; ++guard) {
         double cells = 1.0;
         for (int k = 0; k < 3; ++k) cells *= std::floor(ext[k] / cell) + 1.0;
-        if (cells <= (double)MAX_CELLS) break;
+        if (cells <= (double)max_cells) break;
         if (guard > 400) return 0;  // 1.26^400 exceeds any finite extent: unreachable for finite input
         cell *= 1.26;  // coarser cells stay correct (a superset of candidates), just less selective
     }
@@ -86,6 +84,11 @@ uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float r
     }
     g.inv_cell = (float)(1.0 / cell);
     return (uint32_t)g.dims[0] * (uint32_t)g.dims[1] * (uint32_t)g.dims[2];
+}
+
+int grid_cell_starts(b200ppf_ctx *ctx, const uint32_t *sorted_ids, uint32_t n, uint32_t n_cells, uint32_t *cell_start) {
+    PPF_LAUNCH(ctx, grid_offsets_kernel, (n_cells + 1 + 255) / 256, 256, 0, sorted_ids, n, n_cells, cell_start);
+    return B200PPF_OK;
 }
 
 int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius, SceneGrid *out) {
@@ -116,7 +119,7 @@ int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius,
     }
     const uint32_t *ids_sorted = in_alt ? ids1.p : ids0.p;
     const uint32_t *ord_sorted = in_alt ? ord1.p : ord0.p;
-    PPF_LAUNCH(ctx, grid_offsets_kernel, (out->n_cells + 1 + 255) / 256, 256, 0, ids_sorted, n, out->n_cells, out->cell_start);
+    if (int rc = grid_cell_starts(ctx, ids_sorted, n, out->n_cells, out->cell_start)) return rc;
     if (n) PPF_LAUNCH(ctx, grid_gather_kernel, gb, 256, 0, scene->pos, scene->nrm, ord_sorted, n, out->pos, out->nrm);
     out->orig = in_alt ? ord1.release() : ord0.release();  // sorted position -> original scene index
     return B200PPF_OK;
