@@ -131,6 +131,8 @@ void b200ppf_destroy(b200ppf_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
     if (ctx->d_stats) cudaFree(ctx->d_stats);
     if (ctx->d_peaks) cudaFree(ctx->d_peaks);
+    if (ctx->d_vote_queue) cudaFree(ctx->d_vote_queue);
+    if (ctx->d_fold) cudaFree(ctx->d_fold);
     if (ctx->d_hyps) cudaFree(ctx->d_hyps);
     if (ctx->d_assign) cudaFree(ctx->d_assign);
     if (ctx->stage) cudaFreeHost(ctx->stage);

@@ -6,7 +6,7 @@
 //   pair feature -> bucket -> for every (i, alpha_m) in the bucket acc[i][bin(alpha_m - alpha_s)]++;
 //   first maximum of acc (lowest flat index wins ties) -> pose = T_sg^-1 * Rx(theta) * T_mg.
 //
-// One CTA per (reference point, accumulator slice).  The accumulator slice — up to ~1600 model
+// One task per (reference point, accumulator slice): one CTA each, or persistent CTAs drawing them from a counter.  The accumulator slice — up to ~1600 model
 // rows x n_alpha 32-bit counters — lives in shared memory for the CTA's whole life, votes are
 // shared-memory reductions (red.shared.add), the peak is a warp-shuffle argmax, and slices merge
 // through one 64-bit atomicMax per CTA on a packed (votes, ~flat index) word, which reproduces
@@ -23,11 +23,12 @@
 //             The scene phase's own cell compares phases per entry; tables whose 2*pi/step is not an
 //             integer bin every entry in fixed point with guard bands, the literal double-precision
 //             form inside the bands.
-//   D  fold   tables of 2 M+ entries, flushes of FOLD_MIN_PAIRS+ candidates: a pair on the constant-shift path keeps
-//             only its own cell in phase C and leaves a code (key, q, cell) in the drained candidate queue.  The codes
-//             are sorted; for every (bucket, shift s) they touch, a warp reads off per cell how many pairs vote on it
-//             with that shift (prefix / suffix counts of the cells at q = s and q = s - 1) and walks the cell once,
-//             adding count x pairs.  Sums of integers in any order: the accumulators are those of one walk per pair.
+//   D  fold   tables of 2 M+ entries, tasks that flush more than once or hold FOLD_MIN_PAIRS+ candidates: a pair on the
+//             constant-shift path keeps only its own cell in phase C and leaves a code (key, q, cell) in its CTA's fold
+//             buffer, across flushes.  At the end of the task (or of a scope of FOLD_SCOPE codes) the codes are sorted; for
+//             every (bucket, shift s) they touch, a warp reads off per cell how many pairs vote on it with that shift
+//             (prefix / suffix counts of the cells at q = s and q = s - 1) and walks the cell once, adding count x pairs.
+//             Sums of integers in any order: the accumulators are those of one walk per pair.
 // The accumulator slice is bin-major (word = bin * pitch + row, pitch a multiple of 32): the bank of a vote
 // is (row mod 32) whatever the scene pair, and the table build orders every phase cell so that 32
 // consecutive entries hit 32 different banks.
@@ -71,9 +72,8 @@ static_assert(CAND_CAP >= 2 * VOTE_THREADS_LARGE, "flush threshold must leave on
 #ifndef B200PPF_FOLD_MIN_PAIRS
 #define B200PPF_FOLD_MIN_PAIRS 1024
 #endif
-constexpr uint32_t FOLD_MIN_PAIRS = B200PPF_FOLD_MIN_PAIRS;  // flushes with fewer candidates keep one walk per pair
+constexpr uint32_t FOLD_MIN_PAIRS = B200PPF_FOLD_MIN_PAIRS;  // single-flush tasks with fewer candidates keep one walk per pair
 constexpr size_t FOLD_MIN_ENTRIES = 1u << 21;  // tables below this walk short buckets: folding does not repay its sort
-static_assert((CAND_CAP & (CAND_CAP - 1)) == 0, "the fold codes of a flush are sorted in place (bitonic)");
 
 // One in-radius scene pair with a non-empty bucket.  Phase-sorted tables: the bucket's merged words are
 // [off, off + len); those below k_below lie under the scene pair's phase (shift constant c_below), those from
@@ -96,8 +96,16 @@ struct __align__(16) WorkItem {
 constexpr size_t queue_bytes(int threads) { return CAND_CAP * sizeof(uint32_t) + (size_t)threads * sizeof(WorkItem); }
 constexpr size_t SMALL_SHAPE_SMEM_MAX = 111 * 1024;  // two such CTAs (+ static + system reserve) share one SM
 constexpr size_t STATIC_RESERVE = 2048;  // static shared + the 1 KB the system reserves per CTA
-// the folded groups of a flush (at most two per fold code) live where the consumed work items were
-static_assert(2 * CAND_CAP * sizeof(uint32_t) <= VOTE_THREADS_SMALL * sizeof(WorkItem), "fold groups must fit the item queue");
+// Fold scope: a task's fold codes collect in its CTA's slot of a global buffer (L2-resident) across flushes, and phase D
+// folds them once the next flush might not fit, or at the end of the task.  D sorts the codes where the idle candidate and
+// item queues are, so the scope is the largest power of two of words both launch shapes' queues hold (8 192 words = the
+// 512-thread shape's queues exactly).  The groups (at most two per code) then overwrite the codes in the slot, which the
+// sort has taken into shared memory: a slot is 2 * FOLD_SCOPE words.
+constexpr uint32_t FOLD_SCOPE = 8192;
+constexpr size_t FOLD_SLOT_WORDS = 2 * (size_t)FOLD_SCOPE;
+static_assert(FOLD_SCOPE * sizeof(uint32_t) <= queue_bytes(VOTE_THREADS_SMALL) && (FOLD_SCOPE & (FOLD_SCOPE - 1)) == 0,
+              "the fold codes of a scope are sorted in the idle queues (bitonic)");
+static_assert(FOLD_SCOPE >= CAND_CAP, "a scope must take one whole flush");
 
 struct VoteArgs {
     const float4 *pos, *nrm;    // scene, original order (reference points are addressed by index)
@@ -123,19 +131,21 @@ struct VoteArgs {
     unsigned long long *peaks;
     unsigned long long *stats;
     uint32_t *acc_dump;  // debug: full accumulator of reference 0 (n_model * n_alpha)
-    // Several GPUs sharing ONE work queue (b200ppf_group): persistent CTAs draw (reference, slice) tasks from a counter in
-    // rank 0's memory with system-scope atomics over NVLink — whichever GPU is free takes the next task, so the ranks
-    // finish together whatever the scene's cost distribution — and merge each task's peak into EVERY rank's peak array
-    // with a system-scope 64-bit atomicMax.  When its queue is exhausted, the last CTA of a rank raises that rank's flag
-    // in every rank's flag array.
-    uint32_t *queue;  // nullptr: the grid is (reference, slice) and peaks are local
+    // Persistent CTAs (as many as the device holds at once) draw (reference, slice) tasks from a counter.  One GPU, a
+    // folding table: the counter is the context's, peaks are local.  Several GPUs sharing ONE work queue (b200ppf_group):
+    // the counter is in rank 0's memory, drawn with system-scope atomics over NVLink — whichever GPU is free takes the next task, so the
+    // ranks finish together whatever the scene's cost distribution — and each task's peak is merged into EVERY rank's peak
+    // array with a system-scope 64-bit atomicMax.  When its queue is exhausted, the last CTA of a rank raises that rank's
+    // flag in every rank's flag array.
+    uint32_t *queue;  // nullptr: the grid is (reference, slice)
     unsigned long long *peer_peaks[MAX_PEERS];
     uint32_t *peer_flags[MAX_PEERS];
-    int n_peers;
+    int n_peers;  // 0: one GPU
     uint32_t signal_slot, signal_value;
     uint32_t *done_counter;
     int no_sub_phase;  // debug (B200PPF_NO_SUB_PHASE): compare every own-cell entry in full
     uint32_t fold_qbits;  // bits of q in a fold code (key, q, cell); 0: every pair walks its own bucket
+    uint32_t *fold_buf;   // folding tables: FOLD_SLOT_WORDS per CTA of the launch, slot = blockIdx.x
 };
 
 __device__ __forceinline__ unsigned long long shfl_xor_u64(unsigned long long v, int o) {
@@ -177,6 +187,33 @@ __device__ __forceinline__ void red_shared_inc_if_lt(uint32_t addr, uint32_t k, 
 // count of a merged word times the scene pairs that cast it: one pair's item (the constant 1) or a folded group
 __device__ __forceinline__ uint32_t times(uint32_t cnt, std::integral_constant<uint32_t, 1>) { return cnt; }
 __device__ __forceinline__ uint32_t times(uint32_t cnt, uint32_t pairs) { return cnt * pairs; }
+
+// Phase timing (instrumented builds only: -DB200PPF_PHASE_TIMING, e.g. tools/build_variant.sh).  Thread 0 reads
+// %globaltimer after the barriers that end each phase and sums the CTA's wall time per phase over the launch's tasks,
+// apart for single-flush and multi-flush tasks; lane 0 of every warp sums its own time in phase C's shift ranges and in
+// its own cells.  The last CTA of the launch prints one line per task class and clears the sums.
+#ifdef B200PPF_PHASE_TIMING
+enum { PT_PROLOGUE, PT_SWEEP, PT_PAIRS, PT_VOTES, PT_FOLD, PT_PEAK, PT_C_SHIFT, PT_C_OWN, PT_TASKS, PT_N };
+__device__ unsigned long long g_phase_ns[2][PT_N];
+__device__ unsigned int g_phase_done;
+__device__ __forceinline__ unsigned long long global_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+#define PT_MARK(k)                                      \
+    do {                                                \
+        if (tid == 0) {                                 \
+            const unsigned long long now_ = global_ns(); \
+            pt[k] += now_ - pt_t;                       \
+            pt_t = now_;                                \
+        }                                               \
+    } while (0)
+#else
+#define PT_MARK(k) \
+    do {           \
+    } while (0)
+#endif
 
 // One vote of the per-entry path of tables without phase cells (alpha mode A), in fixed point (ppf_math.cuh,
 // alpha_bin_fixed):  X = A_m - C_s  (wraps like the angle),  hi = mulhi(X, T_fix) = bin.position,
@@ -222,6 +259,11 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
     __shared__ unsigned long long s_stat[4];
 
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+#ifdef B200PPF_PHASE_TIMING
+    __shared__ unsigned long long s_warp_ns[2];
+    unsigned long long pt[PT_N] = {}, pt_t = global_ns(), wt_shift = 0, wt_own = 0;
+    if (tid == 0) s_warp_ns[0] = s_warp_ns[1] = 0;
+#endif
     const uint32_t slice_base = slice * a.kp.slice_rows;
     const uint32_t rows = min(a.kp.slice_rows, a.n_model - slice_base);
     const uint32_t pitch = a.kp.row_pitch;               // words between two alpha columns (multiple of 32)
@@ -271,12 +313,16 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
     for (uint32_t k = tid; k < acc_len; k += THREADS) acc[k] = 0;
     __syncthreads();
     if (draws) *next_task = drawn;  // everyone has read the current task before the barrier above
+    PT_MARK(PT_PROLOGUE);
 
     const uint32_t lf = a.bp.cells_log2;
     const uint32_t *slice_offsets = a.sub_offsets + (((size_t)slice * a.kp.key_space) << lf);
     const uint32_t *slice_moffsets = BULK ? a.msub_offsets + (((size_t)slice * a.kp.key_space) << lf) : nullptr;
     const uint32_t fmask = (1u << a.bp.fix_shift) - 1u;
     uint32_t st_examined = 0, st_in_radius = 0, st_nonempty = 0, st_votes = 0, st_skipped = 0;
+    uint32_t neighbourhood = 0;
+#pragma unroll
+    for (int r = 0; r < 9; ++r) neighbourhood += s_run_end[r] - s_run_start[r];
 
     // shift range [kb, ke) of merged words mp[]: add count * mult at umin(hot word - c, hot word - c + one turn).  The
     // arrays carry ENTRY_PAD readable words past the end, so the partial batch loads unclamped.  mult is the constant 1
@@ -316,12 +362,18 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
         }
     };
 
-    // phases B + C (+ D) over the buffered candidates
-    auto flush = [&]() {
+    // this CTA's fold buffer: the codes of the current scope, then the groups of phase D
+    uint32_t *const fold_slot = FOLD ? a.fold_buf + (size_t)blockIdx.x * FOLD_SLOT_WORDS : nullptr;
+
+    // phases B + C (+ D) over the buffered candidates; `last`: the task's final flush (earlier ones are taken mid-sweep)
+    bool flushed = false;  // an earlier flush was taken: the task flushes more than once
+    auto flush = [&](const bool last) {
+        PT_MARK(PT_SWEEP);
         const uint32_t ncand = s_ncand;
-        // Fold the constant-shift walks of this flush's pairs (D below): on tables of FOLD_MIN_ENTRIES+ entries, when the
-        // flush holds enough pairs to share buckets.  Light reference points keep one walk per pair.
-        const bool fold = FOLD && BULK && ncand >= FOLD_MIN_PAIRS;
+        // Fold the constant-shift walks of the task's pairs (D below) on tables of FOLD_MIN_ENTRIES+ entries, when the task
+        // has enough pairs to share buckets: it flushes more than once (every flush folds, a short last one too) or its
+        // one flush holds FOLD_MIN_PAIRS+ candidates.  Light reference points keep one walk per pair.
+        const bool fold = FOLD && BULK && (!last || flushed || ncand >= FOLD_MIN_PAIRS);
         for (uint32_t c0 = 0; c0 < ncand; c0 += THREADS) {
             // ---- B: pair features -> work items -------------------------------------------------
             const uint32_t c = c0 + tid;
@@ -393,16 +445,16 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                     rank = __shfl_sync(same, rank, leader) + __popc(same & ((1u << lane) - 1u));
                 }
             }
-            __syncthreads();
-            if (fold) {  // every candidate of the round has been read: the fold codes take the front of the queue
+            if (fold) {  // the fold codes join the scope's codes in the CTA's fold buffer
                 const uint32_t fm = __ballot_sync(0xFFFFFFFFu, folds);
                 if (fm) {
                     uint32_t b = 0;
                     if (lane == (uint32_t)(__ffs(fm) - 1)) b = atomicAdd(&s_nfold, __popc(fm));
                     b = __shfl_sync(0xFFFFFFFFu, b, __ffs(fm) - 1);
-                    if (folds) cand[b + __popc(fm & ((1u << lane) - 1u))] = code;
+                    if (folds) fold_slot[b + __popc(fm & ((1u << lane) - 1u))] = code;
                 }
             }
+            __syncthreads();
             if (push) {
                 uint32_t slot = rank;
 #pragma unroll
@@ -429,6 +481,7 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 s_nitems = total;
             }
             __syncthreads();
+            PT_MARK(PT_PAIRS);
             // ---- C: votes ---------------------------------------------------------------------
             const uint32_t nitems = s_nitems;
             for (;;) {
@@ -439,11 +492,21 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 const WorkItem wi = items[w];
                 const uint32_t len = wi.len;
                 const uint32_t *mp = a.merged_w + wi.off;
+#ifdef B200PPF_PHASE_TIMING
+                unsigned long long wt0 = global_ns();
+#endif
                 if (BULK) {
                     const std::integral_constant<uint32_t, 1> one;
                     if (wi.k_below) shift_range(mp, 0u, wi.k_below, wi.c_below, one);
                     if (wi.k_above < len) shift_range(mp, wi.k_above, len, wi.c_below - unit, one);
                 }
+#ifdef B200PPF_PHASE_TIMING
+                {
+                    const unsigned long long t = global_ns();
+                    wt_shift += t - wt0;
+                    wt0 = t;
+                }
+#endif
                 if (wi.e_len) {
                     // per-entry range [0, e_end) of the unmerged entry arrays
                     const uint32_t *wp = a.entry_w + wi.e_off;
@@ -564,8 +627,12 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                                              st_skipped);
                     }
                 }
+#ifdef B200PPF_PHASE_TIMING
+                wt_own += global_ns() - wt0;
+#endif
             }
             __syncthreads();
+            PT_MARK(PT_VOTES);
             if (tid == 0) {
                 s_nitems = 0;
                 s_next = 0;
@@ -573,18 +640,19 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
             if (tid >= 64 && tid < 72) s_cls[tid - 64] = 0;
             __syncthreads();
         }
+        // the scope ends with the task, or when the next flush might not fit the fold buffer
         const uint32_t n = fold ? s_nfold : 0u;
-        if (n) {
+        if (n && (last || n > FOLD_SCOPE - CAND_CAP)) {
             // ---- D: folded shift ranges ------------------------------------------------------------
             // A folding pair (q, c) votes on cell k of its bucket with shift q + 1 below c and q above it, so the pairs
             // of one bucket that vote on cell k with shift s number
             //     m_s(k) = #{q = s, c < k} + #{q = s - 1 (mod N_T), c > k},
             // and one walk of the cell adding count * m_s(k) casts all their votes.  The codes (key, q, c) are sorted
-            // (bitonic, in place), so both terms are differences of lower bounds.
+            // (bitonic, in the idle candidate and item queues), so both terms are differences of lower bounds.
             const uint32_t qb = a.fold_qbits, qmask = (1u << qb) - 1u, ncell = 1u << lf;
             uint32_t np = 32;
             while (np < n) np <<= 1;
-            for (uint32_t i = n + tid; i < np; i += THREADS) cand[i] = 0xFFFFFFFFu;  // codes have at most 31 bits
+            for (uint32_t i = tid; i < np; i += THREADS) cand[i] = i < n ? fold_slot[i] : 0xFFFFFFFFu;  // codes have at most 31 bits
             __syncthreads();
             for (uint32_t k = 2; k <= np; k <<= 1)
                 for (uint32_t j = k >> 1; j > 0; j >>= 1) {
@@ -612,7 +680,7 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 return lo;
             };
             // one group (key, s) per s that some run (key, q) touches: s = q, and s = q + 1 when no run (key, q + 1) exists
-            uint32_t *groups = reinterpret_cast<uint32_t *>(items);  // the round's items are consumed
+            uint32_t *const groups = fold_slot;  // the codes are in shared memory now
             for (uint32_t i = tid; i < n; i += THREADS) {
                 const uint32_t run = cand[i] >> lf;
                 if (i == 0 || (cand[i - 1] >> lf) != run) {
@@ -654,6 +722,7 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 }
             }
             __syncthreads();
+            PT_MARK(PT_FOLD);
             if (tid == 0) {
                 s_next = 0;
                 s_nfold = 0;
@@ -661,6 +730,7 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
             }
         }
         if (tid == 0) s_ncand = 0;
+        if (!last) flushed = true;
         __syncthreads();
     };
 
@@ -684,9 +754,6 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
             if (in) cand[b + __popc(m & ((1u << lane) - 1u))] = s;
         }
     };
-    uint32_t neighbourhood = 0;
-#pragma unroll
-    for (int r = 0; r < 9; ++r) neighbourhood += s_run_end[r] - s_run_start[r];
     if (neighbourhood <= CAND_CAP) {
         // the common case: every point of the 27 cells fits the queue — no barriers inside the sweep
         for (int r = 0; r < 9; ++r) {
@@ -702,11 +769,11 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                 __syncthreads();
                 const uint32_t buffered = s_ncand;
                 __syncthreads();  // nobody may start the next sweep's atomics before everyone has read
-                if (buffered > CAND_CAP - THREADS) flush();
+                if (buffered > CAND_CAP - THREADS) flush(false);
             }
         }
     }
-    flush();
+    flush(true);
 
     // ---- peak: first maximum in (i, bin) order == max of (votes, ~flat) ---------------------------
     // one thread per model row (consecutive threads read consecutive words of a column): the spare column n_alpha
@@ -748,13 +815,27 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
         atomicAdd(&s_stat[2], (unsigned long long)st_nonempty);
         atomicAdd(&s_stat[3], (unsigned long long)st_votes);
         atomicAdd(&s_stat[3], 0ull - (unsigned long long)st_skipped);  // NaN alphas cast no vote
+#ifdef B200PPF_PHASE_TIMING
+        atomicAdd(&s_warp_ns[0], wt_shift);
+        atomicAdd(&s_warp_ns[1], wt_own);
+#endif
     }
     __syncthreads();
+    PT_MARK(PT_PEAK);
+#ifdef B200PPF_PHASE_TIMING
+    if (tid == 0) {
+        unsigned long long *g = g_phase_ns[flushed ? 1 : 0];
+        for (int k = 0; k < PT_C_SHIFT; ++k) atomicAdd(g + k, pt[k]);
+        atomicAdd(g + PT_C_SHIFT, s_warp_ns[0]);
+        atomicAdd(g + PT_C_OWN, s_warp_ns[1]);
+        atomicAdd(g + PT_TASKS, 1ull);
+    }
+#endif
     if (tid == 0) {
 #pragma unroll
         for (int w = 1; w < (THREADS / 32); ++w) best = max(best, s_best[w]);
         if (best) {
-            if (a.queue) {
+            if (a.n_peers) {
                 for (int g = 0; g < a.n_peers; ++g) atomicMax_system(a.peer_peaks[g] + ref_i, best);
             } else {
                 atomicMax(a.peaks + ref_i, best);
@@ -791,9 +872,10 @@ __global__ void ref_cost_kernel(const float4 *__restrict__ pos, const uint32_t *
 template <int MODE, bool SEAM, bool BULK, int THREADS, bool FOLD>
 __global__ void __launch_bounds__(THREADS, THREADS == 1024 ? 1 : B200PPF_VOTE_MINBLOCKS)
 ppf_vote_kernel(const VoteArgs a) {
-    // Either one CTA per (reference point, slice) — the grid is (positions, slices) — or persistent CTAs on a queue
-    // shared by all ranks.  One call site serves both, so the two modes run the same machine code.  Slice-major order
-    // either way: the CTAs in flight share one slice of the table in L2.
+    // Either one CTA per (reference point, slice) — the grid is (positions, slices) — or persistent CTAs drawing those
+    // tasks from a queue counter (folding tables: a CTA owns one slot of the fold buffer for all its tasks; several GPUs:
+    // the queue shared by all ranks).  One call site serves both, so the two modes run the same machine code.  Slice-major
+    // order either way: the CTAs in flight share one slice of the table in L2.
     __shared__ uint32_t s_task;
     const bool persistent = a.queue != nullptr;
     const uint32_t total = a.ref_count * a.kp.n_slices;
@@ -804,9 +886,26 @@ ppf_vote_kernel(const VoteArgs a) {
         if (task >= total) break;
         const uint32_t pos = task % a.ref_count;
         vote_task<MODE, SEAM, BULK, THREADS, FOLD>(a, a.ref_order ? a.ref_order[pos] : pos, task / a.ref_count,
-                                             persistent ? &s_task : nullptr);
+                                                   persistent ? &s_task : nullptr);
         if (!persistent) break;
     }
+#ifdef B200PPF_PHASE_TIMING
+    if (threadIdx.x == 0) {
+        __threadfence();
+        if (atomicAdd(&g_phase_done, 1u) == gridDim.x * gridDim.y - 1) {
+            __threadfence();
+            for (int c = 0; c < 2; ++c) {
+                unsigned long long *g = g_phase_ns[c];
+                printf("k3_phase_ns flushes=%s tasks=%llu prologue=%llu sweep=%llu pairs=%llu votes=%llu fold=%llu peak=%llu "
+                       "votes_shift_warp=%llu votes_own_warp=%llu\n",
+                       c ? "many" : "one", g[PT_TASKS], g[PT_PROLOGUE], g[PT_SWEEP], g[PT_PAIRS], g[PT_VOTES], g[PT_FOLD],
+                       g[PT_PEAK], g[PT_C_SHIFT], g[PT_C_OWN]);
+                for (int k = 0; k < PT_N; ++k) g[k] = 0;
+            }
+            g_phase_done = 0;
+        }
+    }
+#endif
     if (threadIdx.x == 0 && a.done_counter) {
         __threadfence_system();  // this CTA's peaks are visible everywhere before it counts as done
         if (atomicAdd(a.done_counter, 1u) == gridDim.x - 1) {
@@ -998,7 +1097,10 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
         a.peer_flags[g] = nullptr;
     }
     const size_t smem = vote_smem_bytes(t);
-    dim3 grid_dim((unsigned)ref_count, t->info.n_slices);
+    const int threads = vote_threads(t);
+    // persistent: as many CTAs as the device holds at once (one GPU: no more than there are tasks)
+    unsigned ctas = (unsigned)(ctx->sm_count * (threads == VOTE_THREADS_SMALL ? B200PPF_VOTE_MINBLOCKS : 1));
+    dim3 grid_dim(ctas);
     if (queue) {
         a.queue = queue->counter;
         a.n_peers = queue->n_peers;
@@ -1009,8 +1111,21 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
             a.peer_peaks[g] = queue->peer_peaks[g];
             a.peer_flags[g] = queue->flags[g];
         }
-        // persistent: as many CTAs as the device holds at once
-        grid_dim = dim3((unsigned)(ctx->sm_count * (vote_threads(t) == VOTE_THREADS_SMALL ? B200PPF_VOTE_MINBLOCKS : 1)), 1);
+    } else if (a.fold_qbits) {
+        // a folding table on one GPU: persistent CTAs on the context's counter, so that each owns a fold-buffer slot
+        ctas = (unsigned)std::min<size_t>(ctas, ref_count * t->info.n_slices);
+        grid_dim = dim3(ctas);
+        if (!ctx->d_vote_queue) PPF_CUDA(ctx, cudaMalloc(&ctx->d_vote_queue, sizeof(uint32_t)));
+        PPF_CUDA(ctx, cudaMemsetAsync(ctx->d_vote_queue, 0, sizeof(uint32_t), ctx->stream));
+        a.queue = ctx->d_vote_queue;
+    } else {
+        // the other tables on one GPU: one CTA per task (C1's 54 µs vote kernel measured 60-61 µs persistent, DESIGN §3)
+        grid_dim = dim3((unsigned)ref_count, t->info.n_slices);
+    }
+    a.fold_buf = nullptr;
+    if (a.fold_qbits) {
+        PPF_CUDA(ctx, grow_buffer(&ctx->d_fold, &ctx->fold_cap, ctas * FOLD_SLOT_WORDS));
+        a.fold_buf = ctx->d_fold;
     }
     cudaEventRecord(ctx->ev_vote[1], ctx->stream);  // grid build ends, voting starts
     // heaviest neighbourhood first once the launch is several waves deep and the buckets long enough for a task to take
@@ -1043,7 +1158,6 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
         if (threads == VOTE_THREADS_SMALL) LAUNCH_VOTE_T(M, S, B, VOTE_THREADS_SMALL, F);  \
         else LAUNCH_VOTE_T(M, S, B, VOTE_THREADS_LARGE, F);                            \
     } while (0)
-    const int threads = vote_threads(t);
     if (ctx->alpha_mode == ALPHA_MODE_B) LAUNCH_VOTE(ALPHA_MODE_B, false, false, false);
     else if (a.bp.bulk && a.fold_qbits) LAUNCH_VOTE(ALPHA_MODE_A, false, true, true);
     else if (a.bp.bulk) LAUNCH_VOTE(ALPHA_MODE_A, false, true, false);  // an integer T has no separate seam band

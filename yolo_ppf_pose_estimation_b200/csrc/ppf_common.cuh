@@ -43,6 +43,9 @@ struct b200ppf_ctx {
     unsigned long long *d_stats = nullptr;  // [4]
     unsigned long long *d_peaks = nullptr;  // packed (votes<<32 | ~flat) per reference
     size_t peaks_cap = 0;
+    uint32_t *d_vote_queue = nullptr;  // task counter of one-GPU vote launches on folding tables
+    uint32_t *d_fold = nullptr;        // fold codes and groups of folding vote launches, one slot per CTA
+    size_t fold_cap = 0;
     b200ppf_hypothesis *d_hyps = nullptr;  // staging for host-output votes
     size_t hyps_cap = 0;
     // cluster scratch of the last cluster call
