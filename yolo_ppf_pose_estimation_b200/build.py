@@ -16,7 +16,7 @@ CSRC = os.path.join(_HERE, "csrc")
 BUILD_DIR = os.path.join(_HERE, "_build")
 LIB_PATH = os.path.join(BUILD_DIR, "libb200ppf.so")
 
-SOURCES = ["capi.cu", "radix_sort.cu", "k1_features.cu", "k2_table.cu", "k3_vote.cu", "scene_grid.cu", "k4_cluster.cu", "verify.cu",
+SOURCES = ["capi.cu", "sort_scan.cu", "k1_features.cu", "k2_table.cu", "k3_vote.cu", "scene_grid.cu", "k4_cluster.cu", "verify.cu",
            "k5_transform.cu", "k6_icp.cu", "prep.cu", "microbench.cu", "group.cu", "k7_cvppf.cu"]
 HEADERS = ["ppf_common.cuh", "ppf_math.cuh", os.path.join("..", "..", "include", "b200ppf.h")]
 

@@ -162,20 +162,6 @@ keys_from_cloud_kernel(const float4 *__restrict__ pos, const float4 *__restrict_
     if ((threadIdx.x & 31) == 0 && mx >= 0) atomicMax(max_f4_bits, mx);
 }
 
-// offsets[k] = first sorted position whose sort key is >= k << shift, for k in [0, total_keys]
-__global__ void csr_offsets_kernel(const uint32_t *__restrict__ sorted_keys, uint32_t n, uint32_t total_keys,
-                                   uint32_t shift, uint32_t *__restrict__ offsets) {
-    uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k > total_keys) return;
-    const uint32_t want = k << shift;
-    uint32_t lo = 0, hi = n;
-    while (lo < hi) {
-        uint32_t mid = lo + ((hi - lo) >> 1);
-        if (sorted_keys[mid] < want) lo = mid + 1; else hi = mid;
-    }
-    offsets[k] = lo;
-}
-
 // sub_offsets[k'] for k' = key << shift | cell: the search is confined to the key's own bucket; the sort keys carry
 // low_bits more bits below the cell (the bin of alpha_m of tables with merged votes)
 __global__ void csr_sub_offsets_kernel(const uint32_t *__restrict__ sorted_keys, const uint32_t *__restrict__ offsets,
@@ -524,8 +510,8 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
 
     // ---- sort -----------------------------------------------------------------------------------
     bool in_alt = false;
-    int rc = radix_sort_u32(ctx, keys[0], keys[1], idx[0], idx[1], alp[0], alp[1], count, (int)info.key_bits,
-                            /*v0_iota=*/true, &in_alt);
+    int rc = radix_sort_u32(ctx, keys[0], keys[1], idx[0], idx[1], alp[0], alp[1], count,
+                            (1ull << info.key_bits) - 1, /*v0_iota=*/true, &in_alt);
     if (rc) return rc;
     const int s = in_alt ? 1 : 0;
     cudaEventRecord(ctx->ev[2], ctx->stream);
@@ -539,8 +525,8 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
         return B200PPF_OK;
     };
     if ((rc = alloc_arrays(0, 1))) return rc;  // offsets, sub_offsets
-    PPF_LAUNCH(ctx, csr_offsets_kernel, (total_keys + 1 + 255) / 256, 256, 0, keys[s], (uint32_t)count, total_keys,
-               cells_log2 + merge_bits, t->offsets);
+    // offsets[k] = first sorted position whose sort key is >= k << (cells_log2 + merge_bits), for k in [0, total_keys]
+    if ((rc = lower_bounds(ctx, keys[s], (uint32_t)count, nullptr, total_keys, cells_log2 + merge_bits, t->offsets))) return rc;
     if (cells_log2)
         PPF_LAUNCH(ctx, csr_sub_offsets_kernel, (total_sub + 1 + 255) / 256, 256, 0, keys[s], t->offsets, total_sub, cells_log2,
                    merge_bits, t->sub_offsets);
@@ -577,7 +563,7 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
         uint32_t n_merged = n_entries;
         if (merge_bits) {
             PPF_LAUNCH(ctx, merge_heads_kernel, (n_entries + 255) / 256, 256, 0, keys[s], idx[s], n_entries, (uint32_t)n, head);
-            if ((rc = flag_scan_u32(ctx, head, n_entries, rank, &n_merged))) return rc;
+            if ((rc = flag_scan_host(ctx, head, n_entries, rank, &n_merged))) return rc;
         }
         t->n_merged = n_merged;
         if ((rc = alloc_arrays(6, 7))) return rc;  // merged_w, msub_offsets

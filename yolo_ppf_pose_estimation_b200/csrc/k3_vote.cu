@@ -1139,10 +1139,8 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
         PPF_CUDA(ctx, order_alt.alloc(ref_count));
         PPF_LAUNCH(ctx, ref_cost_kernel, (unsigned)((ref_count + 255) / 256), 256, 0, scene->pos, grid.cell_start, grid.gp,
                    (uint32_t)ref_first, (uint32_t)ref_step, (uint32_t)ref_count, (uint32_t)scene->n, cost.p);
-        int bits = 1;
-        while ((scene->n >> bits) != 0) ++bits;  // costs are counts of scene points
-        bool in_alt = false;
-        rc = radix_sort_u32(ctx, cost.p, cost_alt.p, order.p, order_alt.p, nullptr, nullptr, ref_count, bits, /*v0_iota=*/true,
+        bool in_alt = false;  // costs are counts of scene points
+        rc = radix_sort_u32(ctx, cost.p, cost_alt.p, order.p, order_alt.p, nullptr, nullptr, ref_count, scene->n, /*v0_iota=*/true,
                             &in_alt);
         if (rc) return rc;
         a.ref_order = in_alt ? order_alt.p : order.p;

@@ -34,7 +34,7 @@ namespace {
 
 constexpr uint32_t NONE = 0xFFFFFFFFu;
 constexpr uint32_t ST_UNDECIDED = 0, ST_LEADER = 1, ST_MEMBER = 2;
-constexpr int SCAN_BLOCK = 1024;
+static_assert(ST_LEADER == 1, "the leader numbering scans state: flag_scan counts the entries equal to 1");
 
 struct PoseRows {  // 3x4 row-major pose as three float4 rows
     float4 r0, r1, r2;
@@ -89,18 +89,6 @@ __global__ void cluster_gather_kernel(const b200ppf_hypothesis *__restrict__ hyp
     votes[k] = h.votes;
     cell_keys[k] = cell_hash(cell_of(h.pose[3], hp.inv_cell), cell_of(h.pose[7], hp.inv_cell),
                              cell_of(h.pose[11], hp.inv_cell), hp.mask);
-}
-
-__global__ void cluster_cell_offsets_kernel(const uint32_t *__restrict__ sorted_keys, uint32_t n, uint32_t n_cells,
-                                            uint32_t *__restrict__ cell_start) {
-    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c > n_cells) return;
-    uint32_t lo = 0, hi = n;
-    while (lo < hi) {
-        const uint32_t mid = lo + ((hi - lo) >> 1);
-        if (sorted_keys[mid] < c) lo = mid + 1; else hi = mid;
-    }
-    cell_start[c] = lo;
 }
 
 // Walk the earlier (rank < k) entries of the per-cell lists around pose k, in rank order inside every cell, and call
@@ -197,14 +185,19 @@ cluster_round_kernel(const PoseRows *__restrict__ poses, const uint32_t *__restr
     else atomicAdd(undecided, 1u);
 }
 
-// list compaction: keep[s] = the entry's pose is (still) of interest; the scan that follows preserves the order
-__global__ void cluster_keep_flags_kernel(const uint32_t *__restrict__ cell_rank, const uint32_t *__restrict__ n_list,
+// list compaction: keep[s] = the entry's pose is (still) of interest; the scan that follows preserves the order.  n bounds
+// the list's length *n_list on the host: the entries between the two are not kept.
+__global__ void cluster_keep_flags_kernel(const uint32_t *__restrict__ cell_rank, uint32_t n, const uint32_t *__restrict__ n_list,
                                           const uint32_t *__restrict__ state, uint32_t leaders_only,
                                           uint32_t *__restrict__ keep) {
     const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= *n_list) return;
-    const uint32_t st = state[cell_rank[s]];
-    keep[s] = leaders_only ? (st == ST_LEADER) : (st != ST_MEMBER);
+    if (s >= n) return;
+    uint32_t k = 0;
+    if (s < *n_list) {
+        const uint32_t st = state[cell_rank[s]];
+        k = leaders_only ? (st == ST_LEADER) : (st != ST_MEMBER);
+    }
+    keep[s] = k;
 }
 
 __global__ void cluster_compact_kernel(const uint32_t *__restrict__ cell_rank, const uint32_t *__restrict__ cell_keys,
@@ -215,113 +208,6 @@ __global__ void cluster_compact_kernel(const uint32_t *__restrict__ cell_rank, c
     if (s >= *n_list || !keep[s]) return;
     rank_out[pos[s]] = cell_rank[s];
     keys_out[pos[s]] = cell_keys[s];
-}
-
-// cell bounds of a (compacted) list whose length lives on the device
-__global__ void cluster_cell_offsets_dev_kernel(const uint32_t *__restrict__ sorted_keys, const uint32_t *__restrict__ n_list,
-                                                uint32_t n_cells, uint32_t *__restrict__ cell_start) {
-    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c > n_cells) return;
-    uint32_t lo = 0, hi = *n_list;
-    while (lo < hi) {
-        const uint32_t mid = lo + ((hi - lo) >> 1);
-        if (sorted_keys[mid] < c) lo = mid + 1; else hi = mid;
-    }
-    cell_start[c] = lo;
-}
-
-// order-preserving positions of the kept list entries (the list length lives on the device)
-__global__ void __launch_bounds__(SCAN_BLOCK)
-keep_count_kernel(const uint32_t *__restrict__ keep, const uint32_t *__restrict__ n_list, uint32_t *__restrict__ block_sums) {
-    const uint32_t k = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-    const int c = __syncthreads_count(k < *n_list && keep[k] != 0u);
-    if (threadIdx.x == 0) block_sums[blockIdx.x] = (uint32_t)c;
-}
-
-__global__ void __launch_bounds__(SCAN_BLOCK)
-keep_index_kernel(const uint32_t *__restrict__ keep, const uint32_t *__restrict__ n_list,
-                  const uint32_t *__restrict__ block_sums, uint32_t *__restrict__ pos) {
-    __shared__ uint32_t warp_tot[32];
-    const uint32_t k = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-    const uint32_t v = (k < *n_list && keep[k] != 0u) ? 1u : 0u;
-    const uint32_t m = __ballot_sync(0xFFFFFFFFu, v);
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) warp_tot[warp] = __popc(m);
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        uint32_t w = warp_tot[threadIdx.x], wi = w;
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, wi, o);
-            if (threadIdx.x >= (uint32_t)o) wi += t;
-        }
-        warp_tot[threadIdx.x] = wi - w;
-    }
-    __syncthreads();
-    if (k < *n_list) pos[k] = block_sums[blockIdx.x] + warp_tot[warp] + __popc(m & ((1u << lane) - 1u));
-}
-
-// exclusive prefix sum of the leader flags -> cluster creation index of every leader
-__global__ void __launch_bounds__(SCAN_BLOCK)
-leader_count_kernel(const uint32_t *__restrict__ state, uint32_t n, uint32_t *__restrict__ block_sums) {
-    const uint32_t k = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-    const int c = __syncthreads_count(k < n && state[k] == ST_LEADER);
-    if (threadIdx.x == 0) block_sums[blockIdx.x] = (uint32_t)c;
-}
-
-__global__ void __launch_bounds__(SCAN_BLOCK)
-leader_scan_blocks_kernel(uint32_t *__restrict__ block_sums, uint32_t n_blocks, uint32_t *__restrict__ total) {
-    __shared__ uint32_t warp_tot[32];
-    __shared__ uint32_t carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (uint32_t base = 0; base < n_blocks; base += SCAN_BLOCK) {
-        const uint32_t i = base + threadIdx.x;
-        const uint32_t v = i < n_blocks ? block_sums[i] : 0u;
-        uint32_t incl = v;
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, incl, o);
-            if ((threadIdx.x & 31) >= (uint32_t)o) incl += t;
-        }
-        if ((threadIdx.x & 31) == 31) warp_tot[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            uint32_t w = warp_tot[threadIdx.x], wi = w;
-            for (int o = 1; o < 32; o <<= 1) {
-                const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, wi, o);
-                if (threadIdx.x >= (uint32_t)o) wi += t;
-            }
-            warp_tot[threadIdx.x] = wi - w;  // exclusive
-        }
-        __syncthreads();
-        const uint32_t excl = carry + warp_tot[threadIdx.x >> 5] + incl - v;
-        if (i < n_blocks) block_sums[i] = excl;
-        __syncthreads();
-        if (threadIdx.x == SCAN_BLOCK - 1) carry = excl + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *total = carry;
-}
-
-__global__ void __launch_bounds__(SCAN_BLOCK)
-leader_index_kernel(const uint32_t *__restrict__ state, uint32_t n, const uint32_t *__restrict__ block_sums,
-                    uint32_t *__restrict__ leader_id) {
-    __shared__ uint32_t warp_tot[32];
-    const uint32_t k = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-    const uint32_t v = (k < n && state[k] == ST_LEADER) ? 1u : 0u;
-    const uint32_t m = __ballot_sync(0xFFFFFFFFu, v);
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) warp_tot[warp] = __popc(m);
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        uint32_t w = warp_tot[threadIdx.x], wi = w;
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, wi, o);
-            if (threadIdx.x >= (uint32_t)o) wi += t;
-        }
-        warp_tot[threadIdx.x] = wi - w;
-    }
-    __syncthreads();
-    if (k < n) leader_id[k] = v ? block_sums[blockIdx.x] + warp_tot[warp] + __popc(m & ((1u << lane) - 1u)) : NONE;
 }
 
 // every pose -> its cluster (leaders: their own; members: the lowest-ranked leader within bounds).  The lists hold
@@ -475,11 +361,10 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
         hp.mask = (1u << bits) - 1u;
     }
     const uint32_t n_cells = hp.mask + 1u;
-    const uint32_t n_scan_blocks = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
 
     // one pooled allocation for all scratch
     uint32_t *keys[2], *order[2], *ckeys[2], *crank[2];
-    uint32_t *votes, *state, *leader_id, *assign_sorted, *cl_votes, *cl_size, *cell_start, *block_sums, *small;
+    uint32_t *votes, *state, *leader_id, *assign_sorted, *cl_votes, *cl_size, *cell_start, *small;
     PoseRows *poses;
     float *d_out;
     size_t words = 0;
@@ -487,7 +372,7 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
     const size_t o_keys0 = take(n), o_keys1 = take(n), o_ord0 = take(n), o_ord1 = take(n), o_ck0 = take(n),
                  o_ck1 = take(n), o_cr0 = take(n), o_cr1 = take(n), o_votes = take(n), o_state = take(n),
                  o_lid = take(n), o_as = take(n), o_cv = take(n), o_cs = take(n), o_cell = take((size_t)n_cells + 1),
-                 o_bs = take(n_scan_blocks), o_small = take(16), o_out = take(48), o_poses = take((size_t)n * 12),
+                 o_small = take(16), o_out = take(48), o_poses = take((size_t)n * 12),
                  o_lr = take(n), o_lk = take(n), o_lcell = take((size_t)n_cells + 1);
     StreamBuf<uint32_t> pool_owner(ctx);  // returned to the pool on every path out of this function
     PPF_CUDA(ctx, pool_owner.alloc(words));
@@ -495,7 +380,7 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
     keys[0] = pool + o_keys0; keys[1] = pool + o_keys1; order[0] = pool + o_ord0; order[1] = pool + o_ord1;
     ckeys[0] = pool + o_ck0; ckeys[1] = pool + o_ck1; crank[0] = pool + o_cr0; crank[1] = pool + o_cr1;
     votes = pool + o_votes; state = pool + o_state; leader_id = pool + o_lid; assign_sorted = pool + o_as;
-    cl_votes = pool + o_cv; cl_size = pool + o_cs; cell_start = pool + o_cell; block_sums = pool + o_bs;
+    cl_votes = pool + o_cv; cl_size = pool + o_cs; cell_start = pool + o_cell;
     small = pool + o_small; d_out = reinterpret_cast<float *>(pool + o_out);
     poses = reinterpret_cast<PoseRows *>(pool + o_poses);
     uint32_t *lrank = pool + o_lr, *lkeys = pool + o_lk, *lcell_start = pool + o_lcell;
@@ -513,23 +398,18 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
     PPF_CUDA(ctx, cudaMemcpyAsync(h_small, small, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     PPF_CUDA(ctx, cudaStreamSynchronize(st));
     const uint32_t max_votes = h_small[0];
-    int vote_bits = 1;
-    while (vote_bits < 32 && (max_votes >> vote_bits)) ++vote_bits;
     PPF_LAUNCH(ctx, cluster_keys_kernel, g, 256, 0, hyps, n, max_votes, keys[0]);
     bool in_alt = false;
-    int rc = radix_sort_u32(ctx, keys[0], keys[1], order[0], order[1], nullptr, nullptr, n, vote_bits, /*v0_iota=*/true,
+    int rc = radix_sort_u32(ctx, keys[0], keys[1], order[0], order[1], nullptr, nullptr, n, max_votes, /*v0_iota=*/true,
                             &in_alt);
     if (rc) return rc;
     const uint32_t *ord = order[in_alt ? 1 : 0];
     PPF_LAUNCH(ctx, cluster_gather_kernel, g, 256, 0, hyps, ord, n, hp, poses, votes, ckeys[0]);
-    int cell_bits = 0;
-    while ((1u << cell_bits) < n_cells) ++cell_bits;
-    rc = radix_sort_u32(ctx, ckeys[0], ckeys[1], crank[0], crank[1], nullptr, nullptr, n, cell_bits, /*v0_iota=*/true,
+    rc = radix_sort_u32(ctx, ckeys[0], ckeys[1], crank[0], crank[1], nullptr, nullptr, n, n_cells - 1, /*v0_iota=*/true,
                         &in_alt);
     if (rc) return rc;
     const uint32_t *cell_keys_sorted = ckeys[in_alt ? 1 : 0], *cell_rank = crank[in_alt ? 1 : 0];
-    PPF_LAUNCH(ctx, cluster_cell_offsets_kernel, (n_cells + 1 + 255) / 256, 256, 0, cell_keys_sorted, n, n_cells,
-               cell_start);
+    if ((rc = lower_bounds(ctx, cell_keys_sorted, n, nullptr, n_cells, 0, cell_start))) return rc;
 
     // The per-cell lists (cell_rank / cell keys, sorted by cell then rank) start with every pose and are compacted to
     // the non-members after each round, to the leaders at the end.  keep flags and positions live in the first
@@ -541,26 +421,20 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
     // compaction of the current non-member lists: into themselves without the members (mode 0: small[9] <- new length), or
     // into the leaders-only lists (mode 1: small[11] <- their length); n_list bounds the source length on the host
     auto compact = [&](uint32_t leaders_only) -> int {
-        const unsigned gl = (n_list + 255) / 256, gs = (n_list + SCAN_BLOCK - 1) / SCAN_BLOCK;
+        const unsigned gl = (n_list + 255) / 256;
         uint32_t *dst_rank = leaders_only ? lrank : crank[1 - cur], *dst_keys = leaders_only ? lkeys : ckeys[1 - cur];
         uint32_t *dst_n = small + (leaders_only ? 11 : 10);
         if (n_list == 0) {
             PPF_CUDA(ctx, cudaMemsetAsync(dst_n, 0, sizeof(uint32_t), st));
         } else {
-            PPF_LAUNCH(ctx, cluster_keep_flags_kernel, gl, 256, 0, crank[cur], small + 9, state, leaders_only, keep);
-            PPF_LAUNCH(ctx, keep_count_kernel, gs, SCAN_BLOCK, 0, keep, small + 9, block_sums);
-            PPF_LAUNCH(ctx, leader_scan_blocks_kernel, 1, SCAN_BLOCK, 0, block_sums, gs, dst_n);
-            PPF_LAUNCH(ctx, keep_index_kernel, gs, SCAN_BLOCK, 0, keep, small + 9, block_sums, pos);
+            PPF_LAUNCH(ctx, cluster_keep_flags_kernel, gl, 256, 0, crank[cur], n_list, small + 9, state, leaders_only, keep);
+            if (int rc = flag_scan(ctx, keep, n_list, pos, dst_n)) return rc;
             PPF_LAUNCH(ctx, cluster_compact_kernel, gl, 256, 0, crank[cur], ckeys[cur], small + 9, keep, pos, dst_rank, dst_keys);
         }
-        if (leaders_only) {
-            PPF_LAUNCH(ctx, cluster_cell_offsets_dev_kernel, (n_cells + 1 + 255) / 256, 256, 0, lkeys, small + 11, n_cells, lcell_start);
-        } else {
-            PPF_CUDA(ctx, cudaMemcpyAsync(small + 9, small + 10, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
-            cur = 1 - cur;
-            PPF_LAUNCH(ctx, cluster_cell_offsets_dev_kernel, (n_cells + 1 + 255) / 256, 256, 0, ckeys[cur], small + 9, n_cells, cell_start);
-        }
-        return B200PPF_OK;
+        if (leaders_only) return lower_bounds(ctx, lkeys, 0, small + 11, n_cells, 0, lcell_start);
+        PPF_CUDA(ctx, cudaMemcpyAsync(small + 9, small + 10, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+        cur = 1 - cur;
+        return lower_bounds(ctx, ckeys[cur], 0, small + 9, n_cells, 0, cell_start);
     };
     // no leader yet: empty leaders-only lists
     PPF_CUDA(ctx, cudaMemsetAsync(lcell_start, 0, ((size_t)n_cells + 1) * sizeof(uint32_t), st));
@@ -580,10 +454,10 @@ int k4_cluster(b200ppf_ctx *ctx, const b200ppf_hypothesis *hyps, size_t n_, floa
         if (h_small[1] == 0) break;
         if (iter > (int)n) return fail_msg(ctx, B200PPF_ERR_CUDA, "cluster: leader resolution did not converge");
     }
-    // lcell_start / lrank now hold every leader, in rank order inside every cell
-    PPF_LAUNCH(ctx, leader_count_kernel, n_scan_blocks, SCAN_BLOCK, 0, state, n, block_sums);
-    PPF_LAUNCH(ctx, leader_scan_blocks_kernel, 1, SCAN_BLOCK, 0, block_sums, n_scan_blocks, small + 2);
-    PPF_LAUNCH(ctx, leader_index_kernel, n_scan_blocks, SCAN_BLOCK, 0, state, n, block_sums, leader_id);
+    // lcell_start / lrank now hold every leader, in rank order inside every cell.  No pose is undecided any more, so the
+    // entries of state equal to 1 are the leaders: leader_id[k] = leaders before k, the creation index of leader k (the
+    // values at members are never read), small[2] = the number of clusters.
+    if ((rc = flag_scan(ctx, state, n, leader_id, small + 2))) return rc;
     PPF_LAUNCH(ctx, cluster_assign_kernel, gr, 128, 0, poses, lcell_start, lrank, hp, n, pos_thr, rot_thr, state,
                leader_id, votes, ord, assign_sorted, ctx->d_assign, cl_votes, cl_size);
     PPF_LAUNCH(ctx, cluster_top3_kernel, 1, 1024, 0, cl_votes, small + 2, small + 3);

@@ -200,11 +200,6 @@ __global__ void cv_cell_index_kernel(const Points pts, uint32_t n, SampleRange r
     cell[i] = (uint32_t)(xc * r.ns * r.ns + yc * r.ns + zc);
 }
 
-__global__ void cv_cell_heads_kernel(const uint32_t *__restrict__ sorted_cell, uint32_t n, uint32_t *__restrict__ head) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) head[i] = (i == 0 || sorted_cell[i] != sorted_cell[i - 1]) ? 1u : 0u;
-}
-
 // one thread per occupied cell: the cell's points averaged in input order, in double
 template <class Points>
 __global__ void cv_cell_average_kernel(const Points pts, const uint32_t *__restrict__ order, const uint32_t *__restrict__ head,
@@ -267,18 +262,6 @@ cv_train_pairs_kernel(const float *__restrict__ model, uint32_t m, double angle_
     const double alpha = cv_alpha(sR, st, p2, &is_nan);
     alpha_m[idx] = (float)alpha;
     keys[idx] = h & mask;  // hash % table size (a power of two)
-}
-
-__global__ void cv_offsets_kernel(const uint32_t *__restrict__ sorted_keys, uint32_t n, uint32_t table_size,
-                                  uint32_t *__restrict__ offsets) {
-    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b > table_size) return;
-    uint32_t lo = 0, hi = n;
-    while (lo < hi) {
-        const uint32_t mid = lo + ((hi - lo) >> 1);
-        if (sorted_keys[mid] < b) lo = mid + 1; else hi = mid;
-    }
-    offsets[b] = lo;  // keys == CV_INVALID (the diagonal) sort behind every bucket
 }
 
 // ---- match -----------------------------------------------------------------------------------------------------
@@ -480,17 +463,14 @@ int cv_sample_points(b200ppf_ctx *ctx, const Points &pts, size_t n, const float 
     PPF_CUDA(ctx, rank.alloc(n));
     const unsigned g = (nn + 255) / 256;
     PPF_LAUNCH(ctx, cv_cell_index_kernel<Points>, g, 256, 0, pts, nn, r, cell0.p);
-    int bits = 1;
-    const uint64_t max_cell = (uint64_t)(r.ns + 1) * (r.ns + 1) * (r.ns + 1);
-    while ((1ull << bits) < max_cell && bits < 32) ++bits;
+    const uint64_t n_cells = (uint64_t)(r.ns + 1) * (r.ns + 1) * (r.ns + 1);
     bool in_alt = false;
-    int rc = radix_sort_u32(ctx, cell0, cell1, ord0, ord1, nullptr, nullptr, n, bits, /*v0_iota=*/true, &in_alt);
+    int rc = radix_sort_u32(ctx, cell0, cell1, ord0, ord1, nullptr, nullptr, n, n_cells - 1, /*v0_iota=*/true, &in_alt);
     if (rc) return rc;
     const uint32_t *cs = in_alt ? cell1.p : cell0.p, *os = in_alt ? ord1.p : ord0.p;
-    PPF_LAUNCH(ctx, cv_cell_heads_kernel, g, 256, 0, cs, nn, head.p);
+    if ((rc = run_heads(ctx, cs, nn, head))) return rc;
     uint32_t cells = 0;
-    rc = flag_scan_u32(ctx, head, nn, rank, &cells);
-    if (rc) return rc;
+    if ((rc = flag_scan_host(ctx, head, nn, rank, &cells))) return rc;
     float *out = nullptr;
     PPF_CUDA(ctx, cudaMalloc(&out, std::max<size_t>(1, cells) * 6 * sizeof(float)));
     std::unique_ptr<float, cudaError_t (*)(void *)> owner(out, cudaFree);
@@ -848,11 +828,12 @@ int b200cv_detector_train(b200cv_detector *d, const float *model, size_t n, size
     cudaEventRecord(ctx->ev[1], ctx->stream);
     // all 32 key bits: the diagonal's CV_INVALID keys have to end up behind every bucket
     bool in_alt = false;
-    rc = radix_sort_u32(ctx, k0, k1, i0, i1, nullptr, nullptr, count, 32, /*v0_iota=*/true, &in_alt);
+    rc = radix_sort_u32(ctx, k0, k1, i0, i1, nullptr, nullptr, count, 0xFFFFFFFFu, /*v0_iota=*/true, &in_alt);
     if (rc) return rc;
     cudaEventRecord(ctx->ev[2], ctx->stream);
     const uint32_t *ks = in_alt ? k1.p : k0.p, *is = in_alt ? i1.p : i0.p;
-    PPF_LAUNCH(ctx, cv_offsets_kernel, (unsigned)((pow2 + 1 + 255) / 256), 256, 0, ks, (uint32_t)count, (uint32_t)pow2, d->d_offsets);
+    // keys == CV_INVALID (the diagonal) sort behind every bucket
+    if ((rc = lower_bounds(ctx, ks, (uint32_t)count, nullptr, (uint32_t)pow2, 0, d->d_offsets))) return rc;
     d->n_nodes = m * (m - 1);
     PPF_CUDA(ctx, cudaMalloc(&d->d_nodes, std::max<size_t>(1, d->n_nodes) * sizeof(uint32_t)));
     PPF_CUDA(ctx, cudaMemcpyAsync(d->d_nodes, is, d->n_nodes * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));

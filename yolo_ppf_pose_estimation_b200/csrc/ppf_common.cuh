@@ -243,9 +243,6 @@ int verify_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_j
 b200ppf_ctx *cv_detector_context(const b200cv_detector *d);
 bool cv_detector_trained(const b200cv_detector *d);
 
-// exclusive scan of 0/1 flags on the context stream (prep.cu): rank[k] = set flags before k; total on the host
-int flag_scan_u32(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, uint32_t *total_host);
-
 // scene pre-processing (prep.cu): voxel grid, k nearest neighbours, outlier removal, normals, curvature edges
 int prep_upload_xyz(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride, b200ppf_cloud **out);
 int prep_download(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, float *host, size_t stride, size_t noff, size_t coff);
@@ -291,8 +288,6 @@ struct SceneGrid {
 // grid geometry for a bounding box and a search radius (host), coarsened until it has at most max_cells cells; returns the
 // number of cells (0 for a non-finite box or radius)
 uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp, uint32_t max_cells = 1u << 22);
-// cell_start[c] (c = 0 .. n_cells) = the first of the n ascending sorted_ids that is >= c
-int grid_cell_starts(b200ppf_ctx *ctx, const uint32_t *sorted_ids, uint32_t n, uint32_t n_cells, uint32_t *cell_start);
 int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius, SceneGrid *out);
 void scene_grid_free(b200ppf_ctx *ctx, SceneGrid *g);
 struct SceneGridFree {
@@ -300,11 +295,27 @@ struct SceneGridFree {
     void operator()(SceneGrid *g) const { scene_grid_free(ctx, g); }
 };
 
-// hand-written LSD radix sort (radix_sort.cu): keys ascending, stable, two 32-bit payload streams.
+// ---- sorted-key primitives (sort_scan.cu), all on the context stream ----------------------------------------------
+// hand-written LSD radix sort: keys ascending, stable, two 32-bit payload streams.
 // All buffers are device pointers of n elements; *_alt are the ping-pong partners.  On return
-// *result_in_alt tells which set holds the sorted data.  bits = number of key bits to sort.
+// *result_in_alt tells which set holds the sorted data.  max_key = the largest key the caller can produce: the sort
+// orders its bits (at least one 8-bit pass, at most four).
 // v0_iota: treat v0 as the identity permutation on entry (its contents are never read).
 int radix_sort_u32(b200ppf_ctx *ctx, uint32_t *keys, uint32_t *keys_alt, uint32_t *v0, uint32_t *v0_alt,
-                   uint32_t *v1, uint32_t *v1_alt, size_t n, int bits, bool v0_iota, bool *result_in_alt);
+                   uint32_t *v1, uint32_t *v1_alt, size_t n, uint64_t max_key, bool v0_iota, bool *result_in_alt);
+// offsets[k] (k = 0 .. n_keys) = the first i with sorted[i] >= k << shift; the length of sorted is *n_dev when n_dev is
+// non-null (a list whose length only the device knows), else n.  One launch.
+int lower_bounds(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, const uint32_t *n_dev, uint32_t n_keys, uint32_t shift,
+                 uint32_t *offsets);
+// exclusive scan of flags: rank[k] = the flags equal to 1 before k (written for every k < n), *total_dev = all of them.
+// Three launches, no host wait; n == 0 zeroes the total and launches nothing.
+int flag_scan(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, uint32_t *total_dev);
+// the same with the total on the host: one more copy and one stream wait
+int flag_scan_host(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, uint32_t *total_host);
+// in place: each of the n_rows rows of data (row_len words, row-major) becomes its exclusive scan, totals[r] its sum.
+// One launch.
+int scan_rows(b200ppf_ctx *ctx, uint32_t *data, uint32_t n_rows, uint32_t row_len, uint32_t *totals);
+// head[i] = 1 where a run of equal keys starts in sorted[0 .. n), else 0.  One launch.
+int run_heads(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, uint32_t *head);
 
 }  // namespace b200ppf

@@ -35,92 +35,6 @@ namespace b200ppf {
 
 namespace {
 
-constexpr int SCAN_BLOCK = 1024;
-
-// ---- exclusive scan of 0/1 flags (three launches; same shape as K4's leader index) ----------------------------
-__global__ void __launch_bounds__(SCAN_BLOCK)
-flag_count_kernel(const uint32_t *__restrict__ flags, uint32_t n, uint32_t *__restrict__ block_sums) {
-    const uint32_t k = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-    const int c = __syncthreads_count(k < n && flags[k] != 0u);
-    if (threadIdx.x == 0) block_sums[blockIdx.x] = (uint32_t)c;
-}
-
-// block b of the grid scans row b: block_sums[b * n_blocks ...], total[b]
-__global__ void __launch_bounds__(SCAN_BLOCK)
-flag_scan_blocks_kernel(uint32_t *__restrict__ block_sums, uint32_t n_blocks, uint32_t *__restrict__ total) {
-    __shared__ uint32_t warp_tot[32];
-    __shared__ uint32_t carry;
-    block_sums += (size_t)blockIdx.x * n_blocks;
-    total += blockIdx.x;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (uint32_t base = 0; base < n_blocks; base += SCAN_BLOCK) {
-        const uint32_t i = base + threadIdx.x;
-        const uint32_t v = i < n_blocks ? block_sums[i] : 0u;
-        uint32_t incl = v;
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, incl, o);
-            if ((threadIdx.x & 31) >= (uint32_t)o) incl += t;
-        }
-        if ((threadIdx.x & 31) == 31) warp_tot[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            uint32_t w = warp_tot[threadIdx.x], wi = w;
-            for (int o = 1; o < 32; o <<= 1) {
-                const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, wi, o);
-                if (threadIdx.x >= (uint32_t)o) wi += t;
-            }
-            warp_tot[threadIdx.x] = wi - w;  // exclusive
-        }
-        __syncthreads();
-        const uint32_t excl = carry + warp_tot[threadIdx.x >> 5] + incl - v;
-        if (i < n_blocks) block_sums[i] = excl;
-        __syncthreads();
-        if (threadIdx.x == SCAN_BLOCK - 1) carry = excl + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *total = carry;
-}
-
-// rank[k] = number of set flags before k (written for every k)
-__global__ void __launch_bounds__(SCAN_BLOCK)
-flag_rank_kernel(const uint32_t *__restrict__ flags, uint32_t n, const uint32_t *__restrict__ block_sums,
-                 uint32_t *__restrict__ rank) {
-    __shared__ uint32_t warp_tot[32];
-    const uint32_t k = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-    const uint32_t v = (k < n && flags[k] != 0u) ? 1u : 0u;
-    const uint32_t m = __ballot_sync(0xFFFFFFFFu, v);
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) warp_tot[warp] = __popc(m);
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        uint32_t w = warp_tot[threadIdx.x], wi = w;
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, wi, o);
-            if (threadIdx.x >= (uint32_t)o) wi += t;
-        }
-        warp_tot[threadIdx.x] = wi - w;
-    }
-    __syncthreads();
-    if (k < n) rank[k] = block_sums[blockIdx.x] + warp_tot[warp] + __popc(m & ((1u << lane) - 1u));
-}
-
-// flags -> rank (exclusive), *total on the host.  block_sums / d_total come from the stream-ordered pool.
-int flag_scan(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, uint32_t *total_host) {
-    *total_host = 0;
-    if (n == 0) return B200PPF_OK;
-    const uint32_t nb = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
-    StreamBuf<uint32_t> block_sums(ctx);
-    PPF_CUDA(ctx, block_sums.alloc((size_t)nb + 1));
-    uint32_t *d_total = block_sums + nb;
-    PPF_LAUNCH(ctx, flag_count_kernel, nb, SCAN_BLOCK, 0, flags, n, block_sums);
-    PPF_LAUNCH(ctx, flag_scan_blocks_kernel, 1, SCAN_BLOCK, 0, block_sums, nb, d_total);
-    PPF_LAUNCH(ctx, flag_rank_kernel, nb, SCAN_BLOCK, 0, flags, n, block_sums, rank);
-    PPF_CUDA(ctx, cudaMemcpyAsync(total_host, d_total, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return B200PPF_OK;
-}
-
 // ---- bounding box of a device cloud (PCL getMinMax3D) ---------------------------------------------------------
 __device__ __forceinline__ uint32_t float_order(float f) {  // order-preserving float -> uint
     const uint32_t u = __float_as_uint(f);
@@ -199,13 +113,6 @@ voxel_ids_kernel(const float4 *__restrict__ pos, uint32_t n, VoxelParams vp, uin
     const int ijk1 = (int)(floorf(p.y * vp.inv[1]) - (float)vp.min_b[1]);
     const int ijk2 = (int)(floorf(p.z * vp.inv[2]) - (float)vp.min_b[2]);
     ids[i] = (uint32_t)(ijk0 * vp.mul[0] + ijk1 * vp.mul[1] + ijk2 * vp.mul[2]);
-}
-
-__global__ void __launch_bounds__(256)
-voxel_heads_kernel(const uint32_t *__restrict__ sorted_ids, uint32_t n, uint32_t *__restrict__ head) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    head[i] = (i == 0 || sorted_ids[i] != sorted_ids[i - 1]) ? 1u : 0u;
 }
 
 // starts[v] = first sorted position of voxel v; starts[n_voxels] = n
@@ -652,7 +559,7 @@ int compact_cloud(b200ppf_ctx *ctx, const b200ppf_cloud *in, const uint32_t *fla
     StreamBuf<uint32_t> rank(ctx), index(ctx);
     PPF_CUDA(ctx, rank.alloc(n));
     uint32_t m = 0;
-    int rc = flag_scan(ctx, flags, n, rank, &m);
+    int rc = flag_scan_host(ctx, flags, n, rank, &m);
     if (rc != B200PPF_OK) return rc;
     CloudPtr c;
     if ((rc = cloud_alloc(ctx, m, &c)) != B200PPF_OK) return rc;
@@ -687,25 +594,26 @@ pyramid_flag_kernel(const float4 *__restrict__ pos, uint32_t n, PyramidPlanes pl
     flags[i] = pyramid_contains(pl, pos[i]) ? 1u : 0u;
 }
 
-// ---- P0 for up to 64 boxes: one tile of SCAN_BLOCK points per block ------------------------------------------
+// ---- P0 for up to 64 boxes: one tile of CROP_TILE points per block -------------------------------------------
 constexpr int MAX_BOXES = 64;
+constexpr int CROP_TILE = 1024;
 
 // membership mask of every point, the tile's count per box (counts[b * n_tiles + tile]) and each box's bounding box
 // (lo[3 * b ..], hi[3 * b ..] as order-preserving words): the bounds of a box's points are those of its cloud
-__global__ void __launch_bounds__(SCAN_BLOCK)
+__global__ void __launch_bounds__(CROP_TILE)
 pyramids_mask_kernel(const float4 *__restrict__ pos, uint32_t n, const PyramidPlanes *__restrict__ planes, int n_boxes,
                      unsigned long long *__restrict__ mask, uint32_t *__restrict__ counts, uint32_t *__restrict__ lo,
                      uint32_t *__restrict__ hi) {
     __shared__ PyramidPlanes s_pl[MAX_BOXES];
     __shared__ uint32_t s_cnt[MAX_BOXES], s_lo[MAX_BOXES][3], s_hi[MAX_BOXES][3];
-    for (int t = threadIdx.x; t < n_boxes * (int)(sizeof(PyramidPlanes) / sizeof(double)); t += SCAN_BLOCK)
+    for (int t = threadIdx.x; t < n_boxes * (int)(sizeof(PyramidPlanes) / sizeof(double)); t += CROP_TILE)
         reinterpret_cast<double *>(s_pl)[t] = reinterpret_cast<const double *>(planes)[t];
-    for (int b = threadIdx.x; b < n_boxes; b += SCAN_BLOCK) {
+    for (int b = threadIdx.x; b < n_boxes; b += CROP_TILE) {
         s_cnt[b] = 0;
         for (int k = 0; k < 3; ++k) s_lo[b][k] = 0xFFFFFFFFu, s_hi[b][k] = 0u;
     }
     __syncthreads();
-    const uint32_t i = blockIdx.x * SCAN_BLOCK + threadIdx.x, lane = threadIdx.x & 31;
+    const uint32_t i = blockIdx.x * CROP_TILE + threadIdx.x, lane = threadIdx.x & 31;
     const float4 p = i < n ? pos[i] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     unsigned long long m = 0;
     if (i < n)
@@ -725,7 +633,7 @@ pyramids_mask_kernel(const float4 *__restrict__ pos, uint32_t n, const PyramidPl
         if (lane == 0) atomicAdd(&s_cnt[b], (uint32_t)__popc(bal));
     }
     __syncthreads();
-    for (int b = threadIdx.x; b < n_boxes; b += SCAN_BLOCK) {
+    for (int b = threadIdx.x; b < n_boxes; b += CROP_TILE) {
         counts[(size_t)b * gridDim.x + blockIdx.x] = s_cnt[b];
         if (s_cnt[b])
             for (int k = 0; k < 3; ++k) atomicMin(lo + 3 * b + k, s_lo[b][k]), atomicMax(hi + 3 * b + k, s_hi[b][k]);
@@ -734,19 +642,19 @@ pyramids_mask_kernel(const float4 *__restrict__ pos, uint32_t n, const PyramidPl
 
 // every point into each of its boxes' clouds at (scanned tile offset + rank in the tile): input order, as compaction
 // keeps it.  out[b] / out[n_boxes + b] are cloud b's pos / nrm arrays.
-__global__ void __launch_bounds__(SCAN_BLOCK)
+__global__ void __launch_bounds__(CROP_TILE)
 pyramids_scatter_kernel(const float4 *__restrict__ pos, const float4 *__restrict__ nrm, uint32_t n,
                         const unsigned long long *__restrict__ mask, int n_boxes, const uint32_t *__restrict__ tile_off,
                         float4 *const *__restrict__ out) {
     __shared__ uint32_t s_warp[MAX_BOXES][32];  // box b: points of warps before w in this tile
-    const uint32_t i = blockIdx.x * SCAN_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t i = blockIdx.x * CROP_TILE + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const unsigned long long m = i < n ? mask[i] : 0ull;
     for (int b = 0; b < n_boxes; ++b) {
         const uint32_t bal = __ballot_sync(0xFFFFFFFFu, (m >> b) & 1ull);
         if (lane == 0) s_warp[b][warp] = (uint32_t)__popc(bal);
     }
     __syncthreads();
-    for (uint32_t t = threadIdx.x; t < (uint32_t)n_boxes * 32; t += SCAN_BLOCK) {  // one warp per box row: exclusive scan
+    for (uint32_t t = threadIdx.x; t < (uint32_t)n_boxes * 32; t += CROP_TILE) {  // one warp per box row: exclusive scan
         const uint32_t v = s_warp[t >> 5][lane];
         uint32_t incl = v;
         for (int o = 1; o < 32; o <<= 1) {
@@ -808,10 +716,6 @@ struct EventTimer {  // prep_ms of the timings block
 };
 
 }  // namespace
-
-int flag_scan_u32(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, uint32_t *total_host) {
-    return flag_scan(ctx, flags, n, rank, total_host);
-}
 
 // ================================================================================================================
 // host entry points (called from capi.cu)
@@ -891,8 +795,6 @@ int prep_voxel_grid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *leaf
     }
     vp.mul[0] = 1, vp.mul[1] = div_b[0], vp.mul[2] = div_b[0] * div_b[1];
     const uint64_t n_cells = (uint64_t)div_b[0] * (uint64_t)div_b[1] * (uint64_t)div_b[2];
-    int bits = 1;
-    while (bits < 32 && (1ull << bits) < n_cells) ++bits;
 
     StreamBuf<uint32_t> ids0(ctx), ids1(ctx), ord0(ctx), ord1(ctx), head(ctx), rank(ctx), starts(ctx);
     PPF_CUDA(ctx, ids0.alloc(n));
@@ -904,12 +806,12 @@ int prep_voxel_grid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *leaf
     const unsigned gb = (n + 255) / 256;
     PPF_LAUNCH(ctx, voxel_ids_kernel, gb, 256, 0, in->pos, n, vp, ids0);
     bool in_alt = false;
-    int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, n, bits, /*v0_iota=*/true, &in_alt);
+    int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, n, n_cells - 1, /*v0_iota=*/true, &in_alt);
     if (rc != B200PPF_OK) return rc;
     const uint32_t *sorted_ids = in_alt ? ids1 : ids0, *order = in_alt ? ord1 : ord0;
-    PPF_LAUNCH(ctx, voxel_heads_kernel, gb, 256, 0, sorted_ids, n, head);
+    if ((rc = run_heads(ctx, sorted_ids, n, head)) != B200PPF_OK) return rc;
     uint32_t m = 0;
-    if ((rc = flag_scan(ctx, head, n, rank, &m)) != B200PPF_OK) return rc;
+    if ((rc = flag_scan_host(ctx, head, n, rank, &m)) != B200PPF_OK) return rc;
     PPF_CUDA(ctx, starts.alloc((size_t)m + 1));
     CloudPtr c;
     if ((rc = cloud_alloc(ctx, m, &c)) != B200PPF_OK) return rc;
@@ -1095,7 +997,7 @@ int prep_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *c
             return fail_msg(ctx, rc, msg);
         }
     }
-    const uint32_t n = (uint32_t)in->n, K = (uint32_t)n_boxes, T = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    const uint32_t n = (uint32_t)in->n, K = (uint32_t)n_boxes, T = (n + CROP_TILE - 1) / CROP_TILE;
     // scratch: planes, masks, tile counts (box-major, scanned in place), and the words read back: K totals, 6K bounds
     StreamBuf<PyramidPlanes> d_pl(ctx);
     StreamBuf<unsigned long long> mask(ctx);
@@ -1113,8 +1015,8 @@ int prep_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *c
     PPF_CUDA(ctx, cudaMemsetAsync(d_lo, 0xFF, 3 * K * sizeof(uint32_t), ctx->stream));
     PPF_CUDA(ctx, cudaMemsetAsync(d_hi, 0x00, 3 * K * sizeof(uint32_t), ctx->stream));
     if (n) {
-        PPF_LAUNCH(ctx, pyramids_mask_kernel, T, SCAN_BLOCK, 0, in->pos, n, d_pl, (int)K, mask, counts, d_lo, d_hi);
-        PPF_LAUNCH(ctx, flag_scan_blocks_kernel, K, SCAN_BLOCK, 0, counts, T, d_tot);
+        PPF_LAUNCH(ctx, pyramids_mask_kernel, T, CROP_TILE, 0, in->pos, n, d_pl, (int)K, mask, counts, d_lo, d_hi);
+        if (int rc = scan_rows(ctx, counts, K, T, d_tot)) return rc;
     }
     std::vector<uint32_t> h(7 * (size_t)K);
     PPF_CUDA(ctx, cudaMemcpyAsync(h.data(), back, h.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1132,7 +1034,7 @@ int prep_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *c
     }
     if (n) {
         PPF_CUDA(ctx, cudaMemcpyAsync(d_out, ptrs.data(), ptrs.size() * sizeof(float4 *), cudaMemcpyHostToDevice, ctx->stream));
-        PPF_LAUNCH(ctx, pyramids_scatter_kernel, T, SCAN_BLOCK, 0, in->pos, in->nrm, n, mask, (int)K, counts, d_out);
+        PPF_LAUNCH(ctx, pyramids_scatter_kernel, T, CROP_TILE, 0, in->pos, in->nrm, n, mask, (int)K, counts, d_out);
     }
     timer.stop();
     for (uint32_t b = 0; b < K; ++b) out[b] = c[b].release();

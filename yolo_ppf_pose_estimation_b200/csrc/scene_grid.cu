@@ -37,18 +37,6 @@ __global__ void grid_gather_kernel(const float4 *__restrict__ pos, const float4 
     snrm[i] = nrm[o];
 }
 
-__global__ void grid_offsets_kernel(const uint32_t *__restrict__ sorted_ids, uint32_t n, uint32_t n_cells,
-                                    uint32_t *__restrict__ cell_start) {
-    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c > n_cells) return;
-    uint32_t lo = 0, hi = n;
-    while (lo < hi) {
-        const uint32_t mid = lo + ((hi - lo) >> 1);
-        if (sorted_ids[mid] < c) lo = mid + 1; else hi = mid;
-    }
-    cell_start[c] = lo;
-}
-
 }  // namespace
 
 void scene_grid_free(b200ppf_ctx *ctx, SceneGrid *g) {
@@ -86,11 +74,6 @@ uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float r
     return (uint32_t)g.dims[0] * (uint32_t)g.dims[1] * (uint32_t)g.dims[2];
 }
 
-int grid_cell_starts(b200ppf_ctx *ctx, const uint32_t *sorted_ids, uint32_t n, uint32_t n_cells, uint32_t *cell_start) {
-    PPF_LAUNCH(ctx, grid_offsets_kernel, (n_cells + 1 + 255) / 256, 256, 0, sorted_ids, n, n_cells, cell_start);
-    return B200PPF_OK;
-}
-
 int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius, SceneGrid *out) {
     *out = SceneGrid();
     const uint32_t n = (uint32_t)scene->n;
@@ -112,14 +95,12 @@ int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius,
     bool in_alt = false;
     if (n) {
         PPF_LAUNCH(ctx, grid_cell_ids_kernel, gb, 256, 0, scene->pos, n, g, ids0.p);
-        int bits = 1;
-        while ((1u << bits) < out->n_cells) ++bits;
-        int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, n, bits, /*v0_iota=*/true, &in_alt);
+        int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, n, out->n_cells - 1, /*v0_iota=*/true, &in_alt);
         if (rc) return rc;
     }
     const uint32_t *ids_sorted = in_alt ? ids1.p : ids0.p;
     const uint32_t *ord_sorted = in_alt ? ord1.p : ord0.p;
-    if (int rc = grid_cell_starts(ctx, ids_sorted, n, out->n_cells, out->cell_start)) return rc;
+    if (int rc = lower_bounds(ctx, ids_sorted, n, nullptr, out->n_cells, 0, out->cell_start)) return rc;
     if (n) PPF_LAUNCH(ctx, grid_gather_kernel, gb, 256, 0, scene->pos, scene->nrm, ord_sorted, n, out->pos, out->nrm);
     out->orig = in_alt ? ord1.release() : ord0.release();  // sorted position -> original scene index
     return B200PPF_OK;

@@ -272,10 +272,11 @@ int verify_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_j
     const uint32_t n_scenes = (uint32_t)scenes.size();
     PPF_LAUNCH(ctx, verify_cell_ids_kernel, (n + 1 + 255) / 256, 256, 0, d_scenes.p, n_scenes, n, n_cells, ids0.p);
     bool in_alt = false;
-    if (int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, (size_t)n + 1, KEY_BITS, /*v0_iota=*/true, &in_alt))
+    if (int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, (size_t)n + 1, MAX_CELLS_TOTAL, /*v0_iota=*/true,
+                                &in_alt))
         return rc;
     const uint32_t *ids_sorted = in_alt ? ids1.p : ids0.p, *ord_sorted = in_alt ? ord1.p : ord0.p;
-    if (int rc = grid_cell_starts(ctx, ids_sorted, n + 1, n_cells, cell_start)) return rc;
+    if (int rc = lower_bounds(ctx, ids_sorted, n + 1, nullptr, n_cells, 0, cell_start)) return rc;
     PPF_LAUNCH(ctx, verify_gather_kernel, std::max(1u, (n + 255) / 256), 256, 0, d_scenes.p, n_scenes, ord_sorted, n, spos.p, snrm.p);
 
     const double tau = (double)params.inlier_dist;
