@@ -274,6 +274,34 @@ int b200ppf_vote_debug_accumulator(b200ppf_ctx *ctx, const b200ppf_table *t,
 int b200ppf_debug_alpha_bins(b200ppf_ctx *ctx, float angle_step, int alpha_mode, int nalpha_rule, const float *alpha_m,
                              const float *alpha_s, size_t n, uint32_t *fast, uint32_t *exact);
 
+/* Parity hooks of the sorted-key primitives every stage that sorts keys shares (radix sort, bucket offsets, flag scan,
+ * row scan, run heads).  They exist for the parity tests only; no product entry point routes through them.  Each one
+ * mirrors its primitive's arguments with host arrays: every array is copied to the device whole, the words past the
+ * documented range (up to *_cap) included, the primitive runs once on the context stream, every array it may write is
+ * copied back whole, and the call waits for the stream.  The primitive's kernels are the only launches the call adds to
+ * b200ppf_launch_count.  B200PPF_ERR_INVALID, before the context is looked at: a NULL array the call needs, a cap below
+ * the range the primitive writes.
+ *   radix_sort     keys / v0 / v1 ascending by key, stable; a NULL pair (v0, v0_alt) or (v1, v1_alt) is no such payload,
+ *                  half a pair is an error.  max_key: the largest key (the pass count follows from its bits, one to four
+ *                  8-bit passes); v0_iota: v0 is the identity 0..n-1 on entry and its contents are never read.
+ *                  *result_in_alt = 1 when the sorted data is in the *_alt arrays.  n < 2^32 - 4096.
+ *   lower_bounds   offsets[k] = first i < len with sorted[i] >= k << shift, k = 0 .. n_keys (shift < 32); len is n for
+ *                  dev_len < 0, else dev_len (<= n), read from device memory as a compacted list's length is.
+ *   flag_scan      rank[k] = the flags equal to 1 before k, k < n; *total = all of them: from the device total of
+ *                  flag_scan (*total's value on entry is its initial device value) or, host_total != 0, flag_scan_host.
+ *   scan_rows      each of the n_rows >= 1 rows of data (row_len words, row-major) in place to its exclusive scan,
+ *                  totals[r] its sum.
+ *   run_heads      head[i] = 1 where a run of equal keys of sorted[0 .. n) starts, else 0. */
+int b200ppf_debug_radix_sort(b200ppf_ctx *ctx, uint32_t *keys, uint32_t *keys_alt, uint32_t *v0, uint32_t *v0_alt, uint32_t *v1,
+                             uint32_t *v1_alt, size_t n, uint64_t max_key, int v0_iota, int *result_in_alt);
+int b200ppf_debug_lower_bounds(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, int64_t dev_len, uint32_t n_keys,
+                               uint32_t shift, uint32_t *offsets, size_t offsets_cap);
+int b200ppf_debug_flag_scan(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, size_t rank_cap, int host_total,
+                            uint32_t *total);
+int b200ppf_debug_scan_rows(b200ppf_ctx *ctx, uint32_t *data, uint32_t n_rows, uint32_t row_len, size_t data_cap, uint32_t *totals,
+                            size_t totals_cap);
+int b200ppf_debug_run_heads(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, uint32_t *head, size_t head_cap);
+
 /* roofline denominator the HBM/tensor peaks do not cover: measured rate of shared-memory reductions
  * (one per vote).  pattern 0 = conflict-free, 1 = random words (address from an LCG), 2 = one word,
  * 3 / 4 = exactly 2 / 4 lanes per bank; 5 / 6 / 7 = the voting loop's own shape (one coalesced 4-byte gather

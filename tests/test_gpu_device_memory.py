@@ -128,6 +128,13 @@ def test_match_paths_return_their_memory(ctx, pool_used, setup):
         ctx.vote_debug_pairs(table, ds, 0)
         ctx.vote_debug_accumulator(table, ds, 0)
         capi.debug_alpha_bins(np.zeros(8, np.float32), np.linspace(-3, 3, 8).astype(np.float32), ANGLE_STEP, ctx=ctx)
+        keys = np.arange(3000, 0, -1, dtype=np.uint32) // 7
+        ctx.debug_radix_sort(keys, 3000, v0=keys, v1=keys, v0_iota=True)
+        ctx.debug_lower_bounds(np.sort(keys), 100, 2, dev_len=1000)
+        ctx.debug_flag_scan(keys % 2)
+        ctx.debug_flag_scan(keys % 2, host_total=True)
+        ctx.debug_scan_rows(keys, 3, 1000)
+        ctx.debug_run_heads(np.sort(keys))
 
     for run in (vote_cluster, debug_hooks):
         _rounds(pool_used, run)

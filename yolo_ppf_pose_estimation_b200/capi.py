@@ -159,6 +159,11 @@ SYMBOLS = {
     "b200ppf_vote_debug_pairs": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp]),
     "b200ppf_vote_debug_accumulator": (_i, [_vp, _vp, _vp, _sz, _vp]),
     "b200ppf_debug_alpha_bins": (_i, [_vp, _f, _i, _i, _vp, _vp, _sz, _vp, _vp]),
+    "b200ppf_debug_radix_sort": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, C.c_uint64, _i, C.POINTER(_i)]),
+    "b200ppf_debug_lower_bounds": (_i, [_vp, _vp, C.c_uint32, C.c_int64, C.c_uint32, C.c_uint32, _vp, _sz]),
+    "b200ppf_debug_flag_scan": (_i, [_vp, _vp, C.c_uint32, _vp, _sz, _i, C.POINTER(C.c_uint32)]),
+    "b200ppf_debug_scan_rows": (_i, [_vp, _vp, C.c_uint32, C.c_uint32, _sz, _vp, _sz]),
+    "b200ppf_debug_run_heads": (_i, [_vp, _vp, C.c_uint32, _vp, _sz]),
     "b200ppf_microbench_atoms": (_i, [_vp, _i, C.POINTER(C.c_double)]),
     "b200ppf_cluster": (_i, [_vp, _vp, _sz, _f, _f, _vp, _vp, C.POINTER(_sz)]),
     "b200ppf_cluster_device": (_i, [_vp, _vp, _sz, _f, _f, _vp, _vp, C.POINTER(_sz)]),
@@ -662,6 +667,53 @@ class Context:
         v = C.c_double(0.0)
         self.check(lib().b200ppf_microbench_atoms(self._h, pattern, C.byref(v)))
         return v.value
+
+    # ---- sorted-key primitives: parity hooks (copies in, one run, whole arrays back) ------------------
+    def debug_radix_sort(self, keys, max_key, v0=None, v1=None, v0_iota=False):
+        """radix_sort_u32 -> (keys, v0, v1, result_in_alt): the arrays holding the sorted data, None for a payload not
+        given.  v0_iota: the sort takes v0 to be 0..n-1 and never reads the v0 given."""
+        sets = [None if a is None else np.array(a, np.uint32).reshape(-1) for a in (keys, v0, v1)]
+        if any(a is not None and a.size != sets[0].size for a in sets):
+            raise ValueError("payloads must have one word per key")
+        alts = [None if a is None else np.zeros_like(a) for a in sets]
+        alt = C.c_int(0)
+        self.check(lib().b200ppf_debug_radix_sort(self._h, _p(sets[0]), _p(alts[0]), _p(sets[1]), _p(alts[1]), _p(sets[2]),
+                                                  _p(alts[2]), sets[0].size, int(max_key), int(bool(v0_iota)), C.byref(alt)))
+        out = alts if alt.value else sets
+        return out[0], out[1], out[2], bool(alt.value)
+
+    def debug_lower_bounds(self, sorted_keys, n_keys, shift, dev_len=None, offsets=None):
+        """lower_bounds -> offsets, the whole array (default n_keys + 1 zeros; words past n_keys are the caller's canary).
+        dev_len: the list length, read from device memory (None: len(sorted_keys), passed by value)"""
+        s = np.ascontiguousarray(sorted_keys, np.uint32).reshape(-1)
+        off = np.zeros(n_keys + 1, np.uint32) if offsets is None else np.array(offsets, np.uint32).reshape(-1)
+        self.check(lib().b200ppf_debug_lower_bounds(self._h, _p(s), s.size, -1 if dev_len is None else int(dev_len), n_keys,
+                                                    shift, _p(off), off.size))
+        return off
+
+    def debug_flag_scan(self, flags, rank=None, host_total=False, total=0):
+        """flag_scan (host_total: flag_scan_host) -> (rank, total): rank the whole array (default len(flags) zeros), total
+        the device total's value before the call"""
+        f = np.ascontiguousarray(flags, np.uint32).reshape(-1)
+        r = np.zeros(f.size, np.uint32) if rank is None else np.array(rank, np.uint32).reshape(-1)
+        t = C.c_uint32(total)
+        self.check(lib().b200ppf_debug_flag_scan(self._h, _p(f), f.size, _p(r), r.size, int(bool(host_total)), C.byref(t)))
+        return r, t.value
+
+    def debug_scan_rows(self, data, n_rows, row_len, totals=None):
+        """scan_rows -> (data, totals), whole arrays: data is n_rows * row_len words and whatever follows them, totals
+        n_rows words by default"""
+        d = np.array(data, np.uint32).reshape(-1)
+        t = np.zeros(n_rows, np.uint32) if totals is None else np.array(totals, np.uint32).reshape(-1)
+        self.check(lib().b200ppf_debug_scan_rows(self._h, _p(d), n_rows, row_len, d.size, _p(t), t.size))
+        return d, t
+
+    def debug_run_heads(self, sorted_keys, head=None):
+        """run_heads -> head, the whole array (default len(sorted_keys) zeros)"""
+        s = np.ascontiguousarray(sorted_keys, np.uint32).reshape(-1)
+        h = np.zeros(s.size, np.uint32) if head is None else np.array(head, np.uint32).reshape(-1)
+        self.check(lib().b200ppf_debug_run_heads(self._h, _p(s), s.size, _p(h), h.size))
+        return h
 
     # ---- K4 / K5 / align ------------------------------------------------------------------------
     def cluster(self, hyps, pos_thr=0.01, rot_thr=20.0 / 180.0 * np.pi, device_ptr=None, n=None):

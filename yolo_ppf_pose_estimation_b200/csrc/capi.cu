@@ -78,6 +78,19 @@ int verify_params(b200ppf_ctx *ctx, const b200ppf_verify_params *params, b200ppf
     return B200PPF_OK;
 }
 
+// the parity hooks' copies: a host array of n words into a new stream-ordered buffer (none for a NULL array), and back
+int to_device(b200ppf_ctx *ctx, StreamBuf<uint32_t> &d, const uint32_t *host, size_t n) {
+    if (!host) return B200PPF_OK;
+    PPF_CUDA(ctx, d.alloc(n));
+    if (n) PPF_CUDA(ctx, cudaMemcpyAsync(d, host, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    return B200PPF_OK;
+}
+
+int to_host(b200ppf_ctx *ctx, uint32_t *host, const StreamBuf<uint32_t> &d, size_t n) {
+    if (host && n) PPF_CUDA(ctx, cudaMemcpyAsync(host, d, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    return B200PPF_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -828,6 +841,91 @@ int b200ppf_debug_alpha_bins(b200ppf_ctx *ctx, float angle_step, int alpha_mode,
     if (!ctx) return k3_debug_alpha_bins(nullptr, angle_step, alpha_mode, nalpha_rule, alpha_m, alpha_s, n, fast, exact);
     DeviceGuard guard(ctx->device);
     return k3_debug_alpha_bins(ctx, angle_step, alpha_mode, nalpha_rule, alpha_m, alpha_s, n, fast, exact);
+}
+
+/* ---- parity hooks of the sorted-key primitives (sort_scan.cu) ------------------------------- */
+
+int b200ppf_debug_radix_sort(b200ppf_ctx *ctx, uint32_t *keys, uint32_t *keys_alt, uint32_t *v0, uint32_t *v0_alt, uint32_t *v1,
+                             uint32_t *v1_alt, size_t n, uint64_t max_key, int v0_iota, int *result_in_alt) {
+    if (!result_in_alt || (n && (!keys || !keys_alt)) || !v0 != !v0_alt || !v1 != !v1_alt)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "debug radix sort: bad argument");
+    CHECK_CTX(ctx);
+    StreamBuf<uint32_t> k(ctx), ka(ctx), a(ctx), aa(ctx), b(ctx), ba(ctx);
+    StreamBuf<uint32_t> *const dev[6] = {&k, &ka, &a, &aa, &b, &ba};
+    uint32_t *const host[6] = {keys, keys_alt, v0, v0_alt, v1, v1_alt};
+    for (int i = 0; i < 6; ++i)
+        if (int rc = to_device(ctx, *dev[i], host[i], n)) return rc;
+    bool alt = false;
+    if (int rc = radix_sort_u32(ctx, k, ka, a, aa, b, ba, n, max_key, v0_iota != 0, &alt)) return rc;
+    for (int i = 0; i < 6; ++i)
+        if (int rc = to_host(ctx, host[i], *dev[i], n)) return rc;
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    *result_in_alt = alt ? 1 : 0;
+    return B200PPF_OK;
+}
+
+int b200ppf_debug_lower_bounds(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, int64_t dev_len, uint32_t n_keys,
+                               uint32_t shift, uint32_t *offsets, size_t offsets_cap) {
+    if ((n && !sorted) || !offsets || offsets_cap < (size_t)n_keys + 1 || dev_len > (int64_t)n || shift >= 32)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "debug lower bounds: bad argument");
+    CHECK_CTX(ctx);
+    StreamBuf<uint32_t> s(ctx), len(ctx), off(ctx);
+    const uint32_t len_host = dev_len < 0 ? 0u : (uint32_t)dev_len;
+    if (int rc = to_device(ctx, s, sorted, n)) return rc;
+    if (int rc = to_device(ctx, len, dev_len < 0 ? nullptr : &len_host, 1)) return rc;
+    if (int rc = to_device(ctx, off, offsets, offsets_cap)) return rc;
+    if (int rc = lower_bounds(ctx, s, n, len, n_keys, shift, off)) return rc;
+    if (int rc = to_host(ctx, offsets, off, offsets_cap)) return rc;
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B200PPF_OK;
+}
+
+int b200ppf_debug_flag_scan(b200ppf_ctx *ctx, const uint32_t *flags, uint32_t n, uint32_t *rank, size_t rank_cap, int host_total,
+                            uint32_t *total) {
+    if ((n && !flags) || (rank_cap && !rank) || rank_cap < n || !total)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "debug flag scan: bad argument");
+    CHECK_CTX(ctx);
+    StreamBuf<uint32_t> f(ctx), r(ctx), t(ctx);
+    if (int rc = to_device(ctx, f, flags, n)) return rc;
+    if (int rc = to_device(ctx, r, rank, rank_cap)) return rc;
+    if (host_total) {
+        if (int rc = flag_scan_host(ctx, f, n, r, total)) return rc;
+    } else {
+        if (int rc = to_device(ctx, t, total, 1)) return rc;
+        if (int rc = flag_scan(ctx, f, n, r, t)) return rc;
+        if (int rc = to_host(ctx, total, t, 1)) return rc;
+    }
+    if (int rc = to_host(ctx, rank, r, rank_cap)) return rc;
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B200PPF_OK;
+}
+
+int b200ppf_debug_scan_rows(b200ppf_ctx *ctx, uint32_t *data, uint32_t n_rows, uint32_t row_len, size_t data_cap, uint32_t *totals,
+                            size_t totals_cap) {
+    if (!data || !totals || n_rows == 0 || (uint64_t)n_rows * row_len > data_cap || totals_cap < n_rows)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "debug scan rows: bad argument");
+    CHECK_CTX(ctx);
+    StreamBuf<uint32_t> d(ctx), t(ctx);
+    if (int rc = to_device(ctx, d, data, data_cap)) return rc;
+    if (int rc = to_device(ctx, t, totals, totals_cap)) return rc;
+    if (int rc = scan_rows(ctx, d, n_rows, row_len, t)) return rc;
+    if (int rc = to_host(ctx, data, d, data_cap)) return rc;
+    if (int rc = to_host(ctx, totals, t, totals_cap)) return rc;
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B200PPF_OK;
+}
+
+int b200ppf_debug_run_heads(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, uint32_t *head, size_t head_cap) {
+    if ((n && !sorted) || (head_cap && !head) || head_cap < n)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "debug run heads: bad argument");
+    CHECK_CTX(ctx);
+    StreamBuf<uint32_t> s(ctx), h(ctx);
+    if (int rc = to_device(ctx, s, sorted, n)) return rc;
+    if (int rc = to_device(ctx, h, head, head_cap)) return rc;
+    if (int rc = run_heads(ctx, s, n, h)) return rc;
+    if (int rc = to_host(ctx, head, h, head_cap)) return rc;
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B200PPF_OK;
 }
 
 int b200ppf_microbench_atoms(b200ppf_ctx *ctx, int pattern, double *atoms_per_sec) {

@@ -303,8 +303,9 @@ struct SceneGridFree {
 // v0_iota: treat v0 as the identity permutation on entry (its contents are never read).
 int radix_sort_u32(b200ppf_ctx *ctx, uint32_t *keys, uint32_t *keys_alt, uint32_t *v0, uint32_t *v0_alt,
                    uint32_t *v1, uint32_t *v1_alt, size_t n, uint64_t max_key, bool v0_iota, bool *result_in_alt);
-// offsets[k] (k = 0 .. n_keys) = the first i with sorted[i] >= k << shift; the length of sorted is *n_dev when n_dev is
-// non-null (a list whose length only the device knows), else n.  One launch.
+// offsets[k] (k = 0 .. n_keys) = the first i with sorted[i] >= k << shift, the target taken in 64 bits (2^32 and above
+// lie past every key); the length of sorted is *n_dev when n_dev is non-null (a list whose length only the device
+// knows), else n.  One launch.
 int lower_bounds(b200ppf_ctx *ctx, const uint32_t *sorted, uint32_t n, const uint32_t *n_dev, uint32_t n_keys, uint32_t shift,
                  uint32_t *offsets);
 // exclusive scan of flags: rank[k] = the flags equal to 1 before k (written for every k < n), *total_dev = all of them.

@@ -221,16 +221,17 @@ radix_scatter_kernel(const uint32_t *__restrict__ keys, const uint32_t *__restri
 // ---- bucket offsets, flag scan, run heads -------------------------------------------------------------------------
 constexpr int SCAN_BLOCK = 1024;
 
-// n_dev, when non-null, holds the length of the list instead of n
+// n_dev, when non-null, holds the length of the list instead of n.  The target is compared in 64 bits: k << shift may
+// reach 2^32 (offsets[n_keys] of a full key range), which is past every key, not 0.
 __global__ void lower_bounds_kernel(const uint32_t *__restrict__ sorted_keys, uint32_t n, const uint32_t *__restrict__ n_dev,
                                     uint32_t n_keys, uint32_t shift, uint32_t *__restrict__ offsets) {
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k > n_keys) return;
-    const uint32_t want = k << shift;
+    const uint64_t want = (uint64_t)k << shift;
     uint32_t lo = 0, hi = n_dev ? *n_dev : n;
     while (lo < hi) {
         const uint32_t mid = lo + ((hi - lo) >> 1);
-        if (sorted_keys[mid] < want) lo = mid + 1; else hi = mid;
+        if ((uint64_t)sorted_keys[mid] < want) lo = mid + 1; else hi = mid;
     }
     offsets[k] = lo;
 }
