@@ -653,6 +653,75 @@ int b200ppf_match_frame_verified(b200ppf_ctx *ctx, const b200ppf_cloud *scene, s
                                  const b200ppf_object_params *params, const b200ppf_verify_params *verify,
                                  b200ppf_object_result *results, int *status, b200ppf_candidate *candidates);
 
+/* ---- verification against the frame's depth image ----------------------------------------------------------------------
+ * The score above knows only the box's object cloud, so it counts every camera-facing model point as one the scene must
+ * explain: a partly occluded instance loses fit, a model point in space the sensor saw through weighs no more than a hidden
+ * one, and points hidden by the model's own surface count as visible.  The depth image settles all three.
+ *
+ * A depth image on the device: rows x cols float32 metres, row-major (row stride cols); a pixel that is 0, negative or not
+ * finite has no measurement.  K4 = fx, fy, ppx, ppy (fx, fy > 0, all finite).  1 <= rows, cols and rows * cols < 2^31.
+ * b200ppf_cloud_from_depth: the measured pixels back-projected (the reference's include/Camera.h:56-58),
+ * x = (u - ppx) * z / fx, y = (v - ppy) * z / fy in double, rounded to float, in row-major pixel order; zero normals, as
+ * b200ppf_cloud_upload_xyz; the exact bounding box.
+ *
+ * The rule (b200ppf_score_poses_depth), for model point p with normal n under T = [R t] (camera at the origin), tau =
+ * inlier_dist:
+ *   1. p' = R p + t, n' = R n in double, as b200ppf_score_poses moves them.
+ *   2. When z' > 0: u = floor(fx x'/z' + ppx + 0.5), v = floor(fy y'/z' + ppy + 0.5) in double.  IN VIEW: z' > 0 and (u, v)
+ *      inside the image.
+ *   3. A z-buffer per pose: every in-view point j writes z'_j into each pixel of the square of half-width
+ *      h_j = min(floor(fx tau / (2 z'_j)), B200PPF_DEPTH_SPLAT_MAX) around its pixel, clipped to the image; a pixel keeps
+ *      the smallest value.  The models are voxel-sampled at the leaf, tau's default, so a splat of tau covers the gap
+ *      between neighbouring model points.  SELF-OCCLUDED: facing (n'.(-p') > 0, or a zero normal), in view and
+ *      z' > zbuf(u, v) + tau.
+ *   4. VISIBLE: facing, in view, not self-occluded.  With d = D(v, u) at a visible point's pixel: no measurement -> UNKNOWN;
+ *      z' > d + tau -> OCCLUDED (something nearer hides it); z' < d - tau -> VIOLATION (the pose puts a surface where the
+ *      sensor saw through); otherwise the point is judged and consistent, and an INLIER when the nearest-neighbour test of
+ *      b200ppf_score_poses passes (nearest scene point within tau, normals within normal_angle, the lower index on ties).
+ * A pose's record has the same bits alone or in any batch and on every run; the call's launch count does not depend on the
+ * number of jobs, poses or points.  The z-buffer of a pose covers the rectangle its splats touch, 8 bytes a pixel, and
+ * the call holds those of all its poses at once: at most n_poses x rows x cols x 8 bytes of device memory (a pose that
+ * fills a 1280 x 720 image takes 7.4 MB).  Score large sets of hypotheses in batches; when the memory is not there the
+ * call returns B200PPF_ERR_NOMEM. */
+#define B200PPF_DEPTH_SPLAT_MAX 16 /* largest splat half-width, pixels */
+typedef struct b200ppf_depth_image b200ppf_depth_image;
+int b200ppf_depth_upload(b200ppf_ctx *ctx, const float *depth, int rows, int cols, const double K4[4], b200ppf_depth_image **out);
+void b200ppf_depth_free(b200ppf_depth_image *d);
+int b200ppf_cloud_from_depth(b200ppf_ctx *ctx, const b200ppf_depth_image *d, b200ppf_cloud **out);
+typedef struct b200ppf_depth_fit {
+    uint32_t inliers;   /* consistent points whose nearest-neighbour test passes */
+    uint32_t judged;    /* visible - occluded - unknown (violations included) */
+    uint32_t visible, self_occluded, occluded, violations, unknown;
+    float fit;          /* inliers / judged; 0 when judged == 0 */
+    float rms;          /* root mean square of the inliers' nearest-neighbour distances; 0 without inliers */
+} b200ppf_depth_fit;
+/* The jobs of b200ppf_score_poses (poses read only, residuals ignored) scored by the rule above against depth: fits
+ * receives the sum of the jobs' n_poses records, job-major.  B200PPF_ERR_INVALID, before anything is allocated, on the
+ * conditions of b200ppf_score_poses and for a NULL depth image or one of another context. */
+int b200ppf_score_poses_depth(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_depth_image *depth,
+                              const b200ppf_verify_params *params, b200ppf_depth_fit *fits);
+/* The verified frame calls with the score b200ppf_score_poses_depth against the box's object cloud and the frame's depth
+ * image.  Slots, sort order, ties, UINT32_MAX for unused slots, status, return codes and every other result field are as the
+ * verified calls document; depth NULL or of another context is B200PPF_ERR_INVALID.  An application reads violations and
+ * judged beside fit (INTEGRATION.md §3c). */
+typedef struct b200ppf_depth_candidate {
+    double pose[16];  /* row-major 4x4, model -> scene, after ICP when icp_poses > 0 */
+    double residual;  /* its ICP residual (0 without ICP) */
+    uint32_t votes;   /* votes of its pose cluster */
+    uint32_t rank;    /* its position among the clusters, 0 = most voted; UINT32_MAX = unused slot */
+    b200ppf_depth_fit fit;
+} b200ppf_depth_candidate;
+int b200cv_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth,
+                                      size_t n_boxes, const float *corners12, b200cv_detector *const *detectors,
+                                      const b200ppf_cloud *const *models, const b200cv_object_params *params,
+                                      const b200ppf_verify_params *verify, b200ppf_object_result *results, int *status,
+                                      b200ppf_depth_candidate *candidates);
+int b200ppf_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth,
+                                       size_t n_boxes, const float *corners12, const b200ppf_cloud *const *models,
+                                       const b200ppf_table *const *tables, const b200ppf_object_params *params,
+                                       const b200ppf_verify_params *verify, b200ppf_object_result *results, int *status,
+                                       b200ppf_depth_candidate *candidates);
+
 #ifdef __cplusplus
 }
 #endif

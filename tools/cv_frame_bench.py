@@ -21,7 +21,15 @@ the wall time; and b200ppf_score_poses alone on the verified call's candidates o
 from b200cv_match_object), --repeat calls timed with CUDA events on the context's stream.  The verified results must hold
 the plain call's fields and the fits of score_poses.
 
-usage: python tools/cv_frame_bench.py [--repeat 20] [--verify] [--out profiles/r4_cv_frame.jsonl | profiles/r5_verify.jsonl]"""
+--verify-depth: what verification against the depth image adds, on synth.synth_library_depth (1024 x 1024, the scene cloud
+from b200ppf_cloud_from_depth, library boxes and detectors as above, leaf 0.005).  For K = 1, 2, 4, 8 boxes and both match
+steps (match_S2B and Matching): --repeat b200cv_match_frame, _verified and _verified_depth calls, alternated after one warm-up
+of each, medians of the wall time; b200ppf_score_poses_depth against b200ppf_score_poses on the depth-verified call's
+candidates (CUDA events on the context's stream); the instances each call finds within 1 cm / 5 degrees and the best fits.
+Once per run: b200ppf_cloud_from_depth on the 1 Mi-pixel image (CUDA events, median of --repeat).
+
+usage: python tools/cv_frame_bench.py [--repeat 20] [--verify | --verify-depth]
+                                      [--out profiles/r4_cv_frame.jsonl | profiles/r5_verify.jsonl | profiles/r7_verify_depth.jsonl]"""
 import argparse
 import json
 import os
@@ -170,14 +178,87 @@ def bench_verify(c, name, scene, boxes, leaf, K, repeat, gpu):
             "fields_equal_plain": same, "fits_equal_score_poses": fits_match, "gpu": gpu}
 
 
+def _event_ms(c, fn, repeat):
+    """median device time of fn() on the context's stream (CUDA events), after one warm-up"""
+    import torch
+    stream = torch.cuda.ExternalStream(c.stream)
+    fn()
+    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(repeat)]
+    for e0, e1 in ev:
+        e0.record(stream)
+        fn()
+        e1.record(stream)
+    torch.cuda.synchronize()
+    return float(np.median([e0.elapsed_time(e1) for e0, e1 in ev]))
+
+
+def _axis_angle_deg(A, B):
+    R = A[:3, :3].T @ B[:3, :3]
+    return float(np.degrees(np.arccos(np.clip((np.trace(R) - 1) / 2, -1.0, 1.0))))
+
+
+def depth_frame(c):
+    from yolo_ppf_pose_estimation_b200 import capi, synth
+    f = synth.synth_library_depth()
+    dimg = c.upload_depth(f["depth"], f["K"])
+    boxes = []
+    for k in range(8):
+        m = synth.synth_model(2000, 10 + k, k).astype(np.float32)
+        boxes.append((library_box(m, k), capi.CvDetector(c, SAMPLING_STEP, DISTANCE_STEP).train_model(m), c.upload_cloud(m)))
+    return f, dimg, c.cloud_from_depth(dimg), boxes
+
+
+def bench_verify_depth(c, dimg, scene, boxes, K, use_edges, repeat, gpu):
+    from yolo_ppf_pose_estimation_b200 import synth
+    cors = np.stack([b[0] for b in boxes[:K]])
+    dets, mods = [b[1] for b in boxes[:K]], [b[2] for b in boxes[:K]]
+    over = dict(leaf=0.005, use_edges=use_edges, relative_scene_sample_step=0.05 if use_edges else 1.0 / 14.0)
+    calls = {"plain": lambda: c.cv_match_frame(scene, cors, dets, mods, **over),
+             "verified": lambda: c.cv_match_frame_verified(scene, cors, dets, mods, **over),
+             "depth_verified": lambda: c.cv_match_frame_verified_depth(scene, dimg, cors, dets, mods, **over)}
+    wall = {n: [] for n in calls}
+    out = {}
+    for fn in calls.values():
+        fn()  # warm-up
+    for _ in range(repeat):
+        for n, fn in calls.items():
+            t0 = time.perf_counter()
+            out[n] = fn()
+            wall[n].append(1e3 * (time.perf_counter() - t0))
+    for n, o in out.items():
+        assert o[1].tolist() == [0] * K, (n, o[1])
+
+    def found(res):
+        return [k for k in range(K) if np.linalg.norm(res[k]["pose"][:3, 3] - synth.library_pose(k)[:3, 3]) < 0.01 and
+                _axis_angle_deg(res[k]["pose"], synth.library_pose(k)) < 5.0]
+    cands = out["depth_verified"][2]
+    objects = [c.cv_match_object(dets[k], scene, cors[k], mods[k], **over)[1] for k in range(K)]
+    jobs = [(mods[k], objects[k], np.stack([x["pose"] for x in cands[k]])) for k in range(K)]
+    dfits = c.score_poses_depth(jobs, dimg)
+    fits_match = all(f == x["fit"] for k in range(K) for f, x in zip(dfits[k], cands[k]))
+    med = lambda v: float(np.median(v))  # noqa: E731
+    return {"frame": "synth_library_depth 1024x1024", "boxes": K, "match": "match_S2B" if use_edges else "Matching", "calls": repeat,
+            "leaf": 0.005, "verify": {"inlier_dist": 0.01, "normal_angle_deg": 30.0}, "candidates": int(sum(len(x) for x in cands)),
+            "wall_ms_median": {n: med(w) for n, w in wall.items()},
+            "score_poses_depth_device_ms_median": _event_ms(c, lambda: c.score_poses_depth(jobs, dimg), repeat),
+            "score_poses_device_ms_median": _event_ms(c, lambda: c.score_poses(jobs), repeat),
+            "found_1cm_5deg": {n: found(o[0]) for n, o in out.items()},
+            "best_fit": {"verified": [round(float(x[0]["fit"]["fit"]), 4) for x in out["verified"][2]],
+                         "depth_verified": [round(float(x[0]["fit"]["fit"]), 4) for x in cands]},
+            "depth_best": [{k: int(v) if k not in ("fit", "rms") else round(float(v), 4) for k, v in x[0]["fit"].items()} for x in cands],
+            "fits_equal_score_poses_depth": fits_match, "gpu": gpu}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--repeat", type=int, default=20, help="timed frame calls and serial rounds per K (after one warm-up each)")
     ap.add_argument("--verify", action="store_true", help="time the verified frame call and b200ppf_score_poses instead")
+    ap.add_argument("--verify-depth", action="store_true", help="time the depth-verified frame call and b200ppf_score_poses_depth")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if args.out is None:
-        args.out = os.path.join(ROOT, "profiles", "r5_verify.jsonl" if args.verify else "r4_cv_frame.jsonl")
+        args.out = os.path.join(ROOT, "profiles", "r7_verify_depth.jsonl" if args.verify_depth else
+                                "r5_verify.jsonl" if args.verify else "r4_cv_frame.jsonl")
     if args.repeat < 1:
         ap.error("--repeat must be at least 1")
     from yolo_ppf_pose_estimation_b200 import capi
@@ -185,6 +266,19 @@ def main():
     gpu = card()
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
+        if args.verify_depth:
+            fr, dimg, scene, boxes = depth_frame(c)
+            line = json.dumps({"frame": "synth_library_depth 1024x1024", "measured_pixels": int(scene.size),
+                               "cloud_from_depth_device_ms_median": _event_ms(c, lambda: c.cloud_from_depth(dimg), args.repeat),
+                               "calls": args.repeat, "gpu": gpu})
+            print(line, flush=True)
+            f.write(line + "\n")
+            for use_edges in (1, 0):
+                for K in (1, 2, 4, 8):
+                    line = json.dumps(bench_verify_depth(c, dimg, scene, boxes, K, use_edges, args.repeat, gpu))
+                    print(line, flush=True)
+                    f.write(line + "\n")
+            return
         for name, scene, boxes, leaf in frames(c):
             for K in ((1, 8) if args.verify else (1, 2, 4, 8)):
                 line = json.dumps((bench_verify if args.verify else bench)(c, name, scene, boxes, leaf, K, args.repeat, gpu))

@@ -81,6 +81,15 @@ class Candidate(C.Structure):
     _fields_ = [("pose", C.c_double * 16), ("residual", C.c_double), ("votes", C.c_uint32), ("rank", C.c_uint32), ("fit", PoseFit)]
 
 
+class DepthFit(C.Structure):
+    _fields_ = [(n, C.c_uint32) for n in ("inliers", "judged", "visible", "self_occluded", "occluded", "violations", "unknown")] + \
+               [("fit", C.c_float), ("rms", C.c_float)]
+
+
+class DepthCandidate(C.Structure):
+    _fields_ = [("pose", C.c_double * 16), ("residual", C.c_double), ("votes", C.c_uint32), ("rank", C.c_uint32), ("fit", DepthFit)]
+
+
 CANDIDATE_UNUSED = 0xFFFFFFFF  # rank of an unused candidate slot
 
 CV_POSE_DTYPE = np.dtype([("pose", np.float64, (16,)), ("alpha", np.float64), ("residual", np.float64), ("angle", np.float64),
@@ -194,6 +203,14 @@ SYMBOLS = {
                                           C.POINTER(ObjectResult), _vp, C.POINTER(Candidate)]),
     "b200cv_match_frame_verified": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(VerifyParams),
                                          C.POINTER(ObjectResult), _vp, C.POINTER(Candidate)]),
+    "b200ppf_depth_upload": (_i, [_vp, _vp, _i, _i, _vp, C.POINTER(_vp)]),
+    "b200ppf_depth_free": (None, [_vp]),
+    "b200ppf_cloud_from_depth": (_i, [_vp, _vp, C.POINTER(_vp)]),
+    "b200ppf_score_poses_depth": (_i, [_vp, C.POINTER(IcpJob), _sz, _vp, C.POINTER(VerifyParams), C.POINTER(DepthFit)]),
+    "b200ppf_match_frame_verified_depth": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(ObjectParams), C.POINTER(VerifyParams),
+                                                C.POINTER(ObjectResult), _vp, C.POINTER(DepthCandidate)]),
+    "b200cv_match_frame_verified_depth": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(VerifyParams),
+                                               C.POINTER(ObjectResult), _vp, C.POINTER(DepthCandidate)]),
     "b200ppf_register": (_i, [_vp, _vp, _vp, _vp, _sz, _f, _f, _vp, _vp, _vp, C.POINTER(_sz)]),
     "b200cv_detector_create": (_i, [_vp, C.c_double, C.c_double, C.c_double, C.POINTER(_vp)]),
     "b200cv_detector_free": (None, [_vp]),
@@ -347,6 +364,20 @@ class Context:
         self.check(lib().b200ppf_cloud_upload_xyz(self._h, _p(xyz), xyz.shape[0], xyz.shape[1], C.byref(h)))
         return Cloud(self, h)
 
+    def upload_depth(self, depth, K) -> "DepthImage":
+        """(rows, cols) float32 metres (0, negative or non-finite = no measurement) and K = fx, fy, ppx, ppy -> DepthImage"""
+        depth = np.ascontiguousarray(depth, np.float32)
+        K4 = np.ascontiguousarray(K, np.float64).reshape(4)
+        h = C.c_void_p()
+        self.check(lib().b200ppf_depth_upload(self._h, _p(depth), depth.shape[0], depth.shape[1], _p(K4), C.byref(h)))
+        return DepthImage(self, h, depth.shape, K4)
+
+    def cloud_from_depth(self, depth: "DepthImage") -> "Cloud":
+        """the measured pixels back-projected (include/Camera.h:56-58 of the reference), row-major, zero normals"""
+        h = C.c_void_p()
+        self.check(lib().b200ppf_cloud_from_depth(self._h, depth._h, C.byref(h)))
+        return Cloud(self, h)
+
     def crop_pyramid(self, cloud: "Cloud", corners):
         """CloudProcessor::SceneCropping's ConvexHull + CropHull for one box: -> (cropped Cloud, kept indices)"""
         c12 = np.ascontiguousarray(corners, np.float32).reshape(12)
@@ -452,9 +483,9 @@ class Context:
 
     @staticmethod
     def _fit(f):
-        return {"inliers": f.inliers, "visible": f.visible, "fit": f.fit, "rms": f.rms}
+        return {n: getattr(f, n) for n, _ in type(f)._fields_}
 
-    def _verified_frame_call(self, params_cls, default_fn, call, corners, overrides):
+    def _verified_frame_call(self, params_cls, default_fn, call, corners, overrides, cand_cls=Candidate):
         """the verified frame calls: -> (result dicts, int32 status per box, candidate dicts per box (used slots only,
         best first))"""
         c12 = np.ascontiguousarray(corners, np.float32).reshape(-1, 12)
@@ -465,7 +496,7 @@ class Context:
         slots = max(prm.icp_poses, 1)
         res = (ObjectResult * max(1, K))()
         status = np.zeros(max(1, K), np.int32)
-        cand = (Candidate * max(1, K * slots))()
+        cand = (cand_cls * max(1, K * slots))()
         self.check(call(K, _p(c12), C.byref(prm), C.byref(vp), res, _p(status), cand))
         per_box = []
         for b in range(K):
@@ -477,6 +508,16 @@ class Context:
     def score_poses(self, jobs, inlier_dist=None, normal_angle=None):
         """b200ppf_score_poses: jobs = [(model, scene, poses (P,4,4)), ...] -> [list of P fit dicts per job]
         (inliers, visible, fit, rms); None keeps a default (0.01 m, 30 degrees)"""
+        return self._score_call(jobs, inlier_dist, normal_angle, PoseFit,
+                                lambda js, n, vp, fits: lib().b200ppf_score_poses(self._h, js, n, vp, fits))
+
+    def score_poses_depth(self, jobs, depth: "DepthImage", inlier_dist=None, normal_angle=None):
+        """b200ppf_score_poses_depth: score_poses against the depth image -> [list of P depth-fit dicts per job] (inliers,
+        judged, visible, self_occluded, occluded, violations, unknown, fit, rms)"""
+        return self._score_call(jobs, inlier_dist, normal_angle, DepthFit,
+                                lambda js, n, vp, fits: lib().b200ppf_score_poses_depth(self._h, js, n, depth._h, vp, fits))
+
+    def _score_call(self, jobs, inlier_dist, normal_angle, fit_cls, call):
         over = {k: v for k, v in (("inlier_dist", inlier_dist), ("normal_angle", normal_angle)) if v is not None}
         vp = self.verify_params(**over)
         arrays = [np.ascontiguousarray(np.asarray(p, np.float64).reshape(-1, 4, 4)) for _, _, p in jobs]
@@ -484,8 +525,8 @@ class Context:
         for k, ((m, s, _), P) in enumerate(zip(jobs, arrays)):
             js[k] = IcpJob(m._h, s._h, P.ctypes.data, P.shape[0], None)
         total = sum(P.shape[0] for P in arrays)
-        fits = (PoseFit * max(1, total))()
-        self.check(lib().b200ppf_score_poses(self._h, js, len(jobs), C.byref(vp), fits))
+        fits = (fit_cls * max(1, total))()
+        self.check(call(js, len(jobs), C.byref(vp), fits))
         out, at = [], 0
         for P in arrays:
             out.append([self._fit(fits[at + i]) for i in range(P.shape[0])])
@@ -509,6 +550,25 @@ class Context:
         return self._verified_frame_call(
             ObjectParams, lib().b200ppf_object_params_default,
             lambda k, c, *a: lib().b200ppf_match_frame_verified(self._h, scene._h, k, c, mods, tabs, *a), corners, dict(overrides))
+
+    def cv_match_frame_verified_depth(self, scene: "Cloud", depth: "DepthImage", corners, detectors, models, **overrides):
+        """cv_match_frame_verified with the candidates scored against the frame's depth image
+        (b200cv_match_frame_verified_depth): candidates carry depth-fit dicts"""
+        n = len(detectors)
+        dets, mods = self._handles(detectors, n), self._handles(models, n)
+        return self._verified_frame_call(
+            CvObjectParams, lib().b200cv_object_params_default,
+            lambda k, c, *a: lib().b200cv_match_frame_verified_depth(self._h, scene._h, depth._h, k, c, dets, mods, *a), corners,
+            dict(overrides), DepthCandidate)
+
+    def match_frame_verified_depth(self, scene: "Cloud", depth: "DepthImage", corners, models, tables, **overrides):
+        """match_frame_verified with the candidates scored against the frame's depth image (b200ppf_match_frame_verified_depth)"""
+        n = len(models)
+        mods, tabs = self._handles(models, n), self._handles(tables, n)
+        return self._verified_frame_call(
+            ObjectParams, lib().b200ppf_object_params_default,
+            lambda k, c, *a: lib().b200ppf_match_frame_verified_depth(self._h, scene._h, depth._h, k, c, mods, tabs, *a), corners,
+            dict(overrides), DepthCandidate)
 
     @staticmethod
     def _handles(objs, n):
@@ -1040,6 +1100,14 @@ class Cloud(_Handle):
         out = np.zeros((self.size, stride), np.float32)
         self.ctx.check(lib().b200ppf_cloud_download(self.ctx._h, self._h, _p(out), stride, 3, 6 if curvature else 0))
         return out
+
+
+class DepthImage(_Handle):
+    _free = "b200ppf_depth_free"
+
+    def __init__(self, ctx, h, shape, K):
+        super().__init__(ctx, h)
+        self.shape, self.K = tuple(shape), np.array(K, np.float64)
 
 
 class Features(_Handle):

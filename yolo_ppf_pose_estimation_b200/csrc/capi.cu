@@ -78,6 +78,34 @@ int verify_params(b200ppf_ctx *ctx, const b200ppf_verify_params *params, b200ppf
     return B200PPF_OK;
 }
 
+// the job block of the score calls: NULL arrays, clouds of another context and non-finite poses are refused
+int score_jobs_args(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, bool have_fits) {
+    if (n_jobs && !jobs) return fail_msg(ctx, B200PPF_ERR_INVALID, "score poses: null jobs");
+    size_t n_poses = 0;
+    for (size_t j = 0; j < n_jobs; ++j) {
+        char msg[128];
+        const b200ppf_icp_job &jb = jobs[j];
+        const char *why = !jb.model || !jb.scene || (jb.n_poses && !jb.poses16) ? "null argument"
+                          : jb.model->ctx != ctx || jb.scene->ctx != ctx       ? "a cloud belongs to another context"
+                                                                                : nullptr;
+        for (size_t k = 0; !why && k < 16 * jb.n_poses; ++k)
+            if (!std::isfinite(jb.poses16[k])) why = "a pose is not finite";
+        if (why) {
+            snprintf(msg, sizeof(msg), "score poses: job %zu: %s", j, why);
+            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
+        }
+        n_poses += jb.n_poses;
+    }
+    if (n_poses && !have_fits) return fail_msg(ctx, B200PPF_ERR_INVALID, "score poses: null fits");
+    return B200PPF_OK;
+}
+
+int depth_arg(b200ppf_ctx *ctx, const b200ppf_depth_image *depth) {
+    if (!depth) return fail_msg(ctx, B200PPF_ERR_INVALID, "depth score: null depth image");
+    if (depth->ctx != ctx) return fail_msg(ctx, B200PPF_ERR_INVALID, "depth score: the depth image belongs to another context");
+    return B200PPF_OK;
+}
+
 // the parity hooks' copies: a host array of n words into a new stream-ordered buffer (none for a NULL array), and back
 int to_device(b200ppf_ctx *ctx, StreamBuf<uint32_t> &d, const uint32_t *host, size_t n) {
     if (!host) return B200PPF_OK;
@@ -1134,24 +1162,57 @@ int b200ppf_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_
     CHECK_CTX(ctx);
     b200ppf_verify_params p;
     if (int rc = verify_params(ctx, params, &p)) return rc;
-    if (n_jobs && !jobs) return fail_msg(ctx, B200PPF_ERR_INVALID, "score poses: null jobs");
-    size_t n_poses = 0;
-    for (size_t j = 0; j < n_jobs; ++j) {
-        char msg[128];
-        const b200ppf_icp_job &jb = jobs[j];
-        const char *why = !jb.model || !jb.scene || (jb.n_poses && !jb.poses16) ? "null argument"
-                          : jb.model->ctx != ctx || jb.scene->ctx != ctx       ? "a cloud belongs to another context"
-                                                                                : nullptr;
-        for (size_t k = 0; !why && k < 16 * jb.n_poses; ++k)
-            if (!std::isfinite(jb.poses16[k])) why = "a pose is not finite";
-        if (why) {
-            snprintf(msg, sizeof(msg), "score poses: job %zu: %s", j, why);
-            return fail_msg(ctx, B200PPF_ERR_INVALID, msg);
-        }
-        n_poses += jb.n_poses;
-    }
-    if (n_poses && !fits) return fail_msg(ctx, B200PPF_ERR_INVALID, "score poses: null fits");
+    if (int rc = score_jobs_args(ctx, jobs, n_jobs, fits != nullptr)) return rc;
     return verify_score_poses(ctx, jobs, n_jobs, p, fits);
+}
+
+int b200ppf_depth_upload(b200ppf_ctx *ctx, const float *depth, int rows, int cols, const double *K4, b200ppf_depth_image **out) {
+    CHECK_CTX(ctx);
+    if (!depth || !K4 || !out) return fail_msg(ctx, B200PPF_ERR_INVALID, "depth upload: null argument");
+    if (rows < 1 || cols < 1 || (int64_t)rows * (int64_t)cols >= (int64_t)1 << 31)
+        return fail_msg(ctx, B200PPF_ERR_INVALID, "depth upload: rows and cols must be >= 1 with rows * cols < 2^31");
+    for (int k = 0; k < 4; ++k)
+        if (!std::isfinite(K4[k])) return fail_msg(ctx, B200PPF_ERR_INVALID, "depth upload: the intrinsics must be finite");
+    if (!(K4[0] > 0.0) || !(K4[1] > 0.0)) return fail_msg(ctx, B200PPF_ERR_INVALID, "depth upload: fx and fy must be positive");
+    std::unique_ptr<b200ppf_depth_image, FreeWith<b200ppf_depth_free>> d(new (std::nothrow) b200ppf_depth_image());
+    if (!d) return fail_msg(ctx, B200PPF_ERR_NOMEM, "depth upload: out of host memory");
+    d->ctx = ctx;
+    d->rows = rows;
+    d->cols = cols;
+    for (int k = 0; k < 4; ++k) d->K[k] = K4[k];
+    const size_t bytes = (size_t)rows * (size_t)cols * sizeof(float);
+    PPF_CUDA(ctx, cudaMallocAsync(&d->d, bytes, ctx->stream));
+    PPF_CUDA(ctx, cudaMemcpyAsync(d->d, depth, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    *out = d.release();
+    return B200PPF_OK;
+}
+
+void b200ppf_depth_free(b200ppf_depth_image *d) {
+    if (!d) return;
+    DeviceGuard guard(d->ctx ? d->ctx->device : 0);
+    if (d->d) {
+        if (d->ctx) cudaFreeAsync(d->d, d->ctx->stream);
+        else cudaFree(d->d);
+    }
+    delete d;
+}
+
+int b200ppf_cloud_from_depth(b200ppf_ctx *ctx, const b200ppf_depth_image *d, b200ppf_cloud **out) {
+    CHECK_CTX(ctx);
+    if (!d || !out) return fail_msg(ctx, B200PPF_ERR_INVALID, "cloud from depth: null argument");
+    if (d->ctx != ctx) return fail_msg(ctx, B200PPF_ERR_INVALID, "cloud from depth: the image belongs to another context");
+    return prep_cloud_from_depth(ctx, d, out);
+}
+
+int b200ppf_score_poses_depth(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_depth_image *depth,
+                              const b200ppf_verify_params *params, b200ppf_depth_fit *fits) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params p;
+    if (int rc = verify_params(ctx, params, &p)) return rc;
+    if (int rc = score_jobs_args(ctx, jobs, n_jobs, fits != nullptr)) return rc;
+    if (int rc = depth_arg(ctx, depth)) return rc;
+    return verify_score_poses_depth(ctx, jobs, n_jobs, depth, p, fits);
 }
 
 int b200ppf_register(b200ppf_ctx *ctx, const b200ppf_cloud *model, const b200ppf_table *t,
@@ -1211,18 +1272,30 @@ int object_prep(b200ppf_ctx *ctx, const b200ppf_cloud *cropped, const Params &p,
 // a CUDA or memory failure ends a call; any other failure of a box's chain is that box's status
 bool fatal(int rc) { return rc == B200PPF_ERR_CUDA || rc == B200PPF_ERR_NOMEM; }
 
+// the candidates' score: against the object clouds alone, or with the frame's depth image
+int score_candidates(b200ppf_ctx *ctx, const std::vector<b200ppf_icp_job> &jobs, const b200ppf_verify_params &verify,
+                     const b200ppf_depth_image *, b200ppf_pose_fit *fits) {
+    return verify_score_poses(ctx, jobs.data(), jobs.size(), verify, fits);
+}
+int score_candidates(b200ppf_ctx *ctx, const std::vector<b200ppf_icp_job> &jobs, const b200ppf_verify_params &verify,
+                     const b200ppf_depth_image *depth, b200ppf_depth_fit *fits) {
+    return verify_score_poses_depth(ctx, jobs.data(), jobs.size(), depth, verify, fits);
+}
+
 // The chain of every match call, frame or per-object: crop all boxes in one pass, then per box the pre-processing and
 // `match(b, object, edges, &poses, &votes)`, the engine's matching step (it fills the box's match_ms and n_poses and returns
 // its best poses, 16 doubles each, most-voted first, and their clusters' votes), then one batched ICP of the top icp_poses
 // poses of every box that reached it against models[b].  With verify (checked), the candidates of every such box (the
 // refined poses, or the top pose alone without ICP) are then scored in one b200ppf_score_poses against models[b] and the
-// box's object cloud, the best one becomes the box's result, and candidates (may be NULL) receives them all, max(icp_poses,
-// 1) slots per box.  When box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
-template <class Params, class Match>
+// box's object cloud (b200ppf_score_poses_depth with the frame's depth image when Cand is b200ppf_depth_candidate), the
+// best one becomes the box's result, and candidates (may be NULL) receives them all, max(icp_poses, 1) slots per box.  When
+// box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
+template <class Params, class Match, class Cand>
 int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
                 const b200ppf_cloud *const *models, const Params &p, bool with_edges, b200ppf_object_result *results, int *status,
-                b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify,
-                b200ppf_candidate *candidates, Match match) {
+                b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify, Cand *candidates,
+                const b200ppf_depth_image *depth, Match match) {
+    using Fit = decltype(Cand::fit);
     const auto t0 = std::chrono::steady_clock::now();
     for (size_t b = 0; b < n_boxes; ++b) {
         memset(&results[b], 0, sizeof(results[b]));
@@ -1264,7 +1337,7 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
         if (int rc = b200ppf_icp_refine_batch(ctx, jobs.data(), jobs.size(), &p.icp, nullptr)) return rc;
         icp_ms = ctx->timings.icp_ms;
     }
-    std::vector<std::vector<b200ppf_pose_fit>> fits(n_boxes);
+    std::vector<std::vector<Fit>> fits(n_boxes);
     std::vector<size_t> best(n_boxes, 0);  // resultsSub[0] unless verified
     if (verify) {
         std::vector<b200ppf_icp_job> score_jobs;
@@ -1274,8 +1347,8 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
                 score_jobs.push_back(b200ppf_icp_job{models[b], objects[b].get(), refined[b].data(), n_cand[b], nullptr});
                 n_scored += n_cand[b];
             }
-        std::vector<b200ppf_pose_fit> all(n_scored);
-        if (int rc = verify_score_poses(ctx, score_jobs.data(), score_jobs.size(), *verify, all.data())) return rc;
+        std::vector<Fit> all(n_scored);
+        if (int rc = score_candidates(ctx, score_jobs, *verify, depth, all.data())) return rc;
         size_t at = 0;
         for (size_t b = 0; b < n_boxes; ++b) {
             if (status[b]) continue;
@@ -1300,7 +1373,7 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
     if (verify && candidates) {
         const size_t slots = p.icp_poses > 1 ? (size_t)p.icp_poses : 1;
         for (size_t b = 0; b < n_boxes; ++b) {
-            b200ppf_candidate *c = candidates + b * slots;
+            Cand *c = candidates + b * slots;
             memset(c, 0, slots * sizeof(*c));
             for (size_t k = 0; k < slots; ++k) c[k].rank = UINT32_MAX;
             if (status[b]) continue;
@@ -1342,10 +1415,11 @@ int frame_args(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, con
 
 // b200ppf_match_frame; b200ppf_match_object is this on one box.  The PCL matching does not read the edge cloud: it is
 // extracted when the caller wants it (want_edges) and edge_curvature > 0.
+template <class Cand = b200ppf_candidate>
 int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, const b200ppf_cloud *const *models,
               const b200ppf_table *const *tables, const b200ppf_object_params *params, b200ppf_object_result *results, int *status,
               bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify = nullptr,
-              b200ppf_candidate *candidates = nullptr) {
+              Cand *candidates = nullptr, const b200ppf_depth_image *depth = nullptr) {
     CHECK_CTX(ctx);
     if (int rc = frame_args(ctx, scene, n_boxes, corners12, tables, models, results, status)) return rc;
     for (size_t b = 0; b < n_boxes; ++b)
@@ -1375,15 +1449,16 @@ int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, cons
         return B200PPF_OK;
     };
     return match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && want_edges, results, status, object_out,
-                       edges_out, verify, candidates, match);
+                       edges_out, verify, candidates, depth, match);
 }
 
 // b200cv_match_frame; b200cv_match_object is this on one box.  The edge cloud is extracted when edge_curvature > 0 and
 // Matching_S2B needs it (use_edges) or the caller wants it (want_edges).
+template <class Cand = b200ppf_candidate>
 int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, b200cv_detector *const *detectors,
              const b200ppf_cloud *const *models, const b200cv_object_params *params, b200ppf_object_result *results, int *status,
              bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify = nullptr,
-             b200ppf_candidate *candidates = nullptr) {
+             Cand *candidates = nullptr, const b200ppf_depth_image *depth = nullptr) {
     CHECK_CTX(ctx);
     if (int rc = frame_args(ctx, scene, n_boxes, corners12, detectors, models, results, status)) return rc;
     for (size_t b = 0; b < n_boxes; ++b) {
@@ -1433,7 +1508,7 @@ int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const
         return B200PPF_OK;
     };
     const int rc = match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && (p.use_edges || want_edges),
-                               results, status, object_out, edges_out, verify, candidates, match);
+                               results, status, object_out, edges_out, verify, candidates, depth, match);
     cudaEventDestroy(ev[0]);
     cudaEventDestroy(ev[1]);
     return rc;
@@ -1523,6 +1598,30 @@ int b200ppf_match_frame_verified(b200ppf_ctx *ctx, const b200ppf_cloud *scene, s
     b200ppf_verify_params v;
     if (int rc = verify_params(ctx, verify, &v)) return rc;
     return ppf_match(ctx, scene, n_boxes, corners12, models, tables, params, results, status, true, nullptr, nullptr, &v, candidates);
+}
+
+int b200cv_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth, size_t n_boxes,
+                                      const float *corners12, b200cv_detector *const *detectors, const b200ppf_cloud *const *models,
+                                      const b200cv_object_params *params, const b200ppf_verify_params *verify,
+                                      b200ppf_object_result *results, int *status, b200ppf_depth_candidate *candidates) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params v;
+    if (int rc = verify_params(ctx, verify, &v)) return rc;
+    if (int rc = depth_arg(ctx, depth)) return rc;
+    return cv_match(ctx, scene, n_boxes, corners12, detectors, models, params, results, status, true, nullptr, nullptr, &v, candidates,
+                    depth);
+}
+
+int b200ppf_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth, size_t n_boxes,
+                                       const float *corners12, const b200ppf_cloud *const *models, const b200ppf_table *const *tables,
+                                       const b200ppf_object_params *params, const b200ppf_verify_params *verify,
+                                       b200ppf_object_result *results, int *status, b200ppf_depth_candidate *candidates) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params v;
+    if (int rc = verify_params(ctx, verify, &v)) return rc;
+    if (int rc = depth_arg(ctx, depth)) return rc;
+    return ppf_match(ctx, scene, n_boxes, corners12, models, tables, params, results, status, true, nullptr, nullptr, &v, candidates,
+                     depth);
 }
 
 }  // extern "C"

@@ -66,6 +66,13 @@ struct b200ppf_cloud {
     float bbox_min[3] = {0, 0, 0}, bbox_max[3] = {0, 0, 0};  // exact min / max of pos: every producer of a cloud sets them
 };
 
+struct b200ppf_depth_image {
+    b200ppf_ctx *ctx = nullptr;
+    int rows = 0, cols = 0;
+    double K[4] = {0, 0, 0, 0};  // fx fy ppx ppy
+    float *d = nullptr;          // rows x cols, row-major
+};
+
 struct b200ppf_features {
     b200ppf_ctx *ctx = nullptr;
     size_t count = 0;              // n*n
@@ -238,6 +245,9 @@ int k6_icp_refine_batch(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_
 // the pose scores of b200ppf_score_poses (verify.cu) for checked arguments: fits of the jobs' poses, job-major
 int verify_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_verify_params &params,
                        b200ppf_pose_fit *fits);
+// the same jobs scored against a depth image (b200ppf_score_poses_depth) for checked arguments
+int verify_score_poses_depth(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_depth_image *depth,
+                             const b200ppf_verify_params &params, b200ppf_depth_fit *fits);
 
 // the context of an OpenCV-engine detector and whether it holds a trained model (k7_cvppf.cu)
 b200ppf_ctx *cv_detector_context(const b200cv_detector *d);
@@ -258,6 +268,8 @@ void prep_frustum_corners(const float *depth, int rows, int cols, int bx, int by
 int prep_crop_pyramid(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, b200ppf_cloud **out, uint32_t *kept_host);
 // the crop for n_boxes pyramids in one pass over the frame; out[b] as prep_crop_pyramid(corners12 + 12 * b) makes it
 int prep_crop_pyramids(b200ppf_ctx *ctx, const b200ppf_cloud *in, const float *corners12, size_t n_boxes, b200ppf_cloud **out);
+// the measured pixels of a depth image back-projected, in row-major pixel order (b200ppf_cloud_from_depth)
+int prep_cloud_from_depth(b200ppf_ctx *ctx, const b200ppf_depth_image *d, b200ppf_cloud **out);
 int prep_debug_knn_host(const float *xyz, size_t n, size_t stride, int k, int mode, float cell_edge, const float *viewpoint3,
                         int cov_mode, uint32_t *idx, float *d2, float *mean_dist, float *normals4);
 

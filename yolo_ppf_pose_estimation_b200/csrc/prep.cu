@@ -675,6 +675,29 @@ pyramids_scatter_kernel(const float4 *__restrict__ pos, const float4 *__restrict
     }
 }
 
+// ---- the scene cloud of a depth image (include/Camera.h:56-58 of the reference) ----------------------------------
+__device__ __forceinline__ bool depth_measured(float d) { return d > 0.0f && d < INFINITY; }  // NaN fails both
+
+__global__ void __launch_bounds__(256) depth_flag_kernel(const float *__restrict__ depth, uint32_t n, uint32_t *__restrict__ flags) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    flags[i] = depth_measured(depth[i]) ? 1u : 0u;
+}
+
+// x = (u - ppx) * z / fx, y = (v - ppy) * z / fy in double (no product to fuse), rounded to float
+__global__ void __launch_bounds__(256)
+depth_scatter_kernel(const float *__restrict__ depth, uint32_t n, uint32_t cols, double fx, double fy, double ppx, double ppy,
+                     const uint32_t *__restrict__ rank, float4 *__restrict__ out_pos, float4 *__restrict__ out_nrm) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float d = depth[i];
+    if (!depth_measured(d)) return;
+    const double z = (double)d, u = (double)(i % cols), v = (double)(i / cols);
+    const uint32_t r = rank[i];
+    out_pos[r] = make_float4((float)((u - ppx) * z / fx), (float)((v - ppy) * z / fy), d, 1.0f);
+    out_nrm[r] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+}
+
 // ---- P6 ---------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) renormalize_kernel(float4 *__restrict__ nrm, uint32_t n) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -744,6 +767,24 @@ int prep_upload_xyz(b200ppf_ctx *ctx, const float *host, size_t n, size_t stride
     if (m) PPF_CUDA(ctx, cudaMemcpyAsync(c->pos, sp, m * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
     if (m) PPF_CUDA(ctx, cudaMemsetAsync(c->nrm, 0, m * sizeof(float4), ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the staging buffer is reused by the next upload
+    *out = c.release();
+    return B200PPF_OK;
+}
+
+int prep_cloud_from_depth(b200ppf_ctx *ctx, const b200ppf_depth_image *d, b200ppf_cloud **out) {
+    const uint32_t n = (uint32_t)d->rows * (uint32_t)d->cols;
+    StreamBuf<uint32_t> flags(ctx), rank(ctx);
+    PPF_CUDA(ctx, flags.alloc(n));
+    PPF_CUDA(ctx, rank.alloc(n));
+    PPF_LAUNCH(ctx, depth_flag_kernel, (n + 255) / 256, 256, 0, d->d, n, flags.p);
+    uint32_t m = 0;
+    int rc = flag_scan_host(ctx, flags, n, rank, &m);
+    if (rc != B200PPF_OK) return rc;
+    CloudPtr c;
+    if ((rc = cloud_alloc(ctx, m, &c)) != B200PPF_OK) return rc;
+    PPF_LAUNCH(ctx, depth_scatter_kernel, (n + 255) / 256, 256, 0, d->d, n, (uint32_t)d->cols, d->K[0], d->K[1], d->K[2], d->K[3],
+               rank.p, c->pos, c->nrm);
+    if ((rc = cloud_bbox_from_device(ctx, c.get())) != B200PPF_OK) return rc;  // synchronises the stream
     *out = c.release();
     return B200PPF_OK;
 }

@@ -192,3 +192,119 @@ def synth_library_scene(n: int = 1 << 20, seed: int = 3, n_models: int = 8, mode
     s = s[: n] if s.shape[0] >= n else np.concatenate([s, rest[: n - s.shape[0]]], axis=0)
     order = np.argsort(uniform(seed, 71, s.shape[0]), kind="stable")
     return s[order].astype(np.float32)
+
+
+DEPTH_SHAPE = (1024, 1024)
+DEPTH_K = (400.0, 400.0, 511.5, 511.5)  # fx, fy, ppx, ppy: the 8 library instances all in view
+DEPTH_OCCLUDED = (2, 6)  # the library instances a sphere stands in front of: poses whose decoys the unhidden half still tells apart
+
+
+def _sphere_depth(depth, label, lab, centre, radius, K):
+    """render one sphere into depth (z of the nearer intersection per ray; pixel (u, v) looks along ((u - ppx) / fx,
+    (v - ppy) / fy, 1)), writing lab into label where it is nearest; only the pixels of its projected bounding square"""
+    fx, fy, ppx, ppy = K
+    rows, cols = depth.shape
+    c = np.asarray(centre, np.float64)
+    if c[2] <= radius:
+        return
+    reach = radius / (c[2] - radius)
+    u0 = int(max(0, np.floor(fx * (c[0] / c[2] - reach) + ppx)))
+    u1 = int(min(cols - 1, np.ceil(fx * (c[0] / c[2] + reach) + ppx)))
+    v0 = int(max(0, np.floor(fy * (c[1] / c[2] - reach) + ppy)))
+    v1 = int(min(rows - 1, np.ceil(fy * (c[1] / c[2] + reach) + ppy)))
+    if u0 > u1 or v0 > v1:
+        return
+    v, u = np.mgrid[v0:v1 + 1, u0:u1 + 1]
+    wx, wy = (u - ppx) / fx, (v - ppy) / fy
+    a = wx * wx + wy * wy + 1.0
+    b = -2.0 * (wx * c[0] + wy * c[1] + c[2])
+    cc = c @ c - radius * radius
+    disc = b * b - 4 * a * cc
+    hit = disc >= 0
+    t = np.where(hit, (-b - np.sqrt(np.where(hit, disc, 0))) / (2 * a), np.inf)
+    sub, lsub = depth[v0:v1 + 1, u0:u1 + 1], label[v0:v1 + 1, u0:u1 + 1]
+    near = hit & (t > 0) & (t < sub)
+    sub[near] = t[near]
+    lsub[near] = lab
+
+
+def synth_library_depth(seed: int = 3, n_models: int = 8, dense: int = 300_000, occluded=DEPTH_OCCLUDED):
+    """A deterministic depth frame of the library scene: DEPTH_SHAPE float32 metres under DEPTH_K, holding the ground plane
+    and walls of synth_scene (intersected per ray), its clutter spheres (radius 5 cm) except those whose image disc meets an
+    instance's box, the n_models library instances under library_pose(k) (a dense synth_model(dense, 10 + k + 7919, k)
+    splatted one point per pixel, nearest wins) and, in front of each instance of `occluded`, a sphere covering 30-60 % of
+    that instance's visible pixels on the side of its base.  0.5 mm of sensor noise on every measured depth; rays that meet nothing read 0.
+    -> dict(depth, K (4,), occluded_share (n_models,), occluders [(k, centre, radius)])"""
+    rows, cols = DEPTH_SHAPE
+    fx, fy, ppx, ppy = DEPTH_K
+    v, u = np.mgrid[0:rows, 0:cols]
+    wx, wy = (u - ppx) / fx, (v - ppy) / fy
+    depth = np.full(DEPTH_SHAPE, np.inf)
+    label = np.full(DEPTH_SHAPE, -1, np.int64)  # -1 background, k instance k, n_models + j occluder j
+    with np.errstate(divide="ignore", invalid="ignore"):
+        t = 0.45 / wy  # ground y = 0.45, x in [-1, 1], z in [0.5, 2.5]
+        ok = (wy > 0) & (np.abs(t * wx) <= 1.0) & (t >= 0.5) & (t <= 2.5)
+        depth[ok] = np.minimum(depth[ok], t[ok])
+        t = np.full(DEPTH_SHAPE, 2.5)  # back wall z = 2.5, x in [-1, 1], y in [-0.6, 0.45]
+        ok = (np.abs(t * wx) <= 1.0) & (t * wy >= -0.6) & (t * wy <= 0.45)
+        depth[ok] = np.minimum(depth[ok], t[ok])
+        t = -1.0 / wx  # side wall x = -1, y in [-0.6, 0.45], z in [0.5, 2.5]
+        ok = (wx < 0) & (t * wy >= -0.6) & (t * wy <= 0.45) & (t >= 0.5) & (t <= 2.5)
+        depth[ok] = np.minimum(depth[ok], t[ok])
+    # the instances, one dense splat each, and their image boxes
+    boxes = []
+    for k in range(n_models):
+        T = library_pose(k, seed)
+        m = synth_model(dense, 10 + k + 7919, k).astype(np.float64)
+        p = m[:, :3] @ T[:3, :3].T + T[:3, 3]
+        pu = np.floor(fx * p[:, 0] / p[:, 2] + ppx + 0.5).astype(np.int64)
+        pv = np.floor(fy * p[:, 1] / p[:, 2] + ppy + 0.5).astype(np.int64)
+        inside = (pu >= 0) & (pu < cols) & (pv >= 0) & (pv < rows)
+        pu, pv, pz = pu[inside], pv[inside], p[inside, 2]
+        boxes.append((pu.min(), pu.max(), pv.min(), pv.max()))
+        flat = depth.ravel()
+        lab = label.ravel()
+        before = flat.copy()
+        np.minimum.at(flat, pv * cols + pu, pz)
+        lab[flat < before] = k
+    # the clutter spheres of synth_scene (synth_library_scene's share of the points), away from the instances
+    n_rest = (1 << 20) - n_models * int(round(0.015 * (1 << 20)))
+    n_clutter = n_rest - int(round(0.40 * n_rest)) - int(round(0.30 * n_rest))
+    n_blobs = max(1, n_clutter // 400)
+    cs = np.stack([-0.9 + 1.8 * uniform(seed, 30, n_blobs), -0.5 + 0.9 * uniform(seed, 31, n_blobs),
+                   0.6 + 1.8 * uniform(seed, 32, n_blobs)], 1)
+    for c in cs:
+        reach = 0.05 / (c[2] - 0.05)
+        cu0, cu1 = fx * (c[0] / c[2] - reach) + ppx, fx * (c[0] / c[2] + reach) + ppx
+        cv0, cv1 = fy * (c[1] / c[2] - reach) + ppy, fy * (c[1] / c[2] + reach) + ppy
+        if any(cu1 >= b[0] - 2 and cu0 <= b[1] + 2 and cv1 >= b[2] - 2 and cv0 <= b[3] + 2 for b in boxes):
+            continue
+        _sphere_depth(depth, label, -1, c, 0.05, DEPTH_K)
+    # the occluders: a sphere 25 cm in front of the instance, moved from its centre toward its base until it hides at most
+    # half of it; the shoulder and neck, which tell a pose from its shifted and upside-down twins, stay in view
+    share = np.zeros(n_models)
+    occluders = []
+    for j, k in enumerate(occluded):
+        mine = label == k
+        vv, uu = np.nonzero(mine)
+        zc = float(np.median(depth[mine]))
+        ray = np.array([(uu.mean() - ppx) / fx, (vv.mean() - ppy) / fy, 1.0])
+        zo, radius = zc - 0.25, 0.05
+        base = library_pose(k, seed)[:3, 3]  # the model's origin: the centre of its base
+        toward = base / base[2] - ray
+        toward = np.array([toward[0], toward[1], 0.0]) / np.hypot(toward[0], toward[1])
+        for shift in np.arange(0.0, 0.2, 0.004):
+            centre = ray * zo + shift * toward
+            d2, l2 = depth.copy(), label.copy()
+            _sphere_depth(d2, l2, n_models + j, centre, radius, DEPTH_K)
+            s = float(((l2 == n_models + j) & mine).sum()) / mine.sum()
+            if s <= 0.5:
+                break
+        assert 0.3 <= s <= 0.6, (k, s)
+        depth, label = d2, l2
+        share[k] = s
+        occluders.append((k, centre, radius))
+    measured = np.isfinite(depth)
+    noisy = depth + 0.0005 * normal(seed, 300, rows * cols).reshape(DEPTH_SHAPE)
+    out = np.where(measured, noisy, 0.0).astype(np.float32)
+    return dict(depth=out, K=np.array(DEPTH_K, np.float64), occluded_share=share, occluders=occluders)
