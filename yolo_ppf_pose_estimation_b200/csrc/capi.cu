@@ -695,6 +695,8 @@ int b200ppf_table_load(b200ppf_ctx *ctx, const char *path, b200ppf_table **out) 
             PPF_CUDA(ctx, cudaMemcpyAsync(*arrs[a].slot, host[a].data(), arrs[a].words * sizeof(uint32_t), cudaMemcpyHostToDevice,
                                           ctx->stream));
     }
+    // whatever order the file holds inside its phase cells, the loaded table walks its own cells in blocks as a built one
+    if (int rc = b200ppf::k2_order_own_blocks(ctx, t.get())) return rc;
     if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) return fail_msg(ctx, B200PPF_ERR_CUDA, "table load: upload failed");
     *out = t.release();
     return B200PPF_OK;

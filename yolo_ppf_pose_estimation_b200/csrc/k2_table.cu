@@ -332,6 +332,87 @@ bank_order_kernel(const uint32_t *__restrict__ sub_offsets, uint32_t total_sub, 
     }
 }
 
+// Own-cell blocks.  The voting kernel walks the unmerged entries of the scene phase's own cell 32 per step, and a step
+// whose entries all lie below the scene's own sub-phases (or all above them) votes with one shift and no per-entry
+// decision (k3_vote.cu own_step).  Inside every phase cell the entries are therefore stably partitioned by the top
+// OWN_BLOCK_BITS bits of their sub-phase byte (a "block"): only the steps that touch the scene's own block can mix the
+// two sides.  A stable partition, not a sort: inside a block the (bin of alpha_m, i, j) order stays, which keeps the
+// entries of one model row adjacent (one ATOMS.POPC.INC pass for the lanes that share a word) and consecutive rows in
+// consecutive banks.  Entries filed just outside their cell carry sub-phase 0 or 255: first or last block.  The vote
+// counts do not depend on this order; only the speed of the own-cell walk does, and only the folding tables' kernel
+// (k3_fold_qbits) tests its steps: smaller tables keep the sorted order, which their per-entry loop walks faster.  One warp per non-empty cell: a count
+// per block (one per lane), their exclusive scan, then a stable scatter of the four entry arrays.
+#ifndef B200PPF_OWN_BLOCK_BITS
+#define B200PPF_OWN_BLOCK_BITS 5
+#endif
+constexpr uint32_t OWN_BLOCK_BITS = B200PPF_OWN_BLOCK_BITS;
+constexpr uint32_t OWN_BLOCKS = 1u << OWN_BLOCK_BITS;
+static_assert(OWN_BLOCK_BITS >= 1 && OWN_BLOCKS <= 32, "one block counter per lane");
+
+__global__ void __launch_bounds__(SPREAD_WARPS * 32)
+own_block_kernel(const uint32_t *__restrict__ sub_offsets, uint32_t total_sub, const uint32_t *__restrict__ w_in,
+                 const uint32_t *__restrict__ am_in, const uint32_t *__restrict__ alpha_in, const uint32_t *__restrict__ idx_in,
+                 uint32_t *__restrict__ w_out, uint32_t *__restrict__ am_out, uint32_t *__restrict__ alpha_out,
+                 uint32_t *__restrict__ idx_out) {
+    __shared__ uint32_t s_next[SPREAD_WARPS][OWN_BLOCKS];
+    const uint32_t lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    uint32_t *next = s_next[wib];
+    const uint32_t n_warps = gridDim.x * SPREAD_WARPS;
+    for (uint32_t c0 = (blockIdx.x * SPREAD_WARPS + wib) * 32; c0 < total_sub; c0 += n_warps * 32) {
+        const uint32_t c = c0 + lane;
+        uint32_t b = 0, e = 0;
+        if (c < total_sub) {
+            b = sub_offsets[c];
+            e = sub_offsets[c + 1];
+        }
+        uint32_t nonempty = __ballot_sync(0xFFFFFFFFu, e > b);
+        while (nonempty) {
+            const int src = __ffs(nonempty) - 1;
+            nonempty &= nonempty - 1;
+            const uint32_t cb = __shfl_sync(0xFFFFFFFFu, b, src), ce = __shfl_sync(0xFFFFFFFFu, e, src);
+            // entries per block (one shared add per block present in a step), then where each block starts in the cell
+            if (lane < OWN_BLOCKS) next[lane] = 0;
+            __syncwarp();
+            for (uint32_t k0 = cb; k0 < ce; k0 += 32) {
+                const uint32_t k = k0 + lane;
+                const bool valid = k < ce;
+                const uint32_t blk = valid ? w_in[k] >> (32u - OWN_BLOCK_BITS) : OWN_BLOCKS + lane;
+                const uint32_t same = __match_any_sync(0xFFFFFFFFu, blk);
+                if (valid && lane == (uint32_t)(31 - __clz(same))) atomicAdd(&next[blk], (uint32_t)__popc(same));
+            }
+            __syncwarp();
+            const uint32_t cnt = lane < OWN_BLOCKS ? next[lane] : 0u;
+            __syncwarp();
+            uint32_t incl = cnt;
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+                if (lane >= (uint32_t)o) incl += t;
+            }
+            if (lane < OWN_BLOCKS) next[lane] = cb + incl - cnt;
+            __syncwarp();
+            for (uint32_t k0 = cb; k0 < ce; k0 += 32) {
+                const uint32_t k = k0 + lane;
+                const bool valid = k < ce;
+                const uint32_t w = valid ? w_in[k] : 0u;
+                const uint32_t blk = valid ? w >> (32u - OWN_BLOCK_BITS) : OWN_BLOCKS + lane;  // idle lanes match nobody
+                const uint32_t same = __match_any_sync(0xFFFFFFFFu, blk);
+                uint32_t dest = 0;
+                if (valid) dest = next[blk] + __popc(same & ((1u << lane) - 1u));
+                __syncwarp();
+                if (valid && lane == (uint32_t)(31 - __clz(same))) next[blk] = dest + 1;  // highest lane of the block
+                __syncwarp();
+                if (valid) {
+                    w_out[dest] = w;
+                    am_out[dest] = am_in[k];
+                    alpha_out[dest] = alpha_in[k];
+                    idx_out[dest] = idx_in[k];
+                }
+            }
+            __syncwarp();
+        }
+    }
+}
+
 __global__ void alpha_scatter_kernel(const uint32_t *__restrict__ entry_idx, const float *__restrict__ entry_alpha,
                                      uint32_t n_entries, float *__restrict__ out) {
     uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -585,6 +666,8 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
                                           ctx->stream));
         }
     }
+    // the merged words are made from the sorted entry order: the own-cell blocks come after them
+    if ((rc = k2_order_own_blocks(ctx, t.get()))) return rc;
     info.n_merged = t->n_merged;
     unsigned long long h_cnt = 0;
     PPF_CUDA(ctx, cudaMemcpyAsync(&h_cnt, d_cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, ctx->stream));
@@ -598,6 +681,30 @@ int k2_build(b200ppf_ctx *ctx, const b200ppf_features *feat, const b200ppf_cloud
     cudaEventElapsedTime(&ctx->timings.sort_ms, ctx->ev[1], ctx->ev[2]);
     cudaEventElapsedTime(&ctx->timings.csr_ms, ctx->ev[2], ctx->ev[3]);
     *out = t.release();
+    return B200PPF_OK;
+}
+
+int k2_order_own_blocks(b200ppf_ctx *ctx, b200ppf_table *t) {
+    // only the folding kernel tests steps for one side; the smaller tables' per-entry loop is faster in sorted order
+    if (!k3_fold_qbits(t) || getenv("B200PPF_NO_OWN_BLOCKS")) return B200PPF_OK;
+    const std::array<TableArray, 8> arrs = table_arrays(t);
+    // the four entry arrays (file order 2..5) are rewritten into fresh arrays of the same length and pad
+    StreamBuf<uint32_t> fresh[4] = {StreamBuf<uint32_t>(ctx), StreamBuf<uint32_t>(ctx), StreamBuf<uint32_t>(ctx),
+                                    StreamBuf<uint32_t>(ctx)};
+    for (int a = 0; a < 4; ++a) {
+        TableArray f = arrs[2 + a];
+        f.slot = &fresh[a].p;
+        PPF_CUDA(ctx, table_array_alloc(ctx->stream, f));
+    }
+    const uint32_t total_sub = (uint32_t)(((uint64_t)t->info.key_space * t->info.n_slices) << t->bp.cells_log2);
+    const unsigned blocks =
+        (unsigned)std::min<size_t>(((size_t)total_sub + 32 * SPREAD_WARPS - 1) / (32 * SPREAD_WARPS), (size_t)ctx->sm_count * 16);
+    PPF_LAUNCH(ctx, own_block_kernel, blocks, SPREAD_WARPS * 32, 0, t->sub_offsets, total_sub, t->entry_w, t->entry_am,
+               reinterpret_cast<const uint32_t *>(t->entry_alpha), t->entry_idx, fresh[0].p, fresh[1].p, fresh[2].p, fresh[3].p);
+    for (int a = 0; a < 4; ++a) {
+        cudaFreeAsync(*arrs[2 + a].slot, ctx->stream);
+        *arrs[2 + a].slot = fresh[a].release();
+    }
     return B200PPF_OK;
 }
 

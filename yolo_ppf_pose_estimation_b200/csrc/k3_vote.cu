@@ -20,9 +20,10 @@
 //             at (entry's hot word - one constant); the scene phase's own cell is a "per-entry" item;
 //   C  vote   warps pull work items.  Shift items: 8 x 32 hot words in flight per lane, a vote is
 //             load / subtract / add-min / red.shared (ppf_math.cuh "constant-shift voting").
-//             The scene phase's own cell compares phases per entry; tables whose 2*pi/step is not an
-//             integer bin every entry in fixed point with guard bands, the literal double-precision
-//             form inside the bands.
+//             The scene phase's own cell compares phases per entry — on folding tables, whose cells the build
+//             orders by sub-phase block, a group of steps whose entries all lie on one side of the scene phase
+//             votes with one shift; tables whose 2*pi/step is not an integer bin every entry in fixed point
+//             with guard bands, the literal double-precision form inside the bands.
 //   D  fold   tables of 2 M+ entries, tasks that flush more than once or hold FOLD_MIN_PAIRS+ candidates: a pair on the
 //             constant-shift path keeps only its own cell in phase C and leaves a code (key, q, cell) in its CTA's fold
 //             buffer, across flushes.  At the end of the task (or of a scope of FOLD_SCOPE codes) the codes are sorted; for
@@ -525,7 +526,10 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                             const uint32_t acc_own = pin_register(acc_addr), c_hi_own = pin_register(c_hi);
                             // the scene phase's own cell by sub-phase: rel = (entry's sub-phase) - sub_lo.  rel > span
                             // (unsigned) = outside the scene's own sub-phases, and then the sign of rel tells the side.
-                            const uint32_t sub_lo = wi.sub_range & 0xFFu, span = ((wi.sub_range >> 8) & 0xFFu) - sub_lo;
+                            const uint32_t sub_lo = wi.sub_range & 0xFFu, sub_hi = (wi.sub_range >> 8) & 0xFFu, span = sub_hi - sub_lo;
+                            // The sub-phase is the word's top byte: w < below_lim <=> below the scene's own sub-phases,
+                            // w > above_lim <=> above them (never when sub_hi = 255).
+                            const uint32_t below_lim = sub_lo << 24, above_lim = (sub_hi << 24) | HOT_MASK;
                             // The increment stays the +1 form (ATOMS.POPC.INC): the entries of one model row are adjacent
                             // in the cell, and lanes of one instruction that hit the same word are counted in one pass —
                             // adding the decision as a value (ATOMS.ADD) serialises them and measured 2 % slower.
@@ -534,6 +538,31 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
                                 uint32_t w[U], v[U], settled = 0;
 #pragma unroll
                                 for (int u = 0; u < U; ++u) w[u] = __ldg(wp + k0 + u * 32);
+                                // Every live entry of these steps below the scene's own sub-phases (or every one above
+                                // them): all vote with one shift, like a shift range.  The table orders each cell by
+                                // sub-phase block (k2_table.cu), so that this is the case for all steps but those that
+                                // touch the scene's own block; the test reads each entry's own byte and holds in any order.
+                                // Folding tables only (2 M+ entries, long own cells): on small tables the own cells that
+                                // reach this loop are few and short, and the extra code measured 1 % slower on C2.
+                                if constexpr (FOLD) {
+                                    bool below = true, above = true;
+#pragma unroll
+                                    for (int u = 0; u < U; ++u) {
+                                        const bool live = !tail || k0 + u * 32 < e_end;
+                                        below = below && (!live || w[u] < below_lim);
+                                        above = above && (!live || w[u] > above_lim);
+                                    }
+                                    const uint32_t side = __reduce_and_sync(0xFFFFFFFFu, (below ? 1u : 0u) | (above ? 2u : 0u));
+                                    if (side) {  // warp-uniform: the vote of a shift range, with the +1 increment
+                                        const uint32_t c0v = (side & 1u) ? c_lo : c_hi, c1v = c0v - wrap_bytes;
+#pragma unroll
+                                        for (int u = 0; u < U; ++u) {
+                                            const uint32_t off = w[u] & HOT_MASK;
+                                            if (!tail || k0 + u * 32 < e_end) red_shared_inc(acc_addr + min(off - c0v, off - c1v));
+                                        }
+                                        return;
+                                    }
+                                }
 #pragma unroll
                                 for (int u = 0; u < U; ++u) {
                                     const uint32_t rel = (w[u] >> 24) - sub_lo;
@@ -1085,13 +1114,7 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
     a.signal_slot = a.signal_value = 0;
     a.done_counter = nullptr;
     a.no_sub_phase = getenv("B200PPF_NO_SUB_PHASE") ? 1 : 0;
-    // folded shift ranges: phase-sorted tables of FOLD_MIN_ENTRIES+ entries whose fold codes (key, q, cell) fit 31 bits
-    a.fold_qbits = 0;
-    if (a.bp.bulk && a.bp.mode == ALPHA_MODE_A && t->info.n_entries >= FOLD_MIN_ENTRIES) {
-        auto bits = [](uint32_t x) { uint32_t b = 0; while (b < 32 && (x >> b) != 0) ++b; return b; };
-        const uint32_t qbits = bits(a.bp.n_turn - 1u);
-        if (bits(a.kp.key_space - 1u) + qbits + a.bp.cells_log2 <= 31) a.fold_qbits = qbits;
-    }
+    a.fold_qbits = a.bp.mode == ALPHA_MODE_A ? k3_fold_qbits(t) : 0u;
     for (int g = 0; g < MAX_PEERS; ++g) {
         a.peer_peaks[g] = nullptr;
         a.peer_flags[g] = nullptr;
@@ -1188,6 +1211,14 @@ int check_vote_inputs(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cl
 }
 
 }  // namespace
+
+// folded shift ranges: phase-sorted tables of FOLD_MIN_ENTRIES+ entries whose fold codes (key, q, cell) fit 31 bits
+uint32_t k3_fold_qbits(const b200ppf_table *t) {
+    if (!t->bp.bulk || t->info.n_entries < FOLD_MIN_ENTRIES) return 0;
+    auto bits = [](uint32_t x) { uint32_t b = 0; while (b < 32 && (x >> b) != 0) ++b; return b; };
+    const uint32_t qbits = bits(t->bp.n_turn - 1u);
+    return bits(t->kp.key_space - 1u) + qbits + t->bp.cells_log2 <= 31 ? qbits : 0u;
+}
 
 uint32_t num_alpha_bins(float angle_step, int nalpha_rule) {
     const double t = 2.0 * M_PI / (double)angle_step;

@@ -196,6 +196,12 @@ cudaError_t table_array_alloc(cudaStream_t stream, const TableArray &a);
 int k1_features_compute(b200ppf_ctx *ctx, const b200ppf_cloud *model, b200ppf_signature *out);
 int k2_build(b200ppf_ctx *ctx, const b200ppf_features *f, const b200ppf_cloud *model, float angle_step,
              float dist_step, b200ppf_table **out);
+// partitions each phase cell's unmerged entries by sub-phase block (k2_table.cu), after a build and after a load, on the
+// tables whose vote kernel folds (the one that walks own cells in blocks); the vote counts do not depend on it.
+// B200PPF_NO_OWN_BLOCKS (debug) leaves the entries in sorted order.
+int k2_order_own_blocks(b200ppf_ctx *ctx, b200ppf_table *t);
+// bits of q in the fold codes of the table's vote launches (k3_vote.cu); 0: the table does not fold
+uint32_t k3_fold_qbits(const b200ppf_table *t);
 int k2_query_key(b200ppf_ctx *ctx, const b200ppf_table *t, const int32_t *d4, uint64_t *pairs, size_t cap,
                  size_t *n_found);
 int k2_alpha_m(b200ppf_ctx *ctx, const b200ppf_table *t, float *host);
