@@ -110,8 +110,7 @@ static_assert(FOLD_SCOPE >= CAND_CAP, "a scope must take one whole flush");
 
 struct VoteArgs {
     const float4 *pos, *nrm;    // scene, original order (reference points are addressed by index)
-    const float4 *gpos, *gnrm;  // scene, cell-sorted
-    const uint32_t *gorig;      // cell-sorted position -> original index
+    const float4 *gpos, *gnrm;  // scene, cell-sorted (gpos.w: the bits of the point's original index)
     const uint32_t *cell_start;
     GridParams gp;
     uint32_t n_s;
@@ -771,8 +770,9 @@ __device__ __forceinline__ void vote_task(const VoteArgs &a, const uint32_t ref_
             const float dx = p4.x - p_r.x, dy = p4.y - p_r.y, dz = p4.z - p_r.z;
             const float d2 = (dx * dx + dy * dy) + dz * dz;
             // radius predicate on f4 itself (SURVEY.md A.8 rule 7): sqrtf(d2) < radius, evaluated
-            // through the equivalent threshold on d2 (sqrtf is monotone and correctly rounded)
-            in = d2 < a.radius_sq_bound && __ldg(a.gorig + s) != s_r;
+            // through the equivalent threshold on d2 (sqrtf is monotone and correctly rounded); the point's index (w) is
+            // read after the test, as holding p4.w across it costs some instantiations a register
+            in = d2 < a.radius_sq_bound && __float_as_uint(__ldg(&a.gpos[s].w)) != s_r;
             ++st_examined;
         }
         const uint32_t m = __ballot_sync(0xFFFFFFFFu, in);
@@ -1077,18 +1077,15 @@ float radius_sq_bound(float r) {
 int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *scene, size_t ref_first,
                 size_t ref_step, size_t ref_count, uint32_t *acc_dump, const VoteQueue *queue = nullptr) {
     const float radius = t->info.max_dist * 0.5f;
-    SceneGrid grid;
-    std::unique_ptr<SceneGrid, SceneGridFree> grid_owner(&grid, SceneGridFree{ctx});
-    int rc = scene_grid_build(ctx, scene, radius, &grid);
-    if (rc) return rc;
+    SceneGrids grid(ctx);
+    if (int rc = scene_grid_build_one(ctx, scene, radius, &grid)) return rc;
     VoteArgs a;
     a.pos = scene->pos;
     a.nrm = scene->nrm;
     a.gpos = grid.pos;
     a.gnrm = grid.nrm;
-    a.gorig = grid.orig;
     a.cell_start = grid.cell_start;
-    a.gp = grid.gp;
+    a.gp = grid.scenes[0].gp;
     a.n_s = (uint32_t)scene->n;
     a.ref_first = (uint32_t)ref_first;
     a.ref_step = (uint32_t)ref_step;
@@ -1160,12 +1157,12 @@ int launch_vote(b200ppf_ctx *ctx, const b200ppf_table *t, const b200ppf_cloud *s
         PPF_CUDA(ctx, cost_alt.alloc(ref_count));
         PPF_CUDA(ctx, order.alloc(ref_count));
         PPF_CUDA(ctx, order_alt.alloc(ref_count));
-        PPF_LAUNCH(ctx, ref_cost_kernel, (unsigned)((ref_count + 255) / 256), 256, 0, scene->pos, grid.cell_start, grid.gp,
+        PPF_LAUNCH(ctx, ref_cost_kernel, (unsigned)((ref_count + 255) / 256), 256, 0, scene->pos, grid.cell_start.p, a.gp,
                    (uint32_t)ref_first, (uint32_t)ref_step, (uint32_t)ref_count, (uint32_t)scene->n, cost.p);
         bool in_alt = false;  // costs are counts of scene points
-        rc = radix_sort_u32(ctx, cost.p, cost_alt.p, order.p, order_alt.p, nullptr, nullptr, ref_count, scene->n, /*v0_iota=*/true,
-                            &in_alt);
-        if (rc) return rc;
+        if (int rc = radix_sort_u32(ctx, cost.p, cost_alt.p, order.p, order_alt.p, nullptr, nullptr, ref_count, scene->n,
+                                    /*v0_iota=*/true, &in_alt))
+            return rc;
         a.ref_order = in_alt ? order_alt.p : order.p;
     }
 #define LAUNCH_VOTE_T(M, S, B, T, F)                                                                                  \

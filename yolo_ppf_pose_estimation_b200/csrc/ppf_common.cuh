@@ -9,6 +9,7 @@
 #include <array>
 #include <memory>
 #include <string>
+#include <vector>
 
 #include "../../include/b200ppf.h"
 #include "ppf_math.cuh"
@@ -295,23 +296,39 @@ __host__ __device__ __forceinline__ uint32_t grid_cell_linear(const GridParams &
     return ((uint32_t)z * (uint32_t)g.dims[1] + (uint32_t)y) * (uint32_t)g.dims[0] + (uint32_t)x;
 }
 
-struct SceneGrid {
-    GridParams gp{};
-    uint32_t n_cells = 0;
-    uint32_t *cell_start = nullptr;  // [n_cells + 1] into the cell-sorted arrays
-    float4 *pos = nullptr, *nrm = nullptr;  // cell-sorted copies of the scene
-    uint32_t *orig = nullptr;        // cell-sorted position -> original scene index
+// one scene of a grid build: its cloud's points, where they sit in the concatenation of the build's scenes, and its cells
+// (the ids cell_base .. cell_base + cells - 1 of the shared id space)
+struct GridScene {
+    const float4 *pos, *nrm;
+    uint32_t first, n;
+    uint32_t cell_base;
+    GridParams gp;
 };
 
-// grid geometry for a bounding box and a search radius (host), coarsened until it has at most max_cells cells; returns the
-// number of cells (0 for a non-finite box or radius)
-uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp, uint32_t max_cells = 1u << 22);
-int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *scene, float radius, SceneGrid *out);
-void scene_grid_free(b200ppf_ctx *ctx, SceneGrid *g);
-struct SceneGridFree {
-    b200ppf_ctx *ctx;
-    void operator()(SceneGrid *g) const { scene_grid_free(ctx, g); }
+// the cell-sorted grids of one build (scene_grid_build): scene k is scenes[k] (on the device in table when asked for), its
+// cells' points are pos / nrm [cell_start[cell_base + c], cell_start[cell_base + c + 1]), in input order inside a cell,
+// and w of a position holds the bits of the point's index in its own scene (no arithmetic on it)
+struct SceneGrids {
+    std::vector<GridScene> scenes;
+    uint32_t n_cells = 0;  // over all scenes
+    StreamBuf<GridScene> table;
+    StreamBuf<uint32_t> cell_start;  // [n_cells + 1]
+    StreamBuf<float4> pos, nrm;
+    explicit SceneGrids(b200ppf_ctx *ctx) : table(ctx), cell_start(ctx), pos(ctx), nrm(ctx) {}
 };
+
+// grid geometry for a bounding box and a cell edge (host), coarsened until it has at most max_cells cells; returns the
+// number of cells (0 for a non-finite box or edge)
+uint32_t scene_grid_params(const float *bbox_min, const float *bbox_max, float radius, GridParams *gp, uint32_t max_cells = 1u << 22);
+// the grids of n_scenes clouds in one pass: cells of edge >= cell_edge, at most cells_per_scene per scene; the sort orders
+// the bits of max(key_limit, total cells).  With device_table the scene table is uploaded for the caller's kernels.  When
+// no grid fits a scene (a non-finite box or edge, or no cells to give) out->n_cells is 0, nothing runs, and the error is
+// the caller's to report.
+int scene_grid_build(b200ppf_ctx *ctx, const b200ppf_cloud *const *clouds, uint32_t n_scenes, float cell_edge,
+                     uint32_t cells_per_scene, uint32_t key_limit, bool device_table, SceneGrids *out);
+// the grid of one cloud (at most 2^22 cells, the sort over its own cells, no device table); B200PPF_ERR_INVALID when no
+// grid fits it
+int scene_grid_build_one(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, float cell_edge, SceneGrids *out);
 
 // ---- sorted-key primitives (sort_scan.cu), all on the context stream ----------------------------------------------
 // hand-written LSD radix sort: keys ascending, stable, two 32-bit payload streams.

@@ -158,9 +158,8 @@ enum { KNN_EXPORT = 0, KNN_MEAN_DISTANCE = 1, KNN_NORMAL = 2 };
 
 struct KnnArgs {
     const float4 *pos;    // cloud, original order
-    const float4 *gpos;   // cloud, cell-sorted
+    const float4 *gpos;   // cloud, cell-sorted (gpos.w: the bits of the point's original index)
     const uint32_t *cell_start;
-    const uint32_t *orig;  // cell-sorted position -> original index
     GridParams gp;
     float cell;  // cell edge
     uint32_t n;
@@ -326,7 +325,7 @@ __host__ __device__ inline void knn_query(const KnnArgs &a, const uint32_t q, Ke
             float d2 = ex * ex;
             d2 += ey * ey;
             d2 += ez * ez;
-            const unsigned long long key = ((unsigned long long)f32_bits(d2) << 32) | (unsigned long long)ld_ro(a.orig + s);
+            const unsigned long long key = ((unsigned long long)f32_bits(d2) << 32) | (unsigned long long)f32_bits(p.w);
             if (cnt < k) {
                 best[cnt++] = key;
                 if (cnt == k)
@@ -377,7 +376,7 @@ __host__ __device__ inline void knn_query(const KnnArgs &a, const uint32_t q, Ke
         sift_down(0, end, v);
     }
 
-    const uint32_t me = a.orig[q];
+    const uint32_t me = f32_bits(ld_ro(&a.gpos[q].w));  // the query's index, reloaded rather than held through the search
     if (MODE == KNN_EXPORT) {
         for (int j = 0; j < k; ++j) {
             a.out_idx[(size_t)me * k + j] = j < cnt ? (uint32_t)best[j] : 0xFFFFFFFFu;
@@ -439,14 +438,6 @@ __host__ __device__ inline void knn_query(const KnnArgs &a, const uint32_t q, Ke
     }
 }
 
-template <int CAP, int MODE>
-__global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const KnnArgs a) {
-    const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;  // cell-sorted position of the query
-    if (q >= a.n) return;
-    LocalKeys<CAP> best;
-    knn_query<MODE>(a, q, best);
-}
-
 template <int MODE>
 __global__ void __launch_bounds__(KNN_THREADS) knn_smem_kernel(const KnnArgs a) {
     extern __shared__ unsigned long long knn_keys[];  // [k][KNN_THREADS]
@@ -459,15 +450,9 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_smem_kernel(const KnnArgs a) 
 template <int MODE>
 int knn_launch(b200ppf_ctx *ctx, const KnnArgs &a) {
     const unsigned grid = (a.n + KNN_THREADS - 1) / KNN_THREADS;
-    static const bool force_local = getenv("B200PPF_KNN_LOCAL") != nullptr;  // tuning switch: the local-memory variant
-    if (!force_local) {
-        const size_t smem = (size_t)a.k * KNN_THREADS * sizeof(unsigned long long);
-        PPF_CUDA(ctx, cudaFuncSetAttribute(knn_smem_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * KNN_THREADS * 8));
-        PPF_LAUNCH(ctx, knn_smem_kernel<MODE>, grid, KNN_THREADS, smem, a);
-        return B200PPF_OK;
-    }
-    void (*kern)(const KnnArgs) = a.k <= 32 ? knn_kernel<32, MODE> : (a.k <= 64 ? knn_kernel<64, MODE> : knn_kernel<128, MODE>);
-    PPF_LAUNCH(ctx, kern, grid, KNN_THREADS, 0, a);
+    const size_t smem = (size_t)a.k * KNN_THREADS * sizeof(unsigned long long);
+    PPF_CUDA(ctx, cudaFuncSetAttribute(knn_smem_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * KNN_THREADS * 8));
+    PPF_LAUNCH(ctx, knn_smem_kernel<MODE>, grid, KNN_THREADS, smem, a);
     return B200PPF_OK;
 }
 
@@ -487,16 +472,13 @@ float knn_cell_edge(const b200ppf_cloud *c, int k) {
 // grid + neighbour kernel of one mode over `cloud`
 template <int MODE>
 int knn_run(b200ppf_ctx *ctx, const b200ppf_cloud *cloud, KnnArgs a) {
-    SceneGrid grid;
-    std::unique_ptr<SceneGrid, SceneGridFree> grid_owner(&grid, SceneGridFree{ctx});
-    int rc = scene_grid_build(ctx, cloud, knn_cell_edge(cloud, a.k), &grid);
-    if (rc != B200PPF_OK) return rc;
+    SceneGrids grid(ctx);
+    if (int rc = scene_grid_build_one(ctx, cloud, knn_cell_edge(cloud, a.k), &grid)) return rc;
     a.pos = cloud->pos;
     a.gpos = grid.pos;
     a.cell_start = grid.cell_start;
-    a.orig = grid.orig;
-    a.gp = grid.gp;
-    a.cell = 1.0f / grid.gp.inv_cell;
+    a.gp = grid.scenes[0].gp;
+    a.cell = 1.0f / a.gp.inv_cell;
     a.n = (uint32_t)cloud->n;
     return knn_launch<MODE>(ctx, a);
 }
@@ -1110,7 +1092,7 @@ int prep_debug_knn_host(const float *xyz, size_t n, size_t stride, int k, int mo
     KnnArgs a{};
     a.k = k;
     const uint32_t n_cells = scene_grid_params(c.bbox_min, c.bbox_max, cell_edge > 0.0f ? cell_edge : knn_cell_edge(&c, k), &a.gp);
-    std::vector<uint32_t> cell(n), start((size_t)n_cells + 1, 0u), orig(n);
+    std::vector<uint32_t> cell(n), start((size_t)n_cells + 1, 0u);
     for (size_t i = 0; i < n; ++i) {
         cell[i] = grid_cell_linear(a.gp, grid_cell_coord(a.gp, pos[i].x, 0), grid_cell_coord(a.gp, pos[i].y, 1),
                                    grid_cell_coord(a.gp, pos[i].z, 2));
@@ -1121,14 +1103,13 @@ int prep_debug_knn_host(const float *xyz, size_t n, size_t stride, int k, int mo
         std::vector<uint32_t> fill(start.begin(), start.end() - 1);
         for (size_t i = 0; i < n; ++i) {  // stable: original order inside a cell, like the radix sort
             const uint32_t s = fill[cell[i]]++;
-            orig[s] = (uint32_t)i;
             gpos[s] = pos[i];
+            gpos[s].w = bits_f32((uint32_t)i);  // the index in w, as the device grid holds it
         }
     }
     a.pos = pos.data();
     a.gpos = gpos.data();
     a.cell_start = start.data();
-    a.orig = orig.data();
     a.cell = 1.0f / a.gp.inv_cell;
     a.n = (uint32_t)n;
     a.out_idx = idx;

@@ -1,10 +1,9 @@
 // verify.cu — pose verification (b200ppf_score_poses): how much of a pose's visible model surface the scene supports.
 //
-// Every distinct scene of a call gets a uniform grid of cell edge >= inlier_dist, and all of them are built in one pass:
-// cell ids are box-major (scene s owns the ids cell_base[s] .. cell_base[s+1]-1), so one stable radix sort of the
-// concatenated points of all scenes over a fixed 24-bit key orders every scene by cell at once, and one cell_start array
-// indexes them all.  A one-past-the-end key (the total cell count) is appended so that the sort never sees zero elements:
-// the call's launches are the same whatever the number of jobs, poses or scene points.
+// Every distinct scene of a call gets a uniform grid of cell edge >= inlier_dist, and all of them are built in one pass
+// (scene_grid_build, scene_grid.cu): scene s owns the cell ids cell_base[s] ..., the sort runs over a fixed 24-bit key
+// whatever the scenes, and an end key keeps it from ever seeing zero elements, so the call's launches are the same whatever
+// the number of jobs, poses or scene points.  w of a cell-sorted position holds the point's index in its own scene.
 //
 // The score is one block per (pose, chunk of CHUNK model points): each thread moves its points (in double), tests
 // visibility, and searches the 27 cells around the moved point for the nearest scene point within inlier_dist (exact
@@ -28,18 +27,11 @@ namespace b200ppf {
 
 namespace {
 
-constexpr int KEY_BITS = 24;
-constexpr uint32_t MAX_CELLS_TOTAL = (1u << KEY_BITS) - 1;  // leaves the id MAX_CELLS_TOTAL for the end key
+// the scenes of a call share a fixed 24-bit id space, so the sort's passes do not depend on the jobs
+constexpr uint32_t MAX_CELLS_TOTAL = (1u << 24) - 1;
 constexpr uint32_t PER_SCENE_CELLS = 1u << 22;
 constexpr int THREADS = 256;
 constexpr uint32_t CHUNK = 1024;  // model points per block
-
-struct VScene {
-    const float4 *pos, *nrm;
-    uint32_t first, n;  // its points in the call's concatenation
-    uint32_t cell_base;
-    GridParams gp;
-};
 
 struct VPose {
     double R[9], t[3];
@@ -53,16 +45,6 @@ struct Partial {
     double sum_d2;
 };
 
-// the scene of concatenated point i: the last scene that starts at or before it (an empty scene never is that one)
-__device__ __forceinline__ uint32_t scene_of(const VScene *__restrict__ sc, uint32_t n_scenes, uint32_t i) {
-    uint32_t lo = 0, hi = n_scenes;
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (sc[mid].first <= i) lo = mid; else hi = mid;
-    }
-    return lo;
-}
-
 // the cells c-1 .. c+1 around coordinate v's cell c, inside the grid; false when c lies more than one cell outside it
 __device__ __forceinline__ bool cell_range(const GridParams &gp, double v, int axis, int *lo, int *hi) {
     const float f = floorf(((float)v - gp.origin[axis]) * gp.inv_cell);
@@ -71,33 +53,6 @@ __device__ __forceinline__ bool cell_range(const GridParams &gp, double v, int a
     *lo = max(c - 1, 0);
     *hi = min(c + 1, gp.dims[axis] - 1);
     return true;
-}
-
-__global__ void verify_cell_ids_kernel(const VScene *__restrict__ sc, uint32_t n_scenes, uint32_t n_total, uint32_t end_id,
-                                       uint32_t *__restrict__ ids) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i > n_total) return;
-    if (i == n_total) {
-        ids[i] = end_id;
-        return;
-    }
-    const VScene &s = sc[scene_of(sc, n_scenes, i)];
-    const float4 p = s.pos[i - s.first];
-    ids[i] = s.cell_base + grid_cell_linear(s.gp, grid_cell_coord(s.gp, p.x, 0), grid_cell_coord(s.gp, p.y, 1),
-                                            grid_cell_coord(s.gp, p.z, 2));
-}
-
-// cell-sorted copies of the points; w of a position holds the point's index in its own scene (the tie-break)
-__global__ void verify_gather_kernel(const VScene *__restrict__ sc, uint32_t n_scenes, const uint32_t *__restrict__ order,
-                                     uint32_t n_total, float4 *__restrict__ spos, float4 *__restrict__ snrm) {
-    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n_total) return;
-    const uint32_t i = order[j];
-    const VScene &s = sc[scene_of(sc, n_scenes, i)];
-    float4 p = s.pos[i - s.first];
-    p.w = __uint_as_float(i - s.first);
-    spos[j] = p;
-    snrm[j] = s.nrm[i - s.first];
 }
 
 // model point i of pose P moved by it (p' = R p + t, n' = R n in double); true when it faces the camera (n'.(-p') > 0) or
@@ -117,7 +72,7 @@ __device__ __forceinline__ bool move_point(const VPose &P, uint32_t i, double p[
 // the nearest-neighbour test of a moved point: its nearest scene point (exact squared distance in double, the lower original
 // index on ties) lies within inlier_dist and, with use_normals, that point's normal is within the normal angle of n.  *d2
 // receives the squared distance of an inlier.
-__device__ __forceinline__ bool nearest_inlier(const VScene &S, const uint32_t *__restrict__ cell_start, const float4 *__restrict__ spos,
+__device__ __forceinline__ bool nearest_inlier(const GridScene &S, const uint32_t *__restrict__ cell_start, const float4 *__restrict__ spos,
                                                const float4 *__restrict__ snrm, const double p[3], const double n[3], double tau2,
                                                double cos_min, int use_normals, double *d2) {
     if (S.n == 0) return false;
@@ -153,14 +108,14 @@ __device__ __forceinline__ bool nearest_inlier(const VScene &S, const uint32_t *
 }
 
 __global__ void __launch_bounds__(THREADS, 1)
-verify_score_kernel(const VPose *__restrict__ poses, const VScene *__restrict__ scenes, const uint32_t *__restrict__ cell_start,
+verify_score_kernel(const VPose *__restrict__ poses, const GridScene *__restrict__ scenes, const uint32_t *__restrict__ cell_start,
                     const float4 *__restrict__ spos, const float4 *__restrict__ snrm, double tau2, double cos_min, int use_normals,
                     uint32_t n_chunks, Partial *__restrict__ partials) {
     const VPose &P = poses[blockIdx.x];
     const uint32_t begin = blockIdx.y * CHUNK;
     if (begin >= P.n_model) return;  // a chunk past this pose's model: the finalisation never reads it
     const uint32_t end = min(P.n_model, begin + CHUNK);
-    const VScene &S = scenes[P.scene];
+    const GridScene &S = scenes[P.scene];
     uint32_t inliers = 0, visible = 0;
     double sum = 0.0;
     for (uint32_t i = begin + threadIdx.x; i < end; i += THREADS) {
@@ -310,7 +265,7 @@ depth_splat_kernel(const VPose *__restrict__ poses, const ZRect *__restrict__ zr
 
 // the classification of the rule (include/b200ppf.h) and the nearest-neighbour test of the judged, consistent points
 __global__ void __launch_bounds__(THREADS, 1)
-depth_score_kernel(const VPose *__restrict__ poses, const VScene *__restrict__ scenes, const uint32_t *__restrict__ cell_start,
+depth_score_kernel(const VPose *__restrict__ poses, const GridScene *__restrict__ scenes, const uint32_t *__restrict__ cell_start,
                    const float4 *__restrict__ spos, const float4 *__restrict__ snrm, const ZRect *__restrict__ zr, DepthView D,
                    double tau, double tau2, double cos_min, int use_normals, const Proj *__restrict__ proj,
                    const unsigned long long *__restrict__ zbuf, uint32_t n_chunks, DPartial *__restrict__ partials) {
@@ -318,7 +273,7 @@ depth_score_kernel(const VPose *__restrict__ poses, const VScene *__restrict__ s
     const uint32_t begin = blockIdx.y * CHUNK;
     if (begin >= P.n_model) return;
     const uint32_t end = min(P.n_model, begin + CHUNK);
-    const VScene &S = scenes[P.scene];
+    const GridScene &S = scenes[P.scene];
     const ZRect Z = zr[blockIdx.x];
     uint32_t c[7] = {0, 0, 0, 0, 0, 0, 0};  // inliers judged visible self_occluded occluded violations unknown
     double sum = 0.0;
@@ -402,24 +357,21 @@ __global__ void depth_finish_kernel(const VPose *__restrict__ poses, uint32_t n_
 
 namespace {
 
-// the scene grids of a call and its poses on the device: one grid per distinct scene, all built in one pass
+// the scene grids of a call (one per distinct scene, all built in one pass) and its poses on the device
 struct Grids {
     std::vector<VPose> poses;
-    uint32_t n_scenes = 0, max_chunks = 1;
+    uint32_t max_chunks = 1;
     uint64_t n_points = 0;  // model points over all poses
-    StreamBuf<VScene> scenes;
     StreamBuf<VPose> d_poses;
-    StreamBuf<uint32_t> cell_start;
-    StreamBuf<float4> spos, snrm;
-    explicit Grids(b200ppf_ctx *ctx) : scenes(ctx), d_poses(ctx), cell_start(ctx), spos(ctx), snrm(ctx) {}
+    SceneGrids grids;
+    explicit Grids(b200ppf_ctx *ctx) : d_poses(ctx), grids(ctx) {}
 };
 
 // the distinct scenes, in order of first appearance, and the poses, job-major; g->poses stays empty when there is nothing to
 // score, and nothing runs then
 int build_grids(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, const b200ppf_verify_params &params, Grids *g) {
     std::unordered_map<const b200ppf_cloud *, uint32_t> scene_index;
-    std::vector<VScene> scenes;
-    std::vector<const b200ppf_cloud *> scene_clouds;
+    std::vector<const b200ppf_cloud *> scenes;
     std::vector<VPose> &poses = g->poses;
     uint64_t n_total = 0;
     uint32_t max_chunks = 1;
@@ -429,16 +381,10 @@ int build_grids(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, co
         auto it = scene_index.find(jb.scene);
         if (it == scene_index.end()) {
             it = scene_index.emplace(jb.scene, (uint32_t)scenes.size()).first;
-            VScene s{};
-            s.pos = jb.scene->pos;
-            s.nrm = jb.scene->nrm;
-            s.first = (uint32_t)n_total;
-            s.n = (uint32_t)jb.scene->n;
             n_total += jb.scene->n;
             if (n_total >= 0xFFFFFFFFull - (1u << 20))
                 return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "score poses: the scenes hold more than 2^32 points in all");
-            scenes.push_back(s);
-            scene_clouds.push_back(jb.scene);
+            scenes.push_back(jb.scene);
         }
         if (jb.model->n > 0xFFFFFFFFull - CHUNK)
             return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "score poses: a model of more than 2^32 points");
@@ -462,43 +408,16 @@ int build_grids(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_jobs, co
     if (poses.empty()) return B200PPF_OK;
     if (poses.size() > 0x7FFFFFFFull || max_chunks > 65535)
         return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "score poses: too many poses or model points");
+    g->max_chunks = max_chunks;
     // the grids: cells of edge >= inlier_dist, the scenes sharing the 24-bit id space
     const uint32_t budget = std::min<uint32_t>(PER_SCENE_CELLS, MAX_CELLS_TOTAL / (uint32_t)scenes.size());
-    uint32_t n_cells = 0;
-    for (size_t k = 0; k < scenes.size(); ++k) {
-        VScene &s = scenes[k];
-        const b200ppf_cloud *c = scene_clouds[k];
-        const uint32_t cells = budget ? scene_grid_params(c->bbox_min, c->bbox_max, params.inlier_dist, &s.gp, budget) : 0;
-        if (cells == 0) return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "score poses: no grid fits a scene (too many scenes, or a non-finite bounding box)");
-        s.cell_base = n_cells;
-        n_cells += cells;
-    }
-    const uint32_t n = (uint32_t)n_total;
-    g->n_scenes = (uint32_t)scenes.size();
-    g->max_chunks = max_chunks;
-
-    StreamBuf<uint32_t> ids0(ctx), ids1(ctx), ord0(ctx), ord1(ctx);
-    PPF_CUDA(ctx, g->scenes.alloc(scenes.size()));
-    PPF_CUDA(ctx, g->d_poses.alloc(poses.size()));
-    PPF_CUDA(ctx, ids0.alloc(n + 1));
-    PPF_CUDA(ctx, ids1.alloc(n + 1));
-    PPF_CUDA(ctx, ord0.alloc(n + 1));
-    PPF_CUDA(ctx, ord1.alloc(n + 1));
-    PPF_CUDA(ctx, g->cell_start.alloc((size_t)n_cells + 1));
-    PPF_CUDA(ctx, g->spos.alloc(n));
-    PPF_CUDA(ctx, g->snrm.alloc(n));
-    PPF_CUDA(ctx, cudaMemcpyAsync(g->scenes, scenes.data(), scenes.size() * sizeof(VScene), cudaMemcpyHostToDevice, ctx->stream));
-    PPF_CUDA(ctx, cudaMemcpyAsync(g->d_poses, poses.data(), poses.size() * sizeof(VPose), cudaMemcpyHostToDevice, ctx->stream));
-
-    PPF_LAUNCH(ctx, verify_cell_ids_kernel, (n + 1 + 255) / 256, 256, 0, g->scenes.p, g->n_scenes, n, n_cells, ids0.p);
-    bool in_alt = false;
-    if (int rc = radix_sort_u32(ctx, ids0, ids1, ord0, ord1, nullptr, nullptr, (size_t)n + 1, MAX_CELLS_TOTAL, /*v0_iota=*/true,
-                                &in_alt))
+    if (int rc = scene_grid_build(ctx, scenes.data(), (uint32_t)scenes.size(), params.inlier_dist, budget, MAX_CELLS_TOTAL,
+                                  /*device_table=*/true, &g->grids))
         return rc;
-    const uint32_t *ids_sorted = in_alt ? ids1.p : ids0.p, *ord_sorted = in_alt ? ord1.p : ord0.p;
-    if (int rc = lower_bounds(ctx, ids_sorted, n + 1, nullptr, n_cells, 0, g->cell_start)) return rc;
-    PPF_LAUNCH(ctx, verify_gather_kernel, std::max(1u, (n + 255) / 256), 256, 0, g->scenes.p, g->n_scenes, ord_sorted, n, g->spos.p,
-               g->snrm.p);
+    if (g->grids.n_cells == 0)
+        return fail_msg(ctx, B200PPF_ERR_UNSUPPORTED, "score poses: no grid fits a scene (too many scenes, or a non-finite bounding box)");
+    PPF_CUDA(ctx, g->d_poses.alloc(poses.size()));
+    PPF_CUDA(ctx, cudaMemcpyAsync(g->d_poses, poses.data(), poses.size() * sizeof(VPose), cudaMemcpyHostToDevice, ctx->stream));
     return B200PPF_OK;
 }
 
@@ -526,8 +445,8 @@ int verify_score_poses(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size_t n_j
     PPF_CUDA(ctx, d_fits.alloc(n_poses));
     const double tau = (double)params.inlier_dist;
     const NormalTest nt = normal_test(params);
-    PPF_LAUNCH(ctx, verify_score_kernel, dim3(n_poses, g.max_chunks), THREADS, 0, g.d_poses.p, g.scenes.p, g.cell_start.p, g.spos.p,
-               g.snrm.p, tau * tau, nt.cos_min, nt.use_normals, g.max_chunks, partials.p);
+    PPF_LAUNCH(ctx, verify_score_kernel, dim3(n_poses, g.max_chunks), THREADS, 0, g.d_poses.p, g.grids.table.p, g.grids.cell_start.p,
+               g.grids.pos.p, g.grids.nrm.p, tau * tau, nt.cos_min, nt.use_normals, g.max_chunks, partials.p);
     PPF_LAUNCH(ctx, verify_finish_kernel, (n_poses + 127) / 128, 128, 0, g.d_poses.p, n_poses, partials.p, g.max_chunks, d_fits.p);
     PPF_CUDA(ctx, cudaMemcpyAsync(fits, d_fits, (size_t)n_poses * sizeof(b200ppf_pose_fit), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -577,8 +496,8 @@ int verify_score_poses_depth(b200ppf_ctx *ctx, const b200ppf_icp_job *jobs, size
     PPF_CUDA(ctx, cudaMemcpyAsync(d_zr, zr.data(), zr.size() * sizeof(ZRect), cudaMemcpyHostToDevice, ctx->stream));
     PPF_CUDA(ctx, cudaMemsetAsync(zbuf, 0xFF, std::max<uint64_t>(slab, 1) * sizeof(unsigned long long), ctx->stream));  // above any positive double
     PPF_LAUNCH(ctx, depth_splat_kernel, grid, THREADS, 0, g.d_poses.p, d_zr.p, D, tau, proj.p, zbuf.p);
-    PPF_LAUNCH(ctx, depth_score_kernel, grid, THREADS, 0, g.d_poses.p, g.scenes.p, g.cell_start.p, g.spos.p, g.snrm.p, d_zr.p, D, tau,
-               tau * tau, nt.cos_min, nt.use_normals, proj.p, zbuf.p, g.max_chunks, partials.p);
+    PPF_LAUNCH(ctx, depth_score_kernel, grid, THREADS, 0, g.d_poses.p, g.grids.table.p, g.grids.cell_start.p, g.grids.pos.p,
+               g.grids.nrm.p, d_zr.p, D, tau, tau * tau, nt.cos_min, nt.use_normals, proj.p, zbuf.p, g.max_chunks, partials.p);
     PPF_LAUNCH(ctx, depth_finish_kernel, (n_poses + 127) / 128, 128, 0, g.d_poses.p, n_poses, partials.p, g.max_chunks, d_fits.p);
     PPF_CUDA(ctx, cudaMemcpyAsync(fits, d_fits, (size_t)n_poses * sizeof(b200ppf_depth_fit), cudaMemcpyDeviceToHost, ctx->stream));
     PPF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
