@@ -722,6 +722,37 @@ int b200ppf_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *sc
                                        const b200ppf_verify_params *verify, b200ppf_object_result *results, int *status,
                                        b200ppf_depth_candidate *candidates);
 
+/* ---- screening the pose clusters before ICP (OpenCV engine) --------------------------------------------------------------
+ * The verified calls refine the icp_poses most-voted clusters of a box and only then score them, so a correct cluster of a
+ * lower rank never reaches the ICP.  The screened calls let the score choose which clusters the ICP refines.  For every box
+ * that reaches the matching:
+ *   1. The screen: its first S = min(n_clusters, screen_poses) pose clusters, most-voted first (screen_poses = 0: every
+ *      cluster), are scored unrefined against models[b] and the box's pre-processed object cloud with verify (the _depth
+ *      call against the frame's depth image as well): the records b200ppf_score_poses / b200ppf_score_poses_depth give.
+ *   2. Selection: the min(icp_poses, S) clusters of highest screen fit are kept, ties to the lower rank; with icp_poses = 0
+ *      the one of best screen fit.
+ *   3. The kept clusters are refined in the frame's one b200ppf_icp_refine_batch, scored again, and the best is returned as
+ *      the verified calls return it (ties to the lower rank).  With icp_poses = 0 nothing is refined and a candidate's fit is
+ *      its screen fit (the same bits: there is no second scoring).
+ * results[b], status, the candidate slots (max(icp_poses, 1) per box), their order and UINT32_MAX for unused slots are as
+ * the verified calls document; a candidate's rank is its cluster's position among all the box's clusters (0 = most voted)
+ * and n_poses stays the number of clusters.  Every result field but pose, residual, votes and the frame-wide times is the
+ * unverified call's.  screen_poses = max(icp_poses, 1) gives the verified call's results and candidates bit for bit.
+ * The return codes are the verified calls' (bad verify values, a NULL depth image or one of another context:
+ * B200PPF_ERR_INVALID before the crop runs); screen_poses has no invalid value.  The screen is one scoring call over every
+ * box's screened clusters and the final score one more over the refined candidates, so the call's launch count does not
+ * grow with the boxes or with S.  Memory: the _depth screen holds a z-buffer for every screened pose at once, at most
+ * S x rows x cols x 8 bytes per box; when it is not there the call returns B200PPF_ERR_NOMEM (limit screen_poses then). */
+int b200cv_match_frame_screened(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                                b200cv_detector *const *detectors, const b200ppf_cloud *const *models,
+                                const b200cv_object_params *params, const b200ppf_verify_params *verify, size_t screen_poses,
+                                b200ppf_object_result *results, int *status, b200ppf_candidate *candidates);
+int b200cv_match_frame_screened_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth,
+                                      size_t n_boxes, const float *corners12, b200cv_detector *const *detectors,
+                                      const b200ppf_cloud *const *models, const b200cv_object_params *params,
+                                      const b200ppf_verify_params *verify, size_t screen_poses,
+                                      b200ppf_object_result *results, int *status, b200ppf_depth_candidate *candidates);
+
 #ifdef __cplusplus
 }
 #endif

@@ -28,8 +28,20 @@ of each, medians of the wall time; b200ppf_score_poses_depth against b200ppf_sco
 candidates (CUDA events on the context's stream); the instances each call finds within 1 cm / 5 degrees and the best fits.
 Once per run: b200ppf_cloud_from_depth on the 1 Mi-pixel image (CUDA events, median of --repeat).
 
-usage: python tools/cv_frame_bench.py [--repeat 20] [--verify | --verify-depth]
-                                      [--out profiles/r4_cv_frame.jsonl | profiles/r5_verify.jsonl | profiles/r7_verify_depth.jsonl]"""
+--screen: what screening the pose clusters before ICP adds and recovers.  On the synthetic 1Mi frame b200cv_match_frame_screened
+against b200cv_match_frame_verified, and on synth.synth_library_depth the _depth pair, for K = 1 and 8 boxes, both match steps,
+icp_poses 5 and 1 and screen_poses = 0 (every cluster): --repeat calls of each, alternated after one warm-up of each, medians
+of the wall time; the device time of the screen alone (score_poses / score_poses_depth on every cluster of the boxes, each
+box's object cloud from b200cv_match_object and its clusters from CvDetector.match_cloud; CUDA events on the context's
+stream); the instances each call finds within 1 cm / 5 degrees (of the model axis, as the tests judge the library's surfaces of
+revolution, and of the whole rotation, as --verify-depth reports), the best fits, per box the clusters screened and the ranks
+of the kept candidates, and the clusters within 1 cm / 5 degrees (axis) of the truth before ICP (or the nearest one) with
+their screen fit and their position in the screen's order; for the depth screen the z-buffer slab it holds (8 bytes a pixel of every screened pose's splat
+rectangle, restated on the host from the rule in include/b200ppf.h), the whole call's and the largest box's.
+
+usage: python tools/cv_frame_bench.py [--repeat 20] [--verify | --verify-depth | --screen]
+                                      [--out profiles/r4_cv_frame.jsonl | profiles/r5_verify.jsonl | profiles/r7_verify_depth.jsonl |
+                                             profiles/r8_screen.jsonl]"""
 import argparse
 import json
 import os
@@ -197,6 +209,12 @@ def _axis_angle_deg(A, B):
     return float(np.degrees(np.arccos(np.clip((np.trace(R) - 1) / 2, -1.0, 1.0))))
 
 
+def _model_axis_deg(A, B):
+    """the angle between the models' z axes: the library models are surfaces of revolution about z, so the axis is what a
+    pose fixes (tests/test_gpu_frame.py judges the library instances by it)"""
+    return float(np.degrees(np.arccos(np.clip(A[:3, 2] @ B[:3, 2], -1.0, 1.0))))
+
+
 def depth_frame(c):
     from yolo_ppf_pose_estimation_b200 import capi, synth
     f = synth.synth_library_depth()
@@ -249,15 +267,105 @@ def bench_verify_depth(c, dimg, scene, boxes, K, use_edges, repeat, gpu):
             "fits_equal_score_poses_depth": fits_match, "gpu": gpu}
 
 
+def _zbuf_slab_bytes(model_rows, poses, dimg_host, K, tau=0.01):
+    """the z-buffer bytes b200ppf_score_poses_depth holds for these poses: 8 bytes a pixel of each pose's clipped splat rectangle"""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from verify_depth_reference import project, splat_half
+    total = 0
+    m = model_rows[:, :3].astype(np.float64)
+    for T in poses:
+        p = m @ T[:3, :3].T + T[:3, 3]
+        u, v, ok, _, _ = project(p, K, dimg_host.shape)
+        if not ok.any():
+            continue
+        h = splat_half(p[ok, 2], float(K[0]), tau)
+        u, v = u[ok], v[ok]
+        rows, cols = dimg_host.shape
+        w = min(int((u + h).max()), cols - 1) - max(int((u - h).min()), 0) + 1
+        hh = min(int((v + h).max()), rows - 1) - max(int((v - h).min()), 0) + 1
+        total += 8 * w * hh
+    return total
+
+
+def bench_screen(c, frame, scene, boxes, K, use_edges, icp_poses, repeat, gpu, depth=None):
+    """frame: name; depth: None or (device image, host image, K4) for the _depth pair"""
+    from yolo_ppf_pose_estimation_b200 import synth
+    cors = np.stack([b[0] for b in boxes[:K]])
+    dets, mods = [b[1] for b in boxes[:K]], [b[2] for b in boxes[:K]]
+    over = dict(leaf=0.005, use_edges=use_edges, icp_poses=icp_poses, relative_scene_sample_step=0.05 if use_edges else 1.0 / 14.0)
+    if depth is None:
+        calls = {"verified": lambda: c.cv_match_frame_verified(scene, cors, dets, mods, **over),
+                 "screened": lambda: c.cv_match_frame_screened(scene, cors, dets, mods, screen_poses=0, **over)}
+    else:
+        calls = {"verified": lambda: c.cv_match_frame_verified_depth(scene, depth[0], cors, dets, mods, **over),
+                 "screened": lambda: c.cv_match_frame_screened_depth(scene, depth[0], cors, dets, mods, screen_poses=0, **over)}
+    wall = {n: [] for n in calls}
+    out = {}
+    for fn in calls.values():
+        fn()  # warm-up
+    for _ in range(repeat):
+        for n, fn in calls.items():
+            t0 = time.perf_counter()
+            out[n] = fn()
+            wall[n].append(1e3 * (time.perf_counter() - t0))
+    for n, o in out.items():
+        assert o[1].tolist() == [0] * K, (n, o[1])
+
+    def found(res, angle):
+        return [k for k in range(K) if np.linalg.norm(res[k]["pose"][:3, 3] - synth.library_pose(k)[:3, 3]) < 0.01 and
+                angle(res[k]["pose"], synth.library_pose(k)) < 5.0]
+    # the screen alone: every cluster of every box, scored unrefined in one call
+    jobs = []
+    for k in range(K):
+        _, obj, edges = c.cv_match_object(dets[k], scene, cors[k], mods[k], **over)
+        top, n = dets[k].match_cloud(obj, edges if use_edges else None, over["relative_scene_sample_step"], 0.05, max_poses=obj.size)
+        jobs.append((mods[k], obj, np.stack([t["pose"].reshape(4, 4) for t in top]).astype(np.float64)))
+    if depth is None:
+        screen_ms = _event_ms(c, lambda: c.score_poses(jobs), repeat)
+        slab = None
+    else:
+        screen_ms = _event_ms(c, lambda: c.score_poses_depth(jobs, depth[0]), repeat)
+        per_box = [_zbuf_slab_bytes(m.download(), P, depth[1], depth[2]) for m, _, P in jobs]
+        slab = {"call_bytes": int(sum(per_box)), "largest_box_bytes": int(max(per_box))}
+    # the clusters within 1 cm / 5 degrees (axis) of the truth before ICP, or the nearest one: rank and screen-fit position
+    fits = c.score_poses(jobs) if depth is None else c.score_poses_depth(jobs, depth[0])
+    truth = []
+    for k, ((_, _, P), f) in enumerate(zip(jobs, fits)):
+        T = synth.library_pose(k)
+        pos = {r: i for i, r in enumerate(sorted(range(len(f)), key=lambda r: (-f[r]["fit"], r)))}
+        dt = [float(np.linalg.norm(Q[:3, 3] - T[:3, 3])) for Q in P]
+        near = [r for r in range(len(P)) if dt[r] < 0.01 and _model_axis_deg(P[r], T) < 5.0] or [int(np.argmin(dt))]
+        truth.append([{"rank": r, "within": dt[r] < 0.01 and _model_axis_deg(P[r], T) < 5.0, "dt_mm": round(1e3 * dt[r], 1),
+                       "axis_deg": round(_model_axis_deg(P[r], T), 1), "screen_fit": round(float(f[r]["fit"]), 4),
+                       "screen_position": pos[r]} for r in near])
+    med = lambda v: float(np.median(v))  # noqa: E731
+    sres, _, scands = out["screened"]
+    line = {"frame": frame, "boxes": K, "match": "match_S2B" if use_edges else "Matching", "icp_poses": icp_poses, "screen_poses": 0,
+            "calls": repeat, "leaf": 0.005, "verify": {"inlier_dist": 0.01, "normal_angle_deg": 30.0},
+            "wall_ms_median": {n: med(w) for n, w in wall.items()},
+            "added_wall_ms": med(wall["screened"]) - med(wall["verified"]),
+            "screen_device_ms_median": screen_ms, "clusters_screened": [int(x["n_poses"]) for x in sres],
+            "kept_ranks": [sorted(int(x["rank"]) for x in cs) for cs in scands],
+            "found_1cm_5deg_axis": {n: found(o[0], _model_axis_deg) for n, o in out.items()},
+            "found_1cm_5deg_rotation": {n: found(o[0], _axis_angle_deg) for n, o in out.items()},
+            "truth_clusters_before_icp": truth,
+            "best_fit": {n: [round(float(x[0]["fit"]["fit"]), 4) for x in o[2]] for n, o in out.items()},
+            "best_rank": {n: [int(x[0]["rank"]) for x in o[2]] for n, o in out.items()}, "gpu": gpu}
+    if slab is not None:
+        line["depth_screen_zbuf_slab"] = slab
+    return line
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--repeat", type=int, default=20, help="timed frame calls and serial rounds per K (after one warm-up each)")
     ap.add_argument("--verify", action="store_true", help="time the verified frame call and b200ppf_score_poses instead")
     ap.add_argument("--verify-depth", action="store_true", help="time the depth-verified frame call and b200ppf_score_poses_depth")
+    ap.add_argument("--screen", action="store_true", help="compare the screened frame calls with the verified ones")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if args.out is None:
-        args.out = os.path.join(ROOT, "profiles", "r7_verify_depth.jsonl" if args.verify_depth else
+        args.out = os.path.join(ROOT, "profiles", "r8_screen.jsonl" if args.screen else "r7_verify_depth.jsonl" if args.verify_depth else
                                 "r5_verify.jsonl" if args.verify else "r4_cv_frame.jsonl")
     if args.repeat < 1:
         ap.error("--repeat must be at least 1")
@@ -266,6 +374,18 @@ def main():
     gpu = card()
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
+        if args.screen:
+            lib_scene, lib_boxes = frames(c)[0][1:3]
+            fr, dimg, dscene, dboxes = depth_frame(c)
+            for frame, scene, boxes, depth in (("synthetic 1Mi frame", lib_scene, lib_boxes, None),
+                                                ("synth_library_depth 1024x1024", dscene, dboxes, (dimg, fr["depth"], fr["K"]))):
+                for use_edges in (1, 0):
+                    for icp_poses in (5, 1):
+                        for K in (1, 8):
+                            line = json.dumps(bench_screen(c, frame, scene, boxes, K, use_edges, icp_poses, args.repeat, gpu, depth))
+                            print(line, flush=True)
+                            f.write(line + "\n")
+            return
         if args.verify_depth:
             fr, dimg, scene, boxes = depth_frame(c)
             line = json.dumps({"frame": "synth_library_depth 1024x1024", "measured_pixels": int(scene.size),

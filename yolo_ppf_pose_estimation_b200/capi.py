@@ -211,6 +211,10 @@ SYMBOLS = {
                                                 C.POINTER(ObjectResult), _vp, C.POINTER(DepthCandidate)]),
     "b200cv_match_frame_verified_depth": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(VerifyParams),
                                                C.POINTER(ObjectResult), _vp, C.POINTER(DepthCandidate)]),
+    "b200cv_match_frame_screened": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(VerifyParams), _sz,
+                                         C.POINTER(ObjectResult), _vp, C.POINTER(Candidate)]),
+    "b200cv_match_frame_screened_depth": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, C.POINTER(CvObjectParams), C.POINTER(VerifyParams),
+                                               _sz, C.POINTER(ObjectResult), _vp, C.POINTER(DepthCandidate)]),
     "b200ppf_register": (_i, [_vp, _vp, _vp, _vp, _sz, _f, _f, _vp, _vp, _vp, C.POINTER(_sz)]),
     "b200cv_detector_create": (_i, [_vp, C.c_double, C.c_double, C.c_double, C.POINTER(_vp)]),
     "b200cv_detector_free": (None, [_vp]),
@@ -569,6 +573,29 @@ class Context:
             ObjectParams, lib().b200ppf_object_params_default,
             lambda k, c, *a: lib().b200ppf_match_frame_verified_depth(self._h, scene._h, depth._h, k, c, mods, tabs, *a), corners,
             dict(overrides), DepthCandidate)
+
+    def cv_match_frame_screened(self, scene: "Cloud", corners, detectors, models, screen_poses=0, **overrides):
+        """cv_match_frame_verified with the clusters the ICP refines chosen by their fit (b200cv_match_frame_screened): each
+        box's first screen_poses clusters (0: all) are scored unrefined and the icp_poses best-fitting ones refined and scored
+        again -> the tuple cv_match_frame_verified returns; a candidate's rank is its cluster's among all the box's clusters"""
+        n = len(detectors)
+        dets, mods = self._handles(detectors, n), self._handles(models, n)
+        return self._verified_frame_call(
+            CvObjectParams, lib().b200cv_object_params_default,
+            lambda k, c, prm, vp, *a: lib().b200cv_match_frame_screened(self._h, scene._h, k, c, dets, mods, prm, vp, screen_poses, *a),
+            corners, dict(overrides))
+
+    def cv_match_frame_screened_depth(self, scene: "Cloud", depth: "DepthImage", corners, detectors, models, screen_poses=0,
+                                      **overrides):
+        """cv_match_frame_screened with the screen and the final score against the frame's depth image
+        (b200cv_match_frame_screened_depth): candidates carry depth-fit dicts"""
+        n = len(detectors)
+        dets, mods = self._handles(detectors, n), self._handles(models, n)
+        return self._verified_frame_call(
+            CvObjectParams, lib().b200cv_object_params_default,
+            lambda k, c, prm, vp, *a: lib().b200cv_match_frame_screened_depth(self._h, scene._h, depth._h, k, c, dets, mods, prm, vp,
+                                                                              screen_poses, *a),
+            corners, dict(overrides), DepthCandidate)
 
     @staticmethod
     def _handles(objs, n):

@@ -1284,19 +1284,63 @@ int score_candidates(b200ppf_ctx *ctx, const std::vector<b200ppf_icp_job> &jobs,
     return verify_score_poses_depth(ctx, jobs.data(), jobs.size(), depth, verify, fits);
 }
 
+// The screen of the screened calls: the first min(n_clusters, screen) clusters of every box in `poses` (most-voted first)
+// are scored unrefined in one call, and each box keeps the min(icp_poses, S) best-fitting ones (one when icp_poses = 0),
+// ties to the lower rank.  poses / votes shrink to the kept clusters in rank order, ranks receives their ranks and, when
+// nothing is refined (icp_poses = 0), fits their screen fits, which are then the final ones.
+template <class Fit>
+int screen_clusters(b200ppf_ctx *ctx, size_t n_boxes, const b200ppf_cloud *const *models, const std::vector<CloudPtr> &objects,
+                    const int *status, size_t screen, int icp_poses, const b200ppf_verify_params &verify,
+                    const b200ppf_depth_image *depth, std::vector<std::vector<double>> &poses,
+                    std::vector<std::vector<uint32_t>> &votes, std::vector<std::vector<uint32_t>> &ranks,
+                    std::vector<std::vector<Fit>> &fits) {
+    std::vector<b200ppf_icp_job> jobs;
+    std::vector<size_t> n_screen(n_boxes, 0);
+    size_t n_scored = 0;
+    for (size_t b = 0; b < n_boxes; ++b)
+        if (!status[b]) {
+            n_screen[b] = std::min(votes[b].size(), screen);
+            jobs.push_back(b200ppf_icp_job{models[b], objects[b].get(), poses[b].data(), n_screen[b], nullptr});
+            n_scored += n_screen[b];
+        }
+    std::vector<Fit> all(n_scored);
+    if (int rc = score_candidates(ctx, jobs, verify, depth, all.data())) return rc;
+    const Fit *f = all.data();
+    for (size_t b = 0; b < n_boxes; ++b) {
+        if (status[b]) continue;
+        std::vector<uint32_t> order(n_screen[b]);
+        for (size_t k = 0; k < order.size(); ++k) order[k] = (uint32_t)k;
+        std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return f[x].fit > f[y].fit; });
+        order.resize(icp_poses > 0 ? std::min(order.size(), (size_t)icp_poses) : 1);
+        std::sort(order.begin(), order.end());
+        std::vector<double> kept(16 * order.size());
+        for (size_t i = 0; i < order.size(); ++i) {
+            memcpy(kept.data() + 16 * i, poses[b].data() + 16 * order[i], 16 * sizeof(double));
+            votes[b][i] = votes[b][order[i]];
+            if (icp_poses <= 0) fits[b].push_back(f[order[i]]);
+        }
+        poses[b] = std::move(kept);
+        votes[b].resize(order.size());
+        ranks[b] = std::move(order);
+        f += n_screen[b];
+    }
+    return B200PPF_OK;
+}
+
 // The chain of every match call, frame or per-object: crop all boxes in one pass, then per box the pre-processing and
 // `match(b, object, edges, &poses, &votes)`, the engine's matching step (it fills the box's match_ms and n_poses and returns
 // its best poses, 16 doubles each, most-voted first, and their clusters' votes), then one batched ICP of the top icp_poses
 // poses of every box that reached it against models[b].  With verify (checked), the candidates of every such box (the
 // refined poses, or the top pose alone without ICP) are then scored in one b200ppf_score_poses against models[b] and the
 // box's object cloud (b200ppf_score_poses_depth with the frame's depth image when Cand is b200ppf_depth_candidate), the
-// best one becomes the box's result, and candidates (may be NULL) receives them all, max(icp_poses, 1) slots per box.  When
-// box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
+// best one becomes the box's result, and candidates (may be NULL) receives them all, max(icp_poses, 1) slots per box.  With
+// screen > 0 (verify set; `match` returns every cluster) screen_clusters picks the candidates from the first `screen`
+// clusters before the ICP.  When box 0 succeeds, object_out / edges_out (either may be NULL) receive its clouds.
 template <class Params, class Match, class Cand>
 int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
                 const b200ppf_cloud *const *models, const Params &p, bool with_edges, b200ppf_object_result *results, int *status,
                 b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify, Cand *candidates,
-                const b200ppf_depth_image *depth, Match match) {
+                const b200ppf_depth_image *depth, size_t screen, Match match) {
     using Fit = decltype(Cand::fit);
     const auto t0 = std::chrono::steady_clock::now();
     for (size_t b = 0; b < n_boxes; ++b) {
@@ -1328,10 +1372,21 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
             rc = fail_msg(ctx, B200PPF_ERR_STATE, "match: the matching returned no pose");
         if (fatal(rc)) return rc;
         status[b] = rc;
-        if (rc) continue;
-        const size_t n_icp = std::min<size_t>(res->n_poses, p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
+    }
+    std::vector<std::vector<Fit>> fits(n_boxes);
+    std::vector<std::vector<uint32_t>> ranks(n_boxes);  // the candidates' cluster ranks (0, 1, .. unless screened)
+    if (screen) {
+        if (int rc = screen_clusters(ctx, n_boxes, models, objects, status, screen, p.icp_poses, *verify, depth, refined, votes,
+                                     ranks, fits))
+            return rc;
+    }
+    for (size_t b = 0; b < n_boxes; ++b) {
+        if (status[b]) continue;
+        const size_t n_icp = std::min<size_t>(votes[b].size(), p.icp_poses > 0 ? (size_t)p.icp_poses : 0);
         n_cand[b] = std::max<size_t>(n_icp, 1);
         residuals[b].assign(n_cand[b], 0.0);
+        if (!screen)
+            for (uint32_t k = 0; k < n_cand[b]; ++k) ranks[b].push_back(k);
         if (n_icp) jobs.push_back(b200ppf_icp_job{models[b], objects[b].get(), refined[b].data(), n_icp, residuals[b].data()});
     }
     float icp_ms = 0.0f;
@@ -1339,9 +1394,8 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
         if (int rc = b200ppf_icp_refine_batch(ctx, jobs.data(), jobs.size(), &p.icp, nullptr)) return rc;
         icp_ms = ctx->timings.icp_ms;
     }
-    std::vector<std::vector<Fit>> fits(n_boxes);
     std::vector<size_t> best(n_boxes, 0);  // resultsSub[0] unless verified
-    if (verify) {
+    if (verify && !(screen && p.icp_poses <= 0)) {  // a screen without ICP has its final fits already
         std::vector<b200ppf_icp_job> score_jobs;
         size_t n_scored = 0;
         for (size_t b = 0; b < n_boxes; ++b)
@@ -1356,10 +1410,12 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
             if (status[b]) continue;
             fits[b].assign(all.begin() + at, all.begin() + at + n_cand[b]);
             at += n_cand[b];
-            for (size_t k = 1; k < n_cand[b]; ++k)
-                if (fits[b][k].fit > fits[b][best[b]].fit) best[b] = k;
         }
     }
+    if (verify)
+        for (size_t b = 0; b < n_boxes; ++b)
+            for (size_t k = 1; k < fits[b].size(); ++k)
+                if (fits[b][k].fit > fits[b][best[b]].fit) best[b] = k;
     const float wall = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     for (size_t b = 0; b < n_boxes; ++b) {
         b200ppf_object_result *res = &results[b];
@@ -1387,7 +1443,7 @@ int match_boxes(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, co
                 memcpy(c[i].pose, refined[b].data() + 16 * k, 16 * sizeof(double));
                 c[i].residual = residuals[b][k];
                 c[i].votes = votes[b][k];
-                c[i].rank = (uint32_t)k;
+                c[i].rank = ranks[b][k];
                 c[i].fit = fits[b][k];
             }
         }
@@ -1451,7 +1507,7 @@ int ppf_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, cons
         return B200PPF_OK;
     };
     return match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && want_edges, results, status, object_out,
-                       edges_out, verify, candidates, depth, match);
+                       edges_out, verify, candidates, depth, 0, match);
 }
 
 // b200cv_match_frame; b200cv_match_object is this on one box.  The edge cloud is extracted when edge_curvature > 0 and
@@ -1460,7 +1516,7 @@ template <class Cand = b200ppf_candidate>
 int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12, b200cv_detector *const *detectors,
              const b200ppf_cloud *const *models, const b200cv_object_params *params, b200ppf_object_result *results, int *status,
              bool want_edges, b200ppf_cloud **object_out, b200ppf_cloud **edges_out, const b200ppf_verify_params *verify = nullptr,
-             Cand *candidates = nullptr, const b200ppf_depth_image *depth = nullptr) {
+             Cand *candidates = nullptr, const b200ppf_depth_image *depth = nullptr, size_t screen = 0) {
     CHECK_CTX(ctx);
     if (int rc = frame_args(ctx, scene, n_boxes, corners12, detectors, models, results, status)) return rc;
     for (size_t b = 0; b < n_boxes; ++b) {
@@ -1492,14 +1548,17 @@ int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const
         b200ppf_object_result *res = &results[b];
         if (p.use_edges && edges->n == 0)
             return fail_msg(ctx, B200PPF_ERR_STATE, "cv match: the object has no edge point for Matching_S2B to pair with");
+        // a screen takes every cluster: K7 copies back as many as it found, at most one per sampled reference point, and
+        // the sampled scene is a subset of the object cloud
+        if (screen && poses.size() < object->n) poses.resize(object->n);
         size_t n_clusters = 0;
         cudaEventRecord(ev[0], ctx->stream);
         int rc = b200cv_detector_match_cloud(detectors[b], object, p.use_edges ? edges : nullptr, p.relative_scene_sample_step,
-                                             p.relative_scene_distance, poses.data(), cap, &n_clusters);
+                                             p.relative_scene_distance, poses.data(), screen ? poses.size() : cap, &n_clusters);
         cudaEventRecord(ev[1], ctx->stream);
         if (rc == B200PPF_OK && cudaEventSynchronize(ev[1]) == cudaSuccess) cudaEventElapsedTime(&res->match_ms, ev[0], ev[1]);
         if (rc) return rc;
-        const size_t n_kept = std::min(n_clusters, cap);
+        const size_t n_kept = std::min(n_clusters, screen ? poses.size() : cap);
         refined->resize(16 * n_kept);
         cluster_votes->resize(n_kept);
         for (size_t k = 0; k < n_kept; ++k) {
@@ -1510,7 +1569,7 @@ int cv_match(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const
         return B200PPF_OK;
     };
     const int rc = match_boxes(ctx, scene, n_boxes, corners12, models, p, p.edge_curvature > 0.0f && (p.use_edges || want_edges),
-                               results, status, object_out, edges_out, verify, candidates, depth, match);
+                               results, status, object_out, edges_out, verify, candidates, depth, screen, match);
     cudaEventDestroy(ev[0]);
     cudaEventDestroy(ev[1]);
     return rc;
@@ -1612,6 +1671,29 @@ int b200cv_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *sce
     if (int rc = depth_arg(ctx, depth)) return rc;
     return cv_match(ctx, scene, n_boxes, corners12, detectors, models, params, results, status, true, nullptr, nullptr, &v, candidates,
                     depth);
+}
+
+int b200cv_match_frame_screened(b200ppf_ctx *ctx, const b200ppf_cloud *scene, size_t n_boxes, const float *corners12,
+                                b200cv_detector *const *detectors, const b200ppf_cloud *const *models,
+                                const b200cv_object_params *params, const b200ppf_verify_params *verify, size_t screen_poses,
+                                b200ppf_object_result *results, int *status, b200ppf_candidate *candidates) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params v;
+    if (int rc = verify_params(ctx, verify, &v)) return rc;
+    return cv_match(ctx, scene, n_boxes, corners12, detectors, models, params, results, status, true, nullptr, nullptr, &v, candidates,
+                    static_cast<const b200ppf_depth_image *>(nullptr), screen_poses ? screen_poses : SIZE_MAX);
+}
+
+int b200cv_match_frame_screened_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth, size_t n_boxes,
+                                      const float *corners12, b200cv_detector *const *detectors, const b200ppf_cloud *const *models,
+                                      const b200cv_object_params *params, const b200ppf_verify_params *verify, size_t screen_poses,
+                                      b200ppf_object_result *results, int *status, b200ppf_depth_candidate *candidates) {
+    CHECK_CTX(ctx);
+    b200ppf_verify_params v;
+    if (int rc = verify_params(ctx, verify, &v)) return rc;
+    if (int rc = depth_arg(ctx, depth)) return rc;
+    return cv_match(ctx, scene, n_boxes, corners12, detectors, models, params, results, status, true, nullptr, nullptr, &v, candidates,
+                    depth, screen_poses ? screen_poses : SIZE_MAX);
 }
 
 int b200ppf_match_frame_verified_depth(b200ppf_ctx *ctx, const b200ppf_cloud *scene, const b200ppf_depth_image *depth, size_t n_boxes,
